@@ -3,11 +3,15 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--config B8_lowrate] [--images PER_GPU] [--height 512] [--width 768] [--lanes 0|1]
+                    [--dump-outputs DIR]
 
 One "step" = compress + decompress of one batch of synthetic HxW RGB images (default 768x512, the
 Kodak size BASELINE.json quotes) with random-init weights of the named architecture.  Metric: Mpixel/s
 of the encode+decode round trip (a pixel counts once per round trip), whole job over all N GPUs
 (image-sharded, weak scaling, no data-path collective).  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) as DIR/<name>.npy on rank 0.  Inputs
+and weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the reference's CPU implementation of the same path (the oracle port of
 graphs/models/BlockBasedImgCompLossy_net.py:319-452; the Python reference itself cannot travel to
@@ -114,6 +118,31 @@ def synth_batch_gpu(n, H, W, seed, dev):
     return img.mul_(255).round_().to(torch.uint8)
 
 
+DUMP_ELEMENTS = 1 << 22      # per array (16 MB of float32): at most ~48 MB in all, plus 8 bytes per image for lens
+
+
+def dump_outputs(dirname, zhat, lens, streams, zdec):
+    """Writes what one encode + decode step hands its caller, as float32 / float64 arrays DIR/<name>.npy:
+    zhat and zdec (encoder and decoder reconstruction, flattened), lens (bytes of each image's stream) and streams
+    (n, k: the bytes of each stream at k fixed fractions of its length).  An array larger than DUMP_ELEMENTS is a fixed,
+    seeded sample whose positions depend only on the shape, the same in every run and build."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    flat_zhat, flat_zdec = zhat.reshape(-1), zdec.reshape(-1)
+    if flat_zhat.numel() > DUMP_ELEMENTS:
+        pos = np.sort(np.random.default_rng(0).choice(flat_zhat.numel(), DUMP_ELEMENTS, replace=False))
+        pos = torch.from_numpy(pos).to(zhat.device)
+        flat_zhat, flat_zdec = flat_zhat[pos], flat_zdec[pos]
+    k = max(1, min(2048, DUMP_ELEMENTS // lens.shape[0]))
+    frac = np.sort(np.random.default_rng(1).random(k))
+    at = (torch.from_numpy(frac).to(lens.device)[None, :] * lens.double()[:, None]).long()
+    out = dict(zhat=flat_zhat.float(), zdec=flat_zdec.float(), lens=lens.double(),
+               streams=torch.gather(streams, 1, at).float())
+    for name, t in out.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), t.cpu().numpy())
+
+
 def cpu_baseline(cfg, H, W, max_blocks, threads):
     """The oracle port of the reference's compress()/decompress() loops (torch CPU fp32 convs exactly as
     NET:363-398) timed on a bounded sample: the first `max_blocks` blocks in raster order of one image.
@@ -212,7 +241,14 @@ def main():
     ap.add_argument("--no-single-image", action="store_true", help="skip the one-image latency leg")
     ap.add_argument("--refc-images", type=int, default=2048,
                     help="second, larger batch for the reference-container round trip (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    sys.dont_write_bytecode = True          # the tree may be read-only: nothing is cached in it
 
     import lbic_b200
     cfg = lbic_b200.load_config(args.config)
@@ -262,12 +298,14 @@ def main():
             torch.cuda.synchronize()
 
     enc_out = m.encode_device(x, lanes=args.lanes)      # allocates outputs + workspace
+    zdec = None
 
     def step():
+        nonlocal zdec
         if flush is not None:
             flush.zero_()
         o = m.encode_device(x, lanes=args.lanes, out=enc_out)
-        return m.decode_device(o.streams, o.lens, n, Hb, Wb, lanes=args.lanes)
+        zdec = m.decode_device(o.streams, o.lens, n, Hb, Wb, lanes=args.lanes)
 
     def timed(fn, k):
         barrier()
@@ -283,9 +321,8 @@ def main():
         return float(ms.item())
 
     for _ in range(args.warmup):
-        zdec = step()
+        step()
     torch.cuda.synchronize()
-    parity_ok = bool(torch.equal(zdec, enc_out.zhat))
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -293,6 +330,9 @@ def main():
     ms_total = timed(step, args.steps)
     launches = m.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    parity_ok = bool(torch.equal(zdec, enc_out.zhat))   # the last timed step
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, enc_out.zhat, enc_out.lens, enc_out.streams, zdec)
     pixels_step = world * n * H * W
     value = pixels_step * args.steps / (ms_total * 1e-3) / 1e6
 

@@ -1,7 +1,8 @@
 """Import the UNMODIFIED reference model (BlockBasedImgCompLossyNetv9) in this container.
 
-TEST INFRASTRUCTURE ONLY; needs /root/reference (absent on the GPU box), so only fixture
-generation (tests/golden/make_golden.py) and the optional `needs_reference` tests use it.
+TEST INFRASTRUCTURE ONLY; needs a checkout of the reference repository, which is not part of this one:
+LBIC_REFERENCE_ROOT names its directory.  Only fixture generation (tests/golden/make_golden*.py) and the
+`needs_reference` tests use it; those tests skip where the variable is not set.
 
 The reference's package __init__ files import every sibling module (graphs/layers/__init__.py:6-10,
 utils/__init__.py:6-10) and so drag in matplotlib/easydict/bjontegaard/compressai, none of which
@@ -13,13 +14,13 @@ import os
 import sys
 import types
 
-REF = os.environ.get("LBIC_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("LBIC_REFERENCE_ROOT", "")
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _REPO = os.path.dirname(os.path.dirname(_HERE))
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF, "graphs/models/BlockBasedImgCompLossy_net.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "graphs/models/BlockBasedImgCompLossy_net.py"))
 
 
 def _load(name, relpath):
@@ -43,7 +44,7 @@ def _ns(name):
 def load():
     """Returns the reference module graphs.models.BlockBasedImgCompLossy_net."""
     if not available():
-        raise FileNotFoundError(f"reference tree not found at {REF}")
+        raise FileNotFoundError(f"reference tree not found at LBIC_REFERENCE_ROOT={REF!r}")
     for p in (_REPO, _HERE):
         if p not in sys.path:
             sys.path.insert(0, p)

@@ -13,7 +13,8 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real sm_100 GPU (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (skipped where it is absent)")
+    config.addinivalue_line("markers", "needs_reference: needs the reference repository at $LBIC_REFERENCE_ROOT "
+                                       "(skipped where it is not set)")
 
 
 def golden_cases():

@@ -1,8 +1,8 @@
 """Generates the golden fixtures in this directory by running the UNMODIFIED reference model
-(/root/reference, imported through oracle/ref_shim) on seeded synthetic inputs.
+(a checkout of it at $LBIC_REFERENCE_ROOT, imported through oracle/ref_shim) on seeded synthetic inputs.
 
-Run here (the container with /root/reference); the GPU box only reads the committed .npz files.
-    python tests/golden/make_golden.py
+Needs no GPU; the tests only read the committed .npz files.
+    LBIC_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 
 Each case_<name>.npz holds, for one (config, grid) pair with weights = synth_state_dict(cfg, seed):
     x         (1, 3B^2, Hb, Wb) fp32   input blocks in [-0.5, 0.5]

@@ -6,7 +6,7 @@ oracle.nets.forward_open_loop reproduces it, and writes forward_<name>.npz:
     xhat       (1, 3B^2, Hb, Wb) fp32   reference forward output (not clamped)
     selfinfo   (1, M, Hb, Wb)    fp32   -log2 of the Gaussian-conditional likelihoods
     symbols    (Hb, Wb, M)       int16  round(y - means) of the oracle restatement
-Run here (the container with /root/reference): python tests/golden/make_golden_forward.py
+Run with a checkout of the reference: LBIC_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden_forward.py
 """
 import os
 import sys

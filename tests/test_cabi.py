@@ -1,8 +1,9 @@
 """CPU tests: the C-ABI library loads, exports every symbol include/lbic.h declares, and refuses to run
 without an sm_100 GPU (no CPU fallback)."""
-import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 import torch
@@ -40,26 +41,41 @@ def test_option_constants_match_the_header():
 def test_blackwell_instructions_in_sass():
     """The shipped kernels are tcgen05/TMA code, not a legacy mma.sync path."""
     import shutil
-    import subprocess
-    if not shutil.which("cuobjdump"):
-        pytest.skip("cuobjdump not on PATH")
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.SO_PATH], capture_output=True, text=True).stdout
+    from lbic_b200 import build
+    # the cuobjdump of the toolkit that built the library, when it is not on PATH
+    tool = shutil.which("cuobjdump") or os.path.join(os.path.dirname(build.NVCC), "cuobjdump")
+    sass = subprocess.run([tool, "-sass", _lib.SO_PATH], capture_output=True, text=True, check=True).stdout
     assert "UTCHMMA" in sass and "UTMALDG" in sass and "LDTM" in sass
     assert "HMMA.16816" not in sass
 
 
-@pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure path")
+_NO_GPU_CHECK = """
+import ctypes
+import sys
+sys.path.insert(0, %r)
+import pytest
+import torch
+import lbic_b200
+from lbic_b200 import _lib
+assert not torch.cuda.is_available()
+L = _lib.lib()
+cfg = _lib.LbicConfig(8, (ctypes.c_int * 4)(3, 1, 1, 1), 768, 96)
+h = ctypes.c_void_p()
+rc = L.lbic_create(ctypes.byref(cfg), 0, ctypes.byref(h))
+assert rc == -5 and b"no CPU fallback" in L.lbic_last_error()
+m = lbic_b200.BlockBasedImgCompLossyNetv9(lbic_b200.load_config("B8_lowrate"))
+with pytest.raises(RuntimeError):
+    m.update(force=True)
+with pytest.raises(RuntimeError):
+    m.to("cpu")
+"""
+
+
 def test_fails_loudly_without_gpu():
-    L = _lib.lib()
-    cfg = _lib.LbicConfig(8, (ctypes.c_int * 4)(3, 1, 1, 1), 768, 96)
-    h = ctypes.c_void_p()
-    rc = L.lbic_create(ctypes.byref(cfg), 0, ctypes.byref(h))
-    assert rc == -5 and b"no CPU fallback" in L.lbic_last_error()
-    m = lbic_b200.BlockBasedImgCompLossyNetv9(lbic_b200.load_config("B8_lowrate"))
-    with pytest.raises(RuntimeError):
-        m.update(force=True)
-    with pytest.raises(RuntimeError):
-        m.to("cpu")
+    # in a child process that sees no GPU, so that this also runs on a machine that has one
+    out = subprocess.run([sys.executable, "-c", _NO_GPU_CHECK % ROOT], capture_output=True, text=True, timeout=600, cwd=ROOT,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 0, out.stderr[-3000:]
 
 
 def test_config_loader_reads_reference_json(tmp_path):

@@ -39,7 +39,7 @@ def integration_patch_source():
 @pytest.fixture(scope="module")
 def ref_agent():
     if not load_reference.available():
-        pytest.skip("reference tree not present")
+        pytest.skip("reference tree not present (LBIC_REFERENCE_ROOT)")
     return load_reference.load_agent()
 
 

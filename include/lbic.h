@@ -229,6 +229,43 @@ int lbic_rans_decode(lbic_model *m, const uint8_t *streams, const uint32_t *stre
 int lbic_debug_gemm(lbic_model *m, const float *A, const float *W, float *D, int R, int K, int cout,
                     void *stream);
 
+/* Test hook: ONE fused GEMM layer, D = A0 W0^T (+ A1 W1^T), through an explicitly chosen core form and epilogue, on
+ * operands the caller gives in fp32 (split into fp16 hi/lo planes on the device as activations are; the weights are NOT
+ * rescaled: pass them as the layer would store them and undo that with acc_scale).  Row r of the step is block r (QUANT /
+ * RECON outputs land at row r).  Allocates per call and synchronises `stream`.  With LBIC_OPT_CHECK_SATURATION set, the
+ * hi plane is scanned afterwards as a product layer's is (lbic_saturation_count). */
+typedef struct {
+    int mode;                  /* epilogue: 0 LRELU, 1 PREGDN, 2 GDN, 3 IGDN, 4 KSI, 5 QUANT, 6 RECON, 7 RAW, 8 RESID   */
+    int core;                  /* 0 SIMT twin, 1 per-tile tcgen05 kernel, 2 persistent kernel, 3 its CTA-pair form
+                                  (tiles <= 192 wide), 4 CTA pair with tiles <= 256 wide                               */
+    int force_bn;              /* core 1: tile width (multiple of 16, <= 256); 0 = the automatic width                   */
+    int R, cout, nseg;         /* rows, output channels (multiple of 16), K segments (1 or 2)                           */
+    int K[2];                  /* segment widths (multiples of 8)                                                         */
+    const float *A[2];         /* device, (R, K[s]) fp32 row-major                                                        */
+    const float *W[2];         /* device, (cout, K[s]) fp32 row-major                                                     */
+    const float *bias;         /* device [cout] (beta for GDN / IGDN), NULL = zeros                                       */
+    const float *aux;          /* device: pre-GDN activation (GDN, IGDN), ksi = scales | means (QUANT), residual (RESID) */
+    int ld_aux;                /* row stride of aux in elements                                                          */
+    float acc_scale;           /* the epilogue computes acc * acc_scale + bias                                            */
+    int M;                     /* QUANT: means at aux[r * ld_aux + M + c], symbols / indexes with row stride M (>= cout)  */
+    const float *scale_table;  /* QUANT: device, 64 increasing scale levels; NULL = the model's installed table          */
+    int no_clamp;              /* RECON / RESID: 1 = no clamp to [-0.5, 0.5]                                              */
+    float *out_f32;            /* RAW, PREGDN, KSI, RECON, RESID: (R, cout) fp32; QUANT: (R, M) int32 symbols            */
+    uint16_t *out_hi, *out_lo; /* LRELU, PREGDN, GDN, IGDN, QUANT: (R, cout) fp16 bit patterns                           */
+    uint8_t *out_idx;          /* QUANT: (R, M) CDF indexes                                                               */
+} lbic_debug_layer_args;
+int lbic_debug_layer(lbic_model *m, const lbic_debug_layer_args *args, void *stream);
+
+/* Test hook: the rate estimate of lbic_validate for R rows of M channels (row r = block r): ksi (R, ld_ksi) device
+ * fp32 with the scales in columns [0, M), sym (R, M) int32, info (R, M) fp32 = -log2 likelihood.  Synchronises. */
+int lbic_debug_selfinfo(lbic_model *m, const float *ksi, int ld_ksi, const int32_t *sym, int R, int M, float *info,
+                        void *stream);
+
+/* Test hook: the CDF index of n scales (device fp32) as the decoders compute it from `scale_table` (device, 64 levels):
+ * idx_bisect[i] by bisection, idx_hinted[i] by the logarithmic hint with its bisection fallback.  Synchronises. */
+int lbic_debug_scale_index(lbic_model *m, const float *scales, int n, const float *scale_table, int32_t *idx_bisect,
+                           int32_t *idx_hinted, void *stream);
+
 /* Tuning hook: times `iters` back-to-back launches of the D = A W^T tile kernel (EPI_RAW or a PREGDN-style
  * epilogue when with_epilogue != 0) on synthetic operands with CUDA events; returns the mean ms per launch. */
 int lbic_debug_gemm_bench(lbic_model *m, int R, int K, int cout, int with_epilogue, int iters, double *ms_per_launch);

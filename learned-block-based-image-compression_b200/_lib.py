@@ -21,6 +21,15 @@ class LbicTensorDesc(ctypes.Structure):
                 ("shape", ctypes.c_int64 * 4)]
 
 
+class LbicDebugLayerArgs(ctypes.Structure):
+    _fields_ = [("mode", ctypes.c_int), ("core", ctypes.c_int), ("force_bn", ctypes.c_int), ("R", ctypes.c_int),
+                ("cout", ctypes.c_int), ("nseg", ctypes.c_int), ("K", ctypes.c_int * 2), ("A", ctypes.c_void_p * 2),
+                ("W", ctypes.c_void_p * 2), ("bias", ctypes.c_void_p), ("aux", ctypes.c_void_p), ("ld_aux", ctypes.c_int),
+                ("acc_scale", ctypes.c_float), ("M", ctypes.c_int), ("scale_table", ctypes.c_void_p),
+                ("no_clamp", ctypes.c_int), ("out_f32", ctypes.c_void_p), ("out_hi", ctypes.c_void_p),
+                ("out_lo", ctypes.c_void_p), ("out_idx", ctypes.c_void_p)]
+
+
 LBIC_OPT_GEMM_CORE = 1
 LBIC_OPT_FORCE_BN = 3
 LBIC_OPT_WS = 6
@@ -76,6 +85,9 @@ PROTOTYPES = {
     "lbic_rans_encode": (_i, [_vp, _vp, _vp, _i, _i64, _vp, _sz, _vp, _vp]),
     "lbic_rans_decode": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _i64, _vp, _vp]),
     "lbic_debug_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "lbic_debug_layer": (_i, [_vp, ctypes.POINTER(LbicDebugLayerArgs), _vp]),
+    "lbic_debug_selfinfo": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _vp]),
+    "lbic_debug_scale_index": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "lbic_debug_gemm_bench": (_i, [_vp, _i, _i, _i, _i, _i, ctypes.POINTER(ctypes.c_double)]),
     "lbic_saturation_count": (_i, [_vp, _vp, ctypes.POINTER(ctypes.c_int64), _i]),
     "lbic_launch_count": (_i64, [_vp]),

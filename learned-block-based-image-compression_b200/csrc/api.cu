@@ -11,6 +11,7 @@
 #include <string>
 #include <vector>
 
+#include "epilogue.cuh"   // epi_has_f32 / epi_has_hilo (lbic_debug_layer)
 #include "lbic_internal.h"
 
 // ------------------------------------------------------------------------------------------------
@@ -2002,6 +2003,112 @@ extern "C" int lbic_debug_gemm(lbic_model *m, const float *A, const float *W, fl
     free_all(tmp);
     if (rc) return rc;
     if (e != cudaSuccess) return lbic_fail(LBIC_ERR_CUDA, "debug gemm failed: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+extern "C" int lbic_debug_layer(lbic_model *m, const lbic_debug_layer_args *a, void *stream) {
+    if (!m || !a) return lbic_fail(LBIC_ERR_INVALID, "null argument");
+    const int md = a->mode;
+    if (md < EPI_LRELU || md > EPI_RESID || a->core < 0 || a->core > 4 || a->R < 1 || a->cout < 16 || a->cout % 16 ||
+        a->nseg < 1 || a->nseg > 2)
+        return lbic_fail(LBIC_ERR_INVALID, "debug layer: bad mode / core / shape");
+    for (int s = 0; s < a->nseg; ++s)
+        if (!a->A[s] || !a->W[s] || a->K[s] < 8 || a->K[s] % 8)
+            return lbic_fail(LBIC_ERR_INVALID, "debug layer: segment %d needs A, W and K %% 8 == 0", s);
+    const bool needs_aux = md == EPI_GDN || md == EPI_IGDN || md == EPI_QUANT || md == EPI_RESID;
+    if ((epi_has_f32(md) && !a->out_f32) || (epi_has_hilo(md) && (!a->out_hi || !a->out_lo)) ||
+        (md == EPI_QUANT && !a->out_idx) || (needs_aux && !a->aux))
+        return lbic_fail(LBIC_ERR_INVALID, "debug layer: an output or side input of mode %d is missing", md);
+    if (md == EPI_QUANT && (a->M < a->cout || a->ld_aux < a->M + a->cout || (!a->scale_table && !m->tables.d_scale_table)))
+        return lbic_fail(LBIC_ERR_INVALID, "debug layer: QUANT needs M >= cout, ld_aux >= M + cout and a scale table");
+    if (a->core == 1 && a->force_bn && (a->force_bn % 16 || a->force_bn > 256))
+        return lbic_fail(LBIC_ERR_INVALID, "debug layer: bad tile width %d", a->force_bn);
+    Active act(m);
+    cudaStream_t st = (cudaStream_t)stream;
+    std::vector<void *> tmp;
+    int rc = 0;
+    do {
+#define P(call) if ((rc = (call)) != 0) break
+        GemmCall g;
+        memset(&g, 0, sizeof(g));
+        const int pair = a->core >= 3;
+        // activation planes cover whole (pair) tiles, zero beyond row R, as the workspace buffers do (R_cap rows)
+        const int Rp = (a->R + 255) / 256 * 256;
+        g.R = a->R; g.cout = a->cout; g.nseg = a->nseg;
+        if (a->core >= 2) {
+            const int wmax = a->core == 4 ? gemm_pair_max_bn() : gemm_ws_max_bn();
+            const int nt = (a->cout + wmax - 1) / wmax;
+            g.bn = ((a->cout + nt - 1) / nt + 15) / 16 * 16;
+        } else {
+            g.bn = a->force_bn ? a->force_bn : pick_bn(a->cout);
+        }
+        CUtensorMap tm[2][4];   // [segment][A hi, A lo, W hi, W lo]
+        for (int s = 0; s < a->nseg && rc == 0; ++s) {
+            const int K = a->K[s];
+            h16 *ah, *al, *wh, *wl;
+            P(dev_alloc(tmp, (void **)&ah, sizeof(h16) * (size_t)Rp * K, true));
+            P(dev_alloc(tmp, (void **)&al, sizeof(h16) * (size_t)Rp * K, true));
+            P(dev_alloc(tmp, (void **)&wh, sizeof(h16) * (size_t)a->cout * K));
+            P(dev_alloc(tmp, (void **)&wl, sizeof(h16) * (size_t)a->cout * K));
+            P(launch_split_f32(a->A[s], ah, al, (int64_t)a->R * K, st));
+            P(launch_split_f32(a->W[s], wh, wl, (int64_t)a->cout * K, st));
+            // the maps make_view and pack_conv_seg build: 64 k x 128 rows, 64 k x tile width (half of it per CTA of a pair)
+            P(make_tmap_2d(&tm[s][0], ah, K, Rp, K, 64, 128));
+            P(make_tmap_2d(&tm[s][1], al, K, Rp, K, 64, 128));
+            P(make_tmap_2d(&tm[s][2], wh, K, a->cout, K, 64, pair ? g.bn / 2 : g.bn));
+            P(make_tmap_2d(&tm[s][3], wl, K, a->cout, K, 64, pair ? g.bn / 2 : g.bn));
+            g.K[s] = K;
+            g.A[s].hi = ah; g.A[s].lo = al; g.A[s].ld = K; g.A[s].tm_hi = &tm[s][0]; g.A[s].tm_lo = &tm[s][1];
+            g.W[s].hi = wh; g.W[s].lo = wl; g.W[s].ld = K; g.W[s].tm_hi = &tm[s][2]; g.W[s].tm_lo = &tm[s][3];
+        }
+        if (rc) break;
+        float *bias = const_cast<float *>(a->bias);
+        if (!bias) P(dev_alloc(tmp, (void **)&bias, sizeof(float) * a->cout, true));
+        StepDesc raster = {1, 0, 0, 0, a->R, 1};   // raster chunk of one image of R x 1 blocks: row r -> block r
+        EpiParams &e = g.ep;
+        e = epi(md, raster);
+        e.R = a->R; e.cout = a->cout; e.bias = bias; e.acc_scale = a->acc_scale;
+        e.no_clamp = a->no_clamp;
+        e.aux = a->aux; e.ld_aux = a->ld_aux; e.M = a->M;
+        e.scale_tab = a->scale_table ? a->scale_table : m->tables.d_scale_table;
+        e.out_hi = reinterpret_cast<h16 *>(a->out_hi); e.out_lo = reinterpret_cast<h16 *>(a->out_lo); e.ld_out = a->cout;
+        if (md == EPI_QUANT) {
+            e.sym = reinterpret_cast<int32_t *>(a->out_f32);
+            e.idx = a->out_idx;
+        } else if (md == EPI_RECON) {
+            e.zhat = a->out_f32;
+        } else {
+            e.out_f32 = a->out_f32; e.ld_f32 = a->cout;
+        }
+        P(a->core == 0 ? gemm_simt_launch(g, st) : a->core == 1 ? gemm_tc_launch(g, st) : gemm_ws_launch(g, st, pair));
+        if (m->check_sat && m->d_sat && epi_has_hilo(md)) P(launch_sat_scan(e.out_hi, a->R, a->cout, e.ld_out, m->d_sat, st));
+#undef P
+    } while (0);
+    cudaError_t ce = cudaStreamSynchronize(st);
+    free_all(tmp);
+    if (rc) return rc;
+    if (ce != cudaSuccess) return lbic_fail(LBIC_ERR_CUDA, "debug layer failed: %s", cudaGetErrorString(ce));
+    return 0;
+}
+
+extern "C" int lbic_debug_selfinfo(lbic_model *m, const float *ksi, int ld_ksi, const int32_t *sym, int R, int M,
+                                   float *info, void *stream) {
+    if (!m || !ksi || !sym || !info || R < 1 || M < 1 || ld_ksi < M) return lbic_fail(LBIC_ERR_INVALID, "bad argument");
+    Active act(m);
+    cudaStream_t st = (cudaStream_t)stream;
+    const StepDesc raster = {1, 0, 0, 0, R, 1};
+    LBIC_TRY(launch_selfinfo_step(raster, R, M, ksi, ld_ksi, sym, info, st));
+    LBIC_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int lbic_debug_scale_index(lbic_model *m, const float *scales, int n, const float *scale_table,
+                                      int32_t *idx_bisect, int32_t *idx_hinted, void *stream) {
+    if (!m || !scales || !scale_table || !idx_bisect || !idx_hinted || n < 1) return lbic_fail(LBIC_ERR_INVALID, "bad argument");
+    Active act(m);
+    cudaStream_t st = (cudaStream_t)stream;
+    LBIC_TRY(launch_scale_index(scales, n, scale_table, idx_bisect, idx_hinted, st));
+    LBIC_CUDA(cudaStreamSynchronize(st));
     return 0;
 }
 

@@ -293,6 +293,8 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
                          int ld_yq, int32_t *sym_out, cudaStream_t st);
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,
                          cudaStream_t st);
+// CDF index of n scales by both routines of the decoders (bisection; hint with bisection fallback), for tests
+int launch_scale_index(const float *scales, int n, const float *tab, int32_t *idx_bisect, int32_t *idx_hinted, cudaStream_t st);
 int launch_rans_decode_full(const Tables &T, const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride,
                             const uint8_t *idx, int n_streams, int64_t n_sym, int32_t *sym_out, cudaStream_t st);
 

@@ -885,6 +885,29 @@ int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int 
     return 0;
 }
 
+// The two index routines of the decoders on given scales: scale_to_index as the warp-per-row decoders and the wave
+// kernel call it, and the hinted lookup with its bisection fallback as the thread-per-stream decoder does.
+__global__ void scale_index_kernel(const float *__restrict__ scales, int n, const float *__restrict__ tab,
+                                   int32_t *__restrict__ idx_bisect, int32_t *__restrict__ idx_hinted) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    idx_bisect[i] = scale_to_index(scales[i], tab);
+    const float s = fmaxf(scales[i], LBIC_SCALES_MIN);
+    const ScaleHint hint = scale_hint(tab);
+    bool ok;
+    int ci = scale_to_index_hinted(s, tab, hint, &ok);
+    if (!ok) ci = scale_to_index_bisect(s, tab);
+    idx_hinted[i] = ci;
+}
+
+int launch_scale_index(const float *scales, int n, const float *tab, int32_t *idx_bisect, int32_t *idx_hinted, cudaStream_t st) {
+    if (n <= 0) return 0;
+    scale_index_kernel<<<(n + 255) / 256, 256, 0, st>>>(scales, n, tab, idx_bisect, idx_hinted);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
 int launch_rans_decode_full(const Tables &T, const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride,
                             const uint8_t *idx, int n_streams, int64_t n_sym, int32_t *sym_out, cudaStream_t st) {
     if (!T.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");

@@ -466,6 +466,75 @@ class BlockBasedImgCompLossyNetv9:
                                                   A.shape[1], W.shape[0], self._stream()))
         return D
 
+    EPI_MODES = ("lrelu", "pregdn", "gdn", "igdn", "ksi", "quant", "recon", "raw", "resid")   # lbic_debug_layer_args.mode
+    DEBUG_CORES = ("simt", "tc", "ws", "pair", "pair_wide")                                   # lbic_debug_layer_args.core
+
+    def debug_layer(self, mode, A, W, core="tc", force_bn=0, bias=None, aux=None, acc_scale=1.0, M=None,
+                    scale_table=None, no_clamp=False):
+        """ONE fused GEMM layer (test hook, lbic_debug_layer): A / W are lists of one or two fp32 CUDA tensors (R, K_s) /
+        (cout, K_s); aux (R, ld_aux) is the pre-GDN activation, ksi (scales | means) or the residual; scale_table (64,)
+        CUDA fp32 or None for the installed table.  Returns the planes the mode writes: 'f32' (R, cout) fp32 (RAW, PREGDN,
+        KSI, RECON, RESID), 'sym' (R, M) int32 and 'idx' (R, M) uint8 (QUANT), 'hi' / 'lo' (R, cout) fp16."""
+        md = self.EPI_MODES.index(mode)
+        A = [a.contiguous().float() for a in A]
+        W = [w.contiguous().float() for w in W]
+        R, cout, dev = A[0].shape[0], W[0].shape[0], A[0].device
+        M = cout if M is None else int(M)
+        keep = list(A) + list(W)
+        a = _lib.LbicDebugLayerArgs()
+        a.mode, a.core, a.force_bn, a.R, a.cout, a.nseg = md, self.DEBUG_CORES.index(core), int(force_bn), R, cout, len(A)
+        for s in range(len(A)):
+            a.K[s], a.A[s], a.W[s] = A[s].shape[1], A[s].data_ptr(), W[s].data_ptr()
+        if bias is not None:
+            bias = bias.contiguous().float()
+            keep.append(bias)
+            a.bias = bias.data_ptr()
+        if aux is not None:
+            aux = aux.contiguous().float()
+            keep.append(aux)
+            a.aux, a.ld_aux = aux.data_ptr(), aux.shape[1]
+        if scale_table is not None:
+            scale_table = scale_table.contiguous().float().to(dev)
+            keep.append(scale_table)
+            a.scale_table = scale_table.data_ptr()
+        a.acc_scale, a.M, a.no_clamp = float(acc_scale), M, 1 if no_clamp else 0
+        out = {}
+        if mode == "quant":
+            out["sym"] = torch.empty(R, M, dtype=torch.int32, device=dev)
+            out["idx"] = torch.empty(R, M, dtype=torch.uint8, device=dev)
+            a.out_f32, a.out_idx = out["sym"].data_ptr(), out["idx"].data_ptr()
+        elif mode in ("raw", "pregdn", "ksi", "recon", "resid"):
+            out["f32"] = torch.empty(R, cout, dtype=torch.float32, device=dev)
+            a.out_f32 = out["f32"].data_ptr()
+        if mode in ("lrelu", "pregdn", "gdn", "igdn", "quant"):
+            out["hi"] = torch.empty(R, cout, dtype=torch.float16, device=dev)
+            out["lo"] = torch.empty(R, cout, dtype=torch.float16, device=dev)
+            a.out_hi, a.out_lo = out["hi"].data_ptr(), out["lo"].data_ptr()
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().lbic_debug_layer(self._need(), ctypes.byref(a), self._stream()))
+        del keep
+        return out
+
+    def debug_selfinfo(self, ksi, sym):
+        """-log2 likelihood of the symbols sym (R, M) int32 under the scales ksi[:, :M] (test hook, lbic_debug_selfinfo)."""
+        ksi, sym = ksi.contiguous().float(), sym.contiguous().int()
+        R, M = sym.shape
+        info = torch.empty(R, M, dtype=torch.float32, device=sym.device)
+        with torch.cuda.device(sym.device):
+            _lib.check(_lib.lib().lbic_debug_selfinfo(self._need(), ksi.data_ptr(), ksi.shape[1], sym.data_ptr(), R, M,
+                                                      info.data_ptr(), self._stream()))
+        return info
+
+    def debug_scale_index(self, scales, scale_table):
+        """CDF indexes of fp32 CUDA scales by the decoders' bisection and by their hinted lookup (test hook,
+        lbic_debug_scale_index) -> (idx_bisect, idx_hinted) int32."""
+        scales, tab = scales.contiguous().float(), scale_table.contiguous().float().to(scales.device)
+        ib, ih = (torch.empty(scales.numel(), dtype=torch.int32, device=scales.device) for _ in range(2))
+        with torch.cuda.device(scales.device):
+            _lib.check(_lib.lib().lbic_debug_scale_index(self._need(), scales.data_ptr(), scales.numel(), tab.data_ptr(),
+                                                         ib.data_ptr(), ih.data_ptr(), self._stream()))
+        return ib, ih
+
 
 class BlkBasedPostProcessing:
     """Mirror of the reference's optional post-processing module (graphs/models/BlockBasedImgCompLossy_net.py:455-476,

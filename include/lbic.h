@@ -65,12 +65,9 @@ typedef struct {
 #define LBIC_OPT_DEC_SMEM_WARP 20   /* 1 (default): decode steps below LBIC_OPT_DEC_THREAD_ROWS decode one row per warp on shared-memory copies of the compact CDF rows; 0: on the int32 tables in global memory (process-wide) */
 #define LBIC_OPT_ENC_BLOCK_STREAMS 17 /* entropy-encode calls with at most this many streams (default 592) encode one stream per CTA: table lookups by seven warps, the serial state chain on one thread (process-wide; 0 = never) */
 #define LBIC_OPT_FLOW 11         /* 1 (default) = run each large wavefront step's layers as ONE dataflow launch (row-block dependencies instead of kernel boundaries): on single CTAs below LBIC_OPT_FLOW_PAIR_MIN_ROWS block rows, on CTA pairs from there; 2 = always (pairs); 0 = one launch per layer */
-#define LBIC_OPT_FLOW_QUAD 21     /* dataflow launch on clusters of FOUR CTAs: two CTA pairs take adjacent column tiles of one 256-row block and share its activation operand by TMA multicast (each CTA fetches one plane); 0 = CTA pairs only */
-#define LBIC_OPT_TMA_STORE 24     /* 1: in the dataflow launch the layers whose output rows are the step's compact rows store through the TMA engine from swizzled staging tiles (full 128-byte lines where the tile allows); 0 (default): staged copy loops; bit-identical, measured equal (process-wide) */
 #define LBIC_OPT_CHECK_SATURATION 26 /* 1: count the elements of the fp16 operand planes clipped at +-65504 (lbic_saturation_count); debug, per-layer launches */
 #define LBIC_OPT_FLOW_MIN_ROWS 12 /* steps with at least this many block rows take the dataflow launch (default 2560) */
 #define LBIC_OPT_FLOW_PAIR_MIN_ROWS 25 /* dataflow steps with fewer block rows than this (default 8192) run on single CTAs with 128 x 96 tiles, larger ones on CTA pairs with 256 x 192 tiles */
-#define LBIC_OPT_FLOW_SMALL 13    /* 1 = steps below LBIC_OPT_FLOW_MIN_ROWS also run as one dataflow launch, on single CTAs with 128 x 96 tiles; 0 (default) = one launch per layer there */
 #define LBIC_OPT_WAVE 15           /* 1 (default) = calls whose wavefront steps have at most LBIC_OPT_WAVE_MAX_ROWS block rows (single images, small batches; KS[1] = 1) run as ONE persistent cooperative launch per call (gemm_wave.cu): gather, all layers and the rANS decode step are tiles of an in-kernel work list; 0 = one launch per layer */
 #define LBIC_OPT_WAVE_MAX_ROWS 16  /* default 1536, at most 4096 */
 #define LBIC_OPT_WAVE_DEC_MAX_ROWS 18 /* decode calls take the wave kernel up to this many rows per step (default 64): its rANS tiles run one warp per row on 8 entropy CTAs that keep the CDF tables in shared memory */
@@ -79,6 +76,7 @@ typedef struct {
 #define LBIC_OPT_WS 6          /* 1 (default) = persistent warp-specialised kernel for steps with >= 2 tiles per SM */
 #define LBIC_OPT_PDL 7         /* 1 (default) = programmatic dependent launch between consecutive GEMM kernels (process-wide) */
 #define LBIC_OPT_FORCE_BN 3    /* tuning hook: force the GEMM tile width (multiple of 16, <= 256); 0 = automatic */
+/* Option numbers 13, 21 and 24 belonged to removed options and are not reused: lbic_set_option rejects them (LBIC_ERR_INVALID). */
 
 const char *lbic_last_error(void);
 const char *lbic_version(void);

@@ -38,17 +38,14 @@ LBIC_OPT_DEC_THREAD_ROWS = 9
 LBIC_OPT_ENC_THREAD_STREAMS = 10
 LBIC_OPT_FLOW = 11
 LBIC_OPT_FLOW_MIN_ROWS = 12
-LBIC_OPT_FLOW_SMALL = 13
 LBIC_OPT_HOST_BANDS = 14
 LBIC_OPT_WAVE = 15
 LBIC_OPT_ENC_BLOCK_STREAMS = 17
 LBIC_OPT_WAVE_DEC_MAX_ROWS = 18
 LBIC_OPT_WAVE_BN = 19
 LBIC_OPT_DEC_SMEM_WARP = 20
-LBIC_OPT_FLOW_QUAD = 21
 LBIC_OPT_CHECK_SATURATION = 26
 LBIC_OPT_FLOW_PAIR_MIN_ROWS = 25
-LBIC_OPT_TMA_STORE = 24
 LBIC_OPT_WAVE_MAX_ROWS = 16
 LBIC_OPT_PDL = 7
 

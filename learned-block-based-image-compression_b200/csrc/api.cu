@@ -137,10 +137,6 @@ struct lbic_model {
     int use_flow = 1;      // dataflow launch of a whole layer range per step (1 = steps with >= flow_min_rows rows, 2 = always)
     int flow_min_rows = 2560;       // (profiles/r2_midsize.log: 2048 gains 4-8 % at 128-256 images and loses 2 % at 48)
     int flow_pair_min_rows = 8192;   // dataflow steps below this many rows run on single CTAs (128 x 96 tiles), from it on CTA pairs
-    int flow_quad = 0;     // large steps: dataflow launch on clusters of four (activation operand shared by TMA multicast)
-    int flow_small = 0;    // steps below flow_min_rows: 1 = single-CTA dataflow launch with 96-wide tiles, 0 = one launch per
-                           // layer (default: the counter hand-off costs as much as a PDL-chained launch, profiles/r1_dataflow.md)
-    int flow_max_rows = 1 << 30;
     int use_wave = 1;      // persistent wavefront (latency) kernel for steps of at most wave_max_rows rows (KS[1] == 1)
     int wave_max_rows = 1536;
     int wave_dec_max_rows = 64;    // decode: the rANS tiles run one warp per row on 8 entropy CTAs (64 rows at a time)
@@ -202,12 +198,6 @@ void free_all(std::vector<void *> &list) {
 // tile-width variants of a layer, one per split factor (lbic_split): widest first
 int bn_variants(int cout, int *out) {
     for (int i = 0; i < NBN; ++i) {
-        if (i == LBIC_QUAD_VARIANT) {
-            int nt = (cout + gemm_ws_max_bn() - 1) / gemm_ws_max_bn();
-            nt += nt & 1;
-            out[i] = ((cout + nt - 1) / nt + 15) / 16 * 16;
-            continue;
-        }
         if (i >= LBIC_WS_VARIANT) {
             const int wmax = i == LBIC_PAIR_WIDE ? gemm_pair_max_bn()
                              : i == LBIC_SMALL_VARIANT ? gemm_ws_max_bn() / 2
@@ -289,7 +279,7 @@ int pack_conv_seg(lbic_model *m, const SdView &sd, const std::string &prefix, in
     const int nb = bn_variants(cout, bnv);
     (void)bn;
     for (int i = 0; i < nb; ++i) {
-        const int box = (i == LBIC_PAIR_VARIANT || i == LBIC_PAIR_WIDE || i == LBIC_QUAD_VARIANT) ? bnv[i] / 2 : bnv[i];   // a CTA pair loads half the tile per CTA
+        const int box = (i == LBIC_PAIR_VARIANT || i == LBIC_PAIR_WIDE) ? bnv[i] / 2 : bnv[i];   // a CTA pair loads half the tile per CTA
         LBIC_TRY(make_tmap_2d(&seg.tm_hi[i], seg.hi, seg.K, cout, seg.K, 64, box));
         LBIC_TRY(make_tmap_2d(&seg.tm_lo[i], seg.lo, seg.K, cout, seg.K, 64, box));
     }
@@ -378,7 +368,7 @@ int pack_gdn(lbic_model *m, const SdView &sd, int id, const std::string &prefix,
     LBIC_TRY(dev_alloc(tmp, (void **)&seg.weff, sizeof(float) * (size_t)C * C));
     LBIC_TRY(launch_pack_gdn(g, b, C, gbound, gped, bbound, bped, seg.weff, C, L.bias, st));
     for (int i = 0; i < L.n_bn; ++i) {
-        const int box = (i == LBIC_PAIR_VARIANT || i == LBIC_PAIR_WIDE || i == LBIC_QUAD_VARIANT) ? L.bn_v[i] / 2 : L.bn_v[i];
+        const int box = (i == LBIC_PAIR_VARIANT || i == LBIC_PAIR_WIDE) ? L.bn_v[i] / 2 : L.bn_v[i];
         LBIC_TRY(make_tmap_2d(&seg.tm_hi[i], seg.hi, C, C, C, 64, box));
         LBIC_TRY(make_tmap_2d(&seg.tm_lo[i], seg.lo, C, C, C, 64, box));
     }
@@ -499,24 +489,6 @@ int build_chain(lbic_model *m) {
         for (int v = 0; v < L.n_bn; ++v) c.bn_v[v] = L.bn_v[v];
         ep.cout = L.cout; ep.bias = L.bias; ep.scale_tab = m->tables.d_scale_table; ep.acc_scale = L.acc_scale;
         c.ep = ep;
-        // output descriptors for the TMA-store epilogue: layers whose output rows are the step's compact rows
-        const bool row_indexed = (ep.mode == EPI_LRELU && !ep.out_pos && !(id == L_E0 && m->k1 == 3)) || ep.mode == EPI_PREGDN || ep.mode == EPI_GDN ||
-                                 ep.mode == EPI_IGDN || ep.mode == EPI_KSI;
-        c.tma_out = 0;
-        if (row_indexed) {
-            bool ok = true;
-            const bool has_hilo = ep.mode != EPI_KSI, has_f32 = ep.mode == EPI_PREGDN || ep.mode == EPI_KSI;
-            if (has_hilo)
-                ok = make_tmap_2d_ex(&c.tmO[0], ep.out_hi, 2, L.cout, ws.R_cap, ep.ld_out, 16, 128, 32) == 0 &&
-                     make_tmap_2d_ex(&c.tmO[1], ep.out_lo, 2, L.cout, ws.R_cap, ep.ld_out, 16, 128, 32) == 0;
-            if (ok && has_hilo)
-                ok = make_tmap_2d_ex(&c.tmO[3], ep.out_hi, 2, L.cout, ws.R_cap, ep.ld_out, 64, 128, 128) == 0 &&
-                     make_tmap_2d_ex(&c.tmO[4], ep.out_lo, 2, L.cout, ws.R_cap, ep.ld_out, 64, 128, 128) == 0;
-            if (ok && has_f32)
-                ok = make_tmap_2d_ex(&c.tmO[2], ep.out_f32, 4, L.cout, ws.R_cap, ep.ld_f32, 16, 128, 64) == 0 &&
-                     make_tmap_2d_ex(&c.tmO[5], ep.out_f32, 4, L.cout, ws.R_cap, ep.ld_f32, 32, 128, 128) == 0;
-            c.tma_out = ok ? 1 : 0;
-        }
     };
     auto pre = [&]() { return epi_pregdn(m, none); };
     auto gdn = [&](bool inv) {
@@ -574,7 +546,7 @@ const int FLOW_DEP[L_COUNT][2] = {
     {-1, -1}, {L_F0, -1}, {L_G0, -1}, {L_F1, -1}, {L_G1, -1}, {L_F2, -1}, {L_G2, L_E3},          // F0 G0 F1 G1 F2 G2 F3 (ksi)
     {L_F3, -1}, {L_D0, -1}, {L_IG0, -1}, {L_D1, -1}, {L_IG1, -1}, {L_D2, -1}, {L_IG2, -1}};     // D0 IG0 D1 IG1 D2 IG2 D3
 
-// 0: one launch per layer; 1: dataflow launch on CTA pairs (large steps); 2: dataflow launch on single CTAs (small steps)
+// 0: one launch per layer; 1: dataflow launch on CTA pairs (large steps); 2: dataflow launch on single CTAs (mid-size steps)
 int flow_applies(const lbic_model *m, int R) {
     if (m->check_sat) return 0;
     if (m->gemm_core != 0 || !m->use_pair || !m->use_flow || m->force_bn || !gemm_flow_supported()) return 0;
@@ -585,10 +557,9 @@ int flow_applies(const lbic_model *m, int R) {
     // (the threshold is quoted for 768-wide layers and scales with the tiles per row block, i.e. inversely with N).
     // KS[1] = 3 topologies (five-tap second entropy layer, K = 5 E1) measure no gain from the single-CTA window
     // (B8_highrate at 64 / 128 / 256 images: 110 / 153 / 187 against 112 / 152 / 189 Mpixel/s): pairs from 4096 rows as before.
-    if (m->k1 == 3) return (R >= (m->flow_min_rows > 4096 ? m->flow_min_rows : 4096) && R <= m->flow_max_rows) ? 1 : ((m->flow_small && R < m->flow_min_rows) ? 2 : 0);
-    if (R >= m->flow_min_rows && R <= m->flow_max_rows)
-        return (long)R * (m->N > 0 ? m->N : 768) >= (long)m->flow_pair_min_rows * 768 ? 1 : 2;
-    return (m->flow_small && R < m->flow_min_rows) ? 2 : 0;
+    if (m->k1 == 3) return R >= (m->flow_min_rows > 4096 ? m->flow_min_rows : 4096) ? 1 : 0;
+    if (R < m->flow_min_rows) return 0;
+    return (long)R * (m->N > 0 ? m->N : 768) >= (long)m->flow_pair_min_rows * 768 ? 1 : 2;
 }
 
 int run_flow(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStream_t st) {
@@ -603,15 +574,8 @@ int run_flow(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStrea
         rec.layer = -1;
         cudaEventRecord(rec.a, st);
     }
-    const int mode = flow_applies(m, R) == 1 ? 1 : 0;
-    int rc = LBIC_FLOW_REFUSED;
-    if (mode == 1 && m->flow_quad) {
-        rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, FLOW_DEP, R, sd, ws.flow_counters, ws.flow_counters_cap, st, 2);
-        if (rc == LBIC_FLOW_REFUSED) m->flow_quad = 0;       // no clusters of four on this device: CTA pairs from now on
-    }
-    if (rc == LBIC_FLOW_REFUSED)
-        rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, FLOW_DEP, R, sd, ws.flow_counters, ws.flow_counters_cap, st,
-                              mode);
+    const int rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, FLOW_DEP, R, sd, ws.flow_counters,
+                                    ws.flow_counters_cap, st, flow_applies(m, R) == 1 ? 1 : 0);
     if (m->profiling) {
         cudaEventRecord(rec.b, st);
         m->prof.push_back(rec);
@@ -971,10 +935,7 @@ extern "C" int lbic_create(const lbic_config *cfg, int device, lbic_model **out)
     // tuning hooks for benchmarking without code changes (the same switches as lbic_set_option)
     if (const char *e = getenv("LBIC_FLOW")) m->use_flow = atoi(e) < 0 ? 0 : (atoi(e) > 2 ? 2 : atoi(e));
     if (const char *e = getenv("LBIC_FLOW_MIN_ROWS")) m->flow_min_rows = atoi(e) < 1 ? 1 : atoi(e);
-    if (const char *e = getenv("LBIC_FLOW_MAX_ROWS")) m->flow_max_rows = atoi(e) < 1 ? 1 : atoi(e);
-    if (const char *e = getenv("LBIC_FLOW_SMALL")) m->flow_small = atoi(e) ? 1 : 0;
     if (const char *e = getenv("LBIC_FLOW_PAIR_MIN_ROWS")) m->flow_pair_min_rows = atoi(e) < 1 ? 1 : atoi(e);
-    if (const char *e = getenv("LBIC_FLOW_QUAD")) m->flow_quad = atoi(e) ? 1 : 0;
     if (const char *e = getenv("LBIC_WAVE")) m->use_wave = atoi(e) ? 1 : 0;
     if (const char *e = getenv("LBIC_WAVE_MAX_ROWS")) m->wave_max_rows = atoi(e) < 1 ? 1 : atoi(e);
     if (const char *e = getenv("LBIC_WAVE_DEC_MAX_ROWS")) m->wave_dec_max_rows = atoi(e) < 1 ? 1 : atoi(e);
@@ -1076,20 +1037,11 @@ extern "C" int lbic_set_option(lbic_model *m, int option, int value) {
     case LBIC_OPT_HOST_BANDS:
         m->host_bands = value < 1 ? 1 : (value > LBIC_MAX_BANDS ? LBIC_MAX_BANDS : value);
         return 0;
-    case LBIC_OPT_FLOW_SMALL:
-        m->flow_small = value ? 1 : 0;
-        return 0;
-    case LBIC_OPT_FLOW_QUAD:
-        m->flow_quad = value ? 1 : 0;
-        return 0;
     case LBIC_OPT_CHECK_SATURATION:
         m->check_sat = value ? 1 : 0;
         return 0;
     case LBIC_OPT_FLOW_PAIR_MIN_ROWS:
         m->flow_pair_min_rows = value < 1 ? 1 : value;
-        return 0;
-    case LBIC_OPT_TMA_STORE:
-        gemm_set_tma_store(value);
         return 0;
     case LBIC_OPT_PAIR:
         m->use_pair = value < 0 ? 0 : (value > 3 ? 3 : value);   // 2 = narrow (<= 192) tiles only, 3 = wide (<= 256) in the microbench

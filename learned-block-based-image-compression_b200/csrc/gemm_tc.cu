@@ -153,12 +153,6 @@ bool g_use_pdl = true;
 
 }  // namespace
 
-static int g_tma_store = -1;       // -1: not decided yet (env LBIC_TMA_STORE; default off: measured equal to the copy loops)
-void gemm_set_tma_store(int on) { g_tma_store = on ? 1 : 0; }
-int gemm_get_tma_store() {
-    if (g_tma_store < 0) { const char *e = getenv("LBIC_TMA_STORE"); g_tma_store = (e && atoi(e) != 0) ? 1 : 0; }
-    return g_tma_store;
-}
 void gemm_set_pdl(int on) { g_use_pdl = on != 0; }
 int gemm_get_pdl() { return g_use_pdl ? 1 : 0; }
 
@@ -191,26 +185,6 @@ int make_tmap_2d(CUtensorMap *tm, const void *base, uint64_t inner, uint64_t out
     CUresult rc = g_encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(base), gdim, gstride, box,
                                  estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (rc != CUDA_SUCCESS) return lbic_fail(LBIC_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)rc);
-    return 0;
-}
-
-int make_tmap_2d_ex(CUtensorMap *tm, const void *base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t ld_elems,
-                    uint32_t box_inner, uint32_t box_outer, int swizzle_bytes) {
-    LBIC_TRY(gemm_tc_init());
-    if ((reinterpret_cast<uintptr_t>(base) & 15) || ((ld_elems * elem_bytes) & 15))
-        return lbic_fail(LBIC_ERR_INVALID, "TMA operand must be 16-byte aligned (base %p, ld %llu)", base,
-                         (unsigned long long)ld_elems);
-    cuuint64_t gdim[2] = {inner, outer};
-    cuuint64_t gstride[1] = {ld_elems * (uint64_t)elem_bytes};
-    cuuint32_t box[2] = {box_inner, box_outer};
-    cuuint32_t estr[2] = {1, 1};
-    const CUtensorMapSwizzle sw = swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B
-                                  : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                  : swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE;
-    CUresult rc = g_encode_tiled(tm, elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2,
-                                 const_cast<void *>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                                 CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (rc != CUDA_SUCCESS) return lbic_fail(LBIC_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)rc);
     return 0;
 }

@@ -174,7 +174,6 @@ gemm_ws_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant_
             c.stg = stg; c.acc_full_bar = acc_full(a); c.acc_empty_bar = acc_empty(a); c.full_phase = (ti >> 1) & 1u;
             c.tmem_acc = tmem_base + a * WS_ACC_STRIDE; c.sb = sbias + a * 256; c.rt = rt; c.stab = stab; c.rank = rank;
             c.dep_cnt = nullptr; c.dep_target = 0; c.dep2_cnt = nullptr; c.dep2_target = 0;
-            c.hack = p.hack;
             ws_tile_epilogue<PAIR>(p.ep, p.bn, m0, n0, c);
         }
     }
@@ -211,45 +210,26 @@ struct FlowParams {
     const ChainLayer *layers;     // device table indexed by absolute layer id
     int *counters;                // [n_layers][n_rb], zero at launch
     int l0, n_layers, n_rb, R, variant, total_tiles;
-    int tma_store;                // 1: row-indexed layers store through the TMA engine (ws_tile_epilogue)
-    int hack;                     // LBIC_EPI_HACK (timing experiments)
     StepDesc step;
-    int chunk_rb;                 // row blocks per chunk: tiles are ordered chunk by chunk, layer by layer inside a chunk,
-    int tiles_per_chunk;          // so that a chunk's activations are still in L2 when the next layer reads them
-    int pre[FLOW_MAX_LAYERS + 1]; // prefix sums of nts (list slots of one row block over the layers)
-    int nts[FLOW_MAX_LAYERS];     // list slots per (layer, row block): ntn, or ceil(ntn / 2) in the quad form (a slot = two
-                                  // adjacent column tiles, one per CTA pair of the cluster)
+    int pre[FLOW_MAX_LAYERS + 1]; // prefix sums of ntn (tiles of one row block over the layers)
     int ntn[FLOW_MAX_LAYERS];     // column tiles per layer
     int dep[FLOW_MAX_LAYERS][2];  // relative layer indices this layer reads from, -1 = none
 };
 
-// tile index -> (layer, row block, column tile)
+// tile index -> (layer, row block, column tile); the list runs layer by layer, each layer row block by row block
 __device__ __forceinline__ void flow_tile(const FlowParams &p, int t, int &li, int &rb, int &nt) {
-    const int c = t / p.tiles_per_chunk;
-    const int u = t - c * p.tiles_per_chunk;
-    const int rb0 = c * p.chunk_rb;
-    const int crb = (p.n_rb - rb0) < p.chunk_rb ? (p.n_rb - rb0) : p.chunk_rb;   // the last chunk may be short
     li = 0;
-    while (u >= crb * p.pre[li + 1]) ++li;
-    const int v = u - crb * p.pre[li];
-    const int q = v / p.nts[li];
-    rb = rb0 + q;
-    nt = v - q * p.nts[li];
+    while (t >= p.n_rb * p.pre[li + 1]) ++li;
+    const int v = t - p.n_rb * p.pre[li];
+    rb = v / p.ntn[li];
+    nt = v - rb * p.ntn[li];
 }
 
 // MODE 1: 256-row tiles on CTA pairs (large steps).  MODE 0: 128 x (<= 96) tiles on single CTAs for small steps, where a
 // layer has a handful of tiles and what matters is the latency from one layer to the next.
-// MODE 2 (quad): clusters of FOUR = two CTA pairs that work on two adjacent column tiles of the SAME 256-row block and
-// share its activation operand: CTA (pair q, rank r) loads ONE plane of activation rows [128 r, 128 r + 128) -- hi for
-// q = 0, lo for q = 1 -- and TMA-multicasts it to CTAs r and r + 2, so a k-block costs a CTA 16 + 24 KiB from L2 instead
-// of 32 + 24.  A stage is free once BOTH pairs' MMAs have read it (each leader's commit is multicast to all four CTAs),
-// so the two pairs walk the k-blocks in lock step; everything per pair (TMEM, accumulator hand-over, epilogue, counters)
-// is as in MODE 1.  A layer with an odd number of column tiles gives the second pair a dummy tile (zero weights by TMA
-// bounds, nothing stored or published).
 template <int MODE>
 __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowParams p) {
-    constexpr bool PAIR = MODE >= 1;
-    constexpr bool QUAD = MODE == 2;
+    constexpr bool PAIR = MODE == 1;
     static_assert(sizeof(EpiParams) <= 256, "EpiParams must fit its shared-memory slot");
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -272,22 +252,16 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
         if (gtab && threadIdx.x < 64) stab[threadIdx.x] = gtab[threadIdx.x];
     }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t crank = PAIR ? cluster_ctarank() : 0u;
-    const uint32_t rank = crank & 1u;                              // CTA within its pair, 0 = leader
-    const uint32_t pidx = QUAD ? (crank >> 1) : 0u;                // pair within the cluster
-    const uint32_t leader = crank & ~1u;                           // cluster rank of this pair's leader
-    const uint16_t pair_mask = (uint16_t)(3u << leader);           // both CTAs of this pair
-    const uint16_t all_mask = QUAD ? (uint16_t)15 : (uint16_t)3;   // every CTA of the cluster
-    constexpr int CL = QUAD ? 4 : (PAIR ? 2 : 1);
-    const int tile_first = (int)blockIdx.x / CL;
-    const int tile_stride = (int)gridDim.x / CL;
-    constexpr int TILE_ROWS = PAIR ? 2 * BM : BM;
+    const uint32_t rank = PAIR ? cluster_ctarank() : 0u;          // CTA within its pair, 0 = leader
     constexpr int CTAS = PAIR ? 2 : 1;          // CTAs that store (and publish) each tile
+    const int tile_first = (int)blockIdx.x / CTAS;
+    const int tile_stride = (int)gridDim.x / CTAS;
+    constexpr int TILE_ROWS = PAIR ? 2 * BM : BM;
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < FLOW_STAGES; ++s) {
             mbar_init(full_bar(s), CTAS);
-            mbar_init(empty_bar(s), QUAD ? 2 : 1);       // quad: one commit per pair
+            mbar_init(empty_bar(s), 1);
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(acc_full(a), 1);
@@ -320,7 +294,6 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
                 flow_tile(p, t, li, rb, nt);
                 const ChainLayer &Lr = p.layers[p.l0 + li];
                 const int bn = Lr.bn_v[p.variant], w_rows = PAIR ? bn / 2 : bn;
-                if (QUAD) nt = 2 * nt + (int)pidx;          // (a dummy tile past the layer's width loads zero weights)
                 const int m0 = rb * TILE_ROWS + (int)rank * BM;
                 const int n0 = nt * bn + (int)rank * w_rows;
                 // wait until the layers this one reads from have stored this row block (both CTAs of every pair)
@@ -352,15 +325,9 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
                     if (elect_one()) {
                         if (PAIR) {
                             if (rank == 0) mbar_expect_tx(full_bar(s), stage_tx);
-                            else mbar_arrive_remote(full_bar(s), leader);
-                            if (QUAD) {
-                                // this CTA's plane of the shared activation rows, to the same-rank CTA of both pairs
-                                tma_load_2d_pair_mc(sa + pidx * A_PLANE, &Lr.tmA[seg][pidx], full_bar(s), kk, m0,
-                                                    (uint16_t)(5u << rank));
-                            } else {
-                                tma_load_2d_pair(sa, &Lr.tmA[seg][0], full_bar(s), kk, m0);
-                                tma_load_2d_pair(sa + A_PLANE, &Lr.tmA[seg][1], full_bar(s), kk, m0);
-                            }
+                            else mbar_arrive_remote(full_bar(s), 0);
+                            tma_load_2d_pair(sa, &Lr.tmA[seg][0], full_bar(s), kk, m0);
+                            tma_load_2d_pair(sa + A_PLANE, &Lr.tmA[seg][1], full_bar(s), kk, m0);
                             tma_load_2d_pair(sa + 2 * A_PLANE, &Lr.tmW[p.variant][seg][0], full_bar(s), kk, n0);
                             tma_load_2d_pair(sa + 2 * A_PLANE + w_plane, &Lr.tmW[p.variant][seg][1], full_bar(s), kk, n0);
                         } else {
@@ -411,8 +378,8 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
                         for (int k = 0; k < BK / 16; ++k) mma(a_hi + 2 * k, w_lo + 2 * k, 1u);
 #pragma unroll
                         for (int k = 0; k < BK / 16; ++k) mma(a_lo + 2 * k, w_hi + 2 * k, 1u);
-                        if (PAIR) umma_commit_pair(empty_bar(s), all_mask); else umma_commit(empty_bar(s));
-                        if (kb == nkb - 1) { if (PAIR) umma_commit_pair(acc_full(a), pair_mask); else umma_commit(acc_full(a)); }
+                        if (PAIR) umma_commit_pair(empty_bar(s)); else umma_commit(empty_bar(s));
+                        if (kb == nkb - 1) { if (PAIR) umma_commit_pair(acc_full(a)); else umma_commit(acc_full(a)); }
                     }
                     __syncwarp();
                 }
@@ -426,7 +393,6 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
                 int li, rb, nt;
                 flow_tile(p, t, li, rb, nt);
                 mbar_wait(tile_done(ti & 1u), (ti >> 1) & 1u);       // all eight epilogue warps have issued their stores
-                if (QUAD && 2 * nt + (int)pidx >= p.ntn[li]) continue;   // dummy tile: nothing was stored
                 asm volatile("fence.proxy.async;" ::: "memory");
                 asm volatile("fence.acq_rel.gpu;" ::: "memory");
                 asm volatile("red.release.gpu.global.add.s32 [%0], 1;" ::"l"(p.counters + (size_t)li * p.n_rb + rb) : "memory");
@@ -442,7 +408,6 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
             flow_tile(p, t, li, rb, nt);
             const ChainLayer &Lr = p.layers[p.l0 + li];
             const int bn = Lr.bn_v[p.variant];
-            if (QUAD) nt = 2 * nt + (int)pidx;           // (a dummy tile lies past the layer's width: every column is masked)
             const int m0 = rb * TILE_ROWS + (int)rank * BM, n0 = nt * bn;
             if (li != cur) {
                 // a new layer: its epilogue description, with this launch's row count and step, into shared memory
@@ -465,9 +430,6 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
             EpiCtx c;
             c.stg = stg; c.acc_full_bar = acc_full(a); c.acc_empty_bar = acc_empty(a); c.full_phase = (ti >> 1) & 1u;
             c.tmem_acc = tmem_base + a * WS_ACC_STRIDE; c.sb = sbias + a * 256; c.rt = rt; c.stab = stab; c.rank = rank;
-            c.leader = leader;
-            c.tmo = (p.tma_store && Lr.tma_out) ? Lr.tmO : nullptr;
-            c.hack = p.hack;
             const int dl = p.dep[li][0];
             c.dep_cnt = dl >= 0 ? p.counters + (size_t)dl * p.n_rb + rb : nullptr;
             c.dep_target = dl >= 0 ? CTAS * p.ntn[dl] : 0;
@@ -488,7 +450,7 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) gemm_flow_kernel(const FlowPa
     }
 }
 
-unsigned long long g_flow_attr_mask[3] = {0, 0, 0};
+unsigned long long g_flow_attr_mask[2] = {0, 0};
 
 unsigned long long g_ws_attr_mask[2] = {0, 0};
 
@@ -522,17 +484,11 @@ int gemm_ws_launch(const GemmCall &g, cudaStream_t st, int pair) {
     const int avail = SMEM_LIMIT - 1024 - (int)p.stg_bytes - 128 - WS_TAIL;
     int stages = avail / (int)p.slot_bytes;
     stages = stages > MAX_STAGES ? MAX_STAGES : stages;
-    {
-        static int cap = -1;   // tuning hook: LBIC_WS_STAGES caps the pipeline depth
-        if (cap < 0) { const char *e = getenv("LBIC_WS_STAGES"); cap = e ? atoi(e) : 0; }
-        if (cap >= 2 && stages > cap) stages = cap;
-    }
     if (stages < 2) return lbic_fail(LBIC_ERR_INVALID, "ws kernel: tile does not fit shared memory");
     p.stages = stages;
     p.ring_bytes = (uint32_t)stages * p.slot_bytes;
     p.idesc = (1u << 4) | ((uint32_t)(g.bn >> 3) << 17) | ((uint32_t)(tile_rows >> 4) << 24);
     p.ep = g.ep;
-    { static int hack = -1; if (hack < 0) { const char *e = getenv("LBIC_EPI_HACK"); hack = e ? atoi(e) : 0; } p.hack = hack; }
     int n_sm = 148;
     {
         int dev = 0;
@@ -610,43 +566,6 @@ int gemm_flow_supported() {
     return ok;
 }
 
-// Number of clusters of four CTAs of the quad form that are resident at once on this device (the SMs of a GPC that do
-// not make up a whole cluster stay idle: 33-37 clusters on a B200), 0 = not available.
-int gemm_flow_quad_clusters() {
-    static int cache[64];
-    static bool cache_init = false;
-    if (!cache_init) { for (int &c : cache) c = -1; cache_init = true; }
-    int cur = 0;
-    cudaGetDevice(&cur);
-    int &nc = cache[cur & 63];
-    if (nc >= 0) return nc;
-    nc = 0;
-    if (gemm_tc_init() != 0) return nc;
-    if (lbic_first_use_on_device(g_flow_attr_mask[2]) &&
-        (cudaFuncSetAttribute(gemm_flow_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess)) {
-        cudaGetLastError();
-        return nc;
-    }
-    int n_sm = 0;
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, cur);
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(n_sm / 4 * 4, 1, 1);
-    cfg.blockDim = dim3(FLOW_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = 1024 + (size_t)FLOW_STAGES * FLOW_SLOT + WGDN_BYTES + FLOW_TAIL;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 4; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int q = 0;
-    if (cudaOccupancyMaxActiveClusters(&q, gemm_flow_kernel<2>, &cfg) != cudaSuccess) { cudaGetLastError(); q = 0; }
-    if (q > n_sm / 4) q = n_sm / 4;
-    if (const char *e = getenv("LBIC_FLOW_QUAD_CLUSTERS")) { const int v = atoi(e); if (v > 0 && v < q) q = v; }
-    nc = q;
-    return nc;
-}
-
 // Layers [l0, l1) of one wavefront step in a single dataflow launch.  dep: for every absolute layer id the (up to two)
 // layer ids it reads from (-1 = none); layers outside [l0, l1) count as already complete.
 int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int l0, int l1, const int (*dep)[2], int R,
@@ -655,28 +574,18 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
     LBIC_TRY(gemm_tc_init());
     const int nl = l1 - l0;
     if (nl > FLOW_MAX_LAYERS) return lbic_fail(LBIC_ERR_INVALID, "flow kernel: too many layers");
-    // pair: 0 = single CTAs, 1 = CTA pairs, 2 = clusters of four (two pairs sharing the activation operand)
-    pair = pair < 0 ? 0 : (pair > 2 ? 2 : pair);
-    const bool quad = pair == 2;
-    int quad_clusters = 0;
-    if (quad) {
-        quad_clusters = gemm_flow_quad_clusters();
-        if (quad_clusters <= 0) return LBIC_FLOW_REFUSED;
-    }
+    pair = pair ? 1 : 0;     // 0 = single CTAs, 1 = CTA pairs
     if (lbic_first_use_on_device(g_flow_attr_mask[pair])) {
-        if (quad) LBIC_CUDA(cudaFuncSetAttribute(gemm_flow_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        else if (pair) LBIC_CUDA(cudaFuncSetAttribute(gemm_flow_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        if (pair) LBIC_CUDA(cudaFuncSetAttribute(gemm_flow_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
         else LBIC_CUDA(cudaFuncSetAttribute(gemm_flow_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     }
-    const int variant = quad ? LBIC_QUAD_VARIANT : pair ? LBIC_PAIR_VARIANT : LBIC_SMALL_VARIANT;
+    const int variant = pair ? LBIC_PAIR_VARIANT : LBIC_SMALL_VARIANT;
     const int tile_rows = pair ? 2 * BM : BM;
     const int max_bn = pair ? WS_MAX_BN : WS_MAX_BN / 2;     // both fill a 56 KiB stage: 2 x 96 weight rows or 1 x 96
     FlowParams p;
     memset(&p, 0, sizeof(p));
     p.layers = d_layers; p.counters = d_counters; p.l0 = l0; p.n_layers = nl; p.R = R; p.step = step;
     p.variant = variant;
-    p.tma_store = gemm_get_tma_store();
-    { static int hack = -1; if (hack < 0) { const char *e = getenv("LBIC_EPI_HACK"); hack = e ? atoi(e) : 0; } p.hack = hack; }
     p.n_rb = (R + tile_rows - 1) / tile_rows;
     if ((size_t)nl * p.n_rb > counters_cap) return lbic_fail(LBIC_ERR_INVALID, "flow kernel: counter buffer too small");
     int total = 0;
@@ -685,25 +594,14 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
         const int bn = L.bn_v[variant];
         if (bn % 16 || bn < 16 || bn > max_bn) return lbic_fail(LBIC_ERR_INVALID, "flow kernel: bad tile N %d", bn);
         p.ntn[i] = (L.cout + bn - 1) / bn;
-        p.nts[i] = quad ? (p.ntn[i] + 1) / 2 : p.ntn[i];
         p.pre[i] = total;
-        total += p.nts[i];
+        total += p.ntn[i];
         for (int d = 0; d < 2; ++d) {
             const int a = dep[l0 + i][d];
             p.dep[i][d] = (a >= l0 && a < l0 + i) ? a - l0 : -1;
         }
     }
     p.pre[nl] = total;
-    {
-        // tuning hook: LBIC_FLOW_CHUNK = row blocks (of 256 rows) per chunk, 0 = one chunk (default).  Chunks keep a
-        // layer's output in L2 for the next layer (DRAM traffic of a step drops from 4 GB), but a chunk of 16 / 32 / 64
-        // row blocks leaves only 1-4 waves of tiles per layer between producer and consumer and the pairs stall on the
-        // counters: 702 / 959 / 1004 Mpixel/s encode against 989-1043 unchunked (profiles/r1_dataflow.md)
-        static int chunk = -1;
-        if (chunk < 0) { const char *e = getenv("LBIC_FLOW_CHUNK"); chunk = e ? atoi(e) : 0; }
-        p.chunk_rb = (chunk <= 0 || chunk > p.n_rb) ? p.n_rb : chunk;
-    }
-    p.tiles_per_chunk = p.chunk_rb * total;
     total *= p.n_rb;
     p.total_tiles = total;
     LBIC_CUDA(cudaMemsetAsync(d_counters, 0, sizeof(int) * (size_t)nl * p.n_rb, st));
@@ -713,8 +611,7 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
     }
-    const int grid = quad ? 4 * (total < quad_clusters ? total : quad_clusters)
-                          : pair ? 2 * (total < n_sm / 2 ? total : n_sm / 2) : (total < n_sm ? total : n_sm);
+    const int grid = pair ? 2 * (total < n_sm / 2 ? total : n_sm / 2) : (total < n_sm ? total : n_sm);
     const size_t smem = 1024 + (size_t)FLOW_STAGES * FLOW_SLOT + WGDN_BYTES + FLOW_TAIL;
     if (smem > (size_t)SMEM_LIMIT) return lbic_fail(LBIC_ERR_INVALID, "flow kernel: shared memory budget exceeded");
     cudaLaunchConfig_t cfg;
@@ -727,7 +624,7 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
     int na = 0;
     if (pair) {
         attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = quad ? 4 : 2; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
+        attr[na].val.clusterDim.x = 2; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
         ++na;
     }
     // Every CTA (pair) waits for tiles owned by the others, so all of them must be resident at once.  A cooperative
@@ -747,9 +644,8 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
         }
         cfg.attrs = attr;
         cfg.numAttrs = n_attr;
-        const cudaError_t e = quad ? cudaLaunchKernelEx(&cfg, gemm_flow_kernel<2>, p)
-                              : pair ? cudaLaunchKernelEx(&cfg, gemm_flow_kernel<1>, p)
-                                     : cudaLaunchKernelEx(&cfg, gemm_flow_kernel<0>, p);
+        const cudaError_t e = pair ? cudaLaunchKernelEx(&cfg, gemm_flow_kernel<1>, p)
+                                   : cudaLaunchKernelEx(&cfg, gemm_flow_kernel<0>, p);
         if (e == cudaSuccess) {
             count_launch(0);
             return 0;

@@ -118,7 +118,7 @@ struct GemmCall {
 // One layer as the persistent multi-layer kernels see it (gemm_flow_kernel, gemm_wave_kernel), resident in device memory.
 // Tile-width variants per layer, indexed by "split factor" f: the layer's Cout is cut into f * ceil(Cout / (256 f))
 // equal tiles (width rounded up to 16), so a cluster of f CTAs gets the same number of tiles per CTA.
-constexpr int LBIC_NBN = 14;          // 6 split factors + the warp-specialised kernel's tiling (width <= 192) + its CTA-pair forms + small / latency tilings
+constexpr int LBIC_NBN = 13;          // 6 split factors + the warp-specialised kernel's tiling (width <= 192) + its CTA-pair forms + small / latency tilings
 constexpr int LBIC_WS_VARIANT = 6;
 constexpr int LBIC_PAIR_WIDE = 8;     // CTA-pair form with tiles up to 256 wide (2 pipeline stages instead of 3)
 constexpr int LBIC_SMALL_VARIANT = 9;  // tiles of at most 96 columns for the single-CTA dataflow launch of small steps
@@ -129,8 +129,6 @@ constexpr int LBIC_LAT_MAX_BN = 128;
 // rows of the activation TMA box for a tile with `rows` valid rows: class 0..3 = 16 / 32 / 48 / 64, 4 = the full 128
 __host__ __device__ inline int lbic_box_class(int rows) { return rows <= 16 ? 0 : rows <= 32 ? 1 : rows <= 48 ? 2 : rows <= 64 ? 3 : 4; }
 __host__ __device__ inline int lbic_box_rows(int cls) { return cls < 4 ? 16 * (cls + 1) : 128; }
-constexpr int LBIC_QUAD_VARIANT = 13;   // quad form of the dataflow launch: width <= 192 with an EVEN number of column tiles (two pairs
-                                        // of a cluster take adjacent tiles); weight TMA box = half the tile
 constexpr int LBIC_PAIR_VARIANT = 7;  // same tile width as LBIC_WS_VARIANT; weight TMA box = half the tile (one half per CTA)
 __host__ __device__ inline int lbic_split(int i) { return i == 0 ? 1 : i == 1 ? 2 : i == 2 ? 3 : i == 3 ? 4 : i == 4 ? 6 : 8; }
 struct alignas(64) ChainLayer {
@@ -144,11 +142,6 @@ struct alignas(64) ChainLayer {
     int bn_v[LBIC_NBN];
     int n_bn;
     EpiParams ep;                       // R and step are filled in per launch
-    // TMA-store epilogue (ws_tile_epilogue): descriptors of the layer's row-indexed OUTPUT planes, boxes of 16 columns x
-    // 128 rows: [0] hi, [1] lo (fp16, SWIZZLE_32B), [2] fp32 plane (SWIZZLE_64B).  tma_out = 0: the layer scatters its
-    // rows (QUANT symbols / indexes, RECON, the position-indexed g0 store) and keeps the staged copy loops.
-    CUtensorMap tmO[6];                 // [3] hi, [4] lo as 64-column boxes (SWIZZLE_128B), [5] fp32 as a 32-column box (SWIZZLE_128B)
-    int tma_out;
 };
 
 int gemm_ws_launch(const GemmCall &g, cudaStream_t st, int pair = 0);   // persistent warp-specialised kernel (gemm_ws.cu)
@@ -156,7 +149,6 @@ int gemm_flow_launch(const ChainLayer *d_layers, const ChainLayer *h_layers, int
                      const StepDesc &step, int *d_counters, size_t counters_cap, cudaStream_t st, int pair = 1);
 constexpr int LBIC_FLOW_REFUSED = 1000;   // gemm_flow_launch: the (cooperative) launch was refused; use the per-layer path
 int gemm_flow_supported();   // 1 if all CTA pairs of the dataflow launch can be co-resident on this device
-int gemm_flow_quad_clusters();   // clusters of four of the quad form resident at once (0 = not available)
 struct RansStreamState;
 // The latency path (gemm_wave.cu): a range of wavefront steps (or raster blocks) of ONE encode / decode in a single
 // persistent cooperative launch; gather, GEMM layers and (decode) the rANS step are tiles of one in-kernel work list.
@@ -193,14 +185,9 @@ int gemm_ws_max_bn();
 int gemm_pair_max_bn();
 void gemm_set_pdl(int on);   // programmatic dependent launch between consecutive GEMM kernels (default on)
 int gemm_get_pdl();
-void gemm_set_tma_store(int on);   // dataflow launch: row-indexed layers store their outputs through the TMA engine (default on)
-int gemm_get_tma_store();
 int gemm_simt_launch(const GemmCall &g, cudaStream_t st);
 int gemm_tc_launch(const GemmCall &g, cudaStream_t st);
 int gemm_tc_init();   // resolves cuTensorMapEncodeTiled, sets smem attributes
-// general form: element size 2 (fp16) or 4 (fp32), swizzle 32 / 64 / 128 bytes
-int make_tmap_2d_ex(CUtensorMap *tm, const void *base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t ld_elems,
-                    uint32_t box_inner, uint32_t box_outer, int swizzle_bytes);
 int make_tmap_2d(CUtensorMap *tm, const void *base, uint64_t inner, uint64_t outer, uint64_t ld_elems,
                  uint32_t box_inner, uint32_t box_outer);
 

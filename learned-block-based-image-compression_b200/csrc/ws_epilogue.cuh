@@ -32,7 +32,6 @@ struct WsParams {
     int stages;
     uint32_t slot_bytes, ring_bytes, stg_bytes;   // stg_bytes: staging region (+ the GDN pre-activation buffer), multiple of 128
     uint32_t idesc;
-    int hack;                  // LBIC_EPI_HACK (timing experiments, EpiCtx::hack)
     EpiParams ep;
 };
 
@@ -79,27 +78,11 @@ __device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t adesc, u
         ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// completion of all prior MMAs of the pair -> arrive on the barrier at this offset in the CTAs of `mask` (cluster ranks;
-// 3 = both CTAs of a cluster of two)
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t mask = 3) {
+// completion of all prior MMAs of the pair -> arrive on the barrier at this offset in both CTAs of the pair
+__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
     asm volatile(
         "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-        ::"r"(bar), "h"(mask) : "memory");
-}
-// TMA load whose box lands at the same shared-memory offset in every CTA of `mask` (cluster ranks); each destination's
-// bytes are credited to the barrier at this offset in the leader of ITS pair (peer bit cleared, as in tma_load_2d_pair).
-__device__ __forceinline__ void tma_load_2d_pair_mc(uint32_t dst, const CUtensorMap *tm, uint32_t bar, int c0, int c1,
-                                                    uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(tm)), "r"(bar & 0xFEFFFFFFu), "r"(c0), "r"(c1), "h"(mask)
-        : "memory");
-}
-
-// TMA store of a 16-column x 128-row box from a swizzled staging tile (bulk async-group of the calling thread)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap *tm, uint32_t src, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-                 ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(src), "r"(c0), "r"(c1) : "memory");
+        ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
 
 __device__ __forceinline__ int ld_acquire_gpu(const int *p) {
@@ -118,7 +101,6 @@ struct EpiCtx {
     RowTab *rt;
     const float *stab;
     uint32_t rank;            // CTA within its pair (0 = leader)
-    uint32_t leader = 0;      // cluster rank of the pair's leader CTA (2 for the second pair of a cluster of four)
     // dataflow launch only: the epilogue's own side input (GDN pre-activations) is written by another layer of the same
     // launch; it may be fetched once *dep_cnt >= dep_target (the epilogue warps run ahead of the TMA producer)
     const int *dep_cnt;
@@ -127,21 +109,10 @@ struct EpiCtx {
     const int *dep2_cnt;
     int dep2_target;
     unsigned long long *trace_acc = nullptr;   // debug: %globaltimer when the accumulator became available
-    // TMA-store form (ChainLayer::tmO: hi, lo, fp32 output planes as 16 x 128 boxes, then hi, lo as 64 x 128 and fp32 as 32 x 128
-    // boxes; needs 48 KiB of staging): the
-    // threads write their chunks into swizzled staging planes and ONE thread hands whole planes to the TMA engine -- no
-    // row table, no shared -> global copy loops, two barriers per 32-column group in every mode
-    const CUtensorMap *tmo = nullptr;
-    // timing experiments only (LBIC_EPI_HACK, results become garbage): 1 = no staging writes / stores, 2 = no fused
-    // arithmetic, 4 = no GDN side-input fetch, 8 = skip the whole group loop (release the accumulator and return),
-    // 16 = staging kept, only the global stores dropped
-    int hack = 0;
     // the accumulator was produced by M = 64 MMAs (latency kernel, steps of at most 64 rows): row r sits in TMEM lane
     // 32 (r / 16) + r % 16, i.e. each warp's lanes 0-15 hold rows 16 q .. 16 q + 15 (scripts/mma_m64_layout.cu)
     int m64 = 0;
 };
-constexpr uint32_t WTMA_LO = 8192, WTMA_F32 = 16384;   // narrow staging: hi 2 x 4 KiB | lo 2 x 4 KiB | fp32 2 x 8 KiB
-constexpr uint32_t WTMA_LO_W = 16384, WTMA_F32_W = 32768;   // wide staging: hi 16 KiB | lo 16 KiB | fp32 16 KiB
 
 template <bool PAIR>
 __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, int m0, int n0, const EpiCtx &cx) {
@@ -162,8 +133,7 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
     epi_bar();                           // previous tile's stores have finished reading rt / sbias
     if (mode != EPI_RAW)
         for (int i = et; i < bn; i += WS_EPI_THREADS) sb[i] = (n0 + i < ep.cout) ? ep.bias[n0 + i] : 0.0f;
-    const bool tma = cx.tmo != nullptr;
-    if (!tma && sub == 0 && row_ok) {
+    if (sub == 0 && row_ok) {
         const EpiRowDst d = epi_row_dst(ep, r);
         cx.rt->f32[rl] = reinterpret_cast<unsigned long long>(epi_f32_ptr(ep, d, n0));
         cx.rt->hilo[rl] = (unsigned long long)(d.hilo + n0);
@@ -193,7 +163,6 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
     const int hl_stride = gdn ? WGDN_STRIDE : WHL_STRIDE;
     const uint32_t aux_base = stg + BM * WGDN_STRIDE;
     auto aux_issue = [&](int g) {
-        if (cx.hack & 4) { asm volatile("cp.async.commit_group;" ::: "memory"); return; }
         const int nv = group_valid(g);
         const uint32_t buf = aux_base + (uint32_t)(g & 1) * WAUX_BUF;
 #pragma unroll
@@ -220,7 +189,7 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 const int row = ew * 16 + j * 4 + rsub;
-                const bool valid = row < rows_valid && c16 * 4 < nv && !(cx.hack & 4);
+                const bool valid = row < rows_valid && c16 * 4 < nv;
                 const float *src = valid ? ep.aux + (size_t)(m0 + row) * ep.ld_aux + half * ep.M + n0 + g * GC + c16 * 4 : ep.aux;
                 const uint32_t dst = buf + row * 128 + ((uint32_t)(c16 ^ (row & 7)) << 4);
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(valid ? 16 : 0) : "memory");
@@ -263,16 +232,6 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
     mbar_wait(cx.acc_full_bar, cx.full_phase);
     tc_fence_after();
     if (cx.trace_acc) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(*cx.trace_acc));
-    if (cx.hack & 8) {
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-            if (PAIR) mbar_arrive_remote(cx.acc_empty_bar, cx.leader);
-            else mbar_arrive(cx.acc_empty_bar);
-        }
-        return;
-    }
     tmem_ld_issue(lane_base + (uint32_t)(sub * 16), accA);
     for (int g = 0; g < ngroups; ++g) {
         const int g0 = g * GC;
@@ -322,107 +281,16 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) {
-                    if (PAIR) mbar_arrive_remote(cx.acc_empty_bar, cx.leader);
+                    if (PAIR) mbar_arrive_remote(cx.acc_empty_bar, 0);
                     else mbar_arrive(cx.acc_empty_bar);
                 }
             }
-            if (ok && !(cx.hack & 2)) {
+            if (ok) {
                 float v[16];
 #pragma unroll
                 for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(even ? accA[i] : accB[i]);
                 epi_compute<16>(ep, sb + g0 + sub * 16, v, pre, o, cx.stab);
             }
-        }
-        if (tma) {
-            // Full-line stores: a store of half a 128-byte line (one plane of a 32-column group is 64 B per row) costs the
-            // memory system about twice a full line (profiles/r2_flow_epilogue.md).  WIDE form (non-GDN modes, both groups
-            // of an even / odd pair fully inside the tile): the hi / lo chunks of the two groups go into 128-byte staging
-            // rows (SWIZZLE_128B) and leave as ONE 64-column box per plane after the second group; the fp32 plane of a
-            // group is a 32-column box (128 B per row).  NARROW form (GDN modes: the side-input buffers leave no room;
-            // ragged tails): 16-column boxes per chunk.
-            const int p0 = (g & ~1) * GC;
-            const bool wide = !gdn && p0 + 2 * GC <= bn && n0 + p0 + 2 * GC <= ep.cout;
-            const bool wide_f = !gdn && g0 + GC <= bn && n0 + g0 + GC <= ep.cout;
-            // staging planes free?  (non-GDN: the elected thread waits for the previous group's bulk reads here, after its
-            // own arithmetic; GDN: the barrier that ends the previous iteration did it)
-            if (!gdn && g > 0) {
-                if (et == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                epi_bar();
-            }
-            if (ok && !(cx.hack & 1)) {
-                if (has_hilo) {
-                    if (wide) {
-                        const uint32_t sw = (uint32_t)(rl & 7);                          // SWIZZLE_128B: bits 4-6 ^= bits 7-9
-                        const uint32_t c = (uint32_t)((g & 1) * 4 + sub * 2);            // 16-byte chunk within the 128-byte row
-                        const uint32_t hrow = stg + (uint32_t)rl * 128u;
-                        sts128(hrow + (((c + 0u) ^ sw) << 4), o.hi[0], o.hi[1], o.hi[2], o.hi[3]);
-                        sts128(hrow + (((c + 1u) ^ sw) << 4), o.hi[4], o.hi[5], o.hi[6], o.hi[7]);
-                        sts128(hrow + WTMA_LO_W + (((c + 0u) ^ sw) << 4), o.lo[0], o.lo[1], o.lo[2], o.lo[3]);
-                        sts128(hrow + WTMA_LO_W + (((c + 1u) ^ sw) << 4), o.lo[4], o.lo[5], o.lo[6], o.lo[7]);
-                    } else {
-                        const uint32_t sw = (uint32_t)((rl >> 2) & 1);                   // SWIZZLE_32B: bit 4 ^= bit 7
-                        const uint32_t hrow = stg + (uint32_t)sub * 4096u + (uint32_t)rl * 32u;
-                        sts128(hrow + ((0u ^ sw) << 4), o.hi[0], o.hi[1], o.hi[2], o.hi[3]);
-                        sts128(hrow + ((1u ^ sw) << 4), o.hi[4], o.hi[5], o.hi[6], o.hi[7]);
-                        sts128(hrow + WTMA_LO + ((0u ^ sw) << 4), o.lo[0], o.lo[1], o.lo[2], o.lo[3]);
-                        sts128(hrow + WTMA_LO + ((1u ^ sw) << 4), o.lo[4], o.lo[5], o.lo[6], o.lo[7]);
-                    }
-                }
-                if (has_f32) {
-                    if (wide_f) {
-                        const uint32_t sw = (uint32_t)(rl & 7);
-                        const uint32_t frow = stg + WTMA_F32_W + (uint32_t)rl * 128u;
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            sts128(frow + ((((uint32_t)(sub * 4 + i)) ^ sw) << 4), __float_as_uint(o.f[4 * i]),
-                                   __float_as_uint(o.f[4 * i + 1]), __float_as_uint(o.f[4 * i + 2]), __float_as_uint(o.f[4 * i + 3]));
-                    } else {
-                        const uint32_t sw = (uint32_t)((rl >> 1) & 3);                   // SWIZZLE_64B: bits 4-5 ^= bits 7-8
-                        const uint32_t frow = stg + WTMA_F32 + (uint32_t)sub * 8192u + (uint32_t)rl * 64u;
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            sts128(frow + (((uint32_t)i ^ sw) << 4), __float_as_uint(o.f[4 * i]), __float_as_uint(o.f[4 * i + 1]),
-                                   __float_as_uint(o.f[4 * i + 2]), __float_as_uint(o.f[4 * i + 3]));
-                    }
-                }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy writes -> the TMA engine's reads
-            epi_bar();                   // (GDN: every thread has also read its pre-activations of this group)
-            if (gdn && g + 2 < ngroups) aux_issue(g + 2);   // into the buffer this group has just released
-            if (et == 0 && rows_valid > 0 && !(cx.hack & 17)) {
-                if (has_hilo && wide) {
-                    if (g & 1) {
-                        tma_store_2d(cx.tmo + 3, stg, n0 + p0, m0);
-                        tma_store_2d(cx.tmo + 4, stg + WTMA_LO_W, n0 + p0, m0);
-                    }
-                } else if (has_hilo) {
-#pragma unroll
-                    for (int sb2 = 0; sb2 < 2; ++sb2) {
-                        const int c0 = n0 + g0 + sb2 * 16;
-                        if (g0 + sb2 * 16 < bn && c0 < ep.cout) {
-                            tma_store_2d(cx.tmo + 0, stg + (uint32_t)sb2 * 4096u, c0, m0);
-                            tma_store_2d(cx.tmo + 1, stg + WTMA_LO + (uint32_t)sb2 * 4096u, c0, m0);
-                        }
-                    }
-                }
-                if (has_f32 && wide_f) {
-                    tma_store_2d(cx.tmo + 5, stg + WTMA_F32_W, n0 + g0, m0);
-                } else if (has_f32) {
-#pragma unroll
-                    for (int sb2 = 0; sb2 < 2; ++sb2) {
-                        const int c0 = n0 + g0 + sb2 * 16;
-                        if (g0 + sb2 * 16 < bn && c0 < ep.cout) tma_store_2d(cx.tmo + 2, stg + WTMA_F32 + (uint32_t)sb2 * 8192u, c0, m0);
-                    }
-                }
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            }
-            if (gdn && g + 1 < ngroups) {                   // this thread's share of group g+1 has landed
-                if (g + 2 < ngroups) asm volatile("cp.async.wait_group 1;" ::: "memory");
-                else asm volatile("cp.async.wait_group 0;" ::: "memory");
-                if (et == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                epi_bar();               // staging planes free; next pre-activations visible
-            }
-            continue;
         }
         const int gc = sub * 16;
         auto stage_hl = [&]() {
@@ -451,7 +319,7 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
                 }
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
-                    if (ew * 16 + j * 4 + rsub < rows_valid && (!(cx.hack & 16) || v[j].x == 0x7fc12345u))
+                    if (ew * 16 + j * 4 + rsub < rows_valid)
                         *reinterpret_cast<uint4 *>(base + off[j]) = v[j];
             }
             if (mode == EPI_QUANT && ep.idx && c16 < 2 && c16 * 16 < nvalid) {      // 2 x 16 B per row
@@ -469,10 +337,9 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
                         *reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(dst[j]) + g0 + c16 * 16) = v[j];
             }
         };
-        const bool no_store = (cx.hack & 1) != 0;
         if (has_f32) {
             // pass F: stage the fp32 plane, then coalesced stores, 4 rows (128 B each) per warp instruction
-            if (ok && !no_store) {
+            if (ok) {
                 const uint32_t d = stg + rl * WF_STRIDE + gc * 4;
 #pragma unroll
                 for (int i = 0; i < 16; i += 4)
@@ -480,7 +347,7 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
                            __float_as_uint(o.f[i + 2]), __float_as_uint(o.f[i + 3]));
             }
             epi_bar();
-            if (c16 * 4 < nvalid && !no_store) {
+            if (c16 * 4 < nvalid) {
                 uint4 v[4];
                 unsigned long long dst[4];
 #pragma unroll
@@ -491,20 +358,20 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
                 }
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
-                    if (ew * 16 + j * 4 + rsub < rows_valid && (!(cx.hack & 16) || v[j].x == 0x7fc12345u))
+                    if (ew * 16 + j * 4 + rsub < rows_valid)
                         *reinterpret_cast<uint4 *>(reinterpret_cast<float *>(dst[j]) + g0 + c16 * 4) = v[j];
             }
             if (has_hilo) {
                 epi_bar();               // the fp32 stores have read the staging area
-                if (ok && !no_store) stage_hl();
+                if (ok) stage_hl();
                 epi_bar();
-                if (nvalid > 0 && !no_store) store_hl();
+                if (nvalid > 0) store_hl();
             }
         } else {
-            if (ok && !no_store) stage_hl();
+            if (ok) stage_hl();
             epi_bar();                   // (GDN: every thread has also read its pre-activations of this group)
             if (gdn && g + 2 < ngroups) aux_issue(g + 2);   // into the buffer this group has just released
-            if (nvalid > 0 && !no_store) store_hl();
+            if (nvalid > 0) store_hl();
             if (gdn && g + 1 < ngroups) {                   // this thread's share of group g+1 has landed
                 if (g + 2 < ngroups) asm volatile("cp.async.wait_group 1;" ::: "memory");
                 else asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -512,9 +379,6 @@ __device__ __forceinline__ void ws_tile_epilogue(const EpiParams &ep, int bn, in
         }
         if (g + 1 < ngroups) epi_bar();   // stores have read the staging area; next pre-activations visible
     }
-    // TMA-store form: this tile's bulk stores are complete (written, not just read from shared memory) before the caller
-    // publishes the tile / the kernel ends
-    if (tma && et == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
 }  // namespace

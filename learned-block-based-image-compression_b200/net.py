@@ -116,11 +116,11 @@ class BlockBasedImgCompLossyNetv9:
         'pair' (CTA-pair form of the persistent kernel), 'pdl', 'host_bands' (bands of block rows of the host calls),
         'wave' (persistent wavefront kernel for small steps), 'wave_max_rows'."""
         opt = {"force_bn": _lib.LBIC_OPT_FORCE_BN, "wave": _lib.LBIC_OPT_WAVE, "wave_max_rows": _lib.LBIC_OPT_WAVE_MAX_ROWS, "wave_dec_max_rows": _lib.LBIC_OPT_WAVE_DEC_MAX_ROWS,
-               "wave_bn": _lib.LBIC_OPT_WAVE_BN, "dec_smem_warp": _lib.LBIC_OPT_DEC_SMEM_WARP, "flow_quad": _lib.LBIC_OPT_FLOW_QUAD, "check_saturation": _lib.LBIC_OPT_CHECK_SATURATION, "flow_pair_min_rows": _lib.LBIC_OPT_FLOW_PAIR_MIN_ROWS, "tma_store": _lib.LBIC_OPT_TMA_STORE,
+               "wave_bn": _lib.LBIC_OPT_WAVE_BN, "dec_smem_warp": _lib.LBIC_OPT_DEC_SMEM_WARP, "check_saturation": _lib.LBIC_OPT_CHECK_SATURATION, "flow_pair_min_rows": _lib.LBIC_OPT_FLOW_PAIR_MIN_ROWS,
                "ws": _lib.LBIC_OPT_WS, "pdl": _lib.LBIC_OPT_PDL,
                "pair": _lib.LBIC_OPT_PAIR, "dec_thread_rows": _lib.LBIC_OPT_DEC_THREAD_ROWS,
                "enc_thread_streams": _lib.LBIC_OPT_ENC_THREAD_STREAMS, "enc_block_streams": _lib.LBIC_OPT_ENC_BLOCK_STREAMS, "flow": _lib.LBIC_OPT_FLOW,
-               "flow_min_rows": _lib.LBIC_OPT_FLOW_MIN_ROWS, "flow_small": _lib.LBIC_OPT_FLOW_SMALL,
+               "flow_min_rows": _lib.LBIC_OPT_FLOW_MIN_ROWS,
                "host_bands": _lib.LBIC_OPT_HOST_BANDS}[name]
         _lib.check(_lib.lib().lbic_set_option(self._need(), opt, int(value)))
 

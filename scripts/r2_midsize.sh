@@ -12,7 +12,7 @@ d=json.loads(sys.stdin.read()); print('value %.1f enc %.1f dec %.1f sm_mhz %s' %
 }
 for n in 128 256 512; do
   run "pair dataflow (default)" $n "LBIC_DUMMY=0"
-  run "single-CTA dataflow below 16384 rows" $n "LBIC_FLOW_SMALL=1 LBIC_FLOW_MIN_ROWS=16384"
+  run "single-CTA dataflow below 16384 rows" $n "LBIC_FLOW_MIN_ROWS=1 LBIC_FLOW_PAIR_MIN_ROWS=16384"
   run "per-layer launches" $n "LBIC_FLOW=0"
 done
 cat $L

@@ -16,7 +16,7 @@ def run(R, K, C, epi, pair, iters=30):
     ms = ctypes.c_double()
     _lib.check(L.lbic_debug_gemm_bench(m._need(), R, K, C, epi, iters, ctypes.byref(ms)))
     tf = 2.0 * R * K * C / (ms.value * 1e-3) / 1e12
-    print(f"stages<={os.environ.get('LBIC_WS_STAGES','-')} pair={pair} R={R:6d} K={K:5d} C={C:4d} {names[epi]:7s}: {ms.value*1e3:8.1f} us ({3*tf:7.1f} mma)", flush=True)
+    print(f"pair={pair} R={R:6d} K={K:5d} C={C:4d} {names[epi]:7s}: {ms.value*1e3:8.1f} us ({3*tf:7.1f} mma)", flush=True)
 for pair in (1, 3):
     for (K, C, e) in [(768, 768, 0), (768, 768, 1), (768, 768, 2), (1152, 960, 4), (768, 1152, 4), (672, 672, 1), (672, 672, 2), (576, 576, 2), (960, 768, 1)]:
         run(24576, K, C, e, pair)

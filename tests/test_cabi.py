@@ -29,11 +29,13 @@ def test_exports_every_declared_symbol():
     assert sorted(_lib.PROTOTYPES) == names
 
 
-def test_option_constants_match_the_header():
-    """Every LBIC_OPT_* of include/lbic.h has the same value in the python binding and a name in set_option()."""
+def test_option_constants_match_the_header_without_reusing_removed_numbers():
+    """Every LBIC_OPT_* of include/lbic.h has the same value in the python binding and a name in set_option(); the
+    numbers of removed options (13, 21, 24) are not given to new ones."""
     src = open(os.path.join(ROOT, "include", "lbic.h")).read()
     opts = {k: int(v) for k, v in re.findall(r"#define\s+(LBIC_OPT_[A-Z0-9_]+)\s+(\d+)", src)}
-    assert len(opts) >= 20 and len(set(opts.values())) == len(opts), "duplicate option numbers"
+    assert len(opts) >= 18 and len(set(opts.values())) == len(opts), "duplicate option numbers"
+    assert not {13, 21, 24} & set(opts.values()), "numbers of removed options are not reused"
     for k, v in opts.items():
         assert getattr(_lib, k, None) == v, f"{k}: header says {v}, _lib.py says {getattr(_lib, k, None)}"
 

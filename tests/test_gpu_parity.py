@@ -399,9 +399,10 @@ def test_warp_specialised_kernel_equals_per_tile_kernel(dev, cfgname):
 
 
 @pytest.mark.parametrize("cfgname", ["B8_lowrate", "B4_highrate", "B16_lowrate", "B8_highrate"])
-def test_dataflow_launch_equals_per_layer_launches(dev, cfgname):
+def test_dataflow_pair_and_single_cta_forms_equal_per_layer_launches(dev, cfgname):
     """gemm_flow_kernel (all layers of a step in one launch, row-block dependency counters instead of kernel boundaries)
-    must be bit-identical to one launch per layer, encode and decode, including ragged last row blocks."""
+    must be bit-identical to one launch per layer, encode and decode, including ragged last row blocks, in its CTA-pair
+    form and (KS3111) its single-CTA form, and must take fewer launches."""
     m = get_model(cfgname, 1337, False, dev)
     B = m.B
     from lbic_b200.layout import arrange_block_pixels_to_channel_dim
@@ -410,38 +411,34 @@ def test_dataflow_launch_equals_per_layer_launches(dev, cfgname):
     try:
         m.set_option("wave", 0)
         m.set_option("flow", 0)
+        l0 = m.launch_count()
         ref = m.compress_batch(x, lanes=0, return_symbols=True)
+        ref_launches = m.launch_count() - l0
         zref = m.decompress_batch(ref[0], x.shape, lanes=0)
         m.set_option("flow", 2)
-        for tma_store in (1, 0):     # TMA stores from swizzled staging planes / staged copy loops (the default)
-            m.set_option("tma_store", tma_store)
-            got = m.compress_batch(x, lanes=0, return_symbols=True)
-            assert got[0] == ref[0], f"bitstreams differ (tma_store={tma_store})"
-            assert torch.equal(got[1], ref[1]) and torch.equal(got[2], ref[2]) and torch.equal(got[3], ref[3])
-            zdec = m.decompress_batch(got[0], x.shape, lanes=0)
-            assert torch.equal(zdec, zref) and torch.equal(zdec, got[1])
+        l0 = m.launch_count()
+        got = m.compress_batch(x, lanes=0, return_symbols=True)
+        assert m.launch_count() - l0 < ref_launches, "the dataflow launch was not taken"
+        assert got[0] == ref[0], "bitstreams differ"
+        assert torch.equal(got[1], ref[1]) and torch.equal(got[2], ref[2]) and torch.equal(got[3], ref[3])
+        zdec = m.decompress_batch(got[0], x.shape, lanes=0)
+        assert torch.equal(zdec, zref) and torch.equal(zdec, got[1])
         zv, iv = m.validate_recu_reco(x)
         assert torch.equal(zv, got[1])
-        # the quad form: clusters of four CTAs, two pairs on adjacent column tiles sharing the activation operand by
-        # TMA multicast (layers with an odd number of column tiles give the second pair a dummy tile)
-        m.set_option("flow_quad", 1)
-        l0 = m.launch_count()
-        quad = m.compress_batch(x, lanes=0, return_symbols=True)
-        assert quad[0] == ref[0], "bitstreams differ (quad form)"
-        assert torch.equal(quad[1], ref[1]) and torch.equal(quad[2], ref[2]) and torch.equal(quad[3], ref[3])
-        assert torch.equal(m.decompress_batch(quad[0], x.shape, lanes=0), zref)
-        m.set_option("flow_quad", 0)
-        # the single-CTA form for small steps (128 x 96 tiles, off by default)
-        m.set_option("flow", 1)
-        m.set_option("flow_small", 1)
-        small = m.compress_batch(x, lanes=0, return_symbols=True)
-        assert small[0] == ref[0] and torch.equal(small[1], ref[1]) and torch.equal(small[2], ref[2])
-        assert torch.equal(m.decompress_batch(small[0], x.shape, lanes=0), zref)
+        if lbic_b200.load_config(cfgname).KS[1] == 1:
+            # the single-CTA form of mid-size steps (128 x 96 tiles), forced for every step (KS3311 runs pairs only)
+            m.set_option("flow", 1)
+            m.set_option("flow_min_rows", 1)
+            m.set_option("flow_pair_min_rows", 1 << 30)
+            l0 = m.launch_count()
+            small = m.compress_batch(x, lanes=0, return_symbols=True)
+            assert m.launch_count() - l0 < ref_launches, "the single-CTA dataflow launch was not taken"
+            assert small[0] == ref[0] and torch.equal(small[1], ref[1]) and torch.equal(small[2], ref[2])
+            assert torch.equal(m.decompress_batch(small[0], x.shape, lanes=0), zref)
     finally:
         m.set_option("flow", 1)
-        m.set_option("flow_small", 0)
-        m.set_option("flow_quad", 0)
-        m.set_option("tma_store", 0)
+        m.set_option("flow_min_rows", 2560)
+        m.set_option("flow_pair_min_rows", 8192)
         m.set_option("wave", 1)
 
 

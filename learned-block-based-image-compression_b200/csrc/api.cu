@@ -77,6 +77,11 @@ struct ActView {   // an activation buffer seen as a GEMM A operand of logical w
     CUtensorMap tm_small[4][2];       // boxes of 64 k x 16 / 32 / 48 / 64 rows, [class][hi, lo] (latency kernel)
 };
 
+struct LayerWiring {   // one layer of a step: its operand per K segment and its epilogue (R and step are filled in per launch)
+    const ActView *a[2] = {nullptr, nullptr};
+    EpiParams ep;
+};
+
 struct Workspace {
     int n_img = 0, Hb = 0, Wb = 0, R_cap = 0;
     float *x_cl = nullptr, *zhat_cl = nullptr;
@@ -94,7 +99,10 @@ struct Workspace {
     size_t rans_scratch_words = 0;   // total words allocated
     RansStreamState *dec_states = nullptr;
     const uint8_t **lane_ptr = nullptr;
-    std::vector<ChainLayer> h_chain;   // host copy of the per-layer chain descriptors (indexed by LayerId)
+    // the layer table (ensure_workspace), indexed by LayerId: [L_E0, L_COUNT) is a whole encode step
+    LayerWiring net[L_COUNT];
+    int dep[L_COUNT][2] = {};          // the layers each layer reads from (operands and epilogue side inputs), -1 = none
+    std::vector<ChainLayer> h_chain;   // the table as the dataflow and wavefront kernels read it (build_chain)
     ChainLayer *d_chain = nullptr;
     int *flow_counters = nullptr;      // (layer, 256-row block) completion counters of the dataflow launch
     size_t flow_counters_cap = 0;
@@ -141,15 +149,12 @@ struct lbic_model {
     int wave_max_rows = 1536;
     int wave_dec_max_rows = 64;    // decode: the rANS tiles run one warp per row on 8 entropy CTAs (64 rows at a time)
     int wave_bn = 0;               // forced tile width of the wave kernel (32 / 64 / 128), 0 = by rows per step
-    float *selfinfo_cl = nullptr;   // set by lbic_validate for the duration of the call: (n,Hb,Wb,M) self-information
     cudaStream_t hs[3] = {nullptr, nullptr, nullptr};   // host-call pipeline: copies in, compute, copies out
     cudaEvent_t hev[2 * LBIC_MAX_BANDS] = {};            // band b copied in / band b ready to copy out
     // grow-only device temporaries of lbic_validate / lbic_forward (channel-last self-information, reconstruction)
     float *aux[3] = {nullptr, nullptr, nullptr};     // [2]: scratch of lbic_image_metrics
     size_t aux_bytes[3] = {0, 0, 0};
     int host_bands = LBIC_MAX_BANDS;   // host calls: bands of block rows per batch (copy / compute overlap granularity)
-    float *recon_cl = nullptr;      // set by lbic_forward: the decoder net writes here instead of the zhat feedback buffer
-    int recon_no_clamp = 0;
     // block-row-band mode (one large image over several GPUs): geometry of the call in progress
     int band_n = 0, band_Hb = 0, band_Wb = 0, band_decode = 0;
     int64_t launches[2] = {0, 0};
@@ -172,12 +177,13 @@ struct lbic_model {
 
 namespace {
 
-struct Active {   // routes launch counting to the model for the duration of an API call
-    explicit Active(lbic_model *m) {
+struct Active {   // routes launch counting to the model for the duration of an API call (a nested call restores it)
+    explicit Active(lbic_model *m) : prev(g_launch_counter) {
         g_launch_counter = m ? m->launches : nullptr;
         if (m) cudaSetDevice(m->device);
     }
-    ~Active() { g_launch_counter = nullptr; }
+    ~Active() { g_launch_counter = prev; }
+    int64_t *prev;
 };
 
 int dev_alloc(std::vector<void *> &list, void **p, size_t bytes, bool zero = false) {
@@ -395,10 +401,100 @@ int make_view(Workspace &ws, ActView &v, const ActBuf &b, int K) {
     return 0;
 }
 
-int build_chain(lbic_model *m);
-EpiParams epi(int mode, const StepDesc &sd);
-EpiParams epi_hilo(int mode, const StepDesc &sd, const ActBuf &out);
-EpiParams epi_pregdn(lbic_model *m, const StepDesc &sd);
+EpiParams epi(int mode, const StepDesc &sd) {
+    EpiParams e;
+    memset(&e, 0, sizeof(e));
+    e.mode = mode;
+    e.step = sd;
+    return e;
+}
+
+EpiParams epi_hilo(int mode, const StepDesc &sd, const ActBuf &out) {
+    EpiParams e = epi(mode, sd);
+    e.out_hi = out.hi; e.out_lo = out.lo; e.ld_out = out.ld;
+    return e;
+}
+
+// The layer table: the network of one step wired into the workspace.  For every layer its operand view per K segment,
+// its epilogue and the layers it reads from.  run_layers launches it one layer at a time; the dataflow and wavefront
+// kernels read the copy build_chain makes.
+void wire_layers(lbic_model *m) {
+    Workspace &ws = m->ws;
+    const StepDesc none = {};
+    auto wire = [&](int id, const ActView *a0, const ActView *a1, const EpiParams &ep, int d0, int d1 = -1) -> EpiParams & {
+        ws.net[id].a[0] = a0; ws.net[id].a[1] = a1;
+        ws.net[id].ep = ep;
+        ws.dep[id][0] = d0; ws.dep[id][1] = d1;
+        return ws.net[id].ep;
+    };
+    auto lrelu = [&](int id, const ActView *a, const ActBuf &out, int d0) -> EpiParams & {
+        return wire(id, a, nullptr, epi_hilo(EPI_LRELU, none, out), d0);
+    };
+    // a = acc + b: fp32 into A32 for the GDN layer that follows, a * a into S as its operand
+    auto pregdn = [&](int id, const ActView *a0, const ActView *a1, int d0) {
+        EpiParams &e = wire(id, a0, a1, epi_hilo(EPI_PREGDN, none, ws.S), d0);
+        e.out_f32 = ws.A32; e.ld_f32 = ws.ldA32;
+    };
+    // GDN / IGDN stage i (widths N, C2, C3): S (squares) -> U
+    auto gdn = [&](int id, int i, int mode, int d0) {
+        EpiParams &e = wire(id, &ws.vS[i], nullptr, epi_hilo(mode, none, ws.U), d0);
+        e.aux = ws.A32; e.ld_aux = ws.ldA32;
+    };
+    // entropy-parameter net: T -> ksi   (get_meanscale_fast, NET:389-398).  KS[1] = 3: E0 runs on the rows of the
+    // ring-extended step and scatters into the g0 store (run_g0); E1 reads the five g0 taps around each block.
+    if (m->k1 == 3) {
+        lrelu(L_E0, &ws.vText, ws.G0, -1).out_pos = 1;
+        lrelu(L_E1, &ws.vH1x5, ws.H2, L_E0);
+    } else {
+        lrelu(L_E0, &ws.vT, ws.H1, -1);
+        lrelu(L_E1, &ws.vH1, ws.H2, L_E0);
+    }
+    lrelu(L_E2, &ws.vH2, ws.H3, L_E1);
+    EpiParams &ksi = wire(L_E3, &ws.vH3, nullptr, epi(EPI_KSI, none), L_E2);
+    ksi.out_f32 = ws.KSI; ksi.ld_f32 = ws.ldKSI;
+    // encoder net + quantisation: X, T, ksi -> symbols, indexes, y_qnt   (forward_prtr_fast NET:379-382, NET:371-374)
+    pregdn(L_F0, &ws.vX, &ws.vT, -1);
+    gdn(L_G0, 0, EPI_GDN, L_F0);
+    pregdn(L_F1, &ws.vU[0], nullptr, L_G0);
+    gdn(L_G1, 1, EPI_GDN, L_F1);
+    pregdn(L_F2, &ws.vU[1], nullptr, L_G1);
+    gdn(L_G2, 2, EPI_GDN, L_F2);
+    EpiParams &q = wire(L_F3, &ws.vU[2], nullptr, epi_hilo(EPI_QUANT, none, ws.YQ), L_G2, L_E3);
+    q.aux = ws.KSI; q.ld_aux = ws.ldKSI; q.M = m->M; q.sym = ws.sym; q.idx = ws.idx;
+    // decoder net: y_qnt, T -> zhat block, clamped   (inverse_prtr_fast NET:384-387, NET:357)
+    pregdn(L_D0, &ws.vYQ, &ws.vT, L_F3);
+    gdn(L_IG0, 0, EPI_IGDN, L_D0);
+    pregdn(L_D1, &ws.vU[0], nullptr, L_IG0);
+    gdn(L_IG1, 1, EPI_IGDN, L_D1);
+    pregdn(L_D2, &ws.vU[1], nullptr, L_IG1);
+    gdn(L_IG2, 2, EPI_IGDN, L_D2);
+    wire(L_D3, &ws.vU[2], nullptr, epi(EPI_RECON, none), L_IG2).zhat = ws.zhat_cl;
+}
+
+// The layer table as the dataflow and wavefront kernels read it: one ChainLayer per LayerId, in device memory.
+int build_chain(lbic_model *m) {
+    Workspace &ws = m->ws;
+    ws.h_chain.assign(L_COUNT, ChainLayer());
+    for (int id = 0; id < L_COUNT; ++id) {
+        ChainLayer &c = ws.h_chain[id];
+        const PackedLayer &L = m->L[id];
+        memset(&c, 0, sizeof(c));
+        c.nseg = L.nseg; c.cout = L.cout; c.n_bn = L.n_bn;
+        for (int s = 0; s < L.nseg; ++s) {
+            const ActView *a = ws.net[id].a[s];
+            c.kb[s] = (L.seg[s].K + 63) / 64;
+            c.tmA[s][0] = a->tm_hi; c.tmA[s][1] = a->tm_lo;
+            for (int b = 0; b < 4; ++b) { c.tmAs[b][s][0] = a->tm_small[b][0]; c.tmAs[b][s][1] = a->tm_small[b][1]; }
+            for (int v = 0; v < L.n_bn; ++v) { c.tmW[v][s][0] = L.seg[s].tm_hi[v]; c.tmW[v][s][1] = L.seg[s].tm_lo[v]; }
+        }
+        for (int v = 0; v < L.n_bn; ++v) c.bn_v[v] = L.bn_v[v];
+        c.ep = ws.net[id].ep;
+        c.ep.cout = L.cout; c.ep.bias = L.bias; c.ep.scale_tab = m->tables.d_scale_table; c.ep.acc_scale = L.acc_scale;
+    }
+    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.d_chain, sizeof(ChainLayer) * L_COUNT));
+    LBIC_CUDA(cudaMemcpy(ws.d_chain, ws.h_chain.data(), sizeof(ChainLayer) * L_COUNT, cudaMemcpyHostToDevice));
+    return 0;
+}
 
 int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     Workspace &ws = m->ws;
@@ -459,6 +555,7 @@ int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.idx, nblk * m->M));
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.dec_states, sizeof(RansStreamState) * (size_t)n_img * Hb));
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.lane_ptr, sizeof(void *) * (size_t)n_img * Hb));
+    wire_layers(m);
     LBIC_TRY(build_chain(m));
     ws.flow_counters_cap = (size_t)L_COUNT * ((ws.R_cap + 127) / 128 + 1);
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.flow_counters, sizeof(int) * ws.flow_counters_cap, true));
@@ -466,85 +563,6 @@ int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.wave_counters, sizeof(int) * ws.wave_counters_cap, true));
     return 0;
 }
-
-// Per-layer descriptors of the persistent chain kernel: the same operand views and epilogues run_ent / run_enc /
-// run_dec pass to the per-layer path, indexed by LayerId (so [L_E0, L_COUNT) is a whole encode step).
-int build_chain(lbic_model *m) {
-    Workspace &ws = m->ws;
-    ws.h_chain.assign(L_COUNT, ChainLayer());
-    StepDesc none;
-    memset(&none, 0, sizeof(none));
-    auto set = [&](int id, const ActView *a0, const ActView *a1, EpiParams ep) {
-        ChainLayer &c = ws.h_chain[id];
-        const PackedLayer &L = m->L[id];
-        memset(&c, 0, sizeof(c));
-        c.nseg = L.nseg; c.cout = L.cout; c.n_bn = L.n_bn;
-        const ActView *av[2] = {a0, a1};
-        for (int s = 0; s < L.nseg; ++s) {
-            c.kb[s] = (L.seg[s].K + 63) / 64;
-            c.tmA[s][0] = av[s]->tm_hi; c.tmA[s][1] = av[s]->tm_lo;
-            for (int b = 0; b < 4; ++b) { c.tmAs[b][s][0] = av[s]->tm_small[b][0]; c.tmAs[b][s][1] = av[s]->tm_small[b][1]; }
-            for (int v = 0; v < L.n_bn; ++v) { c.tmW[v][s][0] = L.seg[s].tm_hi[v]; c.tmW[v][s][1] = L.seg[s].tm_lo[v]; }
-        }
-        for (int v = 0; v < L.n_bn; ++v) c.bn_v[v] = L.bn_v[v];
-        ep.cout = L.cout; ep.bias = L.bias; ep.scale_tab = m->tables.d_scale_table; ep.acc_scale = L.acc_scale;
-        c.ep = ep;
-    };
-    auto pre = [&]() { return epi_pregdn(m, none); };
-    auto gdn = [&](bool inv) {
-        EpiParams e = epi_hilo(inv ? EPI_IGDN : EPI_GDN, none, ws.U);
-        e.aux = ws.A32; e.ld_aux = ws.ldA32;
-        return e;
-    };
-    if (m->k1 == 3) {
-        {
-            EpiParams e0 = epi_hilo(EPI_LRELU, none, ws.G0);                // rows of the EXTENDED step, scattered into the g0
-            e0.out_pos = 1;                                                 // store (wave kernel; the dataflow launch starts at E1)
-            set(L_E0, &ws.vText, nullptr, e0);
-        }
-        set(L_E1, &ws.vH1x5, nullptr, epi_hilo(EPI_LRELU, none, ws.H2));
-    } else {
-        set(L_E0, &ws.vT, nullptr, epi_hilo(EPI_LRELU, none, ws.H1));
-        set(L_E1, &ws.vH1, nullptr, epi_hilo(EPI_LRELU, none, ws.H2));
-    }
-    set(L_E2, &ws.vH2, nullptr, epi_hilo(EPI_LRELU, none, ws.H3));
-    {
-        EpiParams e = epi(EPI_KSI, none);
-        e.out_f32 = ws.KSI; e.ld_f32 = ws.ldKSI;
-        set(L_E3, &ws.vH3, nullptr, e);
-    }
-    set(L_F0, &ws.vX, &ws.vT, pre());
-    set(L_G0, &ws.vS[0], nullptr, gdn(false));
-    set(L_F1, &ws.vU[0], nullptr, pre());
-    set(L_G1, &ws.vS[1], nullptr, gdn(false));
-    set(L_F2, &ws.vU[1], nullptr, pre());
-    set(L_G2, &ws.vS[2], nullptr, gdn(false));
-    {
-        EpiParams e = epi_hilo(EPI_QUANT, none, ws.YQ);
-        e.aux = ws.KSI; e.ld_aux = ws.ldKSI; e.M = m->M; e.sym = ws.sym; e.idx = ws.idx;
-        set(L_F3, &ws.vU[2], nullptr, e);
-    }
-    set(L_D0, &ws.vYQ, &ws.vT, pre());
-    set(L_IG0, &ws.vS[0], nullptr, gdn(true));
-    set(L_D1, &ws.vU[0], nullptr, pre());
-    set(L_IG1, &ws.vS[1], nullptr, gdn(true));
-    set(L_D2, &ws.vU[1], nullptr, pre());
-    set(L_IG2, &ws.vS[2], nullptr, gdn(true));
-    {
-        EpiParams e = epi(EPI_RECON, none);
-        e.zhat = ws.zhat_cl;
-        set(L_D3, &ws.vU[2], nullptr, e);
-    }
-    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.d_chain, sizeof(ChainLayer) * L_COUNT));
-    LBIC_CUDA(cudaMemcpy(ws.d_chain, ws.h_chain.data(), sizeof(ChainLayer) * L_COUNT, cudaMemcpyHostToDevice));
-    return 0;
-}
-
-// which layers each layer reads from (operands and epilogue side inputs), by LayerId; -1 = inputs of the step
-const int FLOW_DEP[L_COUNT][2] = {
-    {-1, -1}, {L_E0, -1}, {L_E1, -1}, {L_E2, -1},                                              // E0..E3
-    {-1, -1}, {L_F0, -1}, {L_G0, -1}, {L_F1, -1}, {L_G1, -1}, {L_F2, -1}, {L_G2, L_E3},          // F0 G0 F1 G1 F2 G2 F3 (ksi)
-    {L_F3, -1}, {L_D0, -1}, {L_IG0, -1}, {L_D1, -1}, {L_IG1, -1}, {L_D2, -1}, {L_IG2, -1}};     // D0 IG0 D1 IG1 D2 IG2 D3
 
 // 0: one launch per layer; 1: dataflow launch on CTA pairs (large steps); 2: dataflow launch on single CTAs (mid-size steps)
 int flow_applies(const lbic_model *m, int R) {
@@ -562,27 +580,6 @@ int flow_applies(const lbic_model *m, int R) {
     return (long)R * (m->N > 0 ? m->N : 768) >= (long)m->flow_pair_min_rows * 768 ? 1 : 2;
 }
 
-int run_flow(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    ProfRec rec;
-    if (m->profiling) {
-        double fl = 0;
-        for (int l = l0; l < l1; ++l)
-            for (int s = 0; s < m->L[l].nseg; ++s) fl += 2.0 * R * (double)m->L[l].seg[s].K * m->L[l].cout;
-        cudaEventCreate(&rec.a); cudaEventCreate(&rec.b);
-        rec.flops = fl;
-        rec.layer = -1;
-        cudaEventRecord(rec.a, st);
-    }
-    const int rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, FLOW_DEP, R, sd, ws.flow_counters,
-                                    ws.flow_counters_cap, st, flow_applies(m, R) == 1 ? 1 : 0);
-    if (m->profiling) {
-        cudaEventRecord(rec.b, st);
-        m->prof.push_back(rec);
-    }
-    return rc;
-}
-
 int ensure_rans_scratch(lbic_model *m, size_t words) {
     Workspace &ws = m->ws;
     if (ws.rans_scratch_words >= words) return 0;
@@ -593,11 +590,6 @@ int ensure_rans_scratch(lbic_model *m, size_t words) {
 }
 
 // ---- GEMM dispatch --------------------------------------------------------------------------------
-int run_gemm_layer(lbic_model *m, const PackedLayer &L, int id, int R, const ActView *a0, const ActView *a1, EpiParams ep,
-                   cudaStream_t st);
-int run_gemm(lbic_model *m, int id, int R, const ActView *a0, const ActView *a1, EpiParams ep, cudaStream_t st) {
-    return run_gemm_layer(m, m->L[id], id, R, a0, a1, ep, st);
-}
 int run_gemm_layer(lbic_model *m, const PackedLayer &L, int id, int R, const ActView *a0, const ActView *a1, EpiParams ep,
                    cudaStream_t st) {
     GemmCall g;
@@ -672,18 +664,47 @@ int run_gemm_layer(lbic_model *m, const PackedLayer &L, int id, int R, const Act
     return rc;
 }
 
-EpiParams epi(int mode, const StepDesc &sd) {
-    EpiParams e;
-    memset(&e, 0, sizeof(e));
-    e.mode = mode;
-    e.step = sd;
-    return e;
+// Layers [l0, l1) of the layer table for the R rows of step `sd`, one launch each.  F3 writes symbols and indexes only
+// when `syms`; `recon` (if set) takes D3's reconstruction in place of the zhat feedback buffer, clamped unless `no_clamp`.
+int run_layers(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStream_t st, bool syms = true,
+               float *recon = nullptr, int no_clamp = 0) {
+    for (int id = l0; id < l1; ++id) {
+        const LayerWiring &w = m->ws.net[id];
+        EpiParams ep = w.ep;
+        ep.step = sd;
+        if (id == L_F3 && !syms) { ep.sym = nullptr; ep.idx = nullptr; }
+        if (id == L_D3 && recon) { ep.zhat = recon; ep.no_clamp = no_clamp; }
+        LBIC_TRY(run_gemm_layer(m, m->L[id], id, R, w.a[0], w.a[1], ep, st));
+    }
+    return 0;
 }
 
-EpiParams epi_hilo(int mode, const StepDesc &sd, const ActBuf &out) {
-    EpiParams e = epi(mode, sd);
-    e.out_hi = out.hi; e.out_lo = out.lo; e.ld_out = out.ld;
-    return e;
+// Layers [l0, l1) of a step: one dataflow launch where it applies (it always writes F3's symbols and indexes), else one
+// launch per layer.  If the dataflow launch itself is refused (no co-residency: a shared or partitioned GPU), the
+// per-layer path takes over for good.
+int run_range(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, bool syms, cudaStream_t st) {
+    if (const int form = flow_applies(m, R)) {
+        Workspace &ws = m->ws;
+        ProfRec rec;
+        if (m->profiling) {
+            double fl = 0;
+            for (int l = l0; l < l1; ++l)
+                for (int s = 0; s < m->L[l].nseg; ++s) fl += 2.0 * R * (double)m->L[l].seg[s].K * m->L[l].cout;
+            cudaEventCreate(&rec.a); cudaEventCreate(&rec.b);
+            rec.flops = fl;
+            rec.layer = -1;
+            cudaEventRecord(rec.a, st);
+        }
+        const int rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, ws.dep, R, sd, ws.flow_counters,
+                                        ws.flow_counters_cap, st, form == 1 ? 1 : 0);
+        if (m->profiling) {
+            cudaEventRecord(rec.b, st);
+            m->prof.push_back(rec);
+        }
+        if (rc != LBIC_FLOW_REFUSED) return rc;
+        m->use_flow = 0;
+    }
+    return run_layers(m, l0, l1, sd, R, st, syms);
 }
 
 // KS[1] == 3: hidden map g0 = lrelu(E0(zhat taps)) at the ring-extended positions `ext` (single-position or
@@ -694,73 +715,17 @@ int run_g0(lbic_model *m, const StepDesc &ext, int R_ext, cudaStream_t st) {
     if (R_ext > ws.R_ext_cap) return lbic_fail(LBIC_ERR_INVALID, "internal: extended step exceeds its workspace");
     LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, ext, R_ext, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo,
                            ws.Text.ld, st));
-    EpiParams e = epi_hilo(EPI_LRELU, ext, ws.G0);
-    e.out_pos = 1;
-    return run_gemm(m, L_E0, R_ext, &ws.vText, nullptr, e, st);
+    return run_layers(m, L_E0, L_E1, ext, R_ext, st);
 }
 
-// entropy-parameter net: T (or the g0 store) -> ksi   (get_meanscale_fast, NET:389-398)
-int run_ent(lbic_model *m, const StepDesc &sd, int R, cudaStream_t st) {
+// The first layer of a step and its operand: E0 on the zhat taps, or (KS[1] == 3: E0 has run on the ring-extended rows,
+// run_g0) E1 on the five g0 taps around each block, gathered here.
+int step_entry(lbic_model *m, const StepDesc &sd, int R, int *first, cudaStream_t st) {
     Workspace &ws = m->ws;
-    if (m->k1 == 3) {
-        LBIC_TRY(launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st));
-        LBIC_TRY(run_gemm(m, L_E1, R, &ws.vH1x5, nullptr, epi_hilo(EPI_LRELU, sd, ws.H2), st));
-    } else {
-        LBIC_TRY(run_gemm(m, L_E0, R, &ws.vT, nullptr, epi_hilo(EPI_LRELU, sd, ws.H1), st));
-        LBIC_TRY(run_gemm(m, L_E1, R, &ws.vH1, nullptr, epi_hilo(EPI_LRELU, sd, ws.H2), st));
-    }
-    LBIC_TRY(run_gemm(m, L_E2, R, &ws.vH2, nullptr, epi_hilo(EPI_LRELU, sd, ws.H3), st));
-    EpiParams e = epi(EPI_KSI, sd);
-    e.out_f32 = ws.KSI; e.ld_f32 = ws.ldKSI;
-    LBIC_TRY(run_gemm(m, L_E3, R, &ws.vH3, nullptr, e, st));
-    return 0;
-}
-
-// GDN / IGDN stage i (widths N, C2, C3): S (squares) -> U
-int run_gdn(lbic_model *m, int id, int i, bool inverse, const StepDesc &sd, int R, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    EpiParams e = epi_hilo(inverse ? EPI_IGDN : EPI_GDN, sd, ws.U);
-    e.aux = ws.A32; e.ld_aux = ws.ldA32;
-    return run_gemm(m, id, R, &ws.vS[i], nullptr, e, st);
-}
-
-EpiParams epi_pregdn(lbic_model *m, const StepDesc &sd) {
-    Workspace &ws = m->ws;
-    EpiParams e = epi_hilo(EPI_PREGDN, sd, ws.S);
-    e.out_f32 = ws.A32; e.ld_f32 = ws.ldA32;
-    return e;
-}
-
-// encoder net + quantisation: X, T, ksi -> symbols, indexes, y_qnt   (forward_prtr_fast NET:379-382, NET:371-374)
-int run_enc(lbic_model *m, const StepDesc &sd, int R, int32_t *sym, uint8_t *idx, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    LBIC_TRY(run_gemm(m, L_F0, R, &ws.vX, &ws.vT, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_G0, 0, false, sd, R, st));
-    LBIC_TRY(run_gemm(m, L_F1, R, &ws.vU[0], nullptr, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_G1, 1, false, sd, R, st));
-    LBIC_TRY(run_gemm(m, L_F2, R, &ws.vU[1], nullptr, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_G2, 2, false, sd, R, st));
-    EpiParams e = epi_hilo(EPI_QUANT, sd, ws.YQ);
-    e.aux = ws.KSI; e.ld_aux = ws.ldKSI; e.M = m->M;
-    e.sym = sym; e.idx = idx;
-    LBIC_TRY(run_gemm(m, L_F3, R, &ws.vU[2], nullptr, e, st));
-    return 0;
-}
-
-// decoder net: y_qnt, T -> zhat block, clamped   (inverse_prtr_fast NET:384-387, NET:357)
-int run_dec(lbic_model *m, const StepDesc &sd, int R, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    LBIC_TRY(run_gemm(m, L_D0, R, &ws.vYQ, &ws.vT, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_IG0, 0, true, sd, R, st));
-    LBIC_TRY(run_gemm(m, L_D1, R, &ws.vU[0], nullptr, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_IG1, 1, true, sd, R, st));
-    LBIC_TRY(run_gemm(m, L_D2, R, &ws.vU[1], nullptr, epi_pregdn(m, sd), st));
-    LBIC_TRY(run_gdn(m, L_IG2, 2, true, sd, R, st));
-    EpiParams e = epi(EPI_RECON, sd);
-    e.zhat = m->recon_cl ? m->recon_cl : ws.zhat_cl;
-    e.no_clamp = m->recon_no_clamp;
-    LBIC_TRY(run_gemm(m, L_D3, R, &ws.vU[2], nullptr, e, st));
-    return 0;
+    *first = L_E0;
+    if (m->k1 != 3) return 0;
+    *first = L_E1;
+    return launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st);
 }
 
 int floor_div2(int a) { return a >= 0 ? a / 2 : -((-a + 1) / 2); }
@@ -819,8 +784,7 @@ struct RowHooks {
 
 // The persistent wavefront kernel (gemm_wave.cu) takes over when every step of the call has at most wave_max_rows rows.
 bool wave_applies(const lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool decode) {
-    if (!m->use_wave || m->gemm_core != 0 || m->force_bn || m->profiling || m->check_sat || m->selfinfo_cl ||
-        m->recon_cl || !gemm_wave_supported())
+    if (!m->use_wave || m->gemm_core != 0 || m->force_bn || m->profiling || m->check_sat || !gemm_wave_supported())
         return false;
     const int max_nv = Hb < (Wb + 1) / 2 ? Hb : (Wb + 1) / 2;
     if (m->k1 == 3) {
@@ -848,7 +812,6 @@ int run_wave(lbic_model *m, bool decode, bool raster, int s_begin, int s_end, in
     w.d_layers = ws.d_chain; w.h_layers = ws.h_chain.data();
     w.decode = decode ? 1 : 0; w.raster = raster ? 1 : 0;
     w.s_begin = s_begin; w.s_end = s_end; w.n_img = n_img; w.Hb = Hb; w.Wb = Wb;
-    for (int i = 0; i < L_COUNT; ++i) w.ids[i] = i;
     {
         // tile width: 32 columns.  The MMA chain of a tile takes the same time for any width up to ~176 columns (it is
         // bound by the latency of dependent accumulations), but the staged epilogue grows with the width (1.5 us per 32
@@ -878,6 +841,109 @@ int run_wave(lbic_model *m, bool decode, bool raster, int s_begin, int s_end, in
     return gemm_wave_launch(w, st);
 }
 
+// One wavefront step of an encode: entropy net, encoder net + quantisation, decoder net for the R rows of `sd`
+// (NET:363-377 for every block of the diagonal at once).
+int encode_step(lbic_model *m, const StepDesc &sd, int R, bool syms, cudaStream_t st) {
+    Workspace &ws = m->ws;
+    int l0;
+    LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, sd, R, &l0, st));
+    return run_range(m, l0, L_COUNT, sd, R, syms, st);
+}
+
+// One step of a decode: entropy net, rANS decode of y_qnt (and of the symbols into `sym`, if set) from `lanes` streams
+// per image, decoder net (NET:420-450 for every block of the step at once).
+int decode_step(lbic_model *m, const StepDesc &sd, int R, int lanes, int32_t *sym, cudaStream_t st) {
+    Workspace &ws = m->ws;
+    int l0;
+    LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, sd, R, &l0, st));
+    LBIC_TRY(run_range(m, l0, L_F0, sd, R, true, st));
+    LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, lanes, sd, R, m->M, ws.KSI, ws.ldKSI, ws.YQ.hi,
+                                  ws.YQ.lo, ws.YQ.ld, sym, st));
+    return run_range(m, L_D0, L_COUNT, sd, R, true, st);
+}
+
+// Step s of a call: wavefront step t = s, or (raster) block (v, h) of every image with s = v * Wb + h.  False if the
+// step has no block of the image (KS[1] == 3: step -1 has ring positions only).
+bool step_desc(int s, bool raster, int n_img, int Hb, int Wb, StepDesc &sd) {
+    if (!raster) return wave_step(s, n_img, Hb, Wb, sd);
+    const int v = s / Wb, h = s - v * Wb;
+    sd = StepDesc{n_img, 1, v, h + 2 * v, Hb, Wb};
+    return true;
+}
+
+// The step loop of an encode or a decode.  Each step runs through `step(sd, R)` (per-layer or dataflow launches) after
+// the hidden-map ring positions (KS[1] == 3) that become computable with it, or, when `wave` (small steps: single images,
+// small batches), consecutive steps are collected into ONE launch of the persistent wavefront kernel, `wave_range(s0,
+// s1)`, cut only where a host hook has copies or conversions to put between two steps.
+template <class Step, class WaveRange>
+int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, const RowHooks *hk, Step step,
+              WaveRange wave_range, cudaStream_t st) {
+    auto launch_step = [&](int s) -> int {
+        if (m->k1 == 3 && raster) {
+            // hidden-map positions that become computable now: the ring columns of the row start, then (v,h)
+            const int v = s / Wb, h = s - v * Wb;
+            if (h == 0) {
+                if (v >= 1) { StepDesc e{n_img, 1, v - 1, Wb + 2 * (v - 1), Hb, Wb}; LBIC_TRY(run_g0(m, e, n_img, st)); }
+                StepDesc e{n_img, 1, v, -1 + 2 * v, Hb, Wb};
+                LBIC_TRY(run_g0(m, e, n_img, st));
+            }
+            StepDesc e{n_img, 1, v, h + 2 * v, Hb, Wb};
+            LBIC_TRY(run_g0(m, e, n_img, st));
+        } else if (m->k1 == 3) {
+            StepDesc ext;
+            if (wave_step_ext(s, n_img, Hb, Wb, ext)) LBIC_TRY(run_g0(m, ext, n_img * ext.nv, st));
+        }
+        StepDesc sd;
+        if (!step_desc(s, raster, n_img, Hb, Wb, sd)) return 0;
+        return step(sd, n_img * sd.nv);
+    };
+    int pend = -1;                                   // steps [pend, s) wait to be launched
+    auto flush = [&](int s_end) -> int {
+        if (pend < 0) return 0;
+        const int b = pend;
+        pend = -1;
+        const int rc = wave_range(b, s_end);
+        if (rc != LBIC_FLOW_REFUSED) return rc;
+        m->use_wave = 0;                             // no co-residency on this device: per-layer launches from now on
+        wave = false;
+        for (int s = b; s < s_end; ++s) LBIC_TRY(launch_step(s));
+        return 0;
+    };
+    const int s_first = raster ? 0 : (m->k1 == 3 ? -1 : 0);
+    const int s_last = raster ? Hb * Wb : Wb + 2 * (Hb - 1);
+    for (int s = s_first; s < s_last; ++s) {
+        StepDesc sd;
+        const bool has = step_desc(s, raster, n_img, Hb, Wb, sd);
+        if (has && hk && hk->need_rows) {
+            const int v_hi = sd.vmin + sd.nv - 1;
+            if (!wave || !hk->will_need || hk->will_need(hk->ctx, v_hi)) {
+                LBIC_TRY(flush(s));
+                LBIC_TRY(hk->need_rows(hk->ctx, v_hi, st));
+            }
+        }
+        if (wave && has) {
+            if (pend < 0) pend = s;
+        } else {
+            LBIC_TRY(launch_step(s));                // (wave: step -1 of KS[1] = 3 is one small GEMM on the per-layer path)
+        }
+        if (has && hk && hk->rows_done) {
+            int done = 0;                            // zhat block rows [0, done) are final after step s
+            if (raster) {
+                if ((s + 1) % Wb == 0) done = (s + 1) / Wb;
+            } else if (s >= Wb - 1) {
+                done = (s - (Wb - 1)) / 2 + 1;
+                done = done < Hb ? done : Hb;
+            }
+            if (done > 0 && (!wave || !hk->will_done || hk->will_done(hk->ctx, done))) {
+                LBIC_TRY(flush(s + 1));
+                LBIC_TRY(hk->rows_done(hk->ctx, done, st));
+            }
+        }
+    }
+    return flush(s_last);
+}
 
 int ws_acquire(lbic_model *m, cudaStream_t st) {
     if (m->ws_used && st != m->ws_stream) LBIC_CUDA(cudaStreamWaitEvent(st, m->ws_event, 0));
@@ -901,9 +967,23 @@ int ensure_aux(lbic_model *m, int which, size_t bytes, float **out) {
     return 0;
 }
 
+// Reads and clears the error flag of the kernels enqueued since the last encode / decode started: a stream buffer that
+// was too small (LBIC_ERR_OVERFLOW) or a malformed lane container (LBIC_ERR_INVALID).  The caller has synchronised.
+int take_error_flag(lbic_model *m) {
+    int flag = 0;
+    LBIC_CUDA(cudaMemcpy(&flag, m->err_flag, sizeof(int), cudaMemcpyDeviceToHost));
+    if (flag) {
+        cudaMemset(m->err_flag, 0, sizeof(int));
+        return lbic_fail(flag == 1 ? LBIC_ERR_OVERFLOW : LBIC_ERR_INVALID,
+                         flag == 1 ? "bitstream buffer too small (stream_cap)" : "malformed lane container");
+    }
+    return 0;
+}
+
+// info_cl: if set, the (n, Hb, Wb, M) channel-last self-information of the latents (lbic_validate)
 int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out,
                 uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
-                cudaStream_t st, const RowHooks *hk);
+                cudaStream_t st, const RowHooks *hk, float *info_cl = nullptr);
 int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img, int Hb,
                 int Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st, const RowHooks *hk);
 
@@ -1161,26 +1241,9 @@ extern "C" int lbic_encode(lbic_model *m, const float *x, int n_img, int Hb, int
 }
 
 namespace {
-// One encode-side wavefront step: entropy net, encoder net + quantisation, decoder net for the R rows of `sd`
-// (NET:363-377 for every block of the diagonal at once).  The gather of the step's operands has been enqueued.
-int encode_step(lbic_model *m, const StepDesc &sd, int R, bool want_syms, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    if (flow_applies(m, R) && !m->recon_cl) {
-        // the whole step as one dataflow launch; if the launch itself is refused (no co-residency: a shared or
-        // partitioned GPU) the per-layer path below takes over for good
-        if (m->k1 == 3) LBIC_TRY(launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st));
-        const int rc = run_flow(m, m->k1 == 3 ? L_E1 : L_E0, L_COUNT, sd, R, st);
-        if (rc != LBIC_FLOW_REFUSED) return rc;
-        m->use_flow = 0;
-    }
-    LBIC_TRY(run_ent(m, sd, R, st));
-    LBIC_TRY(run_enc(m, sd, R, want_syms ? ws.sym : nullptr, want_syms ? ws.idx : nullptr, st));
-    return run_dec(m, sd, R, st);
-}
-
 int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out,
                 uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
-                cudaStream_t st, const RowHooks *hk) {
+                cudaStream_t st, const RowHooks *hk, float *info_cl) {
     LBIC_TRY(check_ready(m, stream_out != nullptr));
     if ((!x && !(hk && hk->need_rows)) || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
     if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
@@ -1194,62 +1257,16 @@ int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float 
     LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
     if (x) LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, n_img, m->Cin, HW, st));
     LBIC_CUDA(cudaMemsetAsync(ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));   // NET:336
-    const bool want_syms = sym_out || idx_out || stream_out || m->selfinfo_cl;
-    const int T_steps = Wb + 2 * (Hb - 1);
+    const bool want_syms = sym_out || idx_out || stream_out || info_cl;
     if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
-    // one step through the per-layer / dataflow launches
-    auto launch_step = [&](int t) -> int {
-        StepDesc sd, ext;
-        if (m->k1 == 3 && wave_step_ext(t, n_img, Hb, Wb, ext)) LBIC_TRY(run_g0(m, ext, n_img * ext.nv, st));
-        if (!wave_step(t, n_img, Hb, Wb, sd)) return 0;
-        const int R = n_img * sd.nv;
-        LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    auto step = [&](const StepDesc &sd, int R) -> int {
         LBIC_TRY(encode_step(m, sd, R, want_syms, st));
-        if (m->selfinfo_cl)
-            LBIC_TRY(launch_selfinfo_step(sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, m->selfinfo_cl, st));
-        return 0;
+        return info_cl ? launch_selfinfo_step(sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st) : 0;
     };
-    // Small steps (single images, small batches): consecutive steps are collected into ONE launch of the persistent
-    // wavefront kernel, cut only where a host hook has copies or conversions to put between two steps.
-    bool wave = wave_applies(m, n_img, Hb, Wb, false, false);
-    int pend = -1;                                   // steps [pend, t) wait to be launched
-    auto flush = [&](int t_end) -> int {
-        if (pend < 0) return 0;
-        const int b = pend;
-        pend = -1;
-        const int rc = run_wave(m, false, false, b, t_end, n_img, Hb, Wb, 0, nullptr, st);
-        if (rc != LBIC_FLOW_REFUSED) return rc;
-        m->use_wave = 0;                             // no co-residency on this device: per-layer launches from now on
-        wave = false;
-        for (int t = b; t < t_end; ++t) LBIC_TRY(launch_step(t));
-        return 0;
-    };
-    for (int t = (m->k1 == 3 ? -1 : 0); t < T_steps; ++t) {
-        StepDesc sd;
-        const bool has = wave_step(t, n_img, Hb, Wb, sd);
-        if (has && hk && hk->need_rows) {
-            const int v_hi = sd.vmin + sd.nv - 1;
-            if (!wave || !hk->will_need || hk->will_need(hk->ctx, v_hi)) {
-                LBIC_TRY(flush(t));
-                LBIC_TRY(hk->need_rows(hk->ctx, v_hi, st));
-            }
-        }
-        if (wave) {
-            if (!has) LBIC_TRY(launch_step(t));      // KS[1] = 3: step -1 has ring positions only (one small GEMM, per-layer path)
-            else if (pend < 0) pend = t;
-        } else {
-            LBIC_TRY(launch_step(t));
-        }
-        if (has && hk && hk->rows_done && t >= Wb - 1) {
-            int done = (t - (Wb - 1)) / 2 + 1;
-            done = done < Hb ? done : Hb;
-            if (!wave || !hk->will_done || hk->will_done(hk->ctx, done)) {
-                LBIC_TRY(flush(t + 1));
-                LBIC_TRY(hk->rows_done(hk->ctx, done, st));
-            }
-        }
-    }
-    LBIC_TRY(flush(T_steps));
+    auto wave_range = [&](int s0, int s1) { return run_wave(m, false, false, s0, s1, n_img, Hb, Wb, 0, nullptr, st); };
+    // (the wavefront kernel does not compute the self-information)
+    const bool wave = !info_cl && wave_applies(m, n_img, Hb, Wb, false, false);
+    LBIC_TRY(run_steps(m, n_img, Hb, Wb, false, wave, hk, step, wave_range, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
     if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
     if (idx_out) LBIC_CUDA(cudaMemcpyAsync(idx_out, ws.idx, nblk * m->M, cudaMemcpyDeviceToDevice, st));
@@ -1279,10 +1296,7 @@ extern "C" int lbic_validate(lbic_model *m, const float *x, int n_img, int Hb, i
     LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
     float *cl = nullptr;
     LBIC_TRY(ensure_aux(m, 0, sizeof(float) * (size_t)n_img * Hb * Wb * m->M, &cl));
-    m->selfinfo_cl = cl;
-    int rc = lbic_encode(m, x, n_img, Hb, Wb, zhat_out, nullptr, nullptr, nullptr, 0, nullptr, 1, stream);
-    m->selfinfo_cl = nullptr;
-    Active act2(m);
+    int rc = encode_impl(m, x, n_img, Hb, Wb, zhat_out, nullptr, nullptr, nullptr, 0, nullptr, 1, st, nullptr, cl);
     if (rc == 0) rc = launch_cl_to_nchw(cl, selfinfo_out, n_img, m->M, Hb * Wb, st);   // -> (n, M, Hb, Wb) as AGENT:509
     if (rc == 0) rc = ws_release(m, st);
     return rc;
@@ -1323,26 +1337,23 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
             for (long r0 = 0; r0 < nblk && rc == 0; r0 += chunk) {
                 const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
                 const StepDesc sd{n_img, 0, 0, (int)r0, Hb, Wb};
-                P(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
-                EpiParams e = epi_hilo(EPI_LRELU, sd, ws.G0);
-                e.out_pos = 1;
-                P(run_gemm(m, L_E0, R, &ws.vT, nullptr, e, st));
+                // (the taps go to Text, the operand of E0 in the layer table; it has at least R_cap rows)
+                P(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo,
+                                ws.Text.ld, st));
+                P(run_layers(m, L_E0, L_E1, sd, R, st));
             }
             if (rc) break;
         }
-        m->recon_cl = xhat_cl;
-        m->recon_no_clamp = clamp ? 0 : 1;
+        // one launch per layer: the decoder net writes the caller's reconstruction, which the dataflow launch cannot
         for (long r0 = 0; r0 < nblk && rc == 0; r0 += chunk) {
             const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
             const StepDesc sd{n_img, 0, 0, (int)r0, Hb, Wb};
+            int l0;
             P(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
-            P(run_ent(m, sd, R, st));
-            P(run_enc(m, sd, R, ws.sym, ws.idx, st));
-            P(run_dec(m, sd, R, st));
+            P(step_entry(m, sd, R, &l0, st));
+            P(run_layers(m, l0, L_COUNT, sd, R, st, true, xhat_cl, clamp ? 0 : 1));
             if (info_cl) P(launch_selfinfo_step(sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st));
         }
-        m->recon_cl = nullptr;
-        m->recon_no_clamp = 0;
         if (rc) break;
         P(launch_cl_to_nchw(xhat_cl, xhat_out, n_img, m->Cin, HW, st));
         if (info_cl) P(launch_cl_to_nchw(info_cl, selfinfo_out, n_img, m->M, HW, st));
@@ -1351,8 +1362,6 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
         if (rc == 0) rc = ws_release(m, st);
 #undef P
     } while (0);
-    m->recon_cl = nullptr;
-    m->recon_no_clamp = 0;
     return rc;
 }
 
@@ -1368,14 +1377,7 @@ extern "C" int lbic_check_errors(lbic_model *m, void *stream) {
     if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
     Active act(m);
     LBIC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-    int flag = 0;
-    LBIC_CUDA(cudaMemcpy(&flag, m->err_flag, sizeof(int), cudaMemcpyDeviceToHost));
-    if (flag) {
-        cudaMemset(m->err_flag, 0, sizeof(int));
-        return lbic_fail(flag == 1 ? LBIC_ERR_OVERFLOW : LBIC_ERR_INVALID,
-                         flag == 1 ? "bitstream buffer too small (stream_cap)" : "malformed lane container");
-    }
-    return 0;
+    return take_error_flag(m);
 }
 
 namespace {
@@ -1396,89 +1398,13 @@ int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_le
     LBIC_CUDA(cudaMemsetAsync(ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));   // NET:417
     LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, n_img, L, lanes != 1, ws.dec_states, ws.lane_ptr,
                                   m->err_flag, st));
-    auto one_step = [&](const StepDesc &sd, int R) -> int {
-        LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
-        bool flow = flow_applies(m, R) != 0;
-        bool ent_done = false;
-        if (flow) {
-            if (m->k1 == 3) LBIC_TRY(launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st));
-            const int rc = run_flow(m, m->k1 == 3 ? L_E1 : L_E0, L_F0, sd, R, st);
-            if (rc == LBIC_FLOW_REFUSED) { m->use_flow = 0; flow = false; }
-            else if (rc) return rc;
-            else ent_done = true;
-        }
-        if (!ent_done) LBIC_TRY(run_ent(m, sd, R, st));
-        LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, L, sd, R, m->M, ws.KSI, ws.ldKSI, ws.YQ.hi,
-                                      ws.YQ.lo, ws.YQ.ld, sym_out ? ws.sym : nullptr, st));
-        if (flow) {
-            const int rc = run_flow(m, L_D0, L_COUNT, sd, R, st);
-            if (rc != LBIC_FLOW_REFUSED) return rc;
-            m->use_flow = 0;
-        }
-        return run_dec(m, sd, R, st);
-    };
     if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
     const bool raster = (L == 1 && lanes == 1);      // reference container: the rANS state threads through the blocks in
                                                      // raster order (NET:420-450), one block of every image per step
-    // raster step s = v * Wb + h; wavefront step s = t
-    auto launch_step = [&](int s) -> int {
-        if (raster) {
-            const int v = s / Wb, h = s - v * Wb;
-            if (m->k1 == 3) {
-                // hidden-map positions that become computable now: the ring columns of the row start, then (v,h)
-                if (h == 0) {
-                    if (v >= 1) { StepDesc e{n_img, 1, v - 1, Wb + 2 * (v - 1), Hb, Wb}; LBIC_TRY(run_g0(m, e, n_img, st)); }
-                    StepDesc e{n_img, 1, v, -1 + 2 * v, Hb, Wb};
-                    LBIC_TRY(run_g0(m, e, n_img, st));
-                }
-                StepDesc e{n_img, 1, v, h + 2 * v, Hb, Wb};
-                LBIC_TRY(run_g0(m, e, n_img, st));
-            }
-            StepDesc sd{n_img, 1, v, h + 2 * v, Hb, Wb};
-            return one_step(sd, n_img);
-        }
-        StepDesc sd, ext;
-        if (m->k1 == 3 && wave_step_ext(s, n_img, Hb, Wb, ext)) LBIC_TRY(run_g0(m, ext, n_img * ext.nv, st));
-        if (!wave_step(s, n_img, Hb, Wb, sd)) return 0;
-        return one_step(sd, n_img * sd.nv);
-    };
-    bool wave = wave_applies(m, n_img, Hb, Wb, raster, true);
-    int pend = -1;
-    auto flush = [&](int s_end) -> int {
-        if (pend < 0) return 0;
-        const int b = pend;
-        pend = -1;
-        const int rc = run_wave(m, true, raster, b, s_end, n_img, Hb, Wb, L, sym_out ? ws.sym : nullptr, st);
-        if (rc != LBIC_FLOW_REFUSED) return rc;
-        m->use_wave = 0;
-        wave = false;
-        for (int s = b; s < s_end; ++s) LBIC_TRY(launch_step(s));
-        return 0;
-    };
-    const int s_first = raster ? 0 : (m->k1 == 3 ? -1 : 0);
-    const int s_last = raster ? Hb * Wb : Wb + 2 * (Hb - 1);
-    for (int s = s_first; s < s_last; ++s) {
-        if (wave) {
-            if (s < 0) LBIC_TRY(launch_step(s));     // KS[1] = 3: step -1 has ring positions only
-            else if (pend < 0) pend = s;
-        } else {
-            LBIC_TRY(launch_step(s));
-        }
-        if (hk && hk->rows_done) {
-            int done = -1;
-            if (raster) {
-                if ((s + 1) % Wb == 0) done = (s + 1) / Wb;
-            } else if (s >= Wb - 1) {
-                done = (s - (Wb - 1)) / 2 + 1;
-                done = done < Hb ? done : Hb;
-            }
-            if (done > 0 && (!wave || !hk->will_done || hk->will_done(hk->ctx, done))) {
-                LBIC_TRY(flush(s + 1));
-                LBIC_TRY(hk->rows_done(hk->ctx, done, st));
-            }
-        }
-    }
-    LBIC_TRY(flush(s_last));
+    int32_t *sym = sym_out ? ws.sym : nullptr;
+    auto step = [&](const StepDesc &sd, int R) { return decode_step(m, sd, R, L, sym, st); };
+    auto wave_range = [&](int s0, int s1) { return run_wave(m, true, raster, s0, s1, n_img, Hb, Wb, L, sym, st); };
+    LBIC_TRY(run_steps(m, n_img, Hb, Wb, raster, wave_applies(m, n_img, Hb, Wb, raster, true), hk, step, wave_range, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
     if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
     return ws_release(m, st);
@@ -1493,17 +1419,6 @@ int ensure_io(lbic_model *m, size_t bytes) {
     return 0;
 }
 size_t align256(size_t v) { return (v + 255) / 256 * 256; }
-
-int check_async(lbic_model *m) {
-    int flag = 0;
-    LBIC_CUDA(cudaMemcpy(&flag, m->err_flag, sizeof(int), cudaMemcpyDeviceToHost));
-    if (flag) {
-        cudaMemset(m->err_flag, 0, sizeof(int));
-        return lbic_fail(flag == 1 ? LBIC_ERR_OVERFLOW : LBIC_ERR_INVALID,
-                         flag == 1 ? "bitstream buffer too small (stream_cap)" : "malformed lane container");
-    }
-    return 0;
-}
 
 // ---- host-buffer calls -----------------------------------------------------------------------------------------
 // The wavefront reads block row v of the input for the first time at step 2v and writes block row v of the
@@ -1619,13 +1534,12 @@ int encode_host_impl(lbic_model *m, int fmt, const void *in, int n_img, int H, i
     hk.will_need = BandPipe::will_need; hk.will_done = BandPipe::will_done;
     int rc = encode_impl(m, nullptr, n_img, Hb, Wb, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr, stream_cap,
                          (uint32_t *)(io + o_len), lanes, s_cmp, &hk);
-    Active act2(m);
     if (rc == 0 && stream_out && cudaMemcpyAsync(stream_len, io + o_len, 4 * (size_t)n_img, cudaMemcpyDeviceToHost, s_cmp) != cudaSuccess)
         rc = lbic_fail(LBIC_ERR_CUDA, "copy failed");
     cudaError_t e0 = cudaStreamSynchronize(m->hs[0]), e1 = cudaStreamSynchronize(s_cmp);
     if (rc == 0 && (e0 != cudaSuccess || e1 != cudaSuccess))
         rc = lbic_fail(LBIC_ERR_CUDA, "encode failed: %s", cudaGetErrorString(e0 != cudaSuccess ? e0 : e1));
-    if (rc == 0 && stream_out) rc = check_async(m);
+    if (rc == 0 && stream_out) rc = take_error_flag(m);
     if (rc == 0 && stream_out) {
         // one strided copy for all bitstreams: every image's slot up to the longest stream of the batch
         size_t longest = 0;
@@ -1668,12 +1582,11 @@ int decode_host_impl(lbic_model *m, int fmt, const uint8_t *streams, const uint3
     hk.ctx = &bp; hk.rows_done = BandPipe::rows_done; hk.will_done = BandPipe::will_done;
     int rc = decode_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hb, Wb, nullptr, nullptr, lanes,
                          s_cmp, &hk);
-    Active act2(m);
     cudaError_t e1 = cudaStreamSynchronize(s_cmp), e2 = cudaStreamSynchronize(s_out);
     if (rc) return rc;
     if (e1 != cudaSuccess || e2 != cudaSuccess)
         return lbic_fail(LBIC_ERR_CUDA, "decode failed: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
-    return check_async(m);
+    return take_error_flag(m);
 }
 }  // namespace
 
@@ -1831,7 +1744,6 @@ extern "C" int lbic_band_step(lbic_model *m, int t, int v0, int v1, void *stream
     if (!m || !m->band_n) return lbic_fail(LBIC_ERR_STATE, "lbic_band_begin has not been called");
     Active act(m);
     cudaStream_t st = (cudaStream_t)stream;
-    Workspace &ws = m->ws;
     const int n_img = m->band_n, Hb = m->band_Hb, Wb = m->band_Wb;
     StepDesc sd;
     if (!wave_step(t, n_img, Hb, Wb, sd)) return 0;
@@ -1840,15 +1752,7 @@ extern "C" int lbic_band_step(lbic_model *m, int t, int v0, int v1, void *stream
     if (hi <= lo) return 0;
     sd.vmin = lo; sd.nv = hi - lo;
     const int R = n_img * sd.nv;
-    if (m->band_decode) {
-        LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
-        LBIC_TRY(run_ent(m, sd, R, st));
-        LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, Hb, sd, R, m->M, ws.KSI, ws.ldKSI, ws.YQ.hi,
-                                      ws.YQ.lo, ws.YQ.ld, nullptr, st));
-        return run_dec(m, sd, R, st);
-    }
-    LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
-    return encode_step(m, sd, R, true, st);
+    return m->band_decode ? decode_step(m, sd, R, Hb, nullptr, st) : encode_step(m, sd, R, true, st);
 }
 
 // Ends the call for block rows [v0, v1): the band's reconstruction (channel-last rows, (n_img, v1-v0, Wb, 3B^2)) and,

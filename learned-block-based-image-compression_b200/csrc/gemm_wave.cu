@@ -808,7 +808,7 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
     }
     int bn_max = 16;
     for (int i = 0; i < 18; ++i) {
-        const int bn = w.h_layers[w.ids[i]].bn_v[w.variant];
+        const int bn = w.h_layers[i].bn_v[w.variant];
         if (bn % 16 || bn < 16 || bn > LBIC_LAT_MAX_BN) return lbic_fail(LBIC_ERR_INVALID, "wave kernel: bad tile N %d", bn);
         bn_max = bn > bn_max ? bn : bn_max;
     }
@@ -826,7 +826,7 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
         if (cap < 0) { const char *e = getenv("LBIC_WAVE_STAGES"); cap = e ? atoi(e) : 0; }
         if (cap >= 2 && p.stages > cap) p.stages = cap;
     }
-    // the step's list.  ids[0..3] = entropy net, [4..10] = encoder net (F0 G0 F1 G1 F2 G2 F3), [11..17] = decoder net.
+    // the step's list.  h_layers by LayerId: E..E+3 = entropy net, F..F+6 = encoder net (F0 G0 F1 G1 F2 G2 F3), D..D+6 = decoder net.
     // The encoder net (the critical path of an encode step) comes first so that its tiles are never queued behind the
     // entropy net's in a CTA's own list; the entropy net only has to be done when F3 quantises.
     int n = 0;
@@ -840,15 +840,15 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
         const int bn = L.bn_v[w.variant];
         return add(WK_GEMM, id, (L.cout + bn - 1) / bn, bn, d0, d1);
     };
-    const int *E = w.ids, *F = w.ids + 4, *D = w.ids + 11;
+    const int E = 0, F = 4, D = 11;
     int n_sm = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
     // KS[1] = 3: CTAs the other groups need -- one per tile of the widest encoder / decoder-net layer, the rANS CTAs of a decode
     int main_need = WAVE_GATHER_PARTS * 5;
-    for (int i = 4; i < 18; ++i) {
-        if (w.decode && i < 11) continue;
-        const ChainLayer &L = w.h_layers[w.ids[i]];
+    for (int i = F; i < D + 7; ++i) {
+        if (w.decode && i < D) continue;
+        const ChainLayer &L = w.h_layers[i];
         const int bn = L.bn_v[w.variant], nt = (L.cout + bn - 1) / bn;
         main_need = nt > main_need ? nt : main_need;
     }
@@ -863,15 +863,15 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
         // by this step's E0
         const int g5a = add(WK_GATHER5, -1, 4 * WAVE_G5_PARTS, 0, -1, -1);
         const int gx = add(WK_GATHER_EXT, -1, 4 * WAVE_GATHER_PARTS, 0, -1, -1);
-        const int e0 = gemm(E[0], gx, -1);
+        const int e0 = gemm(E, gx, -1);
         p.ord[gx].ext = 1; p.ord[e0].ext = 1;
         const int g5b = add(WK_GATHER5, -1, 1 * WAVE_G5_PARTS, 0, e0, -1);
         p.ord[g5b].tap0 = 4;
-        const int e1 = gemm(E[1], g5a, -1);
+        const int e1 = gemm(E + 1, g5a, -1);
         p.ord[e1].dep_late = g5b;
         p.ord[e1].kb_late = (4 * w.E1) / BK;          // the k-block that holds the first column of tap 4
-        const int e2 = gemm(E[2], e1, -1);
-        const int e3 = gemm(E[3], e2, -1);
+        const int e2 = gemm(E + 2, e1, -1);
+        const int e3 = gemm(E + 3, e2, -1);
         // its own CTAs for this chain, each with at most one tile of every entry: E1 (and g5a, E2, E3) from the group's CTA 0,
         // the E0 sub-chain (gx, E0, g5b) behind E1's CTAs where the grid has room -- an E1 tile then starts as soon as the
         // first four taps are gathered instead of queueing behind an E0 tile of its CTA
@@ -896,14 +896,14 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
     };
     if (p.k3 && !w.decode) {
         // the entropy net is the longer chain here (E1 has K = 5 E1): its tiles first
-        const int f0 = gemm(F[0], g, -1);
+        const int f0 = gemm(F, g, -1);
         last_e = ent_k3();
-        const int g0 = gemm(F[1], f0, -1);
-        const int f1 = gemm(F[2], g0, -1);
-        const int g1 = gemm(F[3], f1, -1);
-        const int f2 = gemm(F[4], g1, -1);
-        const int g2 = gemm(F[5], f2, -1);
-        last = gemm(F[6], g2, last_e);
+        const int g0 = gemm(F + 1, f0, -1);
+        const int f1 = gemm(F + 2, g0, -1);
+        const int g1 = gemm(F + 3, f1, -1);
+        const int f2 = gemm(F + 4, g1, -1);
+        const int g2 = gemm(F + 5, f2, -1);
+        last = gemm(F + 6, g2, last_e);
     } else if (p.k3) {
         last_e = ent_k3();
         last = add(WK_RANS, -1, WAVE_RANS_PARTS, 0, last_e, -1);
@@ -915,22 +915,22 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
             return lbic_fail(LBIC_ERR_INVALID, "wave kernel: entropy tables do not fit shared memory");
     } else if (!w.decode) {
         // interleaved: F0 E0 G0 E1 F1 E2 G1 E3 F2 G2 F3 | D0 .. D3
-        const int f0 = gemm(F[0], g, -1);
-        const int e0 = gemm(E[0], g, -1);
-        const int g0 = gemm(F[1], f0, -1);
-        const int e1 = gemm(E[1], e0, -1);
-        const int f1 = gemm(F[2], g0, -1);
-        const int e2 = gemm(E[2], e1, -1);
-        const int g1 = gemm(F[3], f1, -1);
-        last_e = gemm(E[3], e2, -1);
-        const int f2 = gemm(F[4], g1, -1);
-        const int g2 = gemm(F[5], f2, -1);
-        last = gemm(F[6], g2, last_e);             // QUANT: operand from G2, entropy parameters from E3
+        const int f0 = gemm(F, g, -1);
+        const int e0 = gemm(E, g, -1);
+        const int g0 = gemm(F + 1, f0, -1);
+        const int e1 = gemm(E + 1, e0, -1);
+        const int f1 = gemm(F + 2, g0, -1);
+        const int e2 = gemm(E + 2, e1, -1);
+        const int g1 = gemm(F + 3, f1, -1);
+        last_e = gemm(E + 3, e2, -1);
+        const int f2 = gemm(F + 4, g1, -1);
+        const int g2 = gemm(F + 5, f2, -1);
+        last = gemm(F + 6, g2, last_e);            // QUANT: operand from G2, entropy parameters from E3
     } else {
-        const int e0 = gemm(E[0], g, -1);
-        const int e1 = gemm(E[1], e0, -1);
-        const int e2 = gemm(E[2], e1, -1);
-        last_e = gemm(E[3], e2, -1);
+        const int e0 = gemm(E, g, -1);
+        const int e1 = gemm(E + 1, e0, -1);
+        const int e2 = gemm(E + 2, e1, -1);
+        last_e = gemm(E + 3, e2, -1);
         last = add(WK_RANS, -1, WAVE_RANS_PARTS, 0, last_e, -1);
         p.rans_ord = last;
         p.n_ent = max_rows > 8 * WAVE_ENT_CTAS ? 2 * WAVE_ENT_CTAS : WAVE_ENT_CTAS;   // one warp per row: 64 or 128 rows per round
@@ -939,7 +939,7 @@ int gemm_wave_launch(const WaveLaunch &w, cudaStream_t st) {
             (size_t)w.cdf16_total * 2 + 16 + 3 * 64 * 4 + 8 * (size_t)RANS_ROW_SCRATCH(w.M) > (size_t)WAVE_RING)
             return lbic_fail(LBIC_ERR_INVALID, "wave kernel: entropy tables do not fit shared memory");
     }
-    for (int i = 0; i < 7; ++i) last = gemm(D[i], last, -1);   // D0 IG0 D1 IG1 D2 IG2 D3: each reads the one before
+    for (int i = 0; i < 7; ++i) last = gemm(D + i, last, -1);   // D0 IG0 D1 IG1 D2 IG2 D3: each reads the one before
     p.recon_ord = last;
     p.n_ord = n;
     int total = 0;

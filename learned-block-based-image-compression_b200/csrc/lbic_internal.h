@@ -153,7 +153,7 @@ struct RansStreamState;
 // The latency path (gemm_wave.cu): a range of wavefront steps (or raster blocks) of ONE encode / decode in a single
 // persistent cooperative launch; gather, GEMM layers and (decode) the rANS step are tiles of one in-kernel work list.
 struct WaveLaunch {
-    const ChainLayer *d_layers, *h_layers;
+    const ChainLayer *d_layers, *h_layers;   // by api.cu's LayerId: E0..E3 = 0..3, F0..F3 = 4..10 (7), D0..D3 = 11..17 (7)
     int decode;                 // 0: encode step = gather | entropy net | encoder net + quantisation | decoder net
                                 // 1: decode step = gather | entropy net | rANS | decoder net
     int raster;                 // 1: steps are single blocks in raster order (reference container decode)
@@ -161,7 +161,6 @@ struct WaveLaunch {
     int n_img, Hb, Wb;
     int variant;                // LBIC_LAT*_VARIANT: tile width
     const uint16_t *cdf16; const int32_t *cdf16_off; int cdf16_total;   // compact CDF rows (Tables), decode only
-    int ids[20];                // LayerId of E0..E3, F0..F3 (7), D0..D3 (7) in api.cu's LayerId order (18 entries)
     const float *x_cl, *zhat_cl;
     int Cin;
     h16 *X_hi, *X_lo; int ldX;

@@ -127,6 +127,22 @@ int lbic_encode(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float 
 int lbic_decode(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                 int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out, int lanes, void *stream);
 
+/* lbic_encode / lbic_decode for n_img images of DIFFERENT sizes in one call.  Hb, Wb: host arrays of n_img block-grid
+ * sizes.  Packed layout, with P_i = sum_{j<i} Hb_j * Wb_j the blocks before image i:
+ *   x, zhat_out        image i at float offset 3B^2 * P_i, (3B^2, Hb_i, Wb_i) within
+ *   sym_out, idx_out   image i at M * P_i, (Hb_i, Wb_i, M) within
+ *   streams            slot i at i * stream_cap, one stream_len per image, as lbic_encode / lbic_decode;
+ *                      stream_cap >= the largest lbic_stream_bound(Hb_i, Wb_i, lanes)
+ * Every image comes out exactly as lbic_encode / lbic_decode of that image alone (same bytes, lengths, zhat, symbols,
+ * indexes), so the streams are ordinary per-image streams.  Overflow and malformed containers are reported as by
+ * lbic_encode / lbic_decode (0xFFFFFFFF lengths, lbic_check_errors).  The persistent wavefront kernel is not used. */
+int lbic_encode_mixed(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
+                      int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap,
+                      uint32_t *stream_len, int lanes, void *stream);
+int lbic_decode_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
+                      int n_img, const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes,
+                      void *stream);
+
 /* Closed-loop reconstruction WITHOUT entropy coding plus the rate estimate -- the loop of validate_recu_reco_fast
  * (AGENT:491-549): zhat_out as lbic_encode; selfinfo_out device, (n_img, M, Hb, Wb) fp32 = -log2 of the
  * Gaussian-conditional likelihood of every quantised latent (ENT:615-647).  Block windows follow the codec path's

@@ -63,6 +63,8 @@ PROTOTYPES = {
     "lbic_get_tables": (_i, [_vp, ctypes.POINTER(_i), ctypes.POINTER(_i), _vp, _vp, _vp]),
     "lbic_encode": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp, _i, _vp]),
     "lbic_decode": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _i, _vp]),
+    "lbic_encode_mixed": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _i, _vp]),
+    "lbic_decode_mixed": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _vp, _vp, _vp, _i, _vp]),
     "lbic_validate": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "lbic_encode_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp, _i]),
     "lbic_decode_host": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _vp, _i]),

@@ -160,6 +160,33 @@ class ImageCodec:
             z = self.model.decompress_batch([payload], shape, lanes=0)
         return self._from_blocks(z, meta["H"], meta["W"])
 
+    def encode_many(self, images) -> list:
+        """A list of images of any sizes (as `encode` takes them) -> one container per image, in one mixed-size call.
+        Each container equals `encode` of that image alone."""
+        ts = [self._as_tensor(img) for img in images]
+        xs = [self._to_blocks(t) for t in ts]
+        payloads = self.model.compress_batch(xs, lanes=0 if self.lanes != 1 else 1)[0]
+        return [pack_container(p, H=int(t.shape[2]), W=int(t.shape[3]), B=self.B, KS=self.KS, N=self.N, M=self.M,
+                               lanes=self.lanes) for p, t in zip(payloads, ts)]
+
+    def decode_many(self, blobs) -> list:
+        """Containers (as `decode` takes them) -> list of (1, 3, H, W) images, in one mixed-size call.  All containers
+        must have been written with the same `lanes` and by this model's configuration."""
+        metas, payloads = [], []
+        for blob in blobs:
+            meta, payload = unpack_container(blob)
+            if (meta["B"], meta["KS"], meta["N"], meta["M"]) != (self.B, self.KS, self.N, self.M):
+                raise ValueError(f"container was written by a different model configuration: {meta}")
+            metas.append(meta)
+            payloads.append(payload)
+        if len({m["lanes"] for m in metas}) > 1:
+            raise ValueError("decode_many needs containers of one lanes setting")
+        if not metas:
+            return []
+        shapes = [((m["H"] + self.B - 1) // self.B, (m["W"] + self.B - 1) // self.B) for m in metas]
+        zs = self.model.decompress_batch(payloads, shapes, lanes=1 if metas[0]["lanes"] == 1 else 0)
+        return [self._from_blocks(z, m["H"], m["W"]) for z, m in zip(zs, metas)]
+
     def evaluate(self, img) -> dict:
         """One image through encode + decode with the figures eval_model logs (AGENT:609-619)."""
         t = self._as_tensor(img)

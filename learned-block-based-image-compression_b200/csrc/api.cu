@@ -83,7 +83,8 @@ struct LayerWiring {   // one layer of a step: its operand per K segment and its
 };
 
 struct Workspace {
-    int n_img = 0, Hb = 0, Wb = 0, R_cap = 0;
+    int n_img = 0, Hb = 0, Wb = 0, R_cap = 0;     // (n_img = 0: sized for a mixed-size call, see ensure_workspace_mixed)
+    size_t nblk_cap = 0, npos_cap = 0, lanes_cap = 0;   // blocks, g0 store rows (KS[1] = 3), decoder lanes
     float *x_cl = nullptr, *zhat_cl = nullptr;
     ActBuf X, T, YQ, H1, H2, H3, S, U;
     float *A32 = nullptr, *KSI = nullptr;
@@ -170,6 +171,12 @@ struct lbic_model {
     // host-call staging
     void *io_dev = nullptr;
     size_t io_bytes = 0;
+    // mixed-size calls: the step schedule (host staging, device copy) and the packed symbols / indexes
+    std::vector<char> mix_host;
+    void *mix_dev = nullptr;
+    size_t mix_dev_bytes = 0;
+    void *mix_sym = nullptr;
+    size_t mix_sym_bytes = 0;
     // profiling
     int profiling = 0;
     std::vector<ProfRec> prof;
@@ -496,16 +503,55 @@ int build_chain(lbic_model *m) {
     return 0;
 }
 
+// What a call needs of the workspace: rows of its largest step and of its largest ring-extended step (KS[1] = 3),
+// blocks, rows of the g0 store and decoder lanes.
+struct WsNeed {
+    size_t rows = 0, ext_rows = 0, nblk = 0, npos = 0, lanes = 0;
+};
+
+int alloc_workspace(lbic_model *m, const WsNeed &z, int n_img, int Hb, int Wb);
+
 int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     Workspace &ws = m->ws;
     if (ws.n_img >= n_img && ws.Hb == Hb && ws.Wb == Wb) return 0;
+    const int max_nv = Hb < (Wb + 1) / 2 ? Hb : (Wb + 1) / 2;
+    WsNeed z;
+    z.rows = (size_t)n_img * max_nv;
+    z.ext_rows = (size_t)n_img * (max_nv + 2);
+    z.nblk = (size_t)n_img * Hb * Wb;
+    z.npos = (size_t)n_img * (Hb + 1) * (Wb + 2);
+    z.lanes = (size_t)n_img * Hb;
+    return alloc_workspace(m, z, n_img, Hb, Wb);
+}
+
+// A mixed-size call keeps the workspace if it is large enough (whatever call sized it), else grows every part to at
+// least what it had, so that calls of changing mixes settle on one allocation.
+int ensure_workspace_mixed(lbic_model *m, const WsNeed &need) {
+    Workspace &ws = m->ws;
+    const bool k3 = m->k1 == 3;
+    if ((size_t)ws.R_cap >= need.rows && (!k3 || ((size_t)ws.R_ext_cap >= need.ext_rows && ws.npos_cap >= need.npos)) &&
+        ws.nblk_cap >= need.nblk && ws.lanes_cap >= need.lanes && ws.d_chain)
+        return 0;
+    WsNeed z = need;
+    if (ws.d_chain) {
+        z.rows = z.rows > (size_t)ws.R_cap ? z.rows : (size_t)ws.R_cap;
+        z.ext_rows = z.ext_rows > (size_t)ws.R_ext_cap ? z.ext_rows : (size_t)ws.R_ext_cap;
+        z.nblk = z.nblk > ws.nblk_cap ? z.nblk : ws.nblk_cap;
+        z.npos = z.npos > ws.npos_cap ? z.npos : ws.npos_cap;
+        z.lanes = z.lanes > ws.lanes_cap ? z.lanes : ws.lanes_cap;
+    }
+    return alloc_workspace(m, z, 0, 0, 0);
+}
+
+int alloc_workspace(lbic_model *m, const WsNeed &z, int n_img, int Hb, int Wb) {
+    Workspace &ws = m->ws;
     LBIC_CUDA(cudaDeviceSynchronize());
     free_all(ws.allocs);
     ws = Workspace();
     ws.n_img = n_img; ws.Hb = Hb; ws.Wb = Wb;
-    const int max_nv = Hb < (Wb + 1) / 2 ? Hb : (Wb + 1) / 2;
-    ws.R_cap = ((n_img * max_nv) + 127) / 128 * 128;
-    const size_t nblk = (size_t)n_img * Hb * Wb;
+    ws.R_cap = (int)((z.rows + 127) / 128 * 128);
+    const size_t nblk = z.nblk;
+    ws.nblk_cap = z.nblk; ws.npos_cap = z.npos; ws.lanes_cap = z.lanes;
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.x_cl, sizeof(float) * nblk * m->Cin));
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.zhat_cl, sizeof(float) * nblk * m->Cin));
     LBIC_TRY(alloc_act(ws, ws.X, m->Cin));
@@ -513,8 +559,8 @@ int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     LBIC_TRY(alloc_act(ws, ws.YQ, m->M));
     LBIC_TRY(alloc_act(ws, ws.H1, m->E1));
     if (m->k1 == 3) {
-        ws.R_ext_cap = ((n_img * (max_nv + 2)) + 127) / 128 * 128;
-        const size_t npos = (size_t)n_img * (Hb + 1) * (Wb + 2);
+        ws.R_ext_cap = (int)((z.ext_rows + 127) / 128 * 128);
+        const size_t npos = z.npos;
         ws.G0.ld = m->E1;
         LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.G0.hi, sizeof(h16) * npos * m->E1, true));
         LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.G0.lo, sizeof(h16) * npos * m->E1, true));
@@ -553,8 +599,8 @@ int ensure_workspace(lbic_model *m, int n_img, int Hb, int Wb) {
     }
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.sym, sizeof(int32_t) * nblk * m->M));
     LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.idx, nblk * m->M));
-    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.dec_states, sizeof(RansStreamState) * (size_t)n_img * Hb));
-    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.lane_ptr, sizeof(void *) * (size_t)n_img * Hb));
+    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.dec_states, sizeof(RansStreamState) * z.lanes));
+    LBIC_TRY(dev_alloc(ws.allocs, (void **)&ws.lane_ptr, sizeof(void *) * z.lanes));
     wire_layers(m);
     LBIC_TRY(build_chain(m));
     ws.flow_counters_cap = (size_t)L_COUNT * ((ws.R_cap + 127) / 128 + 1);
@@ -707,6 +753,150 @@ int run_range(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, bool sym
     return run_layers(m, l0, l1, sd, R, st, syms);
 }
 
+// The step schedule of a mixed-size call (lbic_encode_mixed / lbic_decode_mixed), built on the host once per call.
+// Step s (wavefront: h + 2v = s from s = 0, or -1 with KS[1] = 3; raster: block number s of every image that has it)
+// covers schedule rows [row0[k], row0[k+1]), k = s - s_first, in (img, v) order, and with KS[1] = 3 first the
+// ring-extended positions [ext0[k], ext0[k+1]) that become computable with it -- per image the positions the
+// equal-size loop of run_steps computes at that step.  The device copy (`geo` and the d_* pointers) is one upload.
+struct MixedPlan {
+    int n_img = 0, s_first = 0, s_last = 0;
+    int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0, n_lanes = 0, max_lanes = 0;
+    int64_t min_seg = 0;
+    std::vector<int> row0, ext0, lane0;
+    std::vector<int64_t> seg;           // encode: symbols of stream s = [seg[s], seg[s+1]) in packed order
+    std::vector<int4> img, rows, ext;
+    std::vector<int> sched, blk_img, g0row, stream;
+    MixedGeo geo;
+    const int4 *d_rows = nullptr, *d_ext = nullptr;
+    const int *d_stream = nullptr, *d_lane0 = nullptr;
+    const int64_t *d_seg = nullptr;
+};
+
+bool wave_step(int t, int n_img, int Hb, int Wb, StepDesc &sd);
+bool wave_step_ext(int t, int n_img, int Hb, int Wb, StepDesc &sd);
+
+// lanes: 1 = one stream per image (reference container; decode in raster order), 0 = one lane per block row
+void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p) {
+    const bool k3 = m->k1 == 3;
+    p = MixedPlan();
+    p.n_img = n;
+    p.lane0.assign(n + 1, 0);
+    int64_t npos = 0;
+    for (int i = 0; i < n; ++i) {
+        p.img.push_back(make_int4(Hb[i], Wb[i], p.nblk, (int)npos));
+        p.nblk += Hb[i] * Wb[i];
+        npos += (int64_t)(Hb[i] + 1) * (Wb[i] + 2);
+        const int L = lanes == 1 ? 1 : Hb[i];
+        p.lane0[i + 1] = p.lane0[i] + L;
+        p.max_lanes = L > p.max_lanes ? L : p.max_lanes;
+        const int last = raster ? Hb[i] * Wb[i] : Wb[i] + 2 * (Hb[i] - 1);
+        p.s_last = last > p.s_last ? last : p.s_last;
+    }
+    p.n_lanes = p.lane0[n];
+    p.s_first = raster ? 0 : (k3 ? -1 : 0);
+    p.sched.assign(p.nblk, 0);
+    p.blk_img.assign(p.nblk, 0);
+    if (k3) p.g0row.assign(npos, 0);   // row 0 of the g0 store: the top ring row, the same for every image
+    for (int i = 0; i < n; ++i)
+        for (int b = 0; b < Hb[i] * Wb[i]; ++b) p.blk_img[p.img[i].z + b] = i;
+    auto add_ext = [&](int i, int v, int h) {
+        p.g0row[p.img[i].w + (v + 1) * (Wb[i] + 2) + (h + 1)] = 1 + p.n_ext++;
+        p.ext.push_back(make_int4(i, v, h, -1));
+    };
+    auto add_row = [&](int i, int v, int h) {
+        const int b = p.img[i].z + v * Wb[i] + h;
+        p.sched[b] = (int)p.rows.size();
+        p.rows.push_back(make_int4(i, v, h, b));
+        p.stream.push_back(p.lane0[i] + (lanes == 1 ? 0 : v));
+    };
+    for (int s = p.s_first; s < p.s_last; ++s) {
+        p.ext0.push_back(p.n_ext);
+        p.row0.push_back((int)p.rows.size());
+        for (int i = 0; i < n; ++i) {
+            if (raster) {
+                if (s >= Hb[i] * Wb[i]) continue;
+                const int v = s / Wb[i], h = s - v * Wb[i];
+                if (k3) {   // as run_steps: at a row start the right ring column of the row above and the left one
+                    if (h == 0 && v >= 1) add_ext(i, v - 1, Wb[i]);
+                    if (h == 0) add_ext(i, v, -1);
+                    add_ext(i, v, h);
+                }
+                add_row(i, v, h);
+                continue;
+            }
+            if (s >= Wb[i] + 2 * (Hb[i] - 1)) continue;
+            StepDesc e;
+            if (k3 && wave_step_ext(s, 1, Hb[i], Wb[i], e))
+                for (int v = e.vmin; v < e.vmin + e.nv; ++v) add_ext(i, v, s - 2 * v);
+            if (wave_step(s, 1, Hb[i], Wb[i], e))
+                for (int v = e.vmin; v < e.vmin + e.nv; ++v) add_row(i, v, s - 2 * v);
+        }
+        const int k = (int)p.row0.size() - 1;
+        const int R = (int)p.rows.size() - p.row0[k], Re = p.n_ext - p.ext0[k];
+        p.max_rows = R > p.max_rows ? R : p.max_rows;
+        p.max_ext = Re > p.max_ext ? Re : p.max_ext;
+    }
+    p.ext0.push_back(p.n_ext);
+    p.row0.push_back((int)p.rows.size());
+    // streams of the encoder: whole images (lanes = 1) or block rows, in packed symbol order
+    const int M = m->M;
+    p.min_seg = INT64_MAX;
+    for (int i = 0; i < n; ++i) {
+        const int L = lanes == 1 ? 1 : Hb[i];
+        const int64_t len = (int64_t)Hb[i] * Wb[i] * M / L;
+        for (int l = 0; l < L; ++l) p.seg.push_back((int64_t)M * p.img[i].z + l * len);
+        p.min_seg = len < p.min_seg ? len : p.min_seg;
+    }
+    p.seg.push_back((int64_t)M * p.nblk);
+}
+
+// One host-to-device copy of the plan's tables into the model's grow-only schedule buffer (on `st`, after the previous
+// call's kernels that read it: the workspace is held).
+int upload_mixed(lbic_model *m, MixedPlan &p, cudaStream_t st) {
+    size_t off = 0;
+    std::vector<std::pair<const void *, size_t>> parts;
+    std::vector<size_t> at;
+    auto add = [&](const void *src, size_t bytes) {
+        at.push_back(off);
+        parts.push_back({src, bytes});
+        off += (bytes + 15) / 16 * 16;
+    };
+    add(p.img.data(), sizeof(int4) * p.img.size());
+    add(p.rows.data(), sizeof(int4) * p.rows.size());
+    add(p.ext.data(), sizeof(int4) * p.ext.size());
+    add(p.sched.data(), sizeof(int) * p.sched.size());
+    add(p.blk_img.data(), sizeof(int) * p.blk_img.size());
+    add(p.g0row.data(), sizeof(int) * p.g0row.size());
+    add(p.stream.data(), sizeof(int) * p.stream.size());
+    add(p.lane0.data(), sizeof(int) * p.lane0.size());
+    add(p.seg.data(), sizeof(int64_t) * p.seg.size());
+    if (m->mix_dev_bytes < off) {
+        if (m->mix_dev) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->mix_dev); m->mix_dev = nullptr; m->mix_dev_bytes = 0; }
+        cudaError_t e = cudaMalloc(&m->mix_dev, off);
+        if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", off, cudaGetErrorString(e));
+        m->mix_dev_bytes = off;
+    }
+    m->mix_host.resize(off);
+    for (size_t i = 0; i < parts.size(); ++i)
+        if (parts[i].second) memcpy(m->mix_host.data() + at[i], parts[i].first, parts[i].second);
+    LBIC_CUDA(cudaMemcpyAsync(m->mix_dev, m->mix_host.data(), off, cudaMemcpyHostToDevice, st));
+    char *d = (char *)m->mix_dev;
+    p.geo.img = (const int4 *)(d + at[0]);
+    p.geo.rows = p.d_rows = (const int4 *)(d + at[1]);
+    p.d_ext = (const int4 *)(d + at[2]);
+    p.geo.sched = (const int *)(d + at[3]);
+    p.geo.blk_img = (const int *)(d + at[4]);
+    p.geo.g0row = (const int *)(d + at[5]);
+    p.d_stream = (const int *)(d + at[6]);
+    p.d_lane0 = (const int *)(d + at[7]);
+    p.d_seg = (const int64_t *)(d + at[8]);
+    return 0;
+}
+
+// The GEMM layers see schedule rows [row0, row0 + R) as a raster chunk of one "image" of 1 x nblk blocks: the row
+// destinations of their epilogues (epi_row_dst) are then the schedule rows themselves.
+StepDesc mixed_step_desc(const MixedPlan &p, int k) { return StepDesc{1, 0, 0, p.row0[k], 1, p.nblk}; }
+
 // KS[1] == 3: hidden map g0 = lrelu(E0(zhat taps)) at the ring-extended positions `ext` (single-position or
 // diagonal steps with h in [-1, Wb]), scattered into the position-indexed store (SURVEY.md A.3 / A.6).
 int run_g0(lbic_model *m, const StepDesc &ext, int R_ext, cudaStream_t st) {
@@ -718,13 +908,33 @@ int run_g0(lbic_model *m, const StepDesc &ext, int R_ext, cudaStream_t st) {
     return run_layers(m, L_E0, L_E1, ext, R_ext, st);
 }
 
+// The same for step k of a mixed-size call: the store holds the ring-extended rows in schedule order after the top
+// row, so E0 writes its R_ext rows contiguously from row 1 + ext0[k].
+int run_g0_mixed(lbic_model *m, const MixedPlan &p, int k, cudaStream_t st) {
+    Workspace &ws = m->ws;
+    const int e0 = p.ext0[k], R_ext = p.ext0[k + 1] - e0;
+    if (R_ext <= 0) return 0;
+    if (R_ext > ws.R_ext_cap) return lbic_fail(LBIC_ERR_INVALID, "internal: extended step exceeds its workspace");
+    LBIC_TRY(launch_gather_mixed(nullptr, ws.zhat_cl, m->Cin, p.geo, p.d_ext + e0, R_ext, nullptr, nullptr, 0, ws.Text.hi,
+                                 ws.Text.lo, ws.Text.ld, st));
+    const LayerWiring &w = ws.net[L_E0];
+    EpiParams ep = w.ep;
+    ep.out_pos = 0;
+    ep.out_hi += (size_t)(1 + e0) * ep.ld_out;
+    ep.out_lo += (size_t)(1 + e0) * ep.ld_out;
+    return run_gemm_layer(m, m->L[L_E0], L_E0, R_ext, w.a[0], w.a[1], ep, st);
+}
+
 // The first layer of a step and its operand: E0 on the zhat taps, or (KS[1] == 3: E0 has run on the ring-extended rows,
 // run_g0) E1 on the five g0 taps around each block, gathered here.
-int step_entry(lbic_model *m, const StepDesc &sd, int R, int *first, cudaStream_t st) {
+int step_entry(lbic_model *m, const StepDesc &sd, int R, int *first, cudaStream_t st, const MixedPlan *mx = nullptr) {
     Workspace &ws = m->ws;
     *first = L_E0;
     if (m->k1 != 3) return 0;
     *first = L_E1;
+    if (mx)
+        return launch_gather5_mixed(ws.G0.hi, ws.G0.lo, m->E1, mx->geo, mx->d_rows + sd.t, R, ws.H1x5.hi, ws.H1x5.lo,
+                                    ws.H1x5.ld, st);
     return launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st);
 }
 
@@ -842,25 +1052,38 @@ int run_wave(lbic_model *m, bool decode, bool raster, int s_begin, int s_end, in
 }
 
 // One wavefront step of an encode: entropy net, encoder net + quantisation, decoder net for the R rows of `sd`
-// (NET:363-377 for every block of the diagonal at once).
-int encode_step(lbic_model *m, const StepDesc &sd, int R, bool syms, cudaStream_t st) {
+// (NET:363-377 for every block of the diagonal at once).  `mx`: a step of a mixed-size call (mixed_step_desc).
+int encode_step(lbic_model *m, const StepDesc &sd, int R, bool syms, cudaStream_t st, const MixedPlan *mx = nullptr) {
     Workspace &ws = m->ws;
     int l0;
-    LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
-    LBIC_TRY(step_entry(m, sd, R, &l0, st));
+    if (mx)
+        LBIC_TRY(launch_gather_mixed(ws.x_cl, ws.zhat_cl, m->Cin, mx->geo, mx->d_rows + sd.t, R, ws.X.hi, ws.X.lo, ws.X.ld,
+                                     ws.T.hi, ws.T.lo, ws.T.ld, st));
+    else
+        LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, sd, R, &l0, st, mx));
     return run_range(m, l0, L_COUNT, sd, R, syms, st);
 }
 
 // One step of a decode: entropy net, rANS decode of y_qnt (and of the symbols into `sym`, if set) from `lanes` streams
 // per image, decoder net (NET:420-450 for every block of the step at once).
-int decode_step(lbic_model *m, const StepDesc &sd, int R, int lanes, int32_t *sym, cudaStream_t st) {
+int decode_step(lbic_model *m, const StepDesc &sd, int R, int lanes, int32_t *sym, cudaStream_t st,
+                const MixedPlan *mx = nullptr) {
     Workspace &ws = m->ws;
     int l0;
-    LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
-    LBIC_TRY(step_entry(m, sd, R, &l0, st));
+    if (mx)
+        LBIC_TRY(launch_gather_mixed(nullptr, ws.zhat_cl, m->Cin, mx->geo, mx->d_rows + sd.t, R, nullptr, nullptr, 0,
+                                     ws.T.hi, ws.T.lo, ws.T.ld, st));
+    else
+        LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, sd, R, &l0, st, mx));
     LBIC_TRY(run_range(m, l0, L_F0, sd, R, true, st));
-    LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, lanes, sd, R, m->M, ws.KSI, ws.ldKSI, ws.YQ.hi,
-                                  ws.YQ.lo, ws.YQ.ld, sym, st));
+    if (mx)
+        LBIC_TRY(launch_rans_dec_step_mixed(m->tables, ws.dec_states, ws.lane_ptr, mx->d_stream + sd.t, sd.t, R, m->M,
+                                            ws.KSI, ws.ldKSI, ws.YQ.hi, ws.YQ.lo, ws.YQ.ld, sym, st));
+    else
+        LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, lanes, sd, R, m->M, ws.KSI, ws.ldKSI,
+                                      ws.YQ.hi, ws.YQ.lo, ws.YQ.ld, sym, st));
     return run_range(m, L_D0, L_COUNT, sd, R, true, st);
 }
 
@@ -876,11 +1099,25 @@ bool step_desc(int s, bool raster, int n_img, int Hb, int Wb, StepDesc &sd) {
 // The step loop of an encode or a decode.  Each step runs through `step(sd, R)` (per-layer or dataflow launches) after
 // the hidden-map ring positions (KS[1] == 3) that become computable with it, or, when `wave` (small steps: single images,
 // small batches), consecutive steps are collected into ONE launch of the persistent wavefront kernel, `wave_range(s0,
-// s1)`, cut only where a host hook has copies or conversions to put between two steps.
+// s1)`, cut only where a host hook has copies or conversions to put between two steps.  A mixed-size call (`mx`) takes
+// its steps from the schedule; it has no hooks and no wavefront kernel (wave = false).
 template <class Step, class WaveRange>
 int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, const RowHooks *hk, Step step,
-              WaveRange wave_range, cudaStream_t st) {
+              WaveRange wave_range, cudaStream_t st, const MixedPlan *mx = nullptr) {
+    auto desc = [&](int s, StepDesc &sd) -> bool {   // step s of the call; false if it has no block
+        if (!mx) return step_desc(s, raster, n_img, Hb, Wb, sd);
+        const int k = s - mx->s_first;
+        sd = mixed_step_desc(*mx, k);
+        return mx->row0[k + 1] > mx->row0[k];
+    };
     auto launch_step = [&](int s) -> int {
+        if (mx) {
+            const int k = s - mx->s_first;
+            if (m->k1 == 3) LBIC_TRY(run_g0_mixed(m, *mx, k, st));
+            StepDesc sd;
+            if (!desc(s, sd)) return 0;
+            return step(sd, mx->row0[k + 1] - mx->row0[k]);
+        }
         if (m->k1 == 3 && raster) {
             // hidden-map positions that become computable now: the ring columns of the row start, then (v,h)
             const int v = s / Wb, h = s - v * Wb;
@@ -911,11 +1148,11 @@ int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, 
         for (int s = b; s < s_end; ++s) LBIC_TRY(launch_step(s));
         return 0;
     };
-    const int s_first = raster ? 0 : (m->k1 == 3 ? -1 : 0);
-    const int s_last = raster ? Hb * Wb : Wb + 2 * (Hb - 1);
+    const int s_first = mx ? mx->s_first : raster ? 0 : (m->k1 == 3 ? -1 : 0);
+    const int s_last = mx ? mx->s_last : raster ? Hb * Wb : Wb + 2 * (Hb - 1);
     for (int s = s_first; s < s_last; ++s) {
         StepDesc sd;
-        const bool has = step_desc(s, raster, n_img, Hb, Wb, sd);
+        const bool has = desc(s, sd);
         if (has && hk && hk->need_rows) {
             const int v_hi = sd.vmin + sd.nv - 1;
             if (!wave || !hk->will_need || hk->will_need(hk->ctx, v_hi)) {
@@ -986,6 +1223,11 @@ int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float 
                 cudaStream_t st, const RowHooks *hk, float *info_cl = nullptr);
 int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img, int Hb,
                 int Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st, const RowHooks *hk);
+int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
+                      int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
+                      int lanes, cudaStream_t st);
+int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
+                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st);
 
 }  // namespace
 
@@ -1063,6 +1305,8 @@ extern "C" void lbic_destroy(lbic_model *m) {
     if (m->d_sat) cudaFree(m->d_sat);
     if (m->ws_event) cudaEventDestroy(m->ws_event);
     if (m->io_dev) cudaFree(m->io_dev);
+    if (m->mix_dev) cudaFree(m->mix_dev);
+    if (m->mix_sym) cudaFree(m->mix_sym);
     for (auto &a : m->aux) if (a) cudaFree(a);
     for (auto &h : m->hs) if (h) cudaStreamDestroy(h);
     for (auto &ev : m->hev) if (ev) cudaEventDestroy(ev);
@@ -1371,6 +1615,20 @@ extern "C" int lbic_decode(lbic_model *m, const uint8_t *streams, const uint32_t
                        nullptr);
 }
 
+extern "C" int lbic_encode_mixed(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
+                                 int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap,
+                                 uint32_t *stream_len, int lanes, void *stream) {
+    return encode_mixed_impl(m, x, n_img, Hb, Wb, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, lanes,
+                             (cudaStream_t)stream);
+}
+
+extern "C" int lbic_decode_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
+                                 int n_img, const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes,
+                                 void *stream) {
+    return decode_mixed_impl(m, streams, stream_len, stream_cap, n_img, Hb, Wb, zhat_out, sym_out, lanes,
+                             (cudaStream_t)stream);
+}
+
 // Synchronises `stream` and reports what the kernels enqueued on it flagged since the last encode / decode started:
 // a stream buffer that was too small (LBIC_ERR_OVERFLOW) or a malformed lane container (LBIC_ERR_INVALID).
 extern "C" int lbic_check_errors(lbic_model *m, void *stream) {
@@ -1407,6 +1665,111 @@ int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_le
     LBIC_TRY(run_steps(m, n_img, Hb, Wb, raster, wave_applies(m, n_img, Hb, Wb, raster, true), hk, step, wave_range, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
     if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
+    return ws_release(m, st);
+}
+
+// ---- mixed-size batches ------------------------------------------------------------------------------------------
+int check_mixed_args(int n_img, const int *Hb, const int *Wb, int lanes) {
+    if (n_img < 1 || !Hb || !Wb) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
+    int64_t nblk = 0;
+    for (int i = 0; i < n_img; ++i) {
+        if (Hb[i] < 1 || Wb[i] < 1) return lbic_fail(LBIC_ERR_INVALID, "image %d has a %d x %d block grid", i, Hb[i], Wb[i]);
+        nblk += (int64_t)Hb[i] * Wb[i];
+    }
+    if (nblk > INT32_MAX / 4) return lbic_fail(LBIC_ERR_INVALID, "batch of %lld blocks is too large", (long long)nblk);
+    return 0;
+}
+
+WsNeed mixed_need(const lbic_model *m, const MixedPlan &p) {
+    WsNeed z;
+    z.rows = p.max_rows; z.ext_rows = p.max_ext; z.nblk = p.nblk; z.lanes = p.n_lanes;
+    z.npos = m->k1 == 3 ? 1 + (size_t)p.n_ext : 0;
+    return z;
+}
+
+int mixed_begin(lbic_model *m, int n_img, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p,
+                cudaStream_t st) {
+    plan_mixed(m, n_img, Hb, Wb, raster, lanes, p);
+    LBIC_TRY(ensure_workspace_mixed(m, mixed_need(m, p)));
+    LBIC_TRY(ws_acquire(m, st));
+    LBIC_TRY(upload_mixed(m, p, st));
+    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
+    LBIC_CUDA(cudaMemsetAsync(m->ws.zhat_cl, 0, sizeof(float) * (size_t)p.nblk * m->Cin, st));   // NET:336, NET:417
+    if (m->k1 == 3)   // row 0 of the g0 store: the top ring row (fill_g0_top of a single position)
+        LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, 1, 0, -1, m->ws.G0.hi, m->ws.G0.lo, st));
+    return 0;
+}
+
+int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
+                      int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
+                      int lanes, cudaStream_t st) {
+    LBIC_TRY(check_ready(m, stream_out != nullptr));
+    if (!x) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
+    if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    MixedPlan p;
+    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, false, lanes, p, st));
+    Workspace &ws = m->ws;
+    const size_t nblk = p.nblk;
+    LBIC_TRY(launch_nchw_to_cl_mixed(x, ws.x_cl, m->Cin, p.geo, p.nblk, st));
+    const bool want_syms = sym_out || idx_out || stream_out;
+    auto step = [&](const StepDesc &sd, int R) { return encode_step(m, sd, R, want_syms, st, &p); };
+    auto no_wave = [&](int, int) { return 0; };
+    LBIC_TRY(run_steps(m, n_img, 0, 0, false, false, nullptr, step, no_wave, st, &p));
+    if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
+    if (!want_syms) return ws_release(m, st);
+    // symbols and indexes in packed order: into the caller's arrays, or (streams only) a model buffer
+    int32_t *sym_p = sym_out;
+    uint8_t *idx_p = idx_out;
+    if (!sym_p || !idx_p) {
+        const size_t need = nblk * m->M * (sizeof(int32_t) + 1);
+        if (m->mix_sym_bytes < need) {
+            if (m->mix_sym) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->mix_sym); m->mix_sym = nullptr; m->mix_sym_bytes = 0; }
+            cudaError_t e = cudaMalloc(&m->mix_sym, need);
+            if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", need, cudaGetErrorString(e));
+            m->mix_sym_bytes = need;
+        }
+        if (!sym_p) sym_p = (int32_t *)m->mix_sym;
+        if (!idx_p) idx_p = (uint8_t *)m->mix_sym + nblk * m->M * sizeof(int32_t);
+    }
+    LBIC_TRY(launch_unschedule_i32(ws.sym, sym_p, m->M, p.geo, p.nblk, st));
+    LBIC_TRY(launch_unschedule_u8(ws.idx, idx_p, m->M, p.geo, p.nblk, st));
+    if (stream_out) {
+        // scratch words per stream as in encode_impl: the caller's slot (reference container) or a lane's worst case
+        int64_t max_seg = 0;
+        for (size_t s = 0; s + 1 < p.seg.size(); ++s) max_seg = p.seg[s + 1] - p.seg[s] > max_seg ? p.seg[s + 1] - p.seg[s] : max_seg;
+        const size_t per = (lanes == 1 ? stream_cap : lane_bound((size_t)max_seg)) / 4;
+        LBIC_TRY(ensure_rans_scratch(m, (size_t)p.n_lanes * per + 2 * (size_t)p.n_lanes));
+        LBIC_TRY(launch_rans_encode_mixed(m->tables, sym_p, idx_p, p.n_lanes, p.d_seg, p.min_seg, ws.rans_scratch, per,
+                                          lanes == 1 ? stream_out : nullptr, stream_cap, stream_len, m->err_flag, st));
+        if (lanes != 1)
+            LBIC_TRY(launch_lane_pack_mixed(ws.rans_scratch, per, n_img, p.d_lane0, p.n_lanes, p.max_lanes, stream_out,
+                                            stream_cap, stream_len, m->err_flag, st));
+    }
+    return ws_release(m, st);
+}
+
+int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
+                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st) {
+    LBIC_TRY(check_ready(m, true));
+    if (!streams || !stream_len) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
+    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    MixedPlan p;
+    const bool raster = lanes == 1;   // reference container: raster order, one block of every image per step
+    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, raster, lanes, p, st));
+    Workspace &ws = m->ws;
+    LBIC_TRY(launch_rans_dec_init_mixed(streams, stream_len, stream_cap, n_img, p.d_lane0, p.n_lanes, lanes != 1,
+                                        ws.dec_states, ws.lane_ptr, m->err_flag, st));
+    int32_t *sym = sym_out ? ws.sym : nullptr;
+    auto step = [&](const StepDesc &sd, int R) { return decode_step(m, sd, R, 0, sym, st, &p); };
+    auto no_wave = [&](int, int) { return 0; };
+    LBIC_TRY(run_steps(m, n_img, 0, 0, raster, false, nullptr, step, no_wave, st, &p));
+    if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
+    if (sym_out) LBIC_TRY(launch_unschedule_i32(ws.sym, sym_out, m->M, p.geo, p.nblk, st));
     return ws_release(m, st);
 }
 

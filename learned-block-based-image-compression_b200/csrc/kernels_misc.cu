@@ -266,6 +266,110 @@ __global__ void fill_g0_top_kernel(const float *__restrict__ bias, int E1, int n
     }
 }
 
+// ---- mixed-size batches (MixedGeo): x_cl is in packed block order, zhat_cl in schedule order ------------------------
+// gather_kernel for the rows of a mixed step: the borders are those of the row's own image.  Ring-extended rows (h =
+// -1 or Wb, the operand of E0 when KS[1] == 3) come without X.
+__global__ void gather_mixed_kernel(const float *__restrict__ x_cl, const float *__restrict__ zhat_cl, int Cin,
+                                    MixedGeo g, const int4 *__restrict__ rows, int R, h16 *__restrict__ X_hi,
+                                    h16 *__restrict__ X_lo, int ldX, h16 *__restrict__ T_hi, h16 *__restrict__ T_lo,
+                                    int ldT) {
+    const int r = blockIdx.x;
+    if (r >= R) return;
+    const int4 rec = rows[r];
+    const int v = rec.y, h = rec.z;
+    const int4 gi = g.img[rec.x];   // Hb, Wb, P, G
+    const int c4n = Cin >> 2;
+    const int first = X_hi ? 0 : 1;
+    for (int e = threadIdx.x + first * c4n; e < 5 * c4n; e += blockDim.x) {
+        const int seg = e / c4n, c = (e - seg * c4n) << 2;
+        float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
+        h16 *ph, *pl;
+        if (seg == 0) {
+            val = *reinterpret_cast<const float4 *>(x_cl + (size_t)rec.w * Cin + c);
+            ph = X_hi + (size_t)r * ldX + c;
+            pl = X_lo + (size_t)r * ldX + c;
+        } else {
+            const int tap = seg - 1;
+            const int dv = (tap == 3) ? 0 : -1;
+            const int dh = (tap == 3) ? -1 : tap - 1;
+            const int vv = v + dv, hh = h + dh;
+            if (vv >= 0 && vv < gi.x && hh >= 0 && hh < gi.y)
+                val = *reinterpret_cast<const float4 *>(zhat_cl + (size_t)g.sched[gi.z + vv * gi.y + hh] * Cin + c);
+            ph = T_hi + (size_t)r * ldT + tap * Cin + c;
+            pl = T_lo + (size_t)r * ldT + tap * Cin + c;
+        }
+        const float f[4] = {val.x, val.y, val.z, val.w};
+        store_hilo<4>(ph, pl, f);
+    }
+}
+
+// gather5_kernel for the rows of a mixed step: the g0 store holds the ring-extended rows in the order E0 computed them
+// (row 0: the top ring row v = -1, shared by every image), g.g0row maps a ring position to its row.
+__global__ void gather5_mixed_kernel(const h16 *__restrict__ g_hi, const h16 *__restrict__ g_lo, int E1, MixedGeo g,
+                                     const int4 *__restrict__ rows, int R, h16 *__restrict__ o_hi,
+                                     h16 *__restrict__ o_lo, int ld) {
+    const int r = blockIdx.x;
+    if (r >= R) return;
+    const int4 rec = rows[r];
+    const int4 gi = g.img[rec.x];
+    const int c8n = E1 >> 3;
+    for (int e = threadIdx.x; e < 5 * c8n; e += blockDim.x) {
+        const int tap = e / c8n, c = (e - tap * c8n) << 3;
+        const int dv = (tap >= 3) ? 0 : -1;
+        const int dh = (tap >= 3) ? tap - 4 : tap - 1;
+        const int pos = gi.w + (rec.y + dv + 1) * (gi.y + 2) + (rec.z + dh + 1);
+        const size_t src = (size_t)g.g0row[pos] * E1 + c;
+        const size_t dst = (size_t)r * ld + (size_t)tap * E1 + c;
+        *reinterpret_cast<uint4 *>(o_hi + dst) = *reinterpret_cast<const uint4 *>(g_hi + src);
+        *reinterpret_cast<uint4 *>(o_lo + dst) = *reinterpret_cast<const uint4 *>(g_lo + src);
+    }
+}
+
+// Packed NCHW (image i at C * P_i, (C, Hb_i, Wb_i) within) <-> channel-last rows, 32 blocks x 32 channels per tile.
+// TO_CL: row = packed block; otherwise row = the block's schedule row.
+template <bool TO_CL>
+__global__ void nchw_cl_mixed_kernel(const float *__restrict__ src, float *__restrict__ dst, int C, MixedGeo g, int nblk) {
+    __shared__ float tile[32][33];
+    const int b0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
+    const int b = b0 + threadIdx.x;
+    size_t pl = 0, hw = 0;   // this thread's block: offset in its image's NCHW planes, plane size
+    size_t row = 0;
+    if (b < nblk) {
+        const int4 gi = g.img[g.blk_img[b]];
+        hw = (size_t)gi.x * gi.y;
+        pl = (size_t)C * gi.z + (size_t)(b - gi.z);
+        row = TO_CL ? (size_t)b : (size_t)g.sched[b];
+    }
+    if (TO_CL) {
+        for (int j = threadIdx.y; j < 32; j += 8)
+            if (b < nblk && c0 + j < C) tile[j][threadIdx.x] = src[pl + (size_t)(c0 + j) * hw];
+        __syncthreads();
+        const int c = c0 + threadIdx.x;
+        for (int j = threadIdx.y; j < 32; j += 8)
+            if (b0 + j < nblk && c < C) dst[(size_t)(b0 + j) * C + c] = tile[threadIdx.x][j];
+    } else {
+        __shared__ size_t srow[32];
+        if (threadIdx.y == 0) srow[threadIdx.x] = row;
+        __syncthreads();
+        const int c = c0 + threadIdx.x;
+        for (int j = threadIdx.y; j < 32; j += 8)
+            if (b0 + j < nblk && c < C) tile[j][threadIdx.x] = src[srow[j] * C + c];
+        __syncthreads();
+        for (int j = threadIdx.y; j < 32; j += 8)
+            if (b < nblk && c0 + j < C) dst[pl + (size_t)(c0 + j) * hw] = tile[threadIdx.x][j];
+    }
+}
+
+// dst[b * C + c] = src[sched[b] * C + c]: a schedule-ordered (block, C) array in packed block order
+template <class T>
+__global__ void unschedule_kernel(const T *__restrict__ src, T *__restrict__ dst, int C, MixedGeo g, int nblk) {
+    const size_t total = (size_t)nblk * C;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int b = (int)(i / C), c = (int)(i - (size_t)b * C);
+        dst[i] = src[(size_t)g.sched[b] * C + c];
+    }
+}
+
 // ---- weight packing -------------------------------------------------------------------------------
 struct TapList {
     int n;
@@ -448,6 +552,56 @@ int launch_restore_border(const float *z_cl, float *out_cl, int Cin, int n_img, 
 
 int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16 *g_hi, h16 *g_lo, cudaStream_t st) {
     fill_g0_top_kernel<<<n_img * (Wb + 2), 256, 0, st>>>(bias, E1, n_img, Hb, Wb, g_hi, g_lo);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_gather_mixed(const float *x_cl, const float *zhat_cl, int Cin, const MixedGeo &g, const int4 *rows, int R,
+                        h16 *X_hi, h16 *X_lo, int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st) {
+    if (R <= 0) return 0;
+    int threads = 5 * (Cin / 4);
+    threads = threads > 256 ? 256 : ((threads + 31) / 32) * 32;
+    gather_mixed_kernel<<<R, threads, 0, st>>>(x_cl, zhat_cl, Cin, g, rows, R, X_hi, X_lo, ldX, T_hi, T_lo, ldT);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_gather5_mixed(const h16 *g0_hi, const h16 *g0_lo, int E1, const MixedGeo &g, const int4 *rows, int R,
+                         h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st) {
+    if (R <= 0) return 0;
+    gather5_mixed_kernel<<<R, 256, 0, st>>>(g0_hi, g0_lo, E1, g, rows, R, out_hi, out_lo, ld);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_nchw_to_cl_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
+    dim3 grid((nblk + 31) / 32, (C + 31) / 32), block(32, 8);
+    nchw_cl_mixed_kernel<true><<<grid, block, 0, st>>>(src, dst, C, g, nblk);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_cl_to_nchw_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
+    dim3 grid((nblk + 31) / 32, (C + 31) / 32), block(32, 8);
+    nchw_cl_mixed_kernel<false><<<grid, block, 0, st>>>(src, dst, C, g, nblk);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_unschedule_i32(const int32_t *src, int32_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
+    unschedule_kernel<int32_t><<<grid_for((size_t)nblk * C, 256), 256, 0, st>>>(src, dst, C, g, nblk);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_unschedule_u8(const uint8_t *src, uint8_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
+    unschedule_kernel<uint8_t><<<grid_for((size_t)nblk * C, 256), 256, 0, st>>>(src, dst, C, g, nblk);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;

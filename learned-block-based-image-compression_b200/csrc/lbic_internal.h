@@ -64,6 +64,23 @@ __host__ __device__ inline void step_row_to_block(const StepDesc &s, int r, int 
 }
 
 // ------------------------------------------------------------------------------------------------
+// A batch of differently sized images (lbic_encode_mixed / lbic_decode_mixed).  The host lays every step's rows out
+// back to back in one schedule (api.cu: MixedPlan) and keeps the per-step working data in SCHEDULE order: schedule row
+// k holds the k-th block the call computes.  The GEMM layers then see each step as the raster chunk
+//   StepDesc{1, 0, 0, k0, 1, n_rows}      (row r -> block k0 + r, see step_row_to_block)
+// so their epilogues write the symbols, indexes and reconstruction of row r to schedule row k0 + r with the
+// equal-size kernels unchanged.  Only the kernels that look at an image's geometry (the gathers, the rANS decode step,
+// the stream and layout kernels) have mixed forms, which read these tables.
+// ------------------------------------------------------------------------------------------------
+struct MixedGeo {
+    const int4 *rows;      // schedule row -> {img, v, h, packed block}      (packed block = P_img + v * Wb_img + h)
+    const int4 *img;       // image -> {Hb, Wb, P (first packed block), G (first ring position)}
+    const int *sched;      // packed block -> schedule row
+    const int *blk_img;    // packed block -> image
+    const int *g0row;      // KS[1] = 3: ring position G_img + (v + 1) * (Wb + 2) + (h + 1) -> row of the g0 store
+};
+
+// ------------------------------------------------------------------------------------------------
 // Epilogue of a GEMM layer (fused into both GEMM cores).
 // ------------------------------------------------------------------------------------------------
 enum EpiMode {
@@ -227,6 +244,17 @@ int launch_restore_border(const float *z_cl, float *out_cl, int Cin, int n_img, 
 int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepDesc &s, int R, h16 *out_hi, h16 *out_lo,
                    int ld, cudaStream_t st);
 int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16 *g_hi, h16 *g_lo, cudaStream_t st);
+// mixed-size forms (MixedGeo): `rows` are the R row records of the step (main rows, or the ring-extended rows of E0)
+int launch_gather_mixed(const float *x_cl, const float *zhat_cl, int Cin, const MixedGeo &g, const int4 *rows, int R,
+                        h16 *X_hi, h16 *X_lo, int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st);
+int launch_gather5_mixed(const h16 *g0_hi, const h16 *g0_lo, int E1, const MixedGeo &g, const int4 *rows, int R,
+                         h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st);
+// packed NCHW images <-> packed channel-last blocks (to_cl) or schedule-ordered channel-last blocks (from_cl), and a
+// schedule-ordered (block, C) array -> packed order; one launch for the whole batch
+int launch_nchw_to_cl_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
+int launch_cl_to_nchw_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
+int launch_unschedule_i32(const int32_t *src, int32_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
+int launch_unschedule_u8(const uint8_t *src, uint8_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
 int launch_add_vec(const float *a, const float *b, float *out, int n, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------------
@@ -279,6 +307,21 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
                          int ld_yq, int32_t *sym_out, cudaStream_t st);
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,
                          cudaStream_t st);
+// Mixed-size forms.  Encode: stream s holds symbols [seg[s], seg[s+1]) (device array, min_sym = the shortest stream);
+// lane s of image i is stream lane0[i] + s (lane0: device, n_img + 1 entries, max_lanes = the most lanes of one image).
+int launch_rans_encode_mixed(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
+                             int64_t min_sym, uint32_t *scratch_words, size_t scratch_words_per_stream, uint8_t *out,
+                             size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st);
+int launch_lane_pack_mixed(const uint32_t *scratch, size_t scratch_words, int n_img, const int *lane0, int n_lanes,
+                           int max_lanes, uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag,
+                           cudaStream_t st);
+int launch_rans_dec_init_mixed(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
+                               const int *lane0, int n_lanes, int lanes_container, RansStreamState *states,
+                               const uint8_t **lane_ptr, int *err_flag, cudaStream_t st);
+// decode step of schedule rows [row0, row0 + R): row r reads stream `stream[r]` and writes its symbols to row row0 + r
+int launch_rans_dec_step_mixed(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr,
+                               const int *stream, int row0, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi,
+                               h16 *yq_lo, int ld_yq, int32_t *sym_out, cudaStream_t st);
 // CDF index of n scales by both routines of the decoders (bisection; hint with bisection fallback), for tests
 int launch_scale_index(const float *scales, int n, const float *tab, int32_t *idx_bisect, int32_t *idx_hinted, cudaStream_t st);
 int launch_rans_decode_full(const Tables &T, const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride,

@@ -16,6 +16,41 @@ namespace {
 
 constexpr uint32_t LANE_MAGIC = 0x4C4D424Cu;   // "LBML"
 
+// Where the encoder finds the symbols of stream s: equal streams of n_sym symbols every `stride` elements (one
+// geometry per call), or the segments [seg[s], seg[s+1]) of a mixed-size batch.
+struct EqualSegs {
+    long n_sym, stride;
+    __device__ __forceinline__ size_t start(int s) const { return (size_t)s * stride; }
+    __device__ __forceinline__ long count(int) const { return n_sym; }
+};
+struct MixedSegs {
+    const int64_t *seg;
+    __device__ __forceinline__ size_t start(int s) const { return (size_t)seg[s]; }
+    __device__ __forceinline__ long count(int s) const { return (long)(seg[s + 1] - seg[s]); }
+};
+// The lanes of image img: `lanes` per image, or lane0[img] .. lane0[img+1] - 1 (mixed-size batch).
+struct EqualLanes {
+    int lanes;
+    __device__ __forceinline__ size_t first(int img) const { return (size_t)img * lanes; }
+    __device__ __forceinline__ int count(int) const { return lanes; }
+    __device__ __forceinline__ int total(int n_img) const { return n_img * lanes; }
+    __device__ __forceinline__ void lane_of(int i, int n_img, int &img, int &l) const { img = i / lanes; l = i - img * lanes; }
+};
+struct MixedLanes {
+    const int *lane0;
+    __device__ __forceinline__ size_t first(int img) const { return (size_t)lane0[img]; }
+    __device__ __forceinline__ int count(int img) const { return lane0[img + 1] - lane0[img]; }
+    __device__ __forceinline__ int total(int n_img) const { return lane0[n_img]; }
+    __device__ __forceinline__ void lane_of(int i, int n_img, int &img, int &l) const {
+        int lo = 0, hi = n_img - 1;                 // last image whose first lane is <= i
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (lane0[mid] <= i) lo = mid; else hi = mid - 1;
+        }
+        img = lo; l = i - lane0[lo];
+    }
+};
+
 // ---------------------------------------------------------------------------------------------
 // encoder: one thread per stream walks its symbols backwards (flush() pops the pushed symbols in
 // reverse) and writes renormalisation words from the end of its scratch region towards the front.
@@ -60,9 +95,10 @@ __device__ __forceinline__ void enc_put_bits(EncCursor &c, uint32_t val) {
 //     x < 2^63, which covers x < x_max = range << 47);
 //   * then all lanes replay the 32 prepared symbols in order (records broadcast with shuffles, every lane holds the
 //     same state, lane 0 writes the renormalisation words), so no memory latency or division sits on the serial chain.
+template <class Segs>
 __global__ void rans_encode_kernel(const int32_t *__restrict__ cdf, int cdf_stride, const int32_t *__restrict__ cdf_len,
                                    const int32_t *__restrict__ offs, const int32_t *__restrict__ sym,
-                                   const uint8_t *__restrict__ idx, int n_streams, long n_sym, long stream_stride,
+                                   const uint8_t *__restrict__ idx, int n_streams, Segs seg,
                                    uint32_t *__restrict__ scratch, long scratch_words, uint32_t *__restrict__ start_word,
                                    uint32_t *__restrict__ n_words, int *__restrict__ err) {
     const int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -72,8 +108,9 @@ __global__ void rans_encode_kernel(const int32_t *__restrict__ cdf, int cdf_stri
     c.base = scratch + (size_t)s * scratch_words;
     c.pos = scratch_words;
     c.overflow = false;
-    const int32_t *ps = sym + (size_t)s * stream_stride;
-    const uint8_t *pi = idx + (size_t)s * stream_stride;
+    const int32_t *ps = sym + seg.start(s);
+    const uint8_t *pi = idx + seg.start(s);
+    const long n_sym = seg.count(s);
     for (long top = n_sym; top > 0; top -= 32) {
         // lane j prepares symbol top-1-j (the coder walks the symbols backwards)
         const long k = top - 1 - lane;
@@ -311,11 +348,11 @@ __device__ __forceinline__ void enc_symbol_thread(EncCursor &c, int symbol, int 
     enc_put(c, start, range);
 }
 
+template <class Segs>
 __global__ void __launch_bounds__(ENC_T_THREADS)
 rans_encode_thread_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__restrict__ off16, int total,
                           const int32_t *__restrict__ cdf_len, const int32_t *__restrict__ offs,
-                          const int32_t *__restrict__ sym, const uint8_t *__restrict__ idx, int n_streams, long n_sym,
-                          long stream_stride, uint32_t *__restrict__ scratch, long scratch_words,
+                          const int32_t *__restrict__ sym, const uint8_t *__restrict__ idx, int n_streams, Segs seg, uint32_t *__restrict__ scratch, long scratch_words,
                           uint32_t *__restrict__ start_word, uint32_t *__restrict__ n_words, int *__restrict__ err) {
     extern __shared__ uint4 enc_smem[];
     const int nvec = (total + 7) >> 3;
@@ -336,10 +373,10 @@ rans_encode_thread_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__r
     c.base = scratch + (size_t)s * scratch_words;
     c.pos = scratch_words;
     c.overflow = false;
-    const int32_t *ps = sym + (size_t)s * stream_stride;
-    const uint8_t *pi = idx + (size_t)s * stream_stride;
-    // the coder walks the symbols backwards, four at a time (n_sym and stream_stride are multiples of 4)
-    for (long k = n_sym - 4; k >= 0; k -= 4) {
+    const int32_t *ps = sym + seg.start(s);
+    const uint8_t *pi = idx + seg.start(s);
+    // the coder walks the symbols backwards, four at a time (stream lengths and starts are multiples of 4)
+    for (long k = seg.count(s) - 4; k >= 0; k -= 4) {
         const int4 v = *reinterpret_cast<const int4 *>(ps + k);
         const uchar4 ci = *reinterpret_cast<const uchar4 *>(pi + k);
         enc_symbol_thread(c, v.w, ci.w, s_cdf, s_off, s_len, s_offs);
@@ -379,19 +416,21 @@ __global__ void rans_compact_kernel(const uint32_t *__restrict__ scratch, long s
 }
 
 // lane container assembly: one CTA per image
+template <class Lanes>
 __global__ void lane_pack_kernel(const uint32_t *__restrict__ scratch, long scratch_words,
                                  const uint32_t *__restrict__ start_word, const uint32_t *__restrict__ n_words,
-                                 int lanes, uint8_t *__restrict__ out, size_t out_stride, uint32_t *__restrict__ out_len,
+                                 Lanes lm, uint8_t *__restrict__ out, size_t out_stride, uint32_t *__restrict__ out_len,
                                  int *__restrict__ err) {
     extern __shared__ uint32_t lane_off[];   // lanes + 1 word offsets
     const int img = blockIdx.x;
+    const int lanes = lm.count(img);
     __shared__ int bad;
     if (threadIdx.x == 0) {
         bad = 0;
         uint32_t run = 2 + (uint32_t)lanes;
         for (int l = 0; l < lanes; ++l) {
             lane_off[l] = run;
-            const uint32_t nw = n_words[(size_t)img * lanes + l];
+            const uint32_t nw = n_words[lm.first(img) + l];
             if (nw == 0xFFFFFFFFu) bad = 1; else run += nw;
         }
         lane_off[lanes] = run;
@@ -404,9 +443,9 @@ __global__ void lane_pack_kernel(const uint32_t *__restrict__ scratch, long scra
     }
     uint32_t *dst = reinterpret_cast<uint32_t *>(out + (size_t)img * out_stride);
     if (threadIdx.x == 0) { dst[0] = LANE_MAGIC; dst[1] = (uint32_t)lanes; out_len[img] = lane_off[lanes] * 4; }
-    for (int l = threadIdx.x; l < lanes; l += blockDim.x) dst[2 + l] = n_words[(size_t)img * lanes + l] * 4;
+    for (int l = threadIdx.x; l < lanes; l += blockDim.x) dst[2 + l] = n_words[lm.first(img) + l] * 4;
     for (int l = 0; l < lanes; ++l) {
-        const size_t s = (size_t)img * lanes + l;
+        const size_t s = lm.first(img) + l;
         const uint32_t *src = scratch + s * scratch_words + start_word[s];
         const uint32_t nw = n_words[s];
         for (uint32_t i = threadIdx.x; i < nw; i += blockDim.x) dst[lane_off[l] + i] = src[i];
@@ -414,13 +453,16 @@ __global__ void lane_pack_kernel(const uint32_t *__restrict__ scratch, long scra
 }
 
 // Parses the per-image container(s) and initialises one decoder state per lane.
+template <class Lanes>
 __global__ void rans_dec_init_kernel(const uint8_t *__restrict__ streams, const uint32_t *__restrict__ stream_len,
-                                     size_t stream_stride, int n_img, int lanes, int lanes_container,
+                                     size_t stream_stride, int n_img, Lanes lm, int lanes_container,
                                      RansStreamState *__restrict__ states, const uint8_t **__restrict__ lane_ptr,
                                      int *__restrict__ err) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_img * lanes) return;
-    const int img = i / lanes, l = i - img * lanes;
+    if (i >= lm.total(n_img)) return;
+    int img, l;
+    lm.lane_of(i, n_img, img, l);
+    const int lanes = lm.count(img);
     const uint8_t *base = streams + (size_t)img * stream_stride;
     const uint32_t total = stream_len[img];
     const uint8_t *p = base;
@@ -464,19 +506,41 @@ __global__ void rans_dec_init_kernel(const uint8_t *__restrict__ streams, const 
     lane_ptr[i] = p;
 }
 
+// The rows of a decode step: a StepDesc (one geometry; row r -> block (img, v, h), stream img * lanes + v with lanes,
+// img without), or the schedule rows [row0, row0 + R) of a mixed-size batch with a stream per row.  row_at() resolves
+// the row's stream, row_out() where its M symbols go in the (block, M) symbol array.
+struct MixedDecRows {
+    const int *stream;
+    int row0;
+};
+struct DecRow {
+    int img, v, h;
+};
+__device__ __forceinline__ int row_at(const StepDesc &sd, int lanes, int r, DecRow &q) {
+    step_row_to_block(sd, r, q.img, q.v, q.h);
+    return lanes > 1 ? q.img * lanes + q.v : q.img;
+}
+__device__ __forceinline__ size_t row_out(const StepDesc &sd, int, const DecRow &q, int M) {
+    return (((size_t)q.img * sd.Hb + q.v) * sd.Wb + q.h) * M;
+}
+__device__ __forceinline__ int row_at(const MixedDecRows &mr, int, int r, DecRow &) { return mr.stream[r]; }
+__device__ __forceinline__ size_t row_out(const MixedDecRows &mr, int r, const DecRow &, int M) {
+    return (size_t)(mr.row0 + r) * M;
+}
+
 // One warp per row of the step: build_indexes from the predicted scales, decode M symbols from the row's
 // lane, dequantise (sym + mean, ENT:159-168) and emit the decoder-net input as h16 hi/lo planes.
+template <class Rows>
 __global__ void rans_dec_step_kernel(const int32_t *__restrict__ cdf, int cdf_stride,
                                      const int32_t *__restrict__ cdf_len, const int32_t *__restrict__ offs,
                                      const float *__restrict__ scale_tab, RansStreamState *__restrict__ states,
-                                     const uint8_t *const *__restrict__ lane_ptr, int lanes, StepDesc sd, int R, int M,
+                                     const uint8_t *const *__restrict__ lane_ptr, int lanes, Rows sd, int R, int M,
                                      const float *__restrict__ ksi, int ld_ksi, h16 *__restrict__ yq_hi,
                                      h16 *__restrict__ yq_lo, int ld_yq, int32_t *__restrict__ sym_out) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= R) return;
-    int img, v, h;
-    step_row_to_block(sd, warp, img, v, h);
-    const int sidx = lanes > 1 ? img * lanes + v : img;
+    DecRow q;
+    const int sidx = row_at(sd, lanes, warp, q);
     DecCursor d;
     {
         const RansStreamState st = states[sidx];
@@ -502,7 +566,7 @@ __global__ void rans_dec_step_kernel(const int32_t *__restrict__ cdf, int cdf_st
         st.x = d.x; st.pos = d.pos; st.nwords = d.nwords;
         states[sidx] = st;
     }
-    const size_t o = (((size_t)img * sd.Hb + v) * sd.Wb + h) * M;
+    const size_t o = row_out(sd, warp, q, M);
     for (int j = 0; j < per; ++j) {
         const int c = j * 32 + lane;
         if (c < M) {
@@ -523,11 +587,12 @@ __global__ void rans_dec_step_kernel(const int32_t *__restrict__ cdf, int cdf_st
 // rans_dec_step_kernel, whose every symbol waits for two dependent L2 round trips (row lookups) and ~150 instructions.
 constexpr int DEC_S_WARPS = 8;
 
+template <class Rows>
 __global__ void __launch_bounds__(DEC_S_WARPS * 32)
 rans_dec_step_smem_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__restrict__ off16, int total,
                           const int32_t *__restrict__ cdf_len, const int32_t *__restrict__ offs,
                           const float *__restrict__ scale_tab, RansStreamState *__restrict__ states,
-                          const uint8_t *const *__restrict__ lane_ptr, int lanes, StepDesc sd, int R, int M,
+                          const uint8_t *const *__restrict__ lane_ptr, int lanes, Rows sd, int R, int M,
                           const float *__restrict__ ksi, int ld_ksi, h16 *__restrict__ yq_hi, h16 *__restrict__ yq_lo,
                           int ld_yq, int32_t *__restrict__ sym_out) {
     extern __shared__ uint4 dsm[];
@@ -548,9 +613,8 @@ rans_dec_step_smem_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__r
     const uint32_t s_cdf = (uint32_t)__cvta_generic_to_shared(dsm);
     const uint32_t s_met = s_cdf + 16u * (uint32_t)nvec;
     const uint32_t scr = s_met + 1024u + (uint32_t)warp * RANS_ROW_SCRATCH(M);
-    int img, v, h;
-    step_row_to_block(sd, r, img, v, h);
-    const int sidx = lanes > 1 ? img * lanes + v : img;
+    DecRow q;
+    const int sidx = row_at(sd, lanes, r, q);
     DecCursorW d;
     {
         const RansStreamState st = states[sidx];
@@ -565,7 +629,7 @@ rans_dec_step_smem_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__r
         st.x = d.x; st.pos = d.pos; st.nwords = d.nwords;
         states[sidx] = st;
     }
-    const size_t o = (((size_t)img * sd.Hb + v) * sd.Wb + h) * M;
+    const size_t o = row_out(sd, r, q, M);
     for (int c = lane; c < M; c += 32) {
         const int sym = lds_s32(scr + 8u * M + 4u * c);
         h16 hi, lo;
@@ -639,25 +703,26 @@ __device__ __forceinline__ int dec_symbol_thread(DecCursorT &d, const uint16_t *
     return value + off;
 }
 
+template <class Rows>
 __global__ void __launch_bounds__(DEC_T_THREADS)
 rans_dec_step_thread_kernel(const uint16_t *__restrict__ cdf16, const int32_t *__restrict__ off16, int total,
                             const int32_t *__restrict__ cdf_len, const int32_t *__restrict__ offs,
                             const float *__restrict__ scale_tab, RansStreamState *__restrict__ states,
-                            const uint8_t *const *__restrict__ lane_ptr, int lanes, StepDesc sd, int R, int M,
+                            const uint8_t *const *__restrict__ lane_ptr, int lanes, Rows sd, int R, int M,
                             const float *__restrict__ ksi, int ld_ksi, h16 *__restrict__ yq_hi,
                             h16 *__restrict__ yq_lo, int ld_yq, int32_t *__restrict__ sym_out) {
     extern __shared__ uint4 dec_smem[];
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = r < R;
     // this thread's stream state and first operands are requested before the table copy so their latency overlaps it
-    int img = 0, v = 0, h = 0, sidx = 0;
+    DecRow q = {0, 0, 0};
+    int sidx = 0;
     DecCursorT d;
     d.x = 0; d.words = nullptr; d.pos = 0; d.nwords = 0; d.w_next = 0;
     const float *krow = ksi;
     float4 sc = make_float4(0.f, 0.f, 0.f, 0.f), mu = sc;
     if (active) {
-        step_row_to_block(sd, r, img, v, h);
-        sidx = lanes > 1 ? img * lanes + v : img;
+        sidx = row_at(sd, lanes, r, q);
         const RansStreamState st = states[sidx];
         d.x = st.x; d.pos = st.pos; d.nwords = st.nwords;
         d.words = reinterpret_cast<const uint32_t *>(lane_ptr[sidx]);
@@ -681,7 +746,7 @@ rans_dec_step_thread_kernel(const uint16_t *__restrict__ cdf16, const int32_t *_
     if (!active) return;
     const uint16_t *s_cdf = reinterpret_cast<const uint16_t *>(dec_smem);
     const uint16_t *s_lut = s_cdf + total;
-    const size_t o = (((size_t)img * sd.Hb + v) * sd.Wb + h) * M;
+    const size_t o = row_out(sd, r, q, M);
     const ScaleHint hint = scale_hint(s_tab);
     for (int c0 = 0; c0 < M; c0 += 4) {
         const float scs[4] = {sc.x, sc.y, sc.z, sc.w};
@@ -763,34 +828,37 @@ static int g_enc_thread_min_streams = 4096;
 static int g_enc_block_max_streams = 592;     // up to 4 CTAs per SM: one CTA per stream; more (and short) streams: one warp each
 
 // scratch layout: [n_streams * scratch_words] words, then start_word[n_streams], n_words[n_streams]
-int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, int64_t n_sym,
-                       int64_t stream_stride, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
-                       uint32_t *out_len, int *err_flag, cudaStream_t st) {
+// (`aligned`: every stream starts and ends on a multiple of 4 symbols and the arrays are 16 / 4-byte aligned;
+// `min_sym`: the shortest stream)
+// (`block_form`: streams of block_n_sym symbols back to back may take the CTA-per-stream form)
+template <class Segs>
+int rans_encode_any(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, Segs seg, bool aligned,
+                    int64_t min_sym, bool block_form, long block_n_sym, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
+                    uint32_t *out_len, int *err_flag, cudaStream_t st) {
     if (!T.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");
     uint32_t *start_word = scratch + (size_t)n_streams * scratch_words;
     uint32_t *n_words = start_word + n_streams;
     // many streams: one thread per stream with the tables in shared memory; few (single images): one warp per stream
-    const bool thread_form = T.cdf16_total > 0 && n_streams >= g_enc_thread_min_streams && n_sym % 4 == 0 &&
-                             stream_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(sym) & 15) == 0 &&
-                             (reinterpret_cast<uintptr_t>(idx) & 3) == 0;
+    const bool thread_form = T.cdf16_total > 0 && n_streams >= g_enc_thread_min_streams && aligned &&
+                             (reinterpret_cast<uintptr_t>(sym) & 15) == 0 && (reinterpret_cast<uintptr_t>(idx) & 3) == 0;
     if (thread_form) {
         const size_t smem = 16 * (((size_t)T.cdf16_total + 7) / 8) + 3 * 64 * 4;
         static unsigned long long attr_mask = 0;
         if (lbic_first_use_on_device(attr_mask))
-            LBIC_CUDA(cudaFuncSetAttribute(rans_encode_thread_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        rans_encode_thread_kernel<<<(n_streams + ENC_T_THREADS - 1) / ENC_T_THREADS, ENC_T_THREADS, smem, st>>>(
-            T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, sym, idx, n_streams, (long)n_sym,
-            (long)stream_stride, scratch, (long)scratch_words, start_word, n_words, err_flag);
-    } else if (n_streams <= g_enc_block_max_streams && n_sym >= 256) {
+            LBIC_CUDA(cudaFuncSetAttribute(rans_encode_thread_kernel<Segs>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        rans_encode_thread_kernel<Segs><<<(n_streams + ENC_T_THREADS - 1) / ENC_T_THREADS, ENC_T_THREADS, smem, st>>>(
+            T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, sym, idx, n_streams, seg, scratch,
+            (long)scratch_words, start_word, n_words, err_flag);
+    } else if (block_form && n_streams <= g_enc_block_max_streams && min_sym >= 256) {
         // few long streams (single images, the reference container): one CTA per stream, serial chain on one thread
         rans_encode_block_kernel<<<n_streams, ENC_B_THREADS, 0, st>>>(
-            T.cdf, T.stride, T.cdf_length, T.offset, sym, idx, n_streams, (long)n_sym, (long)stream_stride, scratch,
+            T.cdf, T.stride, T.cdf_length, T.offset, sym, idx, n_streams, block_n_sym, block_n_sym, scratch,
             (long)scratch_words, start_word, n_words, err_flag);
     } else {
         const int warps_per_block = 4;
-        rans_encode_kernel<<<(n_streams + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(
-            T.cdf, T.stride, T.cdf_length, T.offset, sym, idx, n_streams, (long)n_sym, (long)stream_stride, scratch,
-            (long)scratch_words, start_word, n_words, err_flag);
+        rans_encode_kernel<Segs><<<(n_streams + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(
+            T.cdf, T.stride, T.cdf_length, T.offset, sym, idx, n_streams, seg, scratch, (long)scratch_words, start_word,
+            n_words, err_flag);
     }
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
@@ -803,13 +871,41 @@ int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, 
     return 0;
 }
 
+int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, int64_t n_sym,
+                       int64_t stream_stride, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
+                       uint32_t *out_len, int *err_flag, cudaStream_t st) {
+    return rans_encode_any(T, sym, idx, n_streams, EqualSegs{(long)n_sym, (long)stream_stride},
+                           n_sym % 4 == 0 && stream_stride % 4 == 0, n_sym, n_sym == stream_stride, (long)n_sym, scratch, scratch_words, out, out_stride,
+                           out_len, err_flag, st);
+}
+
+int launch_rans_encode_mixed(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
+                             int64_t min_sym, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
+                             uint32_t *out_len, int *err_flag, cudaStream_t st) {
+    // (every stream is a whole number of blocks of M symbols, M a multiple of 16; the streams differ in length, so
+    // the CTA-per-stream form, which is for few long streams of one size, is not used)
+    return rans_encode_any(T, sym, idx, n_streams, MixedSegs{seg}, true, min_sym, false, 0L, scratch, scratch_words, out,
+                           out_stride, out_len, err_flag, st);
+}
+
 int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, int n_img, int lanes, uint8_t *out,
                      size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st) {
     const uint32_t *start_word = scratch + (size_t)n_img * lanes * scratch_words;
     const uint32_t *n_words = start_word + (size_t)n_img * lanes;
-    lane_pack_kernel<<<n_img, 256, sizeof(uint32_t) * (lanes + 1), st>>>(scratch, (long)scratch_words, start_word,
-                                                                        n_words, lanes, out, out_stride, out_len,
-                                                                        err_flag);
+    lane_pack_kernel<EqualLanes><<<n_img, 256, sizeof(uint32_t) * (lanes + 1), st>>>(
+        scratch, (long)scratch_words, start_word, n_words, EqualLanes{lanes}, out, out_stride, out_len, err_flag);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_lane_pack_mixed(const uint32_t *scratch, size_t scratch_words, int n_img, const int *lane0, int n_lanes,
+                           int max_lanes, uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag,
+                           cudaStream_t st) {
+    const uint32_t *start_word = scratch + (size_t)n_lanes * scratch_words;
+    const uint32_t *n_words = start_word + (size_t)n_lanes;
+    lane_pack_kernel<MixedLanes><<<n_img, 256, sizeof(uint32_t) * (max_lanes + 1), st>>>(
+        scratch, (long)scratch_words, start_word, n_words, MixedLanes{lane0}, out, out_stride, out_len, err_flag);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
@@ -819,8 +915,20 @@ int launch_rans_dec_init(const uint8_t *streams, const uint32_t *stream_len, siz
                          int lanes_container, RansStreamState *states, const uint8_t **lane_ptr, int *err_flag,
                          cudaStream_t st) {
     const int n = n_img * lanes;
-    rans_dec_init_kernel<<<(n + 127) / 128, 128, 0, st>>>(streams, stream_len, stream_stride, n_img, lanes,
-                                                          lanes_container, states, lane_ptr, err_flag);
+    rans_dec_init_kernel<EqualLanes><<<(n + 127) / 128, 128, 0, st>>>(streams, stream_len, stream_stride, n_img,
+                                                                      EqualLanes{lanes}, lanes_container, states,
+                                                                      lane_ptr, err_flag);
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_rans_dec_init_mixed(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
+                               const int *lane0, int n_lanes, int lanes_container, RansStreamState *states,
+                               const uint8_t **lane_ptr, int *err_flag, cudaStream_t st) {
+    rans_dec_init_kernel<MixedLanes><<<(n_lanes + 127) / 128, 128, 0, st>>>(streams, stream_len, stream_stride, n_img,
+                                                                            MixedLanes{lane0}, lanes_container, states,
+                                                                            lane_ptr, err_flag);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
@@ -833,9 +941,10 @@ void rans_set_dec_thread_min_rows(int rows) { g_dec_thread_min_rows = rows < 1 ?
 void rans_set_enc_thread_min_streams(int n) { g_enc_thread_min_streams = n < 1 ? 1 : n; }
 void rans_set_enc_block_max_streams(int n) { g_enc_block_max_streams = n < 0 ? 0 : n; }
 
-int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
-                         const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo,
-                         int ld_yq, int32_t *sym_out, cudaStream_t st) {
+template <class Rows>
+int rans_dec_step_any(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes, const Rows &s,
+                      int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq, int32_t *sym_out,
+                      cudaStream_t st) {
     if (R <= 0) return 0;
     if (M > 256) return lbic_fail(LBIC_ERR_INVALID, "M > 256 unsupported by the decode step");
     // many streams: one thread per stream with the tables in shared memory; few (single images): one warp per stream
@@ -843,8 +952,8 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
         const size_t smem = 16 * (((size_t)T.cdf16_total + 64 * 257 + 7) / 8) + 4 * 64 * 4;
         static unsigned long long attr_mask = 0;
         if (lbic_first_use_on_device(attr_mask))
-            LBIC_CUDA(cudaFuncSetAttribute(rans_dec_step_thread_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        rans_dec_step_thread_kernel<<<(R + DEC_T_THREADS - 1) / DEC_T_THREADS, DEC_T_THREADS, smem, st>>>(
+            LBIC_CUDA(cudaFuncSetAttribute(rans_dec_step_thread_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        rans_dec_step_thread_kernel<Rows><<<(R + DEC_T_THREADS - 1) / DEC_T_THREADS, DEC_T_THREADS, smem, st>>>(
             T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, T.d_scale_table, states, lane_ptr, lanes, s, R, M,
             ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out);
         count_launch(1);
@@ -856,9 +965,9 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
         const size_t smem = 16 * (((size_t)T.cdf16_total + 7) / 8) + 1024 + (size_t)DEC_S_WARPS * RANS_ROW_SCRATCH(M);
         static unsigned long long attr_mask2 = 0;
         if (lbic_first_use_on_device(attr_mask2))
-            LBIC_CUDA(cudaFuncSetAttribute(rans_dec_step_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            LBIC_CUDA(cudaFuncSetAttribute(rans_dec_step_smem_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         if (smem <= 200 * 1024) {
-            rans_dec_step_smem_kernel<<<(R + DEC_S_WARPS - 1) / DEC_S_WARPS, DEC_S_WARPS * 32, smem, st>>>(
+            rans_dec_step_smem_kernel<Rows><<<(R + DEC_S_WARPS - 1) / DEC_S_WARPS, DEC_S_WARPS * 32, smem, st>>>(
                 T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, T.d_scale_table, states, lane_ptr, lanes, s, R, M,
                 ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out);
             count_launch(1);
@@ -867,12 +976,25 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
         }
     }
     const int warps_per_block = 4;
-    rans_dec_step_kernel<<<(R + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(
+    rans_dec_step_kernel<Rows><<<(R + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(
         T.cdf, T.stride, T.cdf_length, T.offset, T.d_scale_table, states, lane_ptr, lanes, s, R, M, ksi, ld_ksi, yq_hi, yq_lo,
         ld_yq, sym_out);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
+}
+
+int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
+                         const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo,
+                         int ld_yq, int32_t *sym_out, cudaStream_t st) {
+    return rans_dec_step_any(T, states, lane_ptr, lanes, s, R, M, ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
+}
+
+int launch_rans_dec_step_mixed(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr,
+                               const int *stream, int row0, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi,
+                               h16 *yq_lo, int ld_yq, int32_t *sym_out, cudaStream_t st) {
+    return rans_dec_step_any(T, states, lane_ptr, 0, MixedDecRows{stream, row0}, R, M, ksi, ld_ksi, yq_hi, yq_lo,
+                             ld_yq, sym_out, st);
 }
 
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,

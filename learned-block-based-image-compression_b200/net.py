@@ -273,6 +273,69 @@ class BlockBasedImgCompLossyNetv9:
                 o.lens.data_ptr() if o.lens is not None else None, lanes, self._stream()))
         return o
 
+    def encode_device_mixed(self, xs, lanes: int = 1, want_symbols: bool = False, stream_cap: int | None = None):
+        """One encode of differently sized images (lbic_encode_mixed); each image comes out exactly as encode_device of
+        it alone.  xs: list of (1, 3B^2, Hb_i, Wb_i) or (3B^2, Hb_i, Wb_i) fp32 CUDA tensors on one device.  Returns a
+        namespace: zhat / sym / idx (lists of per-image views of the packed outputs), streams (n, cap) uint8, lens (n,)
+        int32, shapes [(Hb_i, Wb_i)]; no host synchronisation."""
+        h = self._need()
+        xs = [x[0] if x.dim() == 4 and x.shape[0] == 1 else x for x in xs]
+        if not xs or any(not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 3 and x.shape[0] == self.Cin) for x in xs):
+            raise ValueError(f"xs must be a non-empty list of CUDA fp32 tensors of shape (1, {self.Cin}, Hb, Wb)")
+        dev = xs[0].device
+        shapes = [(int(x.shape[1]), int(x.shape[2])) for x in xs]
+        n, counts = len(xs), [hb * wb for hb, wb in shapes]
+        x = torch.cat([t.reshape(-1) for t in xs]).to(dev)
+        o = SimpleNamespace(shapes=shapes)
+        zhat = torch.empty_like(x)
+        total = sum(counts)
+        sym = torch.empty(total * self.M, dtype=torch.int32, device=dev) if want_symbols else None
+        idx = torch.empty(total * self.M, dtype=torch.uint8, device=dev) if want_symbols else None
+        cap = stream_cap or max(self.stream_bound(hb, wb, lanes) for hb, wb in shapes)
+        cap = (cap + 3) // 4 * 4
+        o.streams = torch.empty(n, cap, dtype=torch.uint8, device=dev)
+        o.lens = torch.zeros(n, dtype=torch.int32, device=dev)
+        Hb = (ctypes.c_int * n)(*[s[0] for s in shapes])
+        Wb = (ctypes.c_int * n)(*[s[1] for s in shapes])
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().lbic_encode_mixed(
+                h, x.data_ptr(), n, Hb, Wb, zhat.data_ptr(), sym.data_ptr() if sym is not None else None,
+                idx.data_ptr() if idx is not None else None, o.streams.data_ptr(), cap, o.lens.data_ptr(), lanes,
+                self._stream()))
+        o.zhat = self._split(zhat, shapes, lambda hb, wb: (1, self.Cin, hb, wb), self.Cin)
+        o.sym = self._split(sym, shapes, lambda hb, wb: (1, hb, wb, self.M), self.M) if sym is not None else None
+        o.idx = self._split(idx, shapes, lambda hb, wb: (1, hb, wb, self.M), self.M) if idx is not None else None
+        return o
+
+    @staticmethod
+    def _split(flat, shapes, shape_of, per_block):
+        out, at = [], 0
+        for hb, wb in shapes:
+            k = hb * wb * per_block
+            out.append(flat[at: at + k].view(*shape_of(hb, wb)))
+            at += k
+        return out
+
+    def decode_device_mixed(self, streams, lens, shapes, lanes: int = 1, want_symbols: bool = False):
+        """streams (n, cap) uint8 CUDA, lens (n,) int32 CUDA, shapes [(Hb_i, Wb_i)] -> list of zhat (1, 3B^2, Hb_i, Wb_i)
+        [, list of sym (1, Hb_i, Wb_i, M)] (lbic_decode_mixed).  Asynchronous like decode_device."""
+        h = self._need()
+        dev = streams.device
+        shapes = [(int(a), int(b)) for a, b in shapes]
+        n, total = len(shapes), sum(a * b for a, b in shapes)
+        zhat = torch.empty(total * self.Cin, dtype=torch.float32, device=dev)
+        sym = torch.empty(total * self.M, dtype=torch.int32, device=dev) if want_symbols else None
+        Hb = (ctypes.c_int * n)(*[s[0] for s in shapes])
+        Wb = (ctypes.c_int * n)(*[s[1] for s in shapes])
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().lbic_decode_mixed(h, streams.data_ptr(), lens.data_ptr(), streams.shape[1], n, Hb, Wb,
+                                                    zhat.data_ptr(), sym.data_ptr() if sym is not None else None, lanes,
+                                                    self._stream()))
+        z = self._split(zhat, shapes, lambda hb, wb: (1, self.Cin, hb, wb), self.Cin)
+        if want_symbols:
+            return z, self._split(sym, shapes, lambda hb, wb: (1, hb, wb, self.M), self.M)
+        return z
+
     def validate_recu_reco(self, x):
         """Closed loop without entropy coding + rate estimate (validate_recu_reco_fast, AGENT:491-549).
         x: (n, 3B^2, Hb, Wb) CUDA fp32 -> (zhat, self_infos (n, M, Hb, Wb)); rate as the reference's loss computes it
@@ -337,17 +400,35 @@ class BlockBasedImgCompLossyNetv9:
         return [host[i, : lens[i]].tobytes() for i in range(len(lens))]
 
     def compress_batch(self, x, lanes: int = 1, return_symbols: bool = False):
-        """-> (list[bytes], zhat) or (list[bytes], zhat, sym, idx)."""
-        o = self.encode_device(x, lanes=lanes, want_symbols=return_symbols)
+        """-> (list[bytes], zhat) or (list[bytes], zhat, sym, idx).  x: a (n, 3B^2, Hb, Wb) tensor, or a list of
+        differently sized (1, 3B^2, Hb_i, Wb_i) tensors (one mixed-size call; zhat / sym / idx are then lists)."""
+        if isinstance(x, (list, tuple)):
+            o = self.encode_device_mixed(list(x), lanes=lanes, want_symbols=return_symbols)
+        else:
+            o = self.encode_device(x, lanes=lanes, want_symbols=return_symbols)
         strings = self._gather_streams(o)
         return (strings, o.zhat, o.sym, o.idx) if return_symbols else (strings, o.zhat)
 
     def decompress_batch(self, strings, xshape, lanes: int = 1, device=None):
+        """xshape: (n, 3B^2, Hb, Wb) for n images of one size, or a list of per-image shapes ((1, 3B^2, Hb_i, Wb_i) or
+        (Hb_i, Wb_i)) for one mixed-size call, which returns a list of zhat tensors."""
+        self._need()
+        dev = torch.device(device) if device is not None else self._device
+        if isinstance(xshape, (list, tuple)) and len(xshape) > 0 and isinstance(xshape[0], (list, tuple, torch.Size)):
+            shapes = [tuple(int(v) for v in s)[-2:] for s in xshape]
+            if len(strings) != len(shapes) or any(len(s) == 4 and int(s[1]) != self.Cin for s in xshape):
+                raise ValueError("strings / xshape mismatch")
+            cap = (max(len(s) for s in strings) + 3) // 4 * 4
+            host = np.zeros((len(strings), cap), dtype=np.uint8)
+            for i, s in enumerate(strings):
+                host[i, : len(s)] = np.frombuffer(s, dtype=np.uint8)
+            lens = torch.tensor([len(s) for s in strings], dtype=torch.int32, device=dev)
+            zs = self.decode_device_mixed(torch.from_numpy(host).to(dev), lens, shapes, lanes=lanes)
+            self.check_errors()
+            return zs
         n, ch, Hb, Wb = [int(v) for v in xshape]
         if len(strings) != n or ch != self.Cin:
             raise ValueError("strings / xshape mismatch")
-        self._need()
-        dev = torch.device(device) if device is not None else self._device
         cap = (max(len(s) for s in strings) + 3) // 4 * 4
         host = np.zeros((n, cap), dtype=np.uint8)
         for i, s in enumerate(strings):

@@ -710,17 +710,17 @@ int run_gemm_layer(lbic_model *m, const PackedLayer &L, int id, int R, const Act
     return rc;
 }
 
-// Layers [l0, l1) of the layer table for the R rows of step `sd`, one launch each.  F3 writes symbols and indexes only
+// Layers [l0, l1) of the layer table for the rows of a step, one launch each.  F3 writes symbols and indexes only
 // when `syms`; `recon` (if set) takes D3's reconstruction in place of the zhat feedback buffer, clamped unless `no_clamp`.
-int run_layers(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStream_t st, bool syms = true,
+int run_layers(lbic_model *m, int l0, int l1, const StepRows &rows, cudaStream_t st, bool syms = true,
                float *recon = nullptr, int no_clamp = 0) {
     for (int id = l0; id < l1; ++id) {
         const LayerWiring &w = m->ws.net[id];
         EpiParams ep = w.ep;
-        ep.step = sd;
+        ep.step = rows.sd;
         if (id == L_F3 && !syms) { ep.sym = nullptr; ep.idx = nullptr; }
         if (id == L_D3 && recon) { ep.zhat = recon; ep.no_clamp = no_clamp; }
-        LBIC_TRY(run_gemm_layer(m, m->L[id], id, R, w.a[0], w.a[1], ep, st));
+        LBIC_TRY(run_gemm_layer(m, m->L[id], id, rows.R, w.a[0], w.a[1], ep, st));
     }
     return 0;
 }
@@ -728,7 +728,8 @@ int run_layers(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, cudaStr
 // Layers [l0, l1) of a step: one dataflow launch where it applies (it always writes F3's symbols and indexes), else one
 // launch per layer.  If the dataflow launch itself is refused (no co-residency: a shared or partitioned GPU), the
 // per-layer path takes over for good.
-int run_range(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, bool syms, cudaStream_t st) {
+int run_range(lbic_model *m, int l0, int l1, const StepRows &rows, bool syms, cudaStream_t st) {
+    const int R = rows.R;
     if (const int form = flow_applies(m, R)) {
         Workspace &ws = m->ws;
         ProfRec rec;
@@ -741,7 +742,7 @@ int run_range(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, bool sym
             rec.layer = -1;
             cudaEventRecord(rec.a, st);
         }
-        const int rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, ws.dep, R, sd, ws.flow_counters,
+        const int rc = gemm_flow_launch(ws.d_chain, ws.h_chain.data(), l0, l1, ws.dep, R, rows.sd, ws.flow_counters,
                                         ws.flow_counters_cap, st, form == 1 ? 1 : 0);
         if (m->profiling) {
             cudaEventRecord(rec.b, st);
@@ -750,16 +751,18 @@ int run_range(lbic_model *m, int l0, int l1, const StepDesc &sd, int R, bool sym
         if (rc != LBIC_FLOW_REFUSED) return rc;
         m->use_flow = 0;
     }
-    return run_layers(m, l0, l1, sd, R, st, syms);
+    return run_layers(m, l0, l1, rows, st, syms);
 }
 
 // The step schedule of a mixed-size call (lbic_encode_mixed / lbic_decode_mixed), built on the host once per call.
 // Step s (wavefront: h + 2v = s from s = 0, or -1 with KS[1] = 3; raster: block number s of every image that has it)
 // covers schedule rows [row0[k], row0[k+1]), k = s - s_first, in (img, v) order, and with KS[1] = 3 first the
 // ring-extended positions [ext0[k], ext0[k+1]) that become computable with it -- per image the positions the
-// equal-size loop of run_steps computes at that step.  The device copy (`geo` and the d_* pointers) is one upload.
+// equal-size loop of run_steps computes at that step (ring_steps).  The device copy (`geo`, d_ext, d_lane0, d_seg) is
+// one upload.
 struct MixedPlan {
     int n_img = 0, s_first = 0, s_last = 0;
+    bool raster = false;
     int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0, n_lanes = 0, max_lanes = 0;
     int64_t min_seg = 0;
     std::vector<int> row0, ext0, lane0;
@@ -767,19 +770,20 @@ struct MixedPlan {
     std::vector<int4> img, rows, ext;
     std::vector<int> sched, blk_img, g0row, stream;
     MixedGeo geo;
-    const int4 *d_rows = nullptr, *d_ext = nullptr;
-    const int *d_stream = nullptr, *d_lane0 = nullptr;
+    const int4 *d_ext = nullptr;
+    const int *d_lane0 = nullptr;
     const int64_t *d_seg = nullptr;
 };
 
-bool wave_step(int t, int n_img, int Hb, int Wb, StepDesc &sd);
-bool wave_step_ext(int t, int n_img, int Hb, int Wb, StepDesc &sd);
+// steps of a call of one geometry: wavefront steps t = h + 2v, or (raster) blocks v * Wb + h
+int step_count(bool raster, int Hb, int Wb) { return raster ? Hb * Wb : Wb + 2 * (Hb - 1); }
 
 // lanes: 1 = one stream per image (reference container; decode in raster order), 0 = one lane per block row
 void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p) {
     const bool k3 = m->k1 == 3;
     p = MixedPlan();
     p.n_img = n;
+    p.raster = raster;
     p.lane0.assign(n + 1, 0);
     int64_t npos = 0;
     for (int i = 0; i < n; ++i) {
@@ -789,7 +793,7 @@ void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster,
         const int L = lanes == 1 ? 1 : Hb[i];
         p.lane0[i + 1] = p.lane0[i] + L;
         p.max_lanes = L > p.max_lanes ? L : p.max_lanes;
-        const int last = raster ? Hb[i] * Wb[i] : Wb[i] + 2 * (Hb[i] - 1);
+        const int last = step_count(raster, Hb[i], Wb[i]);
         p.s_last = last > p.s_last ? last : p.s_last;
     }
     p.n_lanes = p.lane0[n];
@@ -813,23 +817,13 @@ void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster,
         p.ext0.push_back(p.n_ext);
         p.row0.push_back((int)p.rows.size());
         for (int i = 0; i < n; ++i) {
-            if (raster) {
-                if (s >= Hb[i] * Wb[i]) continue;
-                const int v = s / Wb[i], h = s - v * Wb[i];
-                if (k3) {   // as run_steps: at a row start the right ring column of the row above and the left one
-                    if (h == 0 && v >= 1) add_ext(i, v - 1, Wb[i]);
-                    if (h == 0) add_ext(i, v, -1);
-                    add_ext(i, v, h);
-                }
-                add_row(i, v, h);
-                continue;
-            }
-            if (s >= Wb[i] + 2 * (Hb[i] - 1)) continue;
-            StepDesc e;
-            if (k3 && wave_step_ext(s, 1, Hb[i], Wb[i], e))
-                for (int v = e.vmin; v < e.vmin + e.nv; ++v) add_ext(i, v, s - 2 * v);
-            if (wave_step(s, 1, Hb[i], Wb[i], e))
-                for (int v = e.vmin; v < e.vmin + e.nv; ++v) add_row(i, v, s - 2 * v);
+            if (s >= step_count(raster, Hb[i], Wb[i])) continue;
+            StepDesc e[3];
+            const int n_ring = k3 ? ring_steps(s, raster, 1, Hb[i], Wb[i], e) : 0;
+            for (int j = 0; j < n_ring; ++j)
+                for (int v = e[j].vmin; v < e[j].vmin + e[j].nv; ++v) add_ext(i, v, e[j].t - 2 * v);
+            if (step_desc(s, raster, 1, Hb[i], Wb[i], e[0]))
+                for (int v = e[0].vmin; v < e[0].vmin + e[0].nv; ++v) add_row(i, v, e[0].t - 2 * v);
         }
         const int k = (int)p.row0.size() - 1;
         const int R = (int)p.rows.size() - p.row0[k], Re = p.n_ext - p.ext0[k];
@@ -882,82 +876,88 @@ int upload_mixed(lbic_model *m, MixedPlan &p, cudaStream_t st) {
     LBIC_CUDA(cudaMemcpyAsync(m->mix_dev, m->mix_host.data(), off, cudaMemcpyHostToDevice, st));
     char *d = (char *)m->mix_dev;
     p.geo.img = (const int4 *)(d + at[0]);
-    p.geo.rows = p.d_rows = (const int4 *)(d + at[1]);
+    p.geo.rows = (const int4 *)(d + at[1]);
     p.d_ext = (const int4 *)(d + at[2]);
     p.geo.sched = (const int *)(d + at[3]);
     p.geo.blk_img = (const int *)(d + at[4]);
     p.geo.g0row = (const int *)(d + at[5]);
-    p.d_stream = (const int *)(d + at[6]);
+    p.geo.stream = (const int *)(d + at[6]);
     p.d_lane0 = (const int *)(d + at[7]);
     p.d_seg = (const int64_t *)(d + at[8]);
     return 0;
 }
 
-// The GEMM layers see schedule rows [row0, row0 + R) as a raster chunk of one "image" of 1 x nblk blocks: the row
-// destinations of their epilogues (epi_row_dst) are then the schedule rows themselves.
-StepDesc mixed_step_desc(const MixedPlan &p, int k) { return StepDesc{1, 0, 0, p.row0[k], 1, p.nblk}; }
+// The steps [first, last) of a call.  at(s) gives step s's rows (R = 0: none, as step -1 of KS[1] = 3) and, with
+// KS[1] = 3, the ring-extended steps whose hidden map becomes computable with it (returns how many).  A call of one
+// geometry takes both from the closed forms (step_desc, ring_steps); a mixed-size call from its schedule, in which the
+// GEMM layers see step s as a raster chunk of one "image" of 1 x nblk blocks, so that the row destinations of their
+// epilogues (epi_row_dst) are the schedule rows themselves.
+struct CallSteps {
+    int first = 0, last = 0;
+    bool raster = false, k3 = false;
+    int n_img = 0, Hb = 0, Wb = 0;
+    const MixedPlan *plan = nullptr;
 
-// KS[1] == 3: hidden map g0 = lrelu(E0(zhat taps)) at the ring-extended positions `ext` (single-position or
-// diagonal steps with h in [-1, Wb]), scattered into the position-indexed store (SURVEY.md A.3 / A.6).
-int run_g0(lbic_model *m, const StepDesc &ext, int R_ext, cudaStream_t st) {
-    Workspace &ws = m->ws;
-    if (R_ext <= 0) return 0;
-    if (R_ext > ws.R_ext_cap) return lbic_fail(LBIC_ERR_INVALID, "internal: extended step exceeds its workspace");
-    LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, ext, R_ext, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo,
-                           ws.Text.ld, st));
-    return run_layers(m, L_E0, L_E1, ext, R_ext, st);
+    int at(int s, StepRows &main, StepRows ring[3]) const {
+        if (plan) {
+            const MixedPlan &p = *plan;
+            const int k = s - first, r0 = p.row0[k], e0 = p.ext0[k];
+            main = StepRows{StepDesc{1, 0, 0, r0, 1, p.nblk}, p.row0[k + 1] - r0, &p.geo, p.geo.rows + r0};
+            // the g0 store holds the ring rows in schedule order after its row 0, the top ring row of every image
+            ring[0] = StepRows{StepDesc{}, p.ext0[k + 1] - e0, &p.geo, p.d_ext + e0, 1 + e0};
+            return k3 ? 1 : 0;
+        }
+        main = StepRows{};
+        if (step_desc(s, raster, n_img, Hb, Wb, main.sd)) main.R = n_img * main.sd.nv;
+        StepDesc e[3];
+        const int n = k3 ? ring_steps(s, raster, n_img, Hb, Wb, e) : 0;
+        for (int j = 0; j < n; ++j) ring[j] = StepRows{e[j], n_img * e[j].nv};
+        return n;
+    }
+};
+
+CallSteps call_steps(const lbic_model *m, int n_img, int Hb, int Wb, bool raster) {
+    CallSteps c;
+    c.raster = raster; c.k3 = m->k1 == 3;
+    c.n_img = n_img; c.Hb = Hb; c.Wb = Wb;
+    c.first = !raster && c.k3 ? -1 : 0;
+    c.last = step_count(raster, Hb, Wb);
+    return c;
 }
 
-// The same for step k of a mixed-size call: the store holds the ring-extended rows in schedule order after the top
-// row, so E0 writes its R_ext rows contiguously from row 1 + ext0[k].
-int run_g0_mixed(lbic_model *m, const MixedPlan &p, int k, cudaStream_t st) {
+CallSteps call_steps(const lbic_model *m, const MixedPlan &p) {
+    CallSteps c;
+    c.raster = p.raster; c.k3 = m->k1 == 3;
+    c.first = p.s_first; c.last = p.s_last;
+    c.plan = &p;
+    return c;
+}
+
+// KS[1] == 3: hidden map g0 = lrelu(E0(zhat taps)) at the ring-extended positions of `ext` (single-position or
+// diagonal steps with h in [-1, Wb]), into the g0 store (SURVEY.md A.3 / A.6): scattered by position, or (ring rows of
+// a mixed-size call) written contiguously from store row ext.g0_row0.
+int run_g0(lbic_model *m, const StepRows &ext, cudaStream_t st) {
     Workspace &ws = m->ws;
-    const int e0 = p.ext0[k], R_ext = p.ext0[k + 1] - e0;
-    if (R_ext <= 0) return 0;
-    if (R_ext > ws.R_ext_cap) return lbic_fail(LBIC_ERR_INVALID, "internal: extended step exceeds its workspace");
-    LBIC_TRY(launch_gather_mixed(nullptr, ws.zhat_cl, m->Cin, p.geo, p.d_ext + e0, R_ext, nullptr, nullptr, 0, ws.Text.hi,
-                                 ws.Text.lo, ws.Text.ld, st));
+    if (ext.R <= 0) return 0;
+    if (ext.R > ws.R_ext_cap) return lbic_fail(LBIC_ERR_INVALID, "internal: extended step exceeds its workspace");
+    LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, ext, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo, ws.Text.ld, st));
+    if (ext.g0_row0 < 0) return run_layers(m, L_E0, L_E1, ext, st);
     const LayerWiring &w = ws.net[L_E0];
     EpiParams ep = w.ep;
     ep.out_pos = 0;
-    ep.out_hi += (size_t)(1 + e0) * ep.ld_out;
-    ep.out_lo += (size_t)(1 + e0) * ep.ld_out;
-    return run_gemm_layer(m, m->L[L_E0], L_E0, R_ext, w.a[0], w.a[1], ep, st);
+    ep.out_hi += (size_t)ext.g0_row0 * ep.ld_out;
+    ep.out_lo += (size_t)ext.g0_row0 * ep.ld_out;
+    return run_gemm_layer(m, m->L[L_E0], L_E0, ext.R, w.a[0], w.a[1], ep, st);
 }
 
 // The first layer of a step and its operand: E0 on the zhat taps, or (KS[1] == 3: E0 has run on the ring-extended rows,
 // run_g0) E1 on the five g0 taps around each block, gathered here.
-int step_entry(lbic_model *m, const StepDesc &sd, int R, int *first, cudaStream_t st, const MixedPlan *mx = nullptr) {
+int step_entry(lbic_model *m, const StepRows &rows, int *first, cudaStream_t st) {
     Workspace &ws = m->ws;
     *first = L_E0;
     if (m->k1 != 3) return 0;
     *first = L_E1;
-    if (mx)
-        return launch_gather5_mixed(ws.G0.hi, ws.G0.lo, m->E1, mx->geo, mx->d_rows + sd.t, R, ws.H1x5.hi, ws.H1x5.lo,
-                                    ws.H1x5.ld, st);
-    return launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, sd, R, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st);
-}
-
-int floor_div2(int a) { return a >= 0 ? a / 2 : -((-a + 1) / 2); }
-
-// ring-extended diagonal of step t (KS[1] == 3): positions (v, h = t - 2v) with v in [0, Hb-1], h in [-1, Wb]
-bool wave_step_ext(int t, int n_img, int Hb, int Wb, StepDesc &sd) {
-    int vmin = floor_div2(t - Wb + 1);   // ceil((t - Wb) / 2)
-    if (vmin < 0) vmin = 0;
-    int vmax = floor_div2(t + 1);
-    if (vmax > Hb - 1) vmax = Hb - 1;
-    if (vmax < vmin) return false;
-    sd.n_img = n_img; sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t; sd.Hb = Hb; sd.Wb = Wb;
-    return true;
-}
-
-bool wave_step(int t, int n_img, int Hb, int Wb, StepDesc &sd) {
-    if (t < 0) return false;
-    int vmin = t - (Wb - 1) <= 0 ? 0 : (t - (Wb - 1) + 1) / 2;
-    int vmax = t / 2 < Hb - 1 ? t / 2 : Hb - 1;
-    if (vmax < vmin) return false;
-    sd.n_img = n_img; sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t; sd.Hb = Hb; sd.Wb = Wb;
-    return true;
+    return launch_gather5(ws.G0.hi, ws.G0.lo, m->E1, rows, ws.H1x5.hi, ws.H1x5.lo, ws.H1x5.ld, st);
 }
 
 int check_ready(lbic_model *m, bool need_tables) {
@@ -1051,90 +1051,43 @@ int run_wave(lbic_model *m, bool decode, bool raster, int s_begin, int s_end, in
     return gemm_wave_launch(w, st);
 }
 
-// One wavefront step of an encode: entropy net, encoder net + quantisation, decoder net for the R rows of `sd`
-// (NET:363-377 for every block of the diagonal at once).  `mx`: a step of a mixed-size call (mixed_step_desc).
-int encode_step(lbic_model *m, const StepDesc &sd, int R, bool syms, cudaStream_t st, const MixedPlan *mx = nullptr) {
+// One wavefront step of an encode: entropy net, encoder net + quantisation, decoder net for the rows of the step
+// (NET:363-377 for every block of the diagonal at once).
+int encode_step(lbic_model *m, const StepRows &rows, bool syms, cudaStream_t st) {
     Workspace &ws = m->ws;
     int l0;
-    if (mx)
-        LBIC_TRY(launch_gather_mixed(ws.x_cl, ws.zhat_cl, m->Cin, mx->geo, mx->d_rows + sd.t, R, ws.X.hi, ws.X.lo, ws.X.ld,
-                                     ws.T.hi, ws.T.lo, ws.T.ld, st));
-    else
-        LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
-    LBIC_TRY(step_entry(m, sd, R, &l0, st, mx));
-    return run_range(m, l0, L_COUNT, sd, R, syms, st);
+    LBIC_TRY(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, rows, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, rows, &l0, st));
+    return run_range(m, l0, L_COUNT, rows, syms, st);
 }
 
 // One step of a decode: entropy net, rANS decode of y_qnt (and of the symbols into `sym`, if set) from `lanes` streams
 // per image, decoder net (NET:420-450 for every block of the step at once).
-int decode_step(lbic_model *m, const StepDesc &sd, int R, int lanes, int32_t *sym, cudaStream_t st,
-                const MixedPlan *mx = nullptr) {
+int decode_step(lbic_model *m, const StepRows &rows, int lanes, int32_t *sym, cudaStream_t st) {
     Workspace &ws = m->ws;
     int l0;
-    if (mx)
-        LBIC_TRY(launch_gather_mixed(nullptr, ws.zhat_cl, m->Cin, mx->geo, mx->d_rows + sd.t, R, nullptr, nullptr, 0,
-                                     ws.T.hi, ws.T.lo, ws.T.ld, st));
-    else
-        LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
-    LBIC_TRY(step_entry(m, sd, R, &l0, st, mx));
-    LBIC_TRY(run_range(m, l0, L_F0, sd, R, true, st));
-    if (mx)
-        LBIC_TRY(launch_rans_dec_step_mixed(m->tables, ws.dec_states, ws.lane_ptr, mx->d_stream + sd.t, sd.t, R, m->M,
-                                            ws.KSI, ws.ldKSI, ws.YQ.hi, ws.YQ.lo, ws.YQ.ld, sym, st));
-    else
-        LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, lanes, sd, R, m->M, ws.KSI, ws.ldKSI,
-                                      ws.YQ.hi, ws.YQ.lo, ws.YQ.ld, sym, st));
-    return run_range(m, L_D0, L_COUNT, sd, R, true, st);
+    LBIC_TRY(launch_gather(nullptr, ws.zhat_cl, m->Cin, rows, nullptr, nullptr, 0, ws.T.hi, ws.T.lo, ws.T.ld, st));
+    LBIC_TRY(step_entry(m, rows, &l0, st));
+    LBIC_TRY(run_range(m, l0, L_F0, rows, true, st));
+    LBIC_TRY(launch_rans_dec_step(m->tables, ws.dec_states, ws.lane_ptr, lanes, rows, m->M, ws.KSI, ws.ldKSI, ws.YQ.hi,
+                                  ws.YQ.lo, ws.YQ.ld, sym, st));
+    return run_range(m, L_D0, L_COUNT, rows, true, st);
 }
 
-// Step s of a call: wavefront step t = s, or (raster) block (v, h) of every image with s = v * Wb + h.  False if the
-// step has no block of the image (KS[1] == 3: step -1 has ring positions only).
-bool step_desc(int s, bool raster, int n_img, int Hb, int Wb, StepDesc &sd) {
-    if (!raster) return wave_step(s, n_img, Hb, Wb, sd);
-    const int v = s / Wb, h = s - v * Wb;
-    sd = StepDesc{n_img, 1, v, h + 2 * v, Hb, Wb};
-    return true;
-}
-
-// The step loop of an encode or a decode.  Each step runs through `step(sd, R)` (per-layer or dataflow launches) after
+// The step loop of an encode or a decode.  Each step runs through `step(rows)` (per-layer or dataflow launches) after
 // the hidden-map ring positions (KS[1] == 3) that become computable with it, or, when `wave` (small steps: single images,
 // small batches), consecutive steps are collected into ONE launch of the persistent wavefront kernel, `wave_range(s0,
-// s1)`, cut only where a host hook has copies or conversions to put between two steps.  A mixed-size call (`mx`) takes
-// its steps from the schedule; it has no hooks and no wavefront kernel (wave = false).
+// s1)`, cut only where a host hook has copies or conversions to put between two steps.  (Mixed-size calls have no hooks
+// and no wavefront kernel.)
 template <class Step, class WaveRange>
-int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, const RowHooks *hk, Step step,
-              WaveRange wave_range, cudaStream_t st, const MixedPlan *mx = nullptr) {
-    auto desc = [&](int s, StepDesc &sd) -> bool {   // step s of the call; false if it has no block
-        if (!mx) return step_desc(s, raster, n_img, Hb, Wb, sd);
-        const int k = s - mx->s_first;
-        sd = mixed_step_desc(*mx, k);
-        return mx->row0[k + 1] > mx->row0[k];
-    };
+int run_steps(lbic_model *m, const CallSteps &cs, bool wave, const RowHooks *hk, Step step, WaveRange wave_range,
+              cudaStream_t st) {
+    const int Hb = cs.Hb, Wb = cs.Wb;
     auto launch_step = [&](int s) -> int {
-        if (mx) {
-            const int k = s - mx->s_first;
-            if (m->k1 == 3) LBIC_TRY(run_g0_mixed(m, *mx, k, st));
-            StepDesc sd;
-            if (!desc(s, sd)) return 0;
-            return step(sd, mx->row0[k + 1] - mx->row0[k]);
-        }
-        if (m->k1 == 3 && raster) {
-            // hidden-map positions that become computable now: the ring columns of the row start, then (v,h)
-            const int v = s / Wb, h = s - v * Wb;
-            if (h == 0) {
-                if (v >= 1) { StepDesc e{n_img, 1, v - 1, Wb + 2 * (v - 1), Hb, Wb}; LBIC_TRY(run_g0(m, e, n_img, st)); }
-                StepDesc e{n_img, 1, v, -1 + 2 * v, Hb, Wb};
-                LBIC_TRY(run_g0(m, e, n_img, st));
-            }
-            StepDesc e{n_img, 1, v, h + 2 * v, Hb, Wb};
-            LBIC_TRY(run_g0(m, e, n_img, st));
-        } else if (m->k1 == 3) {
-            StepDesc ext;
-            if (wave_step_ext(s, n_img, Hb, Wb, ext)) LBIC_TRY(run_g0(m, ext, n_img * ext.nv, st));
-        }
-        StepDesc sd;
-        if (!step_desc(s, raster, n_img, Hb, Wb, sd)) return 0;
-        return step(sd, n_img * sd.nv);
+        StepRows rows, ring[3];
+        const int n_ring = cs.at(s, rows, ring);
+        for (int j = 0; j < n_ring; ++j) LBIC_TRY(run_g0(m, ring[j], st));
+        return rows.R > 0 ? step(rows) : 0;
     };
     int pend = -1;                                   // steps [pend, s) wait to be launched
     auto flush = [&](int s_end) -> int {
@@ -1148,11 +1101,11 @@ int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, 
         for (int s = b; s < s_end; ++s) LBIC_TRY(launch_step(s));
         return 0;
     };
-    const int s_first = mx ? mx->s_first : raster ? 0 : (m->k1 == 3 ? -1 : 0);
-    const int s_last = mx ? mx->s_last : raster ? Hb * Wb : Wb + 2 * (Hb - 1);
-    for (int s = s_first; s < s_last; ++s) {
-        StepDesc sd;
-        const bool has = desc(s, sd);
+    for (int s = cs.first; s < cs.last; ++s) {
+        StepRows rows, ring[3];
+        cs.at(s, rows, ring);
+        const StepDesc &sd = rows.sd;
+        const bool has = rows.R > 0;
         if (has && hk && hk->need_rows) {
             const int v_hi = sd.vmin + sd.nv - 1;
             if (!wave || !hk->will_need || hk->will_need(hk->ctx, v_hi)) {
@@ -1167,7 +1120,7 @@ int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, 
         }
         if (has && hk && hk->rows_done) {
             int done = 0;                            // zhat block rows [0, done) are final after step s
-            if (raster) {
+            if (cs.raster) {
                 if ((s + 1) % Wb == 0) done = (s + 1) / Wb;
             } else if (s >= Wb - 1) {
                 done = (s - (Wb - 1)) / 2 + 1;
@@ -1179,11 +1132,20 @@ int run_steps(lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool wave, 
             }
         }
     }
-    return flush(s_last);
+    return flush(cs.last);
 }
 
 int ws_acquire(lbic_model *m, cudaStream_t st) {
     if (m->ws_used && st != m->ws_stream) LBIC_CUDA(cudaStreamWaitEvent(st, m->ws_event, 0));
+    return 0;
+}
+
+// Start of an encode or decode on `st`: hold the workspace, clear the error flag and the zhat feedback buffer of its
+// nblk blocks (NET:336, NET:417).
+int call_begin(lbic_model *m, size_t nblk, cudaStream_t st) {
+    LBIC_TRY(ws_acquire(m, st));
+    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
+    LBIC_CUDA(cudaMemsetAsync(m->ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));
     return 0;
 }
 int ws_release(lbic_model *m, cudaStream_t st) {
@@ -1497,20 +1459,18 @@ int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float 
     Workspace &ws = m->ws;
     const int HW = Hb * Wb;
     const size_t nblk = (size_t)n_img * HW;
-    LBIC_TRY(ws_acquire(m, st));
-    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
+    LBIC_TRY(call_begin(m, nblk, st));
     if (x) LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, n_img, m->Cin, HW, st));
-    LBIC_CUDA(cudaMemsetAsync(ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));   // NET:336
     const bool want_syms = sym_out || idx_out || stream_out || info_cl;
     if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
-    auto step = [&](const StepDesc &sd, int R) -> int {
-        LBIC_TRY(encode_step(m, sd, R, want_syms, st));
-        return info_cl ? launch_selfinfo_step(sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st) : 0;
+    auto step = [&](const StepRows &rows) -> int {
+        LBIC_TRY(encode_step(m, rows, want_syms, st));
+        return info_cl ? launch_selfinfo_step(rows.sd, rows.R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st) : 0;
     };
     auto wave_range = [&](int s0, int s1) { return run_wave(m, false, false, s0, s1, n_img, Hb, Wb, 0, nullptr, st); };
     // (the wavefront kernel does not compute the self-information)
     const bool wave = !info_cl && wave_applies(m, n_img, Hb, Wb, false, false);
-    LBIC_TRY(run_steps(m, n_img, Hb, Wb, false, wave, hk, step, wave_range, st));
+    LBIC_TRY(run_steps(m, call_steps(m, n_img, Hb, Wb, false), wave, hk, step, wave_range, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
     if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
     if (idx_out) LBIC_CUDA(cudaMemcpyAsync(idx_out, ws.idx, nblk * m->M, cudaMemcpyDeviceToDevice, st));
@@ -1580,23 +1540,23 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
             }
             for (long r0 = 0; r0 < nblk && rc == 0; r0 += chunk) {
                 const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
-                const StepDesc sd{n_img, 0, 0, (int)r0, Hb, Wb};
+                const StepRows rows{StepDesc{n_img, 0, 0, (int)r0, Hb, Wb}, R};
                 // (the taps go to Text, the operand of E0 in the layer table; it has at least R_cap rows)
-                P(launch_gather(nullptr, ws.zhat_cl, m->Cin, sd, R, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo,
+                P(launch_gather(nullptr, ws.zhat_cl, m->Cin, rows, nullptr, nullptr, 0, ws.Text.hi, ws.Text.lo,
                                 ws.Text.ld, st));
-                P(run_layers(m, L_E0, L_E1, sd, R, st));
+                P(run_layers(m, L_E0, L_E1, rows, st));
             }
             if (rc) break;
         }
         // one launch per layer: the decoder net writes the caller's reconstruction, which the dataflow launch cannot
         for (long r0 = 0; r0 < nblk && rc == 0; r0 += chunk) {
             const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
-            const StepDesc sd{n_img, 0, 0, (int)r0, Hb, Wb};
+            const StepRows rows{StepDesc{n_img, 0, 0, (int)r0, Hb, Wb}, R};
             int l0;
-            P(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, sd, R, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
-            P(step_entry(m, sd, R, &l0, st));
-            P(run_layers(m, l0, L_COUNT, sd, R, st, true, xhat_cl, clamp ? 0 : 1));
-            if (info_cl) P(launch_selfinfo_step(sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st));
+            P(launch_gather(ws.x_cl, ws.zhat_cl, m->Cin, rows, ws.X.hi, ws.X.lo, ws.X.ld, ws.T.hi, ws.T.lo, ws.T.ld, st));
+            P(step_entry(m, rows, &l0, st));
+            P(run_layers(m, l0, L_COUNT, rows, st, true, xhat_cl, clamp ? 0 : 1));
+            if (info_cl) P(launch_selfinfo_step(rows.sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st));
         }
         if (rc) break;
         P(launch_cl_to_nchw(xhat_cl, xhat_out, n_img, m->Cin, HW, st));
@@ -1651,18 +1611,17 @@ int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_le
     const int HW = Hb * Wb;
     const size_t nblk = (size_t)n_img * HW;
     const int L = lanes == 1 ? 1 : Hb;
-    LBIC_TRY(ws_acquire(m, st));
-    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
-    LBIC_CUDA(cudaMemsetAsync(ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));   // NET:417
+    LBIC_TRY(call_begin(m, nblk, st));
     LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, n_img, L, lanes != 1, ws.dec_states, ws.lane_ptr,
                                   m->err_flag, st));
     if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
     const bool raster = (L == 1 && lanes == 1);      // reference container: the rANS state threads through the blocks in
                                                      // raster order (NET:420-450), one block of every image per step
     int32_t *sym = sym_out ? ws.sym : nullptr;
-    auto step = [&](const StepDesc &sd, int R) { return decode_step(m, sd, R, L, sym, st); };
+    auto step = [&](const StepRows &rows) { return decode_step(m, rows, L, sym, st); };
     auto wave_range = [&](int s0, int s1) { return run_wave(m, true, raster, s0, s1, n_img, Hb, Wb, L, sym, st); };
-    LBIC_TRY(run_steps(m, n_img, Hb, Wb, raster, wave_applies(m, n_img, Hb, Wb, raster, true), hk, step, wave_range, st));
+    LBIC_TRY(run_steps(m, call_steps(m, n_img, Hb, Wb, raster), wave_applies(m, n_img, Hb, Wb, raster, true), hk, step,
+                       wave_range, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
     if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
     return ws_release(m, st);
@@ -1692,10 +1651,8 @@ int mixed_begin(lbic_model *m, int n_img, const int *Hb, const int *Wb, bool ras
                 cudaStream_t st) {
     plan_mixed(m, n_img, Hb, Wb, raster, lanes, p);
     LBIC_TRY(ensure_workspace_mixed(m, mixed_need(m, p)));
-    LBIC_TRY(ws_acquire(m, st));
+    LBIC_TRY(call_begin(m, p.nblk, st));
     LBIC_TRY(upload_mixed(m, p, st));
-    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
-    LBIC_CUDA(cudaMemsetAsync(m->ws.zhat_cl, 0, sizeof(float) * (size_t)p.nblk * m->Cin, st));   // NET:336, NET:417
     if (m->k1 == 3)   // row 0 of the g0 store: the top ring row (fill_g0_top of a single position)
         LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, 1, 0, -1, m->ws.G0.hi, m->ws.G0.lo, st));
     return 0;
@@ -1715,9 +1672,9 @@ int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, c
     const size_t nblk = p.nblk;
     LBIC_TRY(launch_nchw_to_cl_mixed(x, ws.x_cl, m->Cin, p.geo, p.nblk, st));
     const bool want_syms = sym_out || idx_out || stream_out;
-    auto step = [&](const StepDesc &sd, int R) { return encode_step(m, sd, R, want_syms, st, &p); };
+    auto step = [&](const StepRows &rows) { return encode_step(m, rows, want_syms, st); };
     auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, n_img, 0, 0, false, false, nullptr, step, no_wave, st, &p));
+    LBIC_TRY(run_steps(m, call_steps(m, p), false, nullptr, step, no_wave, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
     if (!want_syms) return ws_release(m, st);
     // symbols and indexes in packed order: into the caller's arrays, or (streams only) a model buffer
@@ -1765,9 +1722,9 @@ int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *str
     LBIC_TRY(launch_rans_dec_init_mixed(streams, stream_len, stream_cap, n_img, p.d_lane0, p.n_lanes, lanes != 1,
                                         ws.dec_states, ws.lane_ptr, m->err_flag, st));
     int32_t *sym = sym_out ? ws.sym : nullptr;
-    auto step = [&](const StepDesc &sd, int R) { return decode_step(m, sd, R, 0, sym, st, &p); };
+    auto step = [&](const StepRows &rows) { return decode_step(m, rows, 0, sym, st); };
     auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, n_img, 0, 0, raster, false, nullptr, step, no_wave, st, &p));
+    LBIC_TRY(run_steps(m, call_steps(m, p), false, nullptr, step, no_wave, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
     if (sym_out) LBIC_TRY(launch_unschedule_i32(ws.sym, sym_out, m->M, p.geo, p.nblk, st));
     return ws_release(m, st);
@@ -2051,8 +2008,9 @@ extern "C" int lbic_postprocess(lbic_model *m, const float *z, int n_img, int Hb
     const int chunk = ws.R_cap;
     for (long r0 = 0; r0 < nblk; r0 += chunk) {
         const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
-        const StepDesc sd{n_img, 0, 0, (int)r0, Hb, Wb};                       // raster chunk: row r = block r0 + r
-        LBIC_TRY(launch_gather9(ws.zhat_cl, m->Cin, sd, R, m->PPA.hi, m->PPA.lo, m->PPA.ld, st));
+        const StepRows rows{StepDesc{n_img, 0, 0, (int)r0, Hb, Wb}, R};          // raster chunk: row r = block r0 + r
+        const StepDesc &sd = rows.sd;
+        LBIC_TRY(launch_gather9(ws.zhat_cl, m->Cin, rows, m->PPA.hi, m->PPA.lo, m->PPA.ld, st));
         LBIC_TRY(run_gemm_layer(m, m->PP[0], -1, R, &m->vPPA, nullptr, epi_hilo(EPI_LRELU, sd, m->PPH), st));
         EpiParams e = epi(EPI_RESID, sd);
         e.out_f32 = out_cl + (size_t)r0 * m->Cin; e.ld_f32 = m->Cin;
@@ -2086,10 +2044,7 @@ extern "C" int lbic_band_begin(lbic_model *m, const float *x, int n_img, int Hb,
     cudaStream_t st = (cudaStream_t)stream;
     LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
     Workspace &ws = m->ws;
-    const size_t nblk = (size_t)n_img * Hb * Wb;
-    LBIC_TRY(ws_acquire(m, st));
-    LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
-    LBIC_CUDA(cudaMemsetAsync(ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));
+    LBIC_TRY(call_begin(m, (size_t)n_img * Hb * Wb, st));
     if (decode) {
         if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
         LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, n_img, Hb, 1, ws.dec_states, ws.lane_ptr, m->err_flag, st));
@@ -2108,14 +2063,15 @@ extern "C" int lbic_band_step(lbic_model *m, int t, int v0, int v1, void *stream
     Active act(m);
     cudaStream_t st = (cudaStream_t)stream;
     const int n_img = m->band_n, Hb = m->band_Hb, Wb = m->band_Wb;
-    StepDesc sd;
+    StepRows rows;
+    StepDesc &sd = rows.sd;
     if (!wave_step(t, n_img, Hb, Wb, sd)) return 0;
     const int lo = sd.vmin > v0 ? sd.vmin : v0;
     const int hi = (sd.vmin + sd.nv) < v1 ? (sd.vmin + sd.nv) : v1;
     if (hi <= lo) return 0;
     sd.vmin = lo; sd.nv = hi - lo;
-    const int R = n_img * sd.nv;
-    return m->band_decode ? decode_step(m, sd, R, Hb, nullptr, st) : encode_step(m, sd, R, true, st);
+    rows.R = n_img * sd.nv;
+    return m->band_decode ? decode_step(m, rows, Hb, nullptr, st) : encode_step(m, rows, true, st);
 }
 
 // Ends the call for block rows [v0, v1): the band's reconstruction (channel-last rows, (n_img, v1-v0, Wb, 3B^2)) and,

@@ -114,35 +114,6 @@ __device__ __forceinline__ unsigned long long wave_now() {
     return t;
 }
 
-__device__ __forceinline__ bool wave_step_desc(const WaveParams &p, int s, StepDesc &sd) {
-    sd.n_img = p.n_img; sd.Hb = p.Hb; sd.Wb = p.Wb;
-    if (p.mode == 1) {
-        const int v = s / p.Wb, h = s - v * p.Wb;
-        sd.nv = 1; sd.vmin = v; sd.t = h + 2 * v;
-        return true;
-    }
-    const int t = s;
-    const int vmin = t - (p.Wb - 1) <= 0 ? 0 : (t - (p.Wb - 1) + 1) / 2;
-    const int vmax = t / 2 < p.Hb - 1 ? t / 2 : p.Hb - 1;
-    if (t < 0 || vmax < vmin) return false;
-    sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t;
-    return true;
-}
-
-// extended step of KS[1] = 3 (api.cu: wave_step_ext): the positions (v, h = t - 2 v) with h in [-1, Wb]
-__device__ __forceinline__ bool wave_step_desc_ext(const WaveParams &p, int t, StepDesc &sd) {
-    sd.n_img = p.n_img; sd.Hb = p.Hb; sd.Wb = p.Wb;
-    const int a = t - p.Wb + 1;
-    int vmin = a >= 0 ? a / 2 : -((-a + 1) / 2);          // floor(a / 2)
-    if (vmin < 0) vmin = 0;
-    const int b = t + 1;
-    int vmax = b >= 0 ? b / 2 : -((-b + 1) / 2);
-    if (vmax > p.Hb - 1) vmax = p.Hb - 1;
-    if (vmax < vmin) return false;
-    sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t;
-    return true;
-}
-
 struct WaveTile {
     StepDesc sd;
     StepDesc sd_ext;     // KS[1] = 3
@@ -177,11 +148,11 @@ __device__ __forceinline__ void wave_for_each_tile(const WaveParams &p, F &&f) {
 #pragma unroll 1
     for (int s = p.s_begin; s < p.s_end; ++s) {
         WaveTile w;
-        if (!wave_step_desc(p, s, w.sd)) continue;
+        if (!step_desc(s, p.mode == 1, p.n_img, p.Hb, p.Wb, w.sd)) continue;
         w.R = w.sd.n_img * w.sd.nv;
         w.R_ext = 0;
         if (p.k3) {              // (one row block per step in this mode: the launch is refused otherwise)
-            if (wave_step_desc_ext(p, s, w.sd_ext)) w.R_ext = w.sd_ext.n_img * w.sd_ext.nv;
+            if (wave_step_ext(s, p.n_img, p.Hb, p.Wb, w.sd_ext)) w.R_ext = w.sd_ext.n_img * w.sd_ext.nv;
         }
         w.n_rb = (w.R + BM - 1) / BM;
         w.prev_n_rb = prev_n_rb;

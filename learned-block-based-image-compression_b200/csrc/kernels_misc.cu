@@ -157,17 +157,67 @@ __global__ void split_kernel(const float *__restrict__ src, h16 *__restrict__ hi
     }
 }
 
-// ---- per-step gather ----------------------------------------------------------------------------
-// Row r = block (img, v, h) of the step.  X[r, :] = x(v,h); T[r, tap*Cin + c] = zhat(v+dv, h+dh)[c] for the
-// four live taps of a 3x3 mask-'A' kernel, (dv,dh) = (-1,-1), (-1,0), (-1,+1), (0,-1) (masked_conv2d.py:12-17),
-// zero outside the image (NET:349).
-__global__ void gather_kernel(const float *__restrict__ x_cl, const float *__restrict__ zhat_cl, int Cin, StepDesc s,
+// ---- per-step gathers -----------------------------------------------------------------------------
+// Row sources: row_at(s, r) resolves row r of a step once; the row then answers where its x block is, where its zhat
+// neighbour (dv, dh) is (false: outside the image) and which row of the g0 store its tap (dv, dh) reads.
+//   StepDesc: one geometry, the closed form (x_cl and zhat_cl by block, the g0 store by ring position, g0_pos_index).
+//   MixedRows: the R row records of a mixed-size step (schedule rows, or the ring-extended rows of E0, which have no x
+//   block); x_cl is in packed block order, zhat_cl and the g0 store in schedule order, the borders those of the row's
+//   own image.
+struct StepRow {
+    int img, v, h, Hb, Wb;
+    __device__ size_t x_block() const { return ((size_t)img * Hb + v) * Wb + h; }
+    __device__ bool zhat_block(int dv, int dh, size_t &b) const {
+        const int vv = v + dv, hh = h + dh;
+        if (!(vv >= 0 && vv < Hb && hh >= 0 && hh < Wb)) return false;
+        b = ((size_t)img * Hb + vv) * Wb + hh;
+        return true;
+    }
+    __device__ size_t g0_row(int dv, int dh) const { return g0_pos_index(img, v + dv, h + dh, Hb, Wb); }
+};
+__device__ __forceinline__ StepRow row_at(const StepDesc &s, int r) {
+    StepRow q;
+    step_row_to_block(s, r, q.img, q.v, q.h);
+    q.Hb = s.Hb; q.Wb = s.Wb;
+    return q;
+}
+
+struct MixedRows {
+    MixedGeo g;
+    const int4 *__restrict__ rows;
+};
+struct MixedRow {
+    int4 rec, gi;   // {img, v, h, packed block}, the image's {Hb, Wb, P, G}
+    const int *sched, *g0row;
+    __device__ size_t x_block() const { return (size_t)rec.w; }
+    __device__ bool zhat_block(int dv, int dh, size_t &b) const {
+        const int vv = rec.y + dv, hh = rec.z + dh;
+        if (!(vv >= 0 && vv < gi.x && hh >= 0 && hh < gi.y)) return false;
+        b = (size_t)sched[gi.z + vv * gi.y + hh];
+        return true;
+    }
+    __device__ size_t g0_row(int dv, int dh) const {
+        return (size_t)g0row[gi.w + (rec.y + dv + 1) * (gi.y + 2) + (rec.z + dh + 1)];
+    }
+};
+__device__ __forceinline__ MixedRow row_at(const MixedRows &s, int r) {
+    MixedRow q;
+    q.rec = s.rows[r];
+    q.gi = s.g.img[q.rec.x];
+    q.sched = s.g.sched; q.g0row = s.g.g0row;
+    return q;
+}
+
+// Row r of the step.  X[r, :] = x(v,h); T[r, tap*Cin + c] = zhat(v+dv, h+dh)[c] for the four live taps of a 3x3
+// mask-'A' kernel, (dv,dh) = (-1,-1), (-1,0), (-1,+1), (0,-1) (masked_conv2d.py:12-17), zero outside the image
+// (NET:349).
+template <class Rows>
+__global__ void gather_kernel(const float *__restrict__ x_cl, const float *__restrict__ zhat_cl, int Cin, Rows s,
                               int R, h16 *__restrict__ X_hi, h16 *__restrict__ X_lo, int ldX,
                               h16 *__restrict__ T_hi, h16 *__restrict__ T_lo, int ldT) {
     const int r = blockIdx.x;
     if (r >= R) return;
-    int img, v, h;
-    step_row_to_block(s, r, img, v, h);
+    const auto q = row_at(s, r);
     const int c4n = Cin >> 2;
     const int first = X_hi ? 0 : 1;
     for (int e = threadIdx.x + first * c4n; e < 5 * c4n; e += blockDim.x) {
@@ -175,16 +225,15 @@ __global__ void gather_kernel(const float *__restrict__ x_cl, const float *__res
         float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
         h16 *ph, *pl;
         if (seg == 0) {
-            val = *reinterpret_cast<const float4 *>(x_cl + (((size_t)img * s.Hb + v) * s.Wb + h) * Cin + c);
+            val = *reinterpret_cast<const float4 *>(x_cl + q.x_block() * Cin + c);
             ph = X_hi + (size_t)r * ldX + c;
             pl = X_lo + (size_t)r * ldX + c;
         } else {
             const int tap = seg - 1;
             const int dv = (tap == 3) ? 0 : -1;
             const int dh = (tap == 3) ? -1 : tap - 1;
-            const int vv = v + dv, hh = h + dh;
-            if (vv >= 0 && vv < s.Hb && hh >= 0 && hh < s.Wb)
-                val = *reinterpret_cast<const float4 *>(zhat_cl + (((size_t)img * s.Hb + vv) * s.Wb + hh) * Cin + c);
+            size_t b;
+            if (q.zhat_block(dv, dh, b)) val = *reinterpret_cast<const float4 *>(zhat_cl + b * Cin + c);
             ph = T_hi + (size_t)r * ldT + tap * Cin + c;
             pl = T_lo + (size_t)r * ldT + tap * Cin + c;
         }
@@ -195,18 +244,18 @@ __global__ void gather_kernel(const float *__restrict__ x_cl, const float *__res
 
 // KS[1] == 3: out[r, tap*E1 + c] = g0(v+dv, h+dh)[c] for the five live taps of a 3x3 mask-'B' kernel,
 // (dv,dh) = (-1,-1), (-1,0), (-1,+1), (0,-1), (0,0); every such position lies inside the ring-extended store.
-__global__ void gather5_kernel(const h16 *__restrict__ g_hi, const h16 *__restrict__ g_lo, int E1, StepDesc s, int R,
+template <class Rows>
+__global__ void gather5_kernel(const h16 *__restrict__ g_hi, const h16 *__restrict__ g_lo, int E1, Rows s, int R,
                                h16 *__restrict__ o_hi, h16 *__restrict__ o_lo, int ld) {
     const int r = blockIdx.x;
     if (r >= R) return;
-    int img, v, h;
-    step_row_to_block(s, r, img, v, h);
+    const auto q = row_at(s, r);
     const int c8n = E1 >> 3;   // 16-byte chunks per plane row
     for (int e = threadIdx.x; e < 5 * c8n; e += blockDim.x) {
         const int tap = e / c8n, c = (e - tap * c8n) << 3;
         const int dv = (tap >= 3) ? 0 : -1;
         const int dh = (tap >= 3) ? tap - 4 : tap - 1;
-        const size_t src = g0_pos_index(img, v + dv, h + dh, s.Hb, s.Wb) * E1 + c;
+        const size_t src = q.g0_row(dv, dh) * E1 + c;
         const size_t dst = (size_t)r * ld + (size_t)tap * E1 + c;
         *reinterpret_cast<uint4 *>(o_hi + dst) = *reinterpret_cast<const uint4 *>(g_hi + src);
         *reinterpret_cast<uint4 *>(o_lo + dst) = *reinterpret_cast<const uint4 *>(g_lo + src);
@@ -267,64 +316,6 @@ __global__ void fill_g0_top_kernel(const float *__restrict__ bias, int E1, int n
 }
 
 // ---- mixed-size batches (MixedGeo): x_cl is in packed block order, zhat_cl in schedule order ------------------------
-// gather_kernel for the rows of a mixed step: the borders are those of the row's own image.  Ring-extended rows (h =
-// -1 or Wb, the operand of E0 when KS[1] == 3) come without X.
-__global__ void gather_mixed_kernel(const float *__restrict__ x_cl, const float *__restrict__ zhat_cl, int Cin,
-                                    MixedGeo g, const int4 *__restrict__ rows, int R, h16 *__restrict__ X_hi,
-                                    h16 *__restrict__ X_lo, int ldX, h16 *__restrict__ T_hi, h16 *__restrict__ T_lo,
-                                    int ldT) {
-    const int r = blockIdx.x;
-    if (r >= R) return;
-    const int4 rec = rows[r];
-    const int v = rec.y, h = rec.z;
-    const int4 gi = g.img[rec.x];   // Hb, Wb, P, G
-    const int c4n = Cin >> 2;
-    const int first = X_hi ? 0 : 1;
-    for (int e = threadIdx.x + first * c4n; e < 5 * c4n; e += blockDim.x) {
-        const int seg = e / c4n, c = (e - seg * c4n) << 2;
-        float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
-        h16 *ph, *pl;
-        if (seg == 0) {
-            val = *reinterpret_cast<const float4 *>(x_cl + (size_t)rec.w * Cin + c);
-            ph = X_hi + (size_t)r * ldX + c;
-            pl = X_lo + (size_t)r * ldX + c;
-        } else {
-            const int tap = seg - 1;
-            const int dv = (tap == 3) ? 0 : -1;
-            const int dh = (tap == 3) ? -1 : tap - 1;
-            const int vv = v + dv, hh = h + dh;
-            if (vv >= 0 && vv < gi.x && hh >= 0 && hh < gi.y)
-                val = *reinterpret_cast<const float4 *>(zhat_cl + (size_t)g.sched[gi.z + vv * gi.y + hh] * Cin + c);
-            ph = T_hi + (size_t)r * ldT + tap * Cin + c;
-            pl = T_lo + (size_t)r * ldT + tap * Cin + c;
-        }
-        const float f[4] = {val.x, val.y, val.z, val.w};
-        store_hilo<4>(ph, pl, f);
-    }
-}
-
-// gather5_kernel for the rows of a mixed step: the g0 store holds the ring-extended rows in the order E0 computed them
-// (row 0: the top ring row v = -1, shared by every image), g.g0row maps a ring position to its row.
-__global__ void gather5_mixed_kernel(const h16 *__restrict__ g_hi, const h16 *__restrict__ g_lo, int E1, MixedGeo g,
-                                     const int4 *__restrict__ rows, int R, h16 *__restrict__ o_hi,
-                                     h16 *__restrict__ o_lo, int ld) {
-    const int r = blockIdx.x;
-    if (r >= R) return;
-    const int4 rec = rows[r];
-    const int4 gi = g.img[rec.x];
-    const int c8n = E1 >> 3;
-    for (int e = threadIdx.x; e < 5 * c8n; e += blockDim.x) {
-        const int tap = e / c8n, c = (e - tap * c8n) << 3;
-        const int dv = (tap >= 3) ? 0 : -1;
-        const int dh = (tap >= 3) ? tap - 4 : tap - 1;
-        const int pos = gi.w + (rec.y + dv + 1) * (gi.y + 2) + (rec.z + dh + 1);
-        const size_t src = (size_t)g.g0row[pos] * E1 + c;
-        const size_t dst = (size_t)r * ld + (size_t)tap * E1 + c;
-        *reinterpret_cast<uint4 *>(o_hi + dst) = *reinterpret_cast<const uint4 *>(g_hi + src);
-        *reinterpret_cast<uint4 *>(o_lo + dst) = *reinterpret_cast<const uint4 *>(g_lo + src);
-    }
-}
-
 // Packed NCHW (image i at C * P_i, (C, Hb_i, Wb_i) within) <-> channel-last rows, 32 blocks x 32 channels per tile.
 // TO_CL: row = packed block; otherwise row = the block's schedule row.
 template <bool TO_CL>
@@ -514,29 +505,37 @@ int launch_split_f32(const float *src, h16 *hi, h16 *lo, int64_t n, cudaStream_t
     return 0;
 }
 
-int launch_gather(const float *x_cl, const float *zhat_cl, int Cin, const StepDesc &s, int R, h16 *X_hi, h16 *X_lo,
-                  int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st) {
-    if (R <= 0) return 0;
+// The gathers of a step: the closed form of s.sd, or (mixed-size step) the step's row records.
+int launch_gather(const float *x_cl, const float *zhat_cl, int Cin, const StepRows &s, h16 *X_hi, h16 *X_lo, int ldX,
+                  h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st) {
+    if (s.R <= 0) return 0;
     int threads = 5 * (Cin / 4);
     threads = threads > 256 ? 256 : ((threads + 31) / 32) * 32;
-    gather_kernel<<<R, threads, 0, st>>>(x_cl, zhat_cl, Cin, s, R, X_hi, X_lo, ldX, T_hi, T_lo, ldT);
+    if (s.geo)
+        gather_kernel<<<s.R, threads, 0, st>>>(x_cl, zhat_cl, Cin, MixedRows{*s.geo, s.rows}, s.R, X_hi, X_lo, ldX, T_hi,
+                                               T_lo, ldT);
+    else
+        gather_kernel<<<s.R, threads, 0, st>>>(x_cl, zhat_cl, Cin, s.sd, s.R, X_hi, X_lo, ldX, T_hi, T_lo, ldT);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepDesc &s, int R, h16 *out_hi, h16 *out_lo,
-                   int ld, cudaStream_t st) {
-    if (R <= 0) return 0;
-    gather5_kernel<<<R, 256, 0, st>>>(g0_hi, g0_lo, E1, s, R, out_hi, out_lo, ld);
+int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepRows &s, h16 *out_hi, h16 *out_lo, int ld,
+                   cudaStream_t st) {
+    if (s.R <= 0) return 0;
+    if (s.geo)
+        gather5_kernel<<<s.R, 256, 0, st>>>(g0_hi, g0_lo, E1, MixedRows{*s.geo, s.rows}, s.R, out_hi, out_lo, ld);
+    else
+        gather5_kernel<<<s.R, 256, 0, st>>>(g0_hi, g0_lo, E1, s.sd, s.R, out_hi, out_lo, ld);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_gather9(const float *z_cl, int Cin, const StepDesc &s, int R, h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st) {
-    if (R <= 0) return 0;
-    gather9_kernel<<<R, 256, 0, st>>>(z_cl, Cin, s, R, out_hi, out_lo, ld);
+int launch_gather9(const float *z_cl, int Cin, const StepRows &s, h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st) {
+    if (s.R <= 0) return 0;
+    gather9_kernel<<<s.R, 256, 0, st>>>(z_cl, Cin, s.sd, s.R, out_hi, out_lo, ld);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
@@ -552,26 +551,6 @@ int launch_restore_border(const float *z_cl, float *out_cl, int Cin, int n_img, 
 
 int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16 *g_hi, h16 *g_lo, cudaStream_t st) {
     fill_g0_top_kernel<<<n_img * (Wb + 2), 256, 0, st>>>(bias, E1, n_img, Hb, Wb, g_hi, g_lo);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_gather_mixed(const float *x_cl, const float *zhat_cl, int Cin, const MixedGeo &g, const int4 *rows, int R,
-                        h16 *X_hi, h16 *X_lo, int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st) {
-    if (R <= 0) return 0;
-    int threads = 5 * (Cin / 4);
-    threads = threads > 256 ? 256 : ((threads + 31) / 32) * 32;
-    gather_mixed_kernel<<<R, threads, 0, st>>>(x_cl, zhat_cl, Cin, g, rows, R, X_hi, X_lo, ldX, T_hi, T_lo, ldT);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_gather5_mixed(const h16 *g0_hi, const h16 *g0_lo, int E1, const MixedGeo &g, const int4 *rows, int R,
-                         h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st) {
-    if (R <= 0) return 0;
-    gather5_mixed_kernel<<<R, 256, 0, st>>>(g0_hi, g0_lo, E1, g, rows, R, out_hi, out_lo, ld);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;

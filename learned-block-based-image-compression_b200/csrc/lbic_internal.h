@@ -63,14 +63,63 @@ __host__ __device__ inline void step_row_to_block(const StepDesc &s, int r, int 
     h = s.t - 2 * v;
 }
 
+// The steps of a call of one geometry, shared by the host drivers (api.cu) and the wavefront kernel (gemm_wave.cu).
+// Step s is wavefront step t = s: the blocks (v, h = t - 2v) with v in [0, Hb-1], h in [0, Wb-1] (false if there is
+// none), or (raster, the serial decode of the reference container) block (v, h) of every image with s = v * Wb + h.
+__host__ __device__ inline bool step_desc(int s, bool raster, int n_img, int Hb, int Wb, StepDesc &sd) {
+    sd.n_img = n_img; sd.Hb = Hb; sd.Wb = Wb;
+    if (raster) {
+        const int v = s / Wb, h = s - v * Wb;
+        sd.nv = 1; sd.vmin = v; sd.t = h + 2 * v;
+        return true;
+    }
+    const int t = s;
+    const int vmin = t - (Wb - 1) <= 0 ? 0 : (t - (Wb - 1) + 1) / 2;
+    const int vmax = t / 2 < Hb - 1 ? t / 2 : Hb - 1;
+    if (t < 0 || vmax < vmin) return false;
+    sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t;
+    return true;
+}
+__host__ __device__ inline bool wave_step(int t, int n_img, int Hb, int Wb, StepDesc &sd) {
+    return step_desc(t, false, n_img, Hb, Wb, sd);
+}
+
+// KS[1] == 3, ring-extended diagonal of step t: the positions (v, h = t - 2v) with v in [0, Hb-1], h in [-1, Wb]
+__host__ __device__ inline bool wave_step_ext(int t, int n_img, int Hb, int Wb, StepDesc &sd) {
+    sd.n_img = n_img; sd.Hb = Hb; sd.Wb = Wb;
+    const int a = t - Wb + 1;
+    int vmin = a >= 0 ? a / 2 : -((-a + 1) / 2);          // floor(a / 2)
+    if (vmin < 0) vmin = 0;
+    const int b = t + 1;
+    int vmax = b >= 0 ? b / 2 : -((-b + 1) / 2);
+    if (vmax > Hb - 1) vmax = Hb - 1;
+    if (vmax < vmin) return false;
+    sd.nv = vmax - vmin + 1; sd.vmin = vmin; sd.t = t;
+    return true;
+}
+
+// KS[1] == 3: the ring-extended positions whose hidden map g0 becomes computable with step s, as single-row-band steps
+// in the order they are computed; returns how many.  Wavefront: the extended diagonal.  Raster: at a row start the right
+// ring column of the row above and the left one of this row, then the block itself.
+__host__ __device__ inline int ring_steps(int s, bool raster, int n_img, int Hb, int Wb, StepDesc ext[3]) {
+    if (!raster) return wave_step_ext(s, n_img, Hb, Wb, ext[0]) ? 1 : 0;
+    const int v = s / Wb, h = s - v * Wb;
+    int n = 0;
+    if (h == 0 && v >= 1) ext[n++] = StepDesc{n_img, 1, v - 1, Wb + 2 * (v - 1), Hb, Wb};
+    if (h == 0) ext[n++] = StepDesc{n_img, 1, v, -1 + 2 * v, Hb, Wb};
+    ext[n++] = StepDesc{n_img, 1, v, h + 2 * v, Hb, Wb};
+    return n;
+}
+
 // ------------------------------------------------------------------------------------------------
 // A batch of differently sized images (lbic_encode_mixed / lbic_decode_mixed).  The host lays every step's rows out
 // back to back in one schedule (api.cu: MixedPlan) and keeps the per-step working data in SCHEDULE order: schedule row
 // k holds the k-th block the call computes.  The GEMM layers then see each step as the raster chunk
 //   StepDesc{1, 0, 0, k0, 1, n_rows}      (row r -> block k0 + r, see step_row_to_block)
 // so their epilogues write the symbols, indexes and reconstruction of row r to schedule row k0 + r with the
-// equal-size kernels unchanged.  Only the kernels that look at an image's geometry (the gathers, the rANS decode step,
-// the stream and layout kernels) have mixed forms, which read these tables.
+// equal-size kernels unchanged.  The kernels that look at an image's geometry read these tables: the gathers and the
+// rANS decode step through a row-source template parameter (one kernel body each, instantiated for StepDesc and for
+// the schedule's rows), the stream and layout kernels in mixed forms of their own.
 // ------------------------------------------------------------------------------------------------
 struct MixedGeo {
     const int4 *rows;      // schedule row -> {img, v, h, packed block}      (packed block = P_img + v * Wb_img + h)
@@ -78,6 +127,19 @@ struct MixedGeo {
     const int *sched;      // packed block -> schedule row
     const int *blk_img;    // packed block -> image
     const int *g0row;      // KS[1] = 3: ring position G_img + (v + 1) * (Wb + 2) + (h + 1) -> row of the g0 store
+    const int *stream;     // schedule row -> decoder stream
+};
+
+// The rows of one step as the host launches them.  `sd` is what the GEMM epilogues see: a wavefront or raster step of
+// one geometry, or for a mixed-size call the raster chunk of schedule rows [sd.t, sd.t + R).  A mixed-size step also
+// carries the schedule and its R device row records (schedule rows, or the ring-extended rows of E0); the launchers of
+// the gathers and of the rANS decode step take the closed form of `sd` when it has none.
+struct StepRows {
+    StepDesc sd{};
+    int R = 0;
+    const MixedGeo *geo = nullptr;
+    const int4 *rows = nullptr;
+    int g0_row0 = -1;      // ring rows of a mixed-size call: E0 writes them to g0 store rows g0_row0, ... (-1: by position)
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -224,8 +286,8 @@ int launch_space_to_depth(const float *img, float *blk, int n, int C, int Hb, in
 int launch_depth_to_space(const float *blk, float *img, int n, int C, int Hb, int Wb, int B, cudaStream_t st);
 int launch_split_f32(const float *src, h16 *hi, h16 *lo, int64_t n, cudaStream_t st);
 // per-step gather of x and the four causal neighbour blocks of zhat (SURVEY.md A.1/A.2)
-int launch_gather(const float *x_cl, const float *zhat_cl, int Cin, const StepDesc &s, int R,
-                  h16 *X_hi, h16 *X_lo, int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st);
+int launch_gather(const float *x_cl, const float *zhat_cl, int Cin, const StepRows &s, h16 *X_hi, h16 *X_lo, int ldX,
+                  h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st);
 // weight packing
 // weight packing: effective fp32 weights (mask folded / taps reordered / GDN reparametrised), their max |w|,
 // then the scaled fp16 hi/lo split
@@ -239,16 +301,12 @@ int launch_split_scaled(const float *src, h16 *hi, h16 *lo, int64_t n, float sca
 // KS[1]==3: A operand of get_meanscale[2] = the five mask-'B' taps of g0 around each block of the step
 // post-processing net (NET:455-476): A operand of its 3x3 conv = all nine taps of the reconstruction around each block
 // of a raster chunk, zero outside the image; and the final fix-up: blocks on the image border keep their input
-int launch_gather9(const float *z_cl, int Cin, const StepDesc &s, int R, h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st);
+// (one geometry only: the closed form of s.sd)
+int launch_gather9(const float *z_cl, int Cin, const StepRows &s, h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st);
 int launch_restore_border(const float *z_cl, float *out_cl, int Cin, int n_img, int Hb, int Wb, cudaStream_t st);
-int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepDesc &s, int R, h16 *out_hi, h16 *out_lo,
-                   int ld, cudaStream_t st);
+int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepRows &s, h16 *out_hi, h16 *out_lo, int ld,
+                   cudaStream_t st);
 int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16 *g_hi, h16 *g_lo, cudaStream_t st);
-// mixed-size forms (MixedGeo): `rows` are the R row records of the step (main rows, or the ring-extended rows of E0)
-int launch_gather_mixed(const float *x_cl, const float *zhat_cl, int Cin, const MixedGeo &g, const int4 *rows, int R,
-                        h16 *X_hi, h16 *X_lo, int ldX, h16 *T_hi, h16 *T_lo, int ldT, cudaStream_t st);
-int launch_gather5_mixed(const h16 *g0_hi, const h16 *g0_lo, int E1, const MixedGeo &g, const int4 *rows, int R,
-                         h16 *out_hi, h16 *out_lo, int ld, cudaStream_t st);
 // packed NCHW images <-> packed channel-last blocks (to_cl) or schedule-ordered channel-last blocks (from_cl), and a
 // schedule-ordered (block, C) array -> packed order; one launch for the whole batch
 int launch_nchw_to_cl_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
@@ -302,9 +360,10 @@ void rans_set_enc_block_max_streams(int n);    // encodes of at most this many s
 void rans_set_enc_thread_min_streams(int n);   // encodes of at least this many streams use the thread-per-stream kernel
 void rans_set_dec_smem_warp(int on);           // 1 (default): warp-per-row decode steps run on shared-memory tables
 void rans_set_dec_thread_min_rows(int rows);   // steps with at least this many rows use the thread-per-stream kernel
+// (one geometry: row r reads stream img * lanes + v, or img for lanes <= 1; a mixed-size step: stream geo->stream[row])
 int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
-                         const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo,
-                         int ld_yq, int32_t *sym_out, cudaStream_t st);
+                         const StepRows &s, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq,
+                         int32_t *sym_out, cudaStream_t st);
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,
                          cudaStream_t st);
 // Mixed-size forms.  Encode: stream s holds symbols [seg[s], seg[s+1]) (device array, min_sym = the shortest stream);
@@ -318,10 +377,6 @@ int launch_lane_pack_mixed(const uint32_t *scratch, size_t scratch_words, int n_
 int launch_rans_dec_init_mixed(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
                                const int *lane0, int n_lanes, int lanes_container, RansStreamState *states,
                                const uint8_t **lane_ptr, int *err_flag, cudaStream_t st);
-// decode step of schedule rows [row0, row0 + R): row r reads stream `stream[r]` and writes its symbols to row row0 + r
-int launch_rans_dec_step_mixed(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr,
-                               const int *stream, int row0, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi,
-                               h16 *yq_lo, int ld_yq, int32_t *sym_out, cudaStream_t st);
 // CDF index of n scales by both routines of the decoders (bisection; hint with bisection fallback), for tests
 int launch_scale_index(const float *scales, int n, const float *tab, int32_t *idx_bisect, int32_t *idx_hinted, cudaStream_t st);
 int launch_rans_decode_full(const Tables &T, const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride,

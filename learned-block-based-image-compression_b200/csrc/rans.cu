@@ -985,16 +985,12 @@ int rans_dec_step_any(const Tables &T, RansStreamState *states, const uint8_t *c
 }
 
 int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
-                         const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo,
-                         int ld_yq, int32_t *sym_out, cudaStream_t st) {
-    return rans_dec_step_any(T, states, lane_ptr, lanes, s, R, M, ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
-}
-
-int launch_rans_dec_step_mixed(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr,
-                               const int *stream, int row0, int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi,
-                               h16 *yq_lo, int ld_yq, int32_t *sym_out, cudaStream_t st) {
-    return rans_dec_step_any(T, states, lane_ptr, 0, MixedDecRows{stream, row0}, R, M, ksi, ld_ksi, yq_hi, yq_lo,
-                             ld_yq, sym_out, st);
+                         const StepRows &s, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq,
+                         int32_t *sym_out, cudaStream_t st) {
+    if (s.geo)   // schedule rows [sd.t, sd.t + R)
+        return rans_dec_step_any(T, states, lane_ptr, 0, MixedDecRows{s.geo->stream + s.sd.t, s.sd.t}, s.R, M, ksi,
+                                 ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
+    return rans_dec_step_any(T, states, lane_ptr, lanes, s.sd, s.R, M, ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
 }
 
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,

@@ -1,6 +1,7 @@
-// Device-side pieces shared by the persistent warp-specialised kernels (gemm_ws.cu: gemm_ws_kernel / gemm_flow_kernel;
-// gemm_wave.cu: gemm_wave_kernel): shared-memory budget constants, CTA-pair helpers, and the epilogue of one 128 x bn
-// tile by the eight epilogue warps (TMEM -> fused layer arithmetic -> staged, coalesced row stores).
+// Device-side pieces shared by the persistent warp-specialised kernels (gemm_ws.cu: the one pipeline body behind
+// gemm_ws_kernel and gemm_flow_kernel; gemm_wave.cu: gemm_wave_kernel): shared-memory budget constants, CTA-pair
+// helpers, and the epilogue of one 128 x bn tile by the eight epilogue warps (TMEM -> fused layer arithmetic -> staged,
+// coalesced row stores).
 #pragma once
 #include "tc_common.cuh"
 
@@ -103,11 +104,11 @@ struct EpiCtx {
     uint32_t rank;            // CTA within its pair (0 = leader)
     // dataflow launch only: the epilogue's own side input (GDN pre-activations) is written by another layer of the same
     // launch; it may be fetched once *dep_cnt >= dep_target (the epilogue warps run ahead of the TMA producer)
-    const int *dep_cnt;
-    int dep_target;
+    const int *dep_cnt = nullptr;
+    int dep_target = 0;
     // second side input written inside the same launch: the entropy parameters (ksi) the QUANT epilogue reads
-    const int *dep2_cnt;
-    int dep2_target;
+    const int *dep2_cnt = nullptr;
+    int dep2_target = 0;
     unsigned long long *trace_acc = nullptr;   // debug: %globaltimer when the accumulator became available
     // the accumulator was produced by M = 64 MMAs (latency kernel, steps of at most 64 rows): row r sits in TMEM lane
     // 32 (r / 16) + r % 16, i.e. each warp's lanes 0-15 hold rows 16 q .. 16 q + 15 (scripts/mma_m64_layout.cu)

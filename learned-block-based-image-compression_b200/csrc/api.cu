@@ -57,7 +57,7 @@ struct PackedSeg {
 };
 
 struct PackedLayer {
-    int cout = 0, bn = 0, nseg = 0;
+    int cout = 0, nseg = 0;
     int bn_v[NBN] = {};
     int n_bn = 0;
     PackedSeg seg[2];
@@ -208,6 +208,12 @@ void free_all(std::vector<void *> &list) {
     list.clear();
 }
 
+// width of the tiles when cout is cut into the fewest equal tiles of at most wmax columns, rounded up to 16
+int tile_width(int cout, int wmax) {
+    const int nt = (cout + wmax - 1) / wmax;
+    return ((cout + nt - 1) / nt + 15) / 16 * 16;
+}
+
 // tile-width variants of a layer, one per split factor (lbic_split): widest first
 int bn_variants(int cout, int *out) {
     for (int i = 0; i < NBN; ++i) {
@@ -216,8 +222,7 @@ int bn_variants(int cout, int *out) {
                              : i == LBIC_SMALL_VARIANT ? gemm_ws_max_bn() / 2
                              : i == LBIC_LAT_VARIANT ? 32 : i == LBIC_LAT64_VARIANT ? 64 : i == LBIC_LAT128_VARIANT ? 128
                              : gemm_ws_max_bn();
-            const int nt = (cout + wmax - 1) / wmax;
-            out[i] = ((cout + nt - 1) / nt + 15) / 16 * 16;
+            out[i] = tile_width(cout, wmax);
             continue;
         }
         const int f = lbic_split(i);
@@ -226,13 +231,6 @@ int bn_variants(int cout, int *out) {
         out[i] = bn < 16 ? 16 : bn;
     }
     return NBN;
-}
-
-int pick_bn(int cout) {
-    const int ntiles = (cout + 255) / 256;
-    int bn = (cout + ntiles - 1) / ntiles;
-    bn = (bn + 15) / 16 * 16;
-    return bn;
 }
 
 // ---- weight loading ---------------------------------------------------------------------------
@@ -276,7 +274,7 @@ const int TAPS_1[2] = {0, 0};
 const int TAPS_9[18] = {0, 0, 0, 1, 0, 2, 1, 0, 1, 1, 1, 2, 2, 0, 2, 1, 2, 2};   // plain 3x3 conv (post-processing net)
 
 int pack_conv_seg(lbic_model *m, const SdView &sd, const std::string &prefix, int cout, int cin, int k,
-                  const int *taps, int ntaps, int bn, PackedSeg &seg, float **bias_tmp, std::vector<void *> &tmp,
+                  const int *taps, int ntaps, PackedSeg &seg, float **bias_tmp, std::vector<void *> &tmp,
                   cudaStream_t st) {
     float *w = nullptr, *mask = nullptr;
     const int64_t nw = (int64_t)cout * cin * k * k;
@@ -290,7 +288,6 @@ int pack_conv_seg(lbic_model *m, const SdView &sd, const std::string &prefix, in
     LBIC_TRY(launch_pack_conv(w, mask, cout, cin, k, k, taps, ntaps, seg.weff, seg.K, st));
     int bnv[NBN];
     const int nb = bn_variants(cout, bnv);
-    (void)bn;
     for (int i = 0; i < nb; ++i) {
         const int box = (i == LBIC_PAIR_VARIANT || i == LBIC_PAIR_WIDE) ? bnv[i] / 2 : bnv[i];   // a CTA pair loads half the tile per CTA
         LBIC_TRY(make_tmap_2d(&seg.tm_hi[i], seg.hi, seg.K, cout, seg.K, 64, box));
@@ -330,11 +327,10 @@ int pack_linear(lbic_model *m, const SdView &sd, int id, const std::string &pref
 int pack_linear_into(lbic_model *m, PackedLayer &L, const SdView &sd, const std::string &prefix, int cout, int cin, int k,
                      const int *taps, int ntaps, std::vector<void *> &tmp, cudaStream_t st) {
     L.cout = cout;
-    L.bn = pick_bn(cout);
     L.n_bn = bn_variants(cout, L.bn_v);
     L.nseg = 1;
     float *b = nullptr;
-    LBIC_TRY(pack_conv_seg(m, sd, prefix, cout, cin, k, taps, ntaps, L.bn, L.seg[0], &b, tmp, st));
+    LBIC_TRY(pack_conv_seg(m, sd, prefix, cout, cin, k, taps, ntaps, L.seg[0], &b, tmp, st));
     LBIC_TRY(dev_alloc(m->weight_allocs, (void **)&L.bias, sizeof(float) * cout));
     LBIC_TRY(launch_add_vec(b, nullptr, L.bias, cout, st));
     return finish_layer(m, L, st);
@@ -345,12 +341,11 @@ int pack_dual(lbic_model *m, const SdView &sd, int id, const std::string &p1, in
               int cout, std::vector<void *> &tmp, cudaStream_t st) {
     PackedLayer &L = m->L[id];
     L.cout = cout;
-    L.bn = pick_bn(cout);
     L.n_bn = bn_variants(cout, L.bn_v);
     L.nseg = 2;
     float *b1 = nullptr, *b2 = nullptr;
-    LBIC_TRY(pack_conv_seg(m, sd, p1, cout, cin1, 1, TAPS_1, 1, L.bn, L.seg[0], &b1, tmp, st));
-    LBIC_TRY(pack_conv_seg(m, sd, p2, cout, m->Cin, 3, TAPS_A, 4, L.bn, L.seg[1], &b2, tmp, st));
+    LBIC_TRY(pack_conv_seg(m, sd, p1, cout, cin1, 1, TAPS_1, 1, L.seg[0], &b1, tmp, st));
+    LBIC_TRY(pack_conv_seg(m, sd, p2, cout, m->Cin, 3, TAPS_A, 4, L.seg[1], &b2, tmp, st));
     LBIC_TRY(dev_alloc(m->weight_allocs, (void **)&L.bias, sizeof(float) * cout));
     LBIC_TRY(launch_add_vec(b1, b2, L.bias, cout, st));
     return finish_layer(m, L, st);
@@ -360,7 +355,6 @@ int pack_gdn(lbic_model *m, const SdView &sd, int id, const std::string &prefix,
              cudaStream_t st) {
     PackedLayer &L = m->L[id];
     L.cout = C;
-    L.bn = pick_bn(C);
     L.n_bn = bn_variants(C, L.bn_v);
     L.nseg = 1;
     float *g = nullptr, *b = nullptr;
@@ -2136,6 +2130,37 @@ extern "C" int lbic_rans_decode(lbic_model *m, const uint8_t *streams, const uin
                                    (cudaStream_t)stream);
 }
 
+namespace {
+
+constexpr int TC_MAX_BN = 256;   // widest tile of the per-tile kernel (gemm_tc_launch)
+
+// K segment s of a debug GEMM whose g.R, g.cout and g.bn are set: A [g.R x K] and W [g.cout x K] (fp32, device) split into
+// fp16 hi / lo planes, the activation planes zero beyond row g.R up to whole 256-row (pair) tiles as the workspace buffers
+// are, and the maps make_view and pack_conv_seg build: 64 k x 128 rows, 64 k x tile width (half of it per CTA of a pair).
+// tm receives [A hi, A lo, W hi, W lo].
+int debug_operands(GemmCall &g, int s, const float *A, const float *W, int K, int pair, CUtensorMap (&tm)[4],
+                   std::vector<void *> &tmp, cudaStream_t st) {
+    const int Rp = (g.R + 255) / 256 * 256;
+    h16 *ah, *al, *wh, *wl;
+    LBIC_TRY(dev_alloc(tmp, (void **)&ah, sizeof(h16) * (size_t)Rp * K, true));
+    LBIC_TRY(dev_alloc(tmp, (void **)&al, sizeof(h16) * (size_t)Rp * K, true));
+    LBIC_TRY(dev_alloc(tmp, (void **)&wh, sizeof(h16) * (size_t)g.cout * K));
+    LBIC_TRY(dev_alloc(tmp, (void **)&wl, sizeof(h16) * (size_t)g.cout * K));
+    LBIC_TRY(launch_split_f32(A, ah, al, (int64_t)g.R * K, st));
+    LBIC_TRY(launch_split_f32(W, wh, wl, (int64_t)g.cout * K, st));
+    const int box = pair ? g.bn / 2 : g.bn;
+    LBIC_TRY(make_tmap_2d(&tm[0], ah, K, Rp, K, 64, 128));
+    LBIC_TRY(make_tmap_2d(&tm[1], al, K, Rp, K, 64, 128));
+    LBIC_TRY(make_tmap_2d(&tm[2], wh, K, g.cout, K, 64, box));
+    LBIC_TRY(make_tmap_2d(&tm[3], wl, K, g.cout, K, 64, box));
+    g.K[s] = K;
+    g.A[s] = {ah, al, K, &tm[0], &tm[1]};
+    g.W[s] = {wh, wl, K, &tm[2], &tm[3]};
+    return 0;
+}
+
+}  // namespace
+
 extern "C" int lbic_debug_gemm(lbic_model *m, const float *A, const float *W, float *D, int R, int K, int cout,
                                void *stream) {
     if (!m || !A || !W || !D) return lbic_fail(LBIC_ERR_INVALID, "null argument");
@@ -2143,33 +2168,17 @@ extern "C" int lbic_debug_gemm(lbic_model *m, const float *A, const float *W, fl
     Active act(m);
     cudaStream_t st = (cudaStream_t)stream;
     std::vector<void *> tmp;
-    h16 *ah, *al, *wh, *wl;
     int rc = 0;
     do {
 #define P(call) if ((rc = (call)) != 0) break
-        P(dev_alloc(tmp, (void **)&ah, sizeof(h16) * (size_t)R * K));
-        P(dev_alloc(tmp, (void **)&al, sizeof(h16) * (size_t)R * K));
-        P(dev_alloc(tmp, (void **)&wh, sizeof(h16) * (size_t)cout * K));
-        P(dev_alloc(tmp, (void **)&wl, sizeof(h16) * (size_t)cout * K));
-        P(launch_split_f32(A, ah, al, (int64_t)R * K, st));
-        P(launch_split_f32(W, wh, wl, (int64_t)cout * K, st));
         GemmCall g;
         memset(&g, 0, sizeof(g));
-        g.R = R; g.cout = cout; g.bn = pick_bn(cout); g.nseg = 1; g.K[0] = K;
         const bool ws = m->gemm_core == 0 && m->use_ws == 2;   // forced persistent kernel (optionally its CTA-pair form)
         const int pair = ws && m->use_pair;
-        if (ws) {
-            const int wmax = (pair && m->use_pair == 3) ? gemm_pair_max_bn() : gemm_ws_max_bn();
-            const int nt = (cout + wmax - 1) / wmax;
-            g.bn = ((cout + nt - 1) / nt + 15) / 16 * 16;
-        }
-        CUtensorMap ta_h, ta_l, tw_h, tw_l;
-        P(make_tmap_2d(&ta_h, ah, K, R, K, 64, 128));
-        P(make_tmap_2d(&ta_l, al, K, R, K, 64, 128));
-        P(make_tmap_2d(&tw_h, wh, K, cout, K, 64, pair ? g.bn / 2 : g.bn));
-        P(make_tmap_2d(&tw_l, wl, K, cout, K, 64, pair ? g.bn / 2 : g.bn));
-        g.A[0].hi = ah; g.A[0].lo = al; g.A[0].ld = K; g.A[0].tm_hi = &ta_h; g.A[0].tm_lo = &ta_l;
-        g.W[0].hi = wh; g.W[0].lo = wl; g.W[0].ld = K; g.W[0].tm_hi = &tw_h; g.W[0].tm_lo = &tw_l;
+        g.R = R; g.cout = cout; g.nseg = 1;
+        g.bn = tile_width(cout, !ws ? TC_MAX_BN : (pair && m->use_pair == 3) ? gemm_pair_max_bn() : gemm_ws_max_bn());
+        CUtensorMap tm[4];
+        P(debug_operands(g, 0, A, W, K, pair, tm, tmp, st));
         g.ep.mode = EPI_RAW; g.ep.R = R; g.ep.cout = cout; g.ep.out_f32 = D; g.ep.ld_f32 = cout; g.ep.acc_scale = 1.0f;
         P(m->gemm_core == 1 ? gemm_simt_launch(g, st) : (ws ? gemm_ws_launch(g, st, pair) : gemm_tc_launch(g, st)));
 #undef P
@@ -2207,35 +2216,11 @@ extern "C" int lbic_debug_layer(lbic_model *m, const lbic_debug_layer_args *a, v
         GemmCall g;
         memset(&g, 0, sizeof(g));
         const int pair = a->core >= 3;
-        // activation planes cover whole (pair) tiles, zero beyond row R, as the workspace buffers do (R_cap rows)
-        const int Rp = (a->R + 255) / 256 * 256;
         g.R = a->R; g.cout = a->cout; g.nseg = a->nseg;
-        if (a->core >= 2) {
-            const int wmax = a->core == 4 ? gemm_pair_max_bn() : gemm_ws_max_bn();
-            const int nt = (a->cout + wmax - 1) / wmax;
-            g.bn = ((a->cout + nt - 1) / nt + 15) / 16 * 16;
-        } else {
-            g.bn = a->force_bn ? a->force_bn : pick_bn(a->cout);
-        }
-        CUtensorMap tm[2][4];   // [segment][A hi, A lo, W hi, W lo]
-        for (int s = 0; s < a->nseg && rc == 0; ++s) {
-            const int K = a->K[s];
-            h16 *ah, *al, *wh, *wl;
-            P(dev_alloc(tmp, (void **)&ah, sizeof(h16) * (size_t)Rp * K, true));
-            P(dev_alloc(tmp, (void **)&al, sizeof(h16) * (size_t)Rp * K, true));
-            P(dev_alloc(tmp, (void **)&wh, sizeof(h16) * (size_t)a->cout * K));
-            P(dev_alloc(tmp, (void **)&wl, sizeof(h16) * (size_t)a->cout * K));
-            P(launch_split_f32(a->A[s], ah, al, (int64_t)a->R * K, st));
-            P(launch_split_f32(a->W[s], wh, wl, (int64_t)a->cout * K, st));
-            // the maps make_view and pack_conv_seg build: 64 k x 128 rows, 64 k x tile width (half of it per CTA of a pair)
-            P(make_tmap_2d(&tm[s][0], ah, K, Rp, K, 64, 128));
-            P(make_tmap_2d(&tm[s][1], al, K, Rp, K, 64, 128));
-            P(make_tmap_2d(&tm[s][2], wh, K, a->cout, K, 64, pair ? g.bn / 2 : g.bn));
-            P(make_tmap_2d(&tm[s][3], wl, K, a->cout, K, 64, pair ? g.bn / 2 : g.bn));
-            g.K[s] = K;
-            g.A[s].hi = ah; g.A[s].lo = al; g.A[s].ld = K; g.A[s].tm_hi = &tm[s][0]; g.A[s].tm_lo = &tm[s][1];
-            g.W[s].hi = wh; g.W[s].lo = wl; g.W[s].ld = K; g.W[s].tm_hi = &tm[s][2]; g.W[s].tm_lo = &tm[s][3];
-        }
+        g.bn = (a->core == 1 && a->force_bn) ? a->force_bn
+               : tile_width(a->cout, a->core <= 1 ? TC_MAX_BN : a->core == 4 ? gemm_pair_max_bn() : gemm_ws_max_bn());
+        CUtensorMap tm[2][4];
+        for (int s = 0; s < a->nseg && rc == 0; ++s) P(debug_operands(g, s, a->A[s], a->W[s], a->K[s], pair, tm[s], tmp, st));
         if (rc) break;
         float *bias = const_cast<float *>(a->bias);
         if (!bias) P(dev_alloc(tmp, (void **)&bias, sizeof(float) * a->cout, true));
@@ -2298,35 +2283,23 @@ extern "C" int lbic_debug_gemm_bench(lbic_model *m, int R, int K, int cout, int 
     do {
 #define P(call) if ((rc = (call)) != 0) break
         const int Rp = (R + 127) / 128 * 128;
-        h16 *ah, *al, *wh, *wl, *oh, *ol;
+        h16 *oh, *ol;
         float *A, *W, *D, *bias;
         P(dev_alloc(tmp, (void **)&A, sizeof(float) * (size_t)Rp * K, true));
         P(dev_alloc(tmp, (void **)&W, sizeof(float) * (size_t)cout * K, true));
         P(dev_alloc(tmp, (void **)&D, sizeof(float) * (size_t)Rp * cout, true));
         P(dev_alloc(tmp, (void **)&bias, sizeof(float) * cout, true));
-        P(dev_alloc(tmp, (void **)&ah, sizeof(h16) * (size_t)Rp * K, true));
-        P(dev_alloc(tmp, (void **)&al, sizeof(h16) * (size_t)Rp * K, true));
-        P(dev_alloc(tmp, (void **)&wh, sizeof(h16) * (size_t)cout * K, true));
-        P(dev_alloc(tmp, (void **)&wl, sizeof(h16) * (size_t)cout * K, true));
         P(dev_alloc(tmp, (void **)&oh, sizeof(h16) * (size_t)Rp * cout, true));
         P(dev_alloc(tmp, (void **)&ol, sizeof(h16) * (size_t)Rp * cout, true));
         GemmCall g;
         memset(&g, 0, sizeof(g));
         const bool ws = m->use_ws == 2;
         const int pair = ws && m->use_pair;
-        g.R = R; g.cout = cout; g.bn = m->force_bn ? m->force_bn : pick_bn(cout); g.nseg = 1; g.K[0] = K;
-        if (ws && !m->force_bn) {
-            const int wmax = (pair && m->use_pair == 3) ? gemm_pair_max_bn() : gemm_ws_max_bn();
-            const int nt = (cout + wmax - 1) / wmax;
-            g.bn = ((cout + nt - 1) / nt + 15) / 16 * 16;
-        }
-        CUtensorMap ta_h, ta_l, tw_h, tw_l;
-        P(make_tmap_2d(&ta_h, ah, K, Rp, K, 64, 128));
-        P(make_tmap_2d(&ta_l, al, K, Rp, K, 64, 128));
-        P(make_tmap_2d(&tw_h, wh, K, cout, K, 64, pair ? g.bn / 2 : g.bn));
-        P(make_tmap_2d(&tw_l, wl, K, cout, K, 64, pair ? g.bn / 2 : g.bn));
-        g.A[0].hi = ah; g.A[0].lo = al; g.A[0].ld = K; g.A[0].tm_hi = &ta_h; g.A[0].tm_lo = &ta_l;
-        g.W[0].hi = wh; g.W[0].lo = wl; g.W[0].ld = K; g.W[0].tm_hi = &tw_h; g.W[0].tm_lo = &tw_l;
+        g.R = R; g.cout = cout; g.nseg = 1;
+        g.bn = m->force_bn ? m->force_bn
+                           : tile_width(cout, !ws ? TC_MAX_BN : (pair && m->use_pair == 3) ? gemm_pair_max_bn() : gemm_ws_max_bn());
+        CUtensorMap tm[4];
+        P(debug_operands(g, 0, A, W, K, pair, tm, tmp, st));
         g.ep.R = R; g.ep.cout = cout; g.ep.acc_scale = 1.0f;
         // with_epilogue: 0 RAW, 1 PREGDN, 2 GDN, 3 QUANT, 4 LRELU, 5 KSI, 6 RECON  (synthetic operands; row r = block r)
         g.ep.bias = bias; g.ep.scale_tab = m->tables.d_scale_table;

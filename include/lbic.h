@@ -72,7 +72,7 @@ typedef struct {
 #define LBIC_OPT_WAVE_MAX_ROWS 16  /* default 1536, at most 4096 */
 #define LBIC_OPT_WAVE_DEC_MAX_ROWS 18 /* decode calls take the wave kernel up to this many rows per step (default 64): its rANS tiles run one warp per row on 8 entropy CTAs that keep the CDF tables in shared memory */
 #define LBIC_OPT_WAVE_BN 19        /* tuning hook: forced tile width of the wave kernel (32, 64, 128); 0 = 32 */
-#define LBIC_OPT_HOST_BANDS 14     /* the *_host entry points move a batch in / out in this many bands of block rows, overlapped with the wavefront (1..16, default 16; 1 = copy, compute, copy) */
+#define LBIC_OPT_HOST_BANDS 14     /* the equal-size *_host entry points move a batch in / out in this many bands of block rows, overlapped with the wavefront (1..16, default 16; 1 = copy, compute, copy) */
 #define LBIC_OPT_WS 6          /* 1 (default) = persistent warp-specialised kernel for steps with >= 2 tiles per SM */
 #define LBIC_OPT_PDL 7         /* 1 (default) = programmatic dependent launch between consecutive GEMM kernels (process-wide) */
 #define LBIC_OPT_FORCE_BN 3    /* tuning hook: force the GEMM tile width (multiple of 16, <= 256); 0 = automatic */
@@ -187,6 +187,23 @@ int lbic_encode_images_u8_host(lbic_model *m, const uint8_t *img, int n_img, int
                                uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes);
 int lbic_decode_images_u8_host(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                                int n_img, int H, int W, uint8_t *img_out, int lanes);
+
+/* The same two calls for n_img 8-bit images of DIFFERENT sizes, one wavefront call as lbic_encode_mixed /
+ * lbic_decode_mixed.  H, W: host arrays of per-image pixel sizes.  img, recon_out, img_out: host memory, packed: image i
+ * starts at byte 3 * sum_{j<i} H_j W_j and is (3, H_i, W_i) within (the planar layout of the equal-size calls).  Streams
+ * as lbic_encode_mixed: slot i at i * stream_cap, one stream_len per image.  Every image comes out exactly as
+ * lbic_encode_images_u8_host / lbic_decode_images_u8_host code it alone (same stream bytes and lengths, same 8-bit
+ * images).  The batch moves in one copy each way (copy, compute, copy; LBIC_OPT_HOST_BANDS does not apply): per-image
+ * bands of block rows measured no faster on a B200 (profiles/r3_mixed_u8_*_banded.json).  LBIC_ERR_INVALID for
+ * n_img < 1, NULL size arrays, a size < 1, lanes outside {0, 1}, stream_cap % 4, a stream_len > stream_cap (decode),
+ * a batch beyond lbic_encode_mixed's block limit or a byte total beyond size_t; LBIC_ERR_OVERFLOW / LBIC_ERR_INVALID
+ * for an overflowing stream buffer / a malformed lane container, as the equal-size calls.  The calls synchronise. */
+int lbic_encode_images_u8_host_mixed(lbic_model *m, const uint8_t *img, int n_img, const int *H, const int *W,
+                                     uint8_t *recon_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
+                                     int lanes);
+int lbic_decode_images_u8_host_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len,
+                                     size_t stream_cap, int n_img, const int *H, const int *W, uint8_t *img_out,
+                                     int lanes);
 
 /* The quality figures eval_model logs (AGENT:611-619), computed on the device: per-image MSE of x vs y ((n, C, H, W)
  * fp32 device tensors; PSNR = -10 log10(mse) for the unit-range images the agent compares) and, if msssim_out != NULL,

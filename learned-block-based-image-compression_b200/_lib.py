@@ -71,6 +71,8 @@ PROTOTYPES = {
     "lbic_check_errors": (_i, [_vp, _vp]),
     "lbic_encode_images_u8_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp, _i]),
     "lbic_decode_images_u8_host": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _vp, _i]),
+    "lbic_encode_images_u8_host_mixed": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp, _i]),
+    "lbic_decode_images_u8_host_mixed": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _vp, _vp, _i]),
     "lbic_image_metrics": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp]),
     "lbic_load_postpm_weights": (_i, [_vp, ctypes.POINTER(LbicTensorDesc), _i, _vp]),
     "lbic_postprocess": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp]),

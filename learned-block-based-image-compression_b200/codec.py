@@ -210,10 +210,51 @@ class ImageCodec:
             return self.encode(np.asarray(im.convert("RGB")))
 
     def decode_to_file(self, blob: bytes, path: str):
+        """Writes the decoded image as a PNG, quantised with round-half-to-even (`(x * 255).round()`).  decode_to_files
+        quantises as save_image does (`floor(255 x + 0.5)`), so the two can differ in a pixel that lands exactly on .5."""
         from PIL import Image
         rec = self.decode(blob)[0]
         arr = (rec * 255.0).round().clamp_(0, 255).to(torch.uint8).permute(1, 2, 0).cpu().numpy()
         Image.fromarray(arr, "RGB").save(path)
+
+    def encode_files(self, paths) -> list:
+        """Image files of any sizes -> one container per file, in one mixed-size 8-bit call (the HWC -> CHW transpose
+        happens while the images are packed for the copy).  Each container equals `encode_file` of that path."""
+        from PIL import Image
+        arrs = []
+        for p in paths:
+            with Image.open(p) as im:
+                arrs.append(np.asarray(im.convert("RGB")))
+        if not arrs:
+            return []
+        payloads = self.model._compress_u8_mixed(arrs, True, lanes=1 if self.lanes == 1 else 0)[0]
+        return [pack_container(p, H=int(a.shape[0]), W=int(a.shape[1]), B=self.B, KS=self.KS, N=self.N, M=self.M,
+                               lanes=self.lanes) for p, a in zip(payloads, arrs)]
+
+    def decode_to_files(self, blobs, paths):
+        """Containers -> PNG files, in one mixed-size 8-bit call.  The 8-bit quantisation is save_image's
+        (`floor(255 x + 0.5)`, what the reference saves, AGENT:628); decode_to_file rounds half to even, so the two can
+        differ in a pixel that lands exactly on .5.  All containers must have been written with the same `lanes` and by
+        this model's configuration (ValueError otherwise)."""
+        from PIL import Image
+        blobs, paths = list(blobs), list(paths)
+        if len(blobs) != len(paths):
+            raise ValueError("blobs / paths mismatch")
+        metas, payloads = [], []
+        for blob in blobs:
+            meta, payload = unpack_container(blob)
+            if (meta["B"], meta["KS"], meta["N"], meta["M"]) != (self.B, self.KS, self.N, self.M):
+                raise ValueError(f"container was written by a different model configuration: {meta}")
+            metas.append(meta)
+            payloads.append(payload)
+        if len({m["lanes"] for m in metas}) > 1:
+            raise ValueError("decode_to_files needs containers of one lanes setting")
+        if not metas:
+            return
+        imgs = self.model.decompress_images_u8_mixed(payloads, [(m["H"], m["W"]) for m in metas],
+                                                     lanes=1 if metas[0]["lanes"] == 1 else 0)
+        for img, path in zip(imgs, paths):
+            Image.fromarray(np.ascontiguousarray(img.transpose(1, 2, 0)), "RGB").save(path)
 
     def _as_tensor(self, img) -> torch.Tensor:
         if isinstance(img, np.ndarray):

@@ -757,9 +757,17 @@ int run_range(lbic_model *m, int l0, int l1, const StepRows &rows, bool syms, cu
 struct MixedPlan {
     int n_img = 0, s_first = 0, s_last = 0;
     bool raster = false;
-    int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0, n_lanes = 0, max_lanes = 0;
+    int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0, n_lanes = 0, max_lanes = 0, max_hb = 0;
     int64_t min_seg = 0;
     std::vector<int> row0, ext0, lane0;
+    // per step k: the largest block row of x it reads, and the block rows final in every image after it (an image with
+    // fewer rows counts once all of its rows are final) -- what the host hooks of run_steps are told
+    std::vector<int> x_hi, done;
+    // 8-bit host calls: pixel sizes and plane offsets per image, and the work-item spans of the conversions (BandPipe)
+    std::vector<MixedPix> pix;
+    std::vector<MixedSpan> spans;
+    const MixedPix *d_pix = nullptr;
+    const MixedSpan *d_span = nullptr;
     std::vector<int64_t> seg;           // encode: symbols of stream s = [seg[s], seg[s+1]) in packed order
     std::vector<int4> img, rows, ext;
     std::vector<int> sched, blk_img, g0row, stream;
@@ -789,6 +797,7 @@ void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster,
         p.max_lanes = L > p.max_lanes ? L : p.max_lanes;
         const int last = step_count(raster, Hb[i], Wb[i]);
         p.s_last = last > p.s_last ? last : p.s_last;
+        p.max_hb = Hb[i] > p.max_hb ? Hb[i] : p.max_hb;
     }
     p.n_lanes = p.lane0[n];
     p.s_first = raster ? 0 : (k3 ? -1 : 0);
@@ -810,15 +819,23 @@ void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster,
     for (int s = p.s_first; s < p.s_last; ++s) {
         p.ext0.push_back(p.n_ext);
         p.row0.push_back((int)p.rows.size());
+        int x_hi = -1, done = p.max_hb;
         for (int i = 0; i < n; ++i) {
+            // block rows of image i final after step s (the closed forms of run_steps' equal-size calls)
+            const int d = raster ? (s + 1) / Wb[i] : (s >= Wb[i] - 1 ? (s - (Wb[i] - 1)) / 2 + 1 : 0);
+            if (d < Hb[i]) done = d < done ? d : done;
             if (s >= step_count(raster, Hb[i], Wb[i])) continue;
             StepDesc e[3];
             const int n_ring = k3 ? ring_steps(s, raster, 1, Hb[i], Wb[i], e) : 0;
             for (int j = 0; j < n_ring; ++j)
                 for (int v = e[j].vmin; v < e[j].vmin + e[j].nv; ++v) add_ext(i, v, e[j].t - 2 * v);
-            if (step_desc(s, raster, 1, Hb[i], Wb[i], e[0]))
+            if (step_desc(s, raster, 1, Hb[i], Wb[i], e[0])) {
                 for (int v = e[0].vmin; v < e[0].vmin + e[0].nv; ++v) add_row(i, v, e[0].t - 2 * v);
+                x_hi = e[0].vmin + e[0].nv - 1 > x_hi ? e[0].vmin + e[0].nv - 1 : x_hi;
+            }
         }
+        p.x_hi.push_back(x_hi);
+        p.done.push_back(done);
         const int k = (int)p.row0.size() - 1;
         const int R = (int)p.rows.size() - p.row0[k], Re = p.n_ext - p.ext0[k];
         p.max_rows = R > p.max_rows ? R : p.max_rows;
@@ -858,6 +875,8 @@ int upload_mixed(lbic_model *m, MixedPlan &p, cudaStream_t st) {
     add(p.stream.data(), sizeof(int) * p.stream.size());
     add(p.lane0.data(), sizeof(int) * p.lane0.size());
     add(p.seg.data(), sizeof(int64_t) * p.seg.size());
+    add(p.pix.data(), sizeof(MixedPix) * p.pix.size());
+    add(p.spans.data(), sizeof(MixedSpan) * p.spans.size());
     if (m->mix_dev_bytes < off) {
         if (m->mix_dev) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->mix_dev); m->mix_dev = nullptr; m->mix_dev_bytes = 0; }
         cudaError_t e = cudaMalloc(&m->mix_dev, off);
@@ -878,6 +897,8 @@ int upload_mixed(lbic_model *m, MixedPlan &p, cudaStream_t st) {
     p.geo.stream = (const int *)(d + at[6]);
     p.d_lane0 = (const int *)(d + at[7]);
     p.d_seg = (const int64_t *)(d + at[8]);
+    p.d_pix = (const MixedPix *)(d + at[9]);
+    p.d_span = (const MixedSpan *)(d + at[10]);
     return 0;
 }
 
@@ -907,6 +928,20 @@ struct CallSteps {
         const int n = k3 ? ring_steps(s, raster, n_img, Hb, Wb, e) : 0;
         for (int j = 0; j < n; ++j) ring[j] = StepRows{e[j], n_img * e[j].nv};
         return n;
+    }
+    // the largest block row of x that step s (rows `sd`, from at) reads
+    int x_row_hi(int s, const StepDesc &sd) const { return plan ? plan->x_hi[s - first] : sd.vmin + sd.nv - 1; }
+    // block rows of zhat final in every image after step s (0: none new to report)
+    int rows_final(int s) const {
+        if (plan) return plan->done[s - first];
+        int done = 0;
+        if (raster) {
+            if ((s + 1) % Wb == 0) done = (s + 1) / Wb;
+        } else if (s >= Wb - 1) {
+            done = (s - (Wb - 1)) / 2 + 1;
+            done = done < Hb ? done : Hb;
+        }
+        return done;
     }
 };
 
@@ -984,6 +1019,8 @@ struct RowHooks {
     // launch where a hook has work to put between two steps)
     bool (*will_need)(void *ctx, int v_hi) = nullptr;
     bool (*will_done)(void *ctx, int v_done) = nullptr;
+    // mixed-size calls: adds the hooks' tables to the step schedule before its upload (and keeps the plan for the hooks)
+    void (*add_to_plan)(void *ctx, MixedPlan &p) = nullptr;
 };
 
 // The persistent wavefront kernel (gemm_wave.cu) takes over when every step of the call has at most wave_max_rows rows.
@@ -1071,12 +1108,11 @@ int decode_step(lbic_model *m, const StepRows &rows, int lanes, int32_t *sym, cu
 // The step loop of an encode or a decode.  Each step runs through `step(rows)` (per-layer or dataflow launches) after
 // the hidden-map ring positions (KS[1] == 3) that become computable with it, or, when `wave` (small steps: single images,
 // small batches), consecutive steps are collected into ONE launch of the persistent wavefront kernel, `wave_range(s0,
-// s1)`, cut only where a host hook has copies or conversions to put between two steps.  (Mixed-size calls have no hooks
-// and no wavefront kernel.)
+// s1)`, cut only where a host hook has copies or conversions to put between two steps.  (Mixed-size calls take no
+// wavefront kernel.)
 template <class Step, class WaveRange>
 int run_steps(lbic_model *m, const CallSteps &cs, bool wave, const RowHooks *hk, Step step, WaveRange wave_range,
               cudaStream_t st) {
-    const int Hb = cs.Hb, Wb = cs.Wb;
     auto launch_step = [&](int s) -> int {
         StepRows rows, ring[3];
         const int n_ring = cs.at(s, rows, ring);
@@ -1101,7 +1137,7 @@ int run_steps(lbic_model *m, const CallSteps &cs, bool wave, const RowHooks *hk,
         const StepDesc &sd = rows.sd;
         const bool has = rows.R > 0;
         if (has && hk && hk->need_rows) {
-            const int v_hi = sd.vmin + sd.nv - 1;
+            const int v_hi = cs.x_row_hi(s, sd);
             if (!wave || !hk->will_need || hk->will_need(hk->ctx, v_hi)) {
                 LBIC_TRY(flush(s));
                 LBIC_TRY(hk->need_rows(hk->ctx, v_hi, st));
@@ -1113,13 +1149,7 @@ int run_steps(lbic_model *m, const CallSteps &cs, bool wave, const RowHooks *hk,
             LBIC_TRY(launch_step(s));                // (wave: step -1 of KS[1] = 3 is one small GEMM on the per-layer path)
         }
         if (has && hk && hk->rows_done) {
-            int done = 0;                            // zhat block rows [0, done) are final after step s
-            if (cs.raster) {
-                if ((s + 1) % Wb == 0) done = (s + 1) / Wb;
-            } else if (s >= Wb - 1) {
-                done = (s - (Wb - 1)) / 2 + 1;
-                done = done < Hb ? done : Hb;
-            }
+            const int done = cs.rows_final(s);       // zhat block rows [0, done) are final after step s
             if (done > 0 && (!wave || !hk->will_done || hk->will_done(hk->ctx, done))) {
                 LBIC_TRY(flush(s + 1));
                 LBIC_TRY(hk->rows_done(hk->ctx, done, st));
@@ -1181,9 +1211,10 @@ int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_le
                 int Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st, const RowHooks *hk);
 int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
                       int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
-                      int lanes, cudaStream_t st);
+                      int lanes, cudaStream_t st, const RowHooks *hk);
 int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
-                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st);
+                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st,
+                      const RowHooks *hk);
 
 }  // namespace
 
@@ -1573,14 +1604,14 @@ extern "C" int lbic_encode_mixed(lbic_model *m, const float *x, int n_img, const
                                  int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap,
                                  uint32_t *stream_len, int lanes, void *stream) {
     return encode_mixed_impl(m, x, n_img, Hb, Wb, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, lanes,
-                             (cudaStream_t)stream);
+                             (cudaStream_t)stream, nullptr);
 }
 
 extern "C" int lbic_decode_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                                  int n_img, const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes,
                                  void *stream) {
     return decode_mixed_impl(m, streams, stream_len, stream_cap, n_img, Hb, Wb, zhat_out, sym_out, lanes,
-                             (cudaStream_t)stream);
+                             (cudaStream_t)stream, nullptr);
 }
 
 // Synchronises `stream` and reports what the kernels enqueued on it flagged since the last encode / decode started:
@@ -1642,8 +1673,9 @@ WsNeed mixed_need(const lbic_model *m, const MixedPlan &p) {
 }
 
 int mixed_begin(lbic_model *m, int n_img, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p,
-                cudaStream_t st) {
+                cudaStream_t st, const RowHooks *hk) {
     plan_mixed(m, n_img, Hb, Wb, raster, lanes, p);
+    if (hk && hk->add_to_plan) hk->add_to_plan(hk->ctx, p);
     LBIC_TRY(ensure_workspace_mixed(m, mixed_need(m, p)));
     LBIC_TRY(call_begin(m, p.nblk, st));
     LBIC_TRY(upload_mixed(m, p, st));
@@ -1654,21 +1686,21 @@ int mixed_begin(lbic_model *m, int n_img, const int *Hb, const int *Wb, bool ras
 
 int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
                       int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
-                      int lanes, cudaStream_t st) {
+                      int lanes, cudaStream_t st, const RowHooks *hk) {
     LBIC_TRY(check_ready(m, stream_out != nullptr));
-    if (!x) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    if (!x && !(hk && hk->need_rows)) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
     LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
     if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
     Active act(m);
     MixedPlan p;
-    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, false, lanes, p, st));
+    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, false, lanes, p, st, hk));
     Workspace &ws = m->ws;
     const size_t nblk = p.nblk;
-    LBIC_TRY(launch_nchw_to_cl_mixed(x, ws.x_cl, m->Cin, p.geo, p.nblk, st));
+    if (x) LBIC_TRY(launch_nchw_to_cl_mixed(x, ws.x_cl, m->Cin, p.geo, p.nblk, st));
     const bool want_syms = sym_out || idx_out || stream_out;
     auto step = [&](const StepRows &rows) { return encode_step(m, rows, want_syms, st); };
     auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, call_steps(m, p), false, nullptr, step, no_wave, st));
+    LBIC_TRY(run_steps(m, call_steps(m, p), false, hk, step, no_wave, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
     if (!want_syms) return ws_release(m, st);
     // symbols and indexes in packed order: into the caller's arrays, or (streams only) a model buffer
@@ -1703,7 +1735,8 @@ int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, c
 }
 
 int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
-                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st) {
+                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st,
+                      const RowHooks *hk) {
     LBIC_TRY(check_ready(m, true));
     if (!streams || !stream_len) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
     LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
@@ -1711,14 +1744,14 @@ int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *str
     Active act(m);
     MixedPlan p;
     const bool raster = lanes == 1;   // reference container: raster order, one block of every image per step
-    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, raster, lanes, p, st));
+    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, raster, lanes, p, st, hk));
     Workspace &ws = m->ws;
     LBIC_TRY(launch_rans_dec_init_mixed(streams, stream_len, stream_cap, n_img, p.d_lane0, p.n_lanes, lanes != 1,
                                         ws.dec_states, ws.lane_ptr, m->err_flag, st));
     int32_t *sym = sym_out ? ws.sym : nullptr;
     auto step = [&](const StepRows &rows) { return decode_step(m, rows, 0, sym, st); };
     auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, call_steps(m, p), false, nullptr, step, no_wave, st));
+    LBIC_TRY(run_steps(m, call_steps(m, p), false, hk, step, no_wave, st));
     if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
     if (sym_out) LBIC_TRY(launch_unschedule_i32(ws.sym, sym_out, m->M, p.geo, p.nblk, st));
     return ws_release(m, st);
@@ -1757,6 +1790,14 @@ struct BandPipe {
     int H = 0, W = 0, B = 0;                      // fmt 1
     const uint8_t *h_in = nullptr; uint8_t *d_in = nullptr;
     uint8_t *h_out = nullptr; uint8_t *d_out = nullptr;
+    // mixed-size u8 call: per-image pixel sizes and plane offsets.  It moves in ONE band (copy, compute, copy): on a
+    // B200 host_bands 16 measured no faster than 1 for mixed batches (profiles/r3_mixed_u8_*.json), so the per-image
+    // band copies were not kept.  The plan's spans are the n images for the input conversion (tin work items), then
+    // the n images again for the output conversion (tout).
+    const int *Hs = nullptr, *Ws = nullptr, *Hbs = nullptr;
+    std::vector<size_t> off;
+    const MixedPlan *mp = nullptr;
+    long long tin = 0, tout = 0;
     int rc = 0;
 
     void plan(lbic_model *model, int n_img, int hb, int wb) {
@@ -1764,22 +1805,56 @@ struct BandPipe {
         nb = hb < m->host_bands ? hb : m->host_bands;
         for (int b = 0; b <= nb; ++b) vb[b] = (int)((long)hb * b / nb);
     }
+    void plan_mixed(lbic_model *model, int n_img, const int *h, const int *w, const int *hb) {
+        int max_hb = 0;
+        Hs = h; Ws = w; Hbs = hb;
+        off.assign(n_img + 1, 0);
+        for (int i = 0; i < n_img; ++i) {
+            max_hb = hb[i] > max_hb ? hb[i] : max_hb;
+            off[i + 1] = off[i] + (size_t)3 * h[i] * w[i];
+        }
+        m = model; n = n_img; Hb = max_hb;
+        nb = 1; vb[0] = 0; vb[1] = max_hb;
+    }
+    static void add_to_plan(void *ctx, MixedPlan &p) {
+        BandPipe *q = (BandPipe *)ctx;
+        q->mp = &p;
+        for (int i = 0; i < q->n; ++i) p.pix.push_back(MixedPix{q->Hs[i], q->Ws[i], (long long)q->off[i]});
+        q->tin = q->tout = 0;
+        for (int i = 0; i < q->n; ++i) {              // padded pixels of the image
+            p.spans.push_back(MixedSpan{q->tin, i, 0});
+            q->tin += (long long)q->Hbs[i] * q->B * ((q->Ws[i] + q->B - 1) / q->B) * q->B;
+        }
+        for (int i = 0; i < q->n; ++i) {              // quads of output pixels of the image
+            p.spans.push_back(MixedSpan{q->tout, i, 0});
+            q->tout += (long long)q->Hs[i] * ((q->Ws[i] + 3) / 4);
+        }
+    }
     // plane geometry of a band for the 2-D copies: `planes` rows of `pitch` bytes, the band is bytes [off, off + width)
-    void geom(int b, size_t &planes, size_t &pitch, size_t &off, size_t &width) const {
+    void geom(int b, size_t &planes, size_t &pitch, size_t &o, size_t &width) const {
         if (fmt == 0) {
             planes = (size_t)n * m->Cin; pitch = sizeof(float) * (size_t)Hb * Wb;
-            off = sizeof(float) * (size_t)vb[b] * Wb; width = sizeof(float) * (size_t)(vb[b + 1] - vb[b]) * Wb;
+            o = sizeof(float) * (size_t)vb[b] * Wb; width = sizeof(float) * (size_t)(vb[b + 1] - vb[b]) * Wb;
         } else {
             const int y0 = vb[b] * B, y1 = vb[b + 1] * B < H ? vb[b + 1] * B : H;
             planes = (size_t)n * 3; pitch = (size_t)H * W;
-            off = (size_t)y0 * W; width = y1 > y0 ? (size_t)(y1 - y0) * W : 0;
+            o = (size_t)y0 * W; width = y1 > y0 ? (size_t)(y1 - y0) * W : 0;
         }
+    }
+    // band b between host and device: one 2-D copy, or (mixed, one band) the packed images in one copy
+    int copy(int b, uint8_t *dst, const uint8_t *src, cudaMemcpyKind kind, cudaStream_t st) const {
+        if (Hs) {
+            LBIC_CUDA(cudaMemcpyAsync(dst, src, off[n], kind, st));
+            return 0;
+        }
+        size_t planes, pitch, o, width;
+        geom(b, planes, pitch, o, width);
+        if (width) LBIC_CUDA(cudaMemcpy2DAsync(dst + o, pitch, src + o, pitch, width, planes, kind, st));
+        return 0;
     }
     int queue_inputs() {
         for (int b = 0; b < nb; ++b) {
-            size_t planes, pitch, off, width;
-            geom(b, planes, pitch, off, width);
-            if (width) LBIC_CUDA(cudaMemcpy2DAsync(d_in + off, pitch, h_in + off, pitch, width, planes, cudaMemcpyHostToDevice, m->hs[0]));
+            LBIC_TRY(copy(b, d_in, h_in, cudaMemcpyHostToDevice, m->hs[0]));
             LBIC_CUDA(cudaEventRecord(m->hev[b], m->hs[0]));
         }
         return 0;
@@ -1797,7 +1872,10 @@ struct BandPipe {
         while (p->next_in < p->nb && p->vb[p->next_in] <= v_hi) {
             const int b = p->next_in++;
             LBIC_CUDA(cudaStreamWaitEvent(st, p->m->hev[b], 0));
-            if (p->fmt == 0)
+            if (p->mp)
+                LBIC_TRY(launch_u8_to_xcl_mixed(p->d_in, p->m->ws.x_cl, p->mp->geo, p->mp->d_pix, p->mp->d_span, p->n,
+                                                p->tin, p->B, st));
+            else if (p->fmt == 0)
                 LBIC_TRY(launch_nchw_to_cl_band((const float *)p->d_in, p->m->ws.x_cl, p->n, p->m->Cin, p->Hb, p->Wb, p->vb[b], p->vb[b + 1], st));
             else
                 LBIC_TRY(launch_u8_to_xcl(p->d_in, p->m->ws.x_cl, p->n, p->H, p->W, p->Hb, p->Wb, p->B, p->vb[b], p->vb[b + 1], st));
@@ -1808,46 +1886,55 @@ struct BandPipe {
         BandPipe *p = (BandPipe *)ctx;
         while (p->next_out < p->nb && p->vb[p->next_out + 1] <= v_done) {
             const int b = p->next_out++;
-            if (p->fmt == 0)
+            if (p->mp)
+                LBIC_TRY(launch_zcl_to_u8_mixed(p->m->ws.zhat_cl, p->d_out, p->mp->geo, p->mp->d_pix, p->mp->d_span + p->n,
+                                                p->n, p->tout, p->B, st));
+            else if (p->fmt == 0)
                 LBIC_TRY(launch_cl_to_nchw_band(p->m->ws.zhat_cl, (float *)p->d_out, p->n, p->m->Cin, p->Hb, p->Wb, p->vb[b], p->vb[b + 1], st));
             else
                 LBIC_TRY(launch_zcl_to_u8(p->m->ws.zhat_cl, p->d_out, p->n, p->H, p->W, p->Hb, p->Wb, p->B, p->vb[b], p->vb[b + 1], st));
             LBIC_CUDA(cudaEventRecord(p->m->hev[LBIC_MAX_BANDS + b], st));
             LBIC_CUDA(cudaStreamWaitEvent(p->m->hs[2], p->m->hev[LBIC_MAX_BANDS + b], 0));
-            size_t planes, pitch, off, width;
-            p->geom(b, planes, pitch, off, width);
-            if (width) LBIC_CUDA(cudaMemcpy2DAsync(p->h_out + off, pitch, p->d_out + off, pitch, width, planes, cudaMemcpyDeviceToHost, p->m->hs[2]));
+            LBIC_TRY(p->copy(b, p->h_out, p->d_out, cudaMemcpyDeviceToHost, p->m->hs[2]));
         }
         return 0;
     }
 };
 
-// fmt 0: x / zhat are fp32 (n, 3B^2, Hb, Wb) block tensors; fmt 1: 8-bit (n, 3, H, W) images (pad / crop fused)
+// fmt 0: x / zhat are fp32 (n, 3B^2, Hb, Wb) block tensors; fmt 1: 8-bit (n, 3, H, W) images (pad / crop fused), or
+// with Hv / Wv (mixed-size u8 call) the packed 8-bit images of pixel sizes Hv[i] x Wv[i] and block grids Hb[i] x Wb[i]
+// (Hbv / Wbv), `in_bytes` in all
 int encode_host_impl(lbic_model *m, int fmt, const void *in, int n_img, int H, int W, int Hb, int Wb, void *recon_out,
-                     uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes) {
+                     uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
+                     const int *Hv = nullptr, const int *Wv = nullptr, const int *Hbv = nullptr, const int *Wbv = nullptr,
+                     size_t in_bytes = 0) {
     LBIC_TRY(check_ready(m, stream_out != nullptr));
-    if (!in || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    if (!in || n_img < 1 || (!Hv && (Hb < 1 || Wb < 1))) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
     if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
     Active act(m);
     LBIC_TRY(host_pipeline_init(m));
-    const size_t nin = fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
+    const size_t nin = Hv ? in_bytes : fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
     const size_t o_in = 0, o_out = align256(nin), o_len = o_out + (recon_out ? align256(nin) : 0),
                  o_s = o_len + align256(4 * (size_t)n_img);
     LBIC_TRY(ensure_io(m, o_s + (stream_out ? (size_t)n_img * stream_cap : 0)));
-    LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
+    if (!Hv) LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
     uint8_t *io = (uint8_t *)m->io_dev;
     cudaStream_t s_cmp = m->hs[1], s_out = m->hs[2];
     BandPipe bp;
-    bp.plan(m, n_img, Hb, Wb);
     bp.fmt = fmt; bp.H = H; bp.W = W; bp.B = m->cfg.block_size;
+    if (Hv) bp.plan_mixed(m, n_img, Hv, Wv, Hbv);
+    else bp.plan(m, n_img, Hb, Wb);
     bp.h_in = (const uint8_t *)in; bp.d_in = io + o_in;
     bp.h_out = (uint8_t *)recon_out; bp.d_out = io + o_out;
     LBIC_TRY(bp.queue_inputs());
     RowHooks hk;
     hk.ctx = &bp; hk.need_rows = BandPipe::need_rows; hk.rows_done = recon_out ? BandPipe::rows_done : nullptr;
     hk.will_need = BandPipe::will_need; hk.will_done = BandPipe::will_done;
-    int rc = encode_impl(m, nullptr, n_img, Hb, Wb, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr, stream_cap,
-                         (uint32_t *)(io + o_len), lanes, s_cmp, &hk);
+    if (Hv) hk.add_to_plan = BandPipe::add_to_plan;
+    int rc = Hv ? encode_mixed_impl(m, nullptr, n_img, Hbv, Wbv, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr,
+                                    stream_cap, (uint32_t *)(io + o_len), lanes, s_cmp, &hk)
+                : encode_impl(m, nullptr, n_img, Hb, Wb, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr, stream_cap,
+                              (uint32_t *)(io + o_len), lanes, s_cmp, &hk);
     if (rc == 0 && stream_out && cudaMemcpyAsync(stream_len, io + o_len, 4 * (size_t)n_img, cudaMemcpyDeviceToHost, s_cmp) != cudaSuccess)
         rc = lbic_fail(LBIC_ERR_CUDA, "copy failed");
     cudaError_t e0 = cudaStreamSynchronize(m->hs[0]), e1 = cudaStreamSynchronize(s_cmp);
@@ -1869,38 +1956,64 @@ int encode_host_impl(lbic_model *m, int fmt, const void *in, int n_img, int H, i
 }
 
 int decode_host_impl(lbic_model *m, int fmt, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
-                     int n_img, int H, int W, int Hb, int Wb, void *out, int lanes) {
+                     int n_img, int H, int W, int Hb, int Wb, void *out, int lanes, const int *Hv = nullptr,
+                     const int *Wv = nullptr, const int *Hbv = nullptr, const int *Wbv = nullptr, size_t out_bytes = 0) {
     LBIC_TRY(check_ready(m, true));
-    if (!streams || !stream_len || !out || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "null argument");
+    if (!streams || !stream_len || !out || n_img < 1 || (!Hv && (Hb < 1 || Wb < 1))) return lbic_fail(LBIC_ERR_INVALID, "null argument");
     if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
     Active act(m);
     LBIC_TRY(host_pipeline_init(m));
-    const size_t nout = fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
+    const size_t nout = Hv ? out_bytes : fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
     const size_t o_out = 0, o_len = align256(nout), o_s = o_len + align256(4 * (size_t)n_img);
-    LBIC_TRY(ensure_io(m, o_s + (size_t)n_img * stream_cap));
-    LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
-    uint8_t *io = (uint8_t *)m->io_dev;
-    cudaStream_t s_cmp = m->hs[1], s_out = m->hs[2];
     size_t longest = 0;
     for (int i = 0; i < n_img; ++i) {
         if (stream_len[i] > stream_cap) return lbic_fail(LBIC_ERR_INVALID, "stream %d longer than stream_cap", i);
         longest = stream_len[i] > longest ? stream_len[i] : longest;
     }
+    LBIC_TRY(ensure_io(m, o_s + (size_t)n_img * stream_cap));
+    if (!Hv) LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
+    uint8_t *io = (uint8_t *)m->io_dev;
+    cudaStream_t s_cmp = m->hs[1], s_out = m->hs[2];
     LBIC_CUDA(cudaMemcpyAsync(io + o_len, stream_len, 4 * (size_t)n_img, cudaMemcpyHostToDevice, s_cmp));
     if (longest) LBIC_CUDA(cudaMemcpy2DAsync(io + o_s, stream_cap, streams, stream_cap, longest, n_img, cudaMemcpyHostToDevice, s_cmp));
     BandPipe bp;
-    bp.plan(m, n_img, Hb, Wb);
     bp.fmt = fmt; bp.H = H; bp.W = W; bp.B = m->cfg.block_size;
+    if (Hv) bp.plan_mixed(m, n_img, Hv, Wv, Hbv);
+    else bp.plan(m, n_img, Hb, Wb);
     bp.h_out = (uint8_t *)out; bp.d_out = io + o_out;
     RowHooks hk;
     hk.ctx = &bp; hk.rows_done = BandPipe::rows_done; hk.will_done = BandPipe::will_done;
-    int rc = decode_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hb, Wb, nullptr, nullptr, lanes,
-                         s_cmp, &hk);
+    if (Hv) hk.add_to_plan = BandPipe::add_to_plan;
+    int rc = Hv ? decode_mixed_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hbv, Wbv, nullptr,
+                                    nullptr, lanes, s_cmp, &hk)
+                : decode_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hb, Wb, nullptr, nullptr, lanes,
+                              s_cmp, &hk);
     cudaError_t e1 = cudaStreamSynchronize(s_cmp), e2 = cudaStreamSynchronize(s_out);
     if (rc) return rc;
     if (e1 != cudaSuccess || e2 != cudaSuccess)
         return lbic_fail(LBIC_ERR_CUDA, "decode failed: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
     return take_error_flag(m);
+}
+
+// Arguments of the mixed-size u8 host calls: per-image block grids and the byte total of the packed images.
+int u8_mixed_args(const lbic_model *m, int n_img, const int *H, const int *W, int lanes, std::vector<int> &Hb,
+                  std::vector<int> &Wb, size_t *bytes) {
+    if (n_img < 1 || !H || !W) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    const int B = m->cfg.block_size;
+    size_t total = 0;
+    Hb.resize(n_img); Wb.resize(n_img);
+    for (int i = 0; i < n_img; ++i) {
+        if (H[i] < 1 || W[i] < 1) return lbic_fail(LBIC_ERR_INVALID, "image %d has size %d x %d", i, H[i], W[i]);
+        size_t px = 0;
+        if (__builtin_mul_overflow((size_t)H[i], (size_t)W[i], &px) || __builtin_mul_overflow(px, (size_t)3, &px) ||
+            __builtin_add_overflow(total, px, &total))
+            return lbic_fail(LBIC_ERR_INVALID, "batch of images exceeds the address space");
+        Hb[i] = (int)(((long long)H[i] + B - 1) / B);
+        Wb[i] = (int)(((long long)W[i] + B - 1) / B);
+    }
+    LBIC_TRY(check_mixed_args(n_img, Hb.data(), Wb.data(), lanes));
+    *bytes = total;
+    return 0;
 }
 }  // namespace
 
@@ -1930,6 +2043,28 @@ extern "C" int lbic_decode_images_u8_host(lbic_model *m, const uint8_t *streams,
     const int B = m->cfg.block_size;
     return decode_host_impl(m, 1, streams, stream_len, stream_cap, n_img, H, W, (H + B - 1) / B, (W + B - 1) / B, img_out,
                             lanes);
+}
+
+extern "C" int lbic_encode_images_u8_host_mixed(lbic_model *m, const uint8_t *img, int n_img, const int *H, const int *W,
+                                                uint8_t *recon_out, uint8_t *stream_out, size_t stream_cap,
+                                                uint32_t *stream_len, int lanes) {
+    if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
+    std::vector<int> Hb, Wb;
+    size_t bytes = 0;
+    LBIC_TRY(u8_mixed_args(m, n_img, H, W, lanes, Hb, Wb, &bytes));
+    return encode_host_impl(m, 1, img, n_img, 0, 0, 0, 0, recon_out, stream_out, stream_cap, stream_len, lanes, H, W,
+                            Hb.data(), Wb.data(), bytes);
+}
+
+extern "C" int lbic_decode_images_u8_host_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len,
+                                                size_t stream_cap, int n_img, const int *H, const int *W, uint8_t *img_out,
+                                                int lanes) {
+    if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
+    std::vector<int> Hb, Wb;
+    size_t bytes = 0;
+    LBIC_TRY(u8_mixed_args(m, n_img, H, W, lanes, Hb, Wb, &bytes));
+    return decode_host_impl(m, 1, streams, stream_len, stream_cap, n_img, 0, 0, 0, 0, img_out, lanes, H, W, Hb.data(),
+                            Wb.data(), bytes);
 }
 
 // ------------------------------------------------------------------------------------------------

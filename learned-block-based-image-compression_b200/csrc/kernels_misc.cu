@@ -43,55 +43,125 @@ __global__ void space_depth_kernel(const float *__restrict__ src, float *__restr
 }
 
 // ---- 8-bit image <-> channel-last block tensors (eval_model's per-image body, AGENT:581-589 and 610-628) ---------
-// Block rows [v0, v1) of every image of the batch, so that the host wrappers can convert band by band while the rest
-// of the batch is still in flight over PCIe.
+// The kernels are templated on where an image's pixels and blocks are:
+//   U8Batch: n images of one size, block rows [v0, v1) of each, so that the host wrappers can convert band by band
+//            while the rest of the batch is still in flight over PCIe; image b's planes at b * 3HW, its blocks from
+//            b * Hb * Wb in x_cl and zhat_cl;
+//   U8Mixed: the whole images of a mixed-size call (a host list, MixedSpan), their planes at the packed byte offsets
+//            (MixedPix), x_cl in packed block order and zhat_cl in schedule order (MixedGeo).
+// Both number their work items image after image: begin_*() gives the count (and fixes what one geometry shares across
+// images), at(i) resolves item i to its image and the item within that image's part.
+struct U8Img {
+    int b, H, W;       // image, pixel size
+    int Wp, W4;        // padded width (to x_cl), quads of output pixels per row (to u8)
+    bool vec;          // (to u8) rows of whole 4-byte words
+    size_t q;          // work item within the image's part of the band
+    long long off;     // (mixed) byte offset of the image's planes
+    int P, Wb;         // (mixed) first packed block and block columns of the image
+};
+struct U8Batch {
+    int n, H, W, Hb, Wb, B, v0, v1;
+    size_t per_img;
+    int Wp, W4;
+    bool vec;
+    __device__ size_t begin_xcl() {
+        Wp = Wb * B;
+        per_img = (size_t)(v1 - v0) * B * Wp;
+        return (size_t)n * per_img;
+    }
+    __device__ size_t begin_u8() {
+        const int y0 = v0 * B, y1 = (v1 * B < H) ? v1 * B : H;
+        if (y1 <= y0) return 0;
+        W4 = (W + 3) >> 2;
+        per_img = (size_t)(y1 - y0) * W4;
+        vec = (W & 3) == 0 && (B & 3) == 0;
+        return (size_t)n * per_img;
+    }
+    __device__ U8Img at(size_t i) const {
+        U8Img p;
+        p.b = (int)(i / per_img);
+        p.q = i - (size_t)p.b * per_img;
+        p.H = H; p.W = W; p.Wp = Wp; p.W4 = W4; p.vec = vec;
+        return p;
+    }
+    __device__ size_t plane(const U8Img &p, int c, int y) const { return (((size_t)p.b * 3 + c) * H + y) * W; }
+    __device__ size_t x_block(const U8Img &p, int v, int h) const { return ((size_t)p.b * Hb + v) * Wb + h; }
+    __device__ size_t z_block(const U8Img &p, int v, int h) const { return ((size_t)p.b * Hb + v) * Wb + h; }
+};
+struct U8Mixed {
+    MixedGeo g;
+    const MixedPix *__restrict__ pix;
+    const MixedSpan *__restrict__ span;
+    int n_span, B, v0;
+    long long n_items;
+    __device__ size_t begin_xcl() const { return (size_t)n_items; }
+    __device__ size_t begin_u8() const { return (size_t)n_items; }
+    __device__ U8Img at(size_t i) const {
+        int lo = 0, hi = n_span - 1;   // the last image whose first item is <= i
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if ((size_t)span[mid].item0 <= i) lo = mid; else hi = mid - 1;
+        }
+        const MixedSpan s = span[lo];
+        const MixedPix px = pix[s.img];
+        const int4 gi = g.img[s.img];
+        U8Img p;
+        p.b = s.img; p.q = i - (size_t)s.item0;
+        p.H = px.H; p.W = px.W;
+        p.Wp = gi.y * B; p.W4 = (px.W + 3) >> 2;
+        // whole 4-byte words only where the image's planes start on one: packed offsets are 3 * sum H_j W_j
+        p.vec = (px.W & 3) == 0 && (B & 3) == 0 && (px.off & 3) == 0;
+        p.off = px.off; p.P = gi.z; p.Wb = gi.y;
+        return p;
+    }
+    __device__ size_t plane(const U8Img &p, int c, int y) const { return (size_t)p.off + ((size_t)c * p.H + y) * p.W; }
+    __device__ size_t x_block(const U8Img &p, int v, int h) const { return (size_t)p.P + v * p.Wb + h; }
+    __device__ size_t z_block(const U8Img &p, int v, int h) const { return (size_t)g.sched[p.P + v * p.Wb + h]; }
+};
+
 //   x_cl[(img, v, h)][(bv*B + bh)*3 + c] = img[c][min(v*B+bv, H-1)][min(h*B+bh, W-1)] / 255 - 0.5
 // = ToTensor() (u8 / 255 in fp32), `x - 0.5` (AGENT:581), replicate padding to a multiple of B (AGENT:583-586) and
 // arrange_block_pixels_to_channel_dim (AGENT:853-860) in one pass.  One thread per padded pixel, bh fastest.
-__global__ void u8_to_xcl_kernel(const uint8_t *__restrict__ img, float *__restrict__ x_cl, int n, int H, int W, int Hb,
-                                 int Wb, int B, int v0, int v1) {
-    const int Wp = Wb * B;
-    const size_t per_img = (size_t)(v1 - v0) * B * Wp;
-    const size_t total = (size_t)n * per_img;
+template <class Geo>
+__global__ void u8_to_xcl_kernel(const uint8_t *__restrict__ img, float *__restrict__ x_cl, Geo g) {
+    const int B = g.B, v0 = g.v0;
+    const size_t total = g.begin_xcl();
     const int Cin = 3 * B * B;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const int b = (int)(i / per_img);
-        const size_t q = i - (size_t)b * per_img;
-        const int yy = (int)(q / Wp), x = (int)(q - (size_t)yy * Wp);
+        const U8Img p = g.at(i);
+        const int yy = (int)(p.q / p.Wp), x = (int)(p.q - (size_t)yy * p.Wp);
         const int y = v0 * B + yy;
         const int v = y / B, bv = y - v * B, h = x / B, bh = x - h * B;
-        const int ys = y < H ? y : H - 1, xs = x < W ? x : W - 1;
-        const uint8_t *src = img + ((size_t)b * 3 * H + ys) * W + xs;
-        float *dst = x_cl + (((size_t)b * Hb + v) * Wb + h) * Cin + (bv * B + bh) * 3;
+        const int ys = y < p.H ? y : p.H - 1, xs = x < p.W ? x : p.W - 1;
+        const uint8_t *src = img + g.plane(p, 0, ys) + xs;
+        float *dst = x_cl + g.x_block(p, v, h) * Cin + (bv * B + bh) * 3;
 #pragma unroll
         for (int c = 0; c < 3; ++c)
-            dst[c] = __fsub_rn(__fdiv_rn((float)src[(size_t)c * H * W], 255.0f), 0.5f);
+            dst[c] = __fsub_rn(__fdiv_rn((float)src[(size_t)c * p.H * p.W], 255.0f), 0.5f);
     }
 }
 
 // out[c][y][x] = uint8(clamp((z + 0.5) * 255 + 0.5, 0, 255)) for y < H, x < W: arrange_channel_dim_to_block_pixels
 // (AGENT:863-873), the crop of the padding, `+ 0.5` (AGENT:628) and torchvision's save_image quantisation
 // (mul(255).add_(0.5).clamp_(0, 255).to(uint8)) in one pass.  One thread per 4 horizontally adjacent pixels.
-__global__ void zcl_to_u8_kernel(const float *__restrict__ z_cl, uint8_t *__restrict__ out, int n, int H, int W, int Hb,
-                                 int Wb, int B, int v0, int v1) {
-    const int y0 = v0 * B, y1 = (v1 * B < H) ? v1 * B : H;
-    if (y1 <= y0) return;
-    const int W4 = (W + 3) >> 2;
-    const size_t per_img = (size_t)(y1 - y0) * W4;
-    const size_t total = (size_t)n * per_img;
+template <class Geo>
+__global__ void zcl_to_u8_kernel(const float *__restrict__ z_cl, uint8_t *__restrict__ out, Geo g) {
+    const int B = g.B, v0 = g.v0;
+    const size_t total = g.begin_u8();
+    if (total == 0) return;
+    const int y0 = v0 * B;
     const int Cin = 3 * B * B;
-    const bool vec = (W & 3) == 0 && (B & 3) == 0;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const int b = (int)(i / per_img);
-        const size_t q = i - (size_t)b * per_img;
-        const int yy = (int)(q / W4), x4 = (int)(q - (size_t)yy * W4) << 2;
+        const U8Img p = g.at(i);
+        const int W = p.W, W4 = p.W4;
+        const int yy = (int)(p.q / W4), x4 = (int)(p.q - (size_t)yy * W4) << 2;
         const int y = y0 + yy, v = y / B, bv = y - v * B;
         uint8_t px[3][4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int x = x4 + j < W ? x4 + j : W - 1;
             const int h = x / B, bh = x - h * B;
-            const float *src = z_cl + (((size_t)b * Hb + v) * Wb + h) * Cin + (bv * B + bh) * 3;
+            const float *src = z_cl + g.z_block(p, v, h) * Cin + (bv * B + bh) * 3;
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
                 float t = __fadd_rn(__fmul_rn(__fadd_rn(src[c], 0.5f), 255.0f), 0.5f);
@@ -101,8 +171,8 @@ __global__ void zcl_to_u8_kernel(const float *__restrict__ z_cl, uint8_t *__rest
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            uint8_t *dst = out + (((size_t)b * 3 + c) * H + y) * W + x4;
-            if (vec) {
+            uint8_t *dst = out + g.plane(p, c, y) + x4;
+            if (p.vec) {
                 *reinterpret_cast<uchar4 *>(dst) = make_uchar4(px[c][0], px[c][1], px[c][2], px[c][3]);
             } else {
                 for (int j = 0; j < 4 && x4 + j < W; ++j) dst[j] = px[c][j];
@@ -448,7 +518,7 @@ int launch_u8_to_xcl(const uint8_t *img, float *x_cl, int n, int H, int W, int H
                      cudaStream_t st) {
     if (v1 <= v0) return 0;
     const size_t total = (size_t)n * (v1 - v0) * B * Wb * B;
-    u8_to_xcl_kernel<<<grid_for(total, 256), 256, 0, st>>>(img, x_cl, n, H, W, Hb, Wb, B, v0, v1);
+    u8_to_xcl_kernel<<<grid_for(total, 256), 256, 0, st>>>(img, x_cl, U8Batch{n, H, W, Hb, Wb, B, v0, v1});
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
@@ -458,7 +528,25 @@ int launch_zcl_to_u8(const float *z_cl, uint8_t *img, int n, int H, int W, int H
                      cudaStream_t st) {
     if (v1 <= v0 || v0 * B >= H) return 0;
     const size_t total = (size_t)n * ((size_t)(v1 - v0) * B) * ((W + 3) / 4);
-    zcl_to_u8_kernel<<<grid_for(total, 256), 256, 0, st>>>(z_cl, img, n, H, W, Hb, Wb, B, v0, v1);
+    zcl_to_u8_kernel<<<grid_for(total, 256), 256, 0, st>>>(z_cl, img, U8Batch{n, H, W, Hb, Wb, B, v0, v1});
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_u8_to_xcl_mixed(const uint8_t *img, float *x_cl, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
+                           int n_span, long long total, int B, cudaStream_t st) {
+    if (n_span < 1 || total < 1) return 0;
+    u8_to_xcl_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(img, x_cl, U8Mixed{g, pix, span, n_span, B, 0, total});
+    count_launch(1);
+    LBIC_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_zcl_to_u8_mixed(const float *z_cl, uint8_t *img, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
+                           int n_span, long long total, int B, cudaStream_t st) {
+    if (n_span < 1 || total < 1) return 0;
+    zcl_to_u8_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(z_cl, img, U8Mixed{g, pix, span, n_span, B, 0, total});
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;

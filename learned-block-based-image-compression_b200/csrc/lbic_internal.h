@@ -130,6 +130,18 @@ struct MixedGeo {
     const int *stream;     // schedule row -> decoder stream
 };
 
+// 8-bit host calls of a mixed-size batch (lbic_*_images_u8_host_mixed): image i's pixel size and the byte offset of its
+// (3, H, W) planes in the packed buffer, and a list of images with the first work item of each (the conversion kernels
+// number their work items image after image and find an item's image by bisection).
+struct MixedPix {
+    int H, W;
+    long long off;
+};
+struct MixedSpan {
+    long long item0;
+    int img, pad;
+};
+
 // The rows of one step as the host launches them.  `sd` is what the GEMM epilogues see: a wavefront or raster step of
 // one geometry, or for a mixed-size call the raster chunk of schedule rows [sd.t, sd.t + R).  A mixed-size step also
 // carries the schedule and its R device row records (schedule rows, or the ring-extended rows of E0); the launchers of
@@ -282,6 +294,12 @@ int launch_u8_to_xcl(const uint8_t *img, float *x_cl, int n, int H, int W, int H
                      cudaStream_t st);
 int launch_zcl_to_u8(const float *z_cl, uint8_t *img, int n, int H, int W, int Hb, int Wb, int B, int v0, int v1,
                      cudaStream_t st);
+// the same for the whole images of the n_span entries of `span` (device; `total` work items: padded pixels in, output
+// pixel quads out) of a mixed-size batch: x_cl in packed block order, zhat_cl in schedule order
+int launch_u8_to_xcl_mixed(const uint8_t *img, float *x_cl, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
+                           int n_span, long long total, int B, cudaStream_t st);
+int launch_zcl_to_u8_mixed(const float *z_cl, uint8_t *img, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
+                           int n_span, long long total, int B, cudaStream_t st);
 int launch_space_to_depth(const float *img, float *blk, int n, int C, int Hb, int Wb, int B, cudaStream_t st);
 int launch_depth_to_space(const float *blk, float *img, int n, int C, int Hb, int Wb, int B, cudaStream_t st);
 int launch_split_f32(const float *src, h16 *hi, h16 *lo, int64_t n, cudaStream_t st);

@@ -475,6 +475,81 @@ class BlockBasedImgCompLossyNetv9:
                                                              out.ctypes.data, lanes))
         return out
 
+    # ---- 8-bit images of different sizes (lbic_encode_images_u8_host_mixed / lbic_decode_images_u8_host_mixed) ----
+    def _pinned(self, name, nbytes):
+        """Grow-only pinned host staging buffer (uint8), so that the call's band copies are asynchronous."""
+        buf = getattr(self, name, None)
+        if buf is None or buf.numel() < nbytes:
+            buf = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, pin_memory=True)
+            setattr(self, name, buf)
+        return buf
+
+    def _pack_u8(self, images, hwc):
+        """images -> (pinned packed (3, H_i, W_i) planes, [(H_i, W_i)]); hwc: (H, W, 3) arrays, transposed while packing."""
+        arrs = [im.numpy() if isinstance(im, torch.Tensor) else np.asarray(im) for im in images]
+        if not arrs or any(a.dtype != np.uint8 or a.ndim != 3 or a.shape[2 if hwc else 0] != 3 for a in arrs):
+            raise ValueError("images must be a non-empty list of uint8 arrays of shape " + ("(H, W, 3)" if hwc else "(3, H, W)"))
+        sizes = [(int(a.shape[0]), int(a.shape[1])) if hwc else (int(a.shape[1]), int(a.shape[2])) for a in arrs]
+        total = sum(3 * H * W for H, W in sizes)
+        buf = self._pinned("_pin_in", total)
+        at = 0
+        for a, (H, W) in zip(arrs, sizes):
+            t = torch.from_numpy(np.ascontiguousarray(a))
+            buf[at: at + 3 * H * W].view(3, H, W).copy_(t.permute(2, 0, 1) if hwc else t)
+            at += 3 * H * W
+        return buf, sizes
+
+    def _unpack_u8(self, buf, sizes):
+        out, at = [], 0
+        for H, W in sizes:
+            out.append(buf[at: at + 3 * H * W].view(3, H, W).numpy().copy())
+            at += 3 * H * W
+        return out
+
+    def _compress_u8_mixed(self, images, hwc, lanes=1, return_recon=False, stream_cap=None):
+        h = self._need()
+        buf, sizes = self._pack_u8(images, hwc)
+        n = len(sizes)
+        grids = [(-(-H // self.B), -(-W // self.B)) for H, W in sizes]
+        cap = (int(stream_cap or max(self.stream_bound(hb, wb, lanes) for hb, wb in grids)) + 3) // 4 * 4
+        streams = np.empty((n, cap), dtype=np.uint8)
+        lens = np.zeros(n, dtype=np.uint32)
+        rec = self._pinned("_pin_out", sum(3 * H * W for H, W in sizes)) if return_recon else None
+        Hs = (ctypes.c_int * n)(*[s[0] for s in sizes])
+        Ws = (ctypes.c_int * n)(*[s[1] for s in sizes])
+        with torch.cuda.device(self._device):
+            _lib.check(_lib.lib().lbic_encode_images_u8_host_mixed(
+                h, buf.data_ptr(), n, Hs, Ws, rec.data_ptr() if rec is not None else None, streams.ctypes.data, cap,
+                lens.ctypes.data, lanes))
+        return [streams[i, : lens[i]].tobytes() for i in range(n)], (self._unpack_u8(rec, sizes) if return_recon else None)
+
+    def compress_images_u8_mixed(self, images, lanes: int = 1, return_recon: bool = False, stream_cap: int | None = None):
+        """images: list of (3, H_i, W_i) uint8 numpy arrays or CPU tensors of any sizes -> (list[bytes], list of
+        (3, H_i, W_i) uint8 reconstructions or None), in one call (lbic_encode_images_u8_host_mixed).  Each image comes
+        out exactly as compress_images_u8 of that image alone.  The images are packed into a pinned staging buffer."""
+        return self._compress_u8_mixed(images, False, lanes, return_recon, stream_cap)
+
+    def decompress_images_u8_mixed(self, strings, sizes, lanes: int = 1):
+        """list[bytes], [(H_i, W_i)] -> list of (3, H_i, W_i) uint8 arrays, in one call; each equals
+        decompress_images_u8 of that stream alone."""
+        h = self._need()
+        sizes = [(int(a), int(b)) for a, b in sizes]
+        n = len(strings)
+        if n == 0 or len(sizes) != n:
+            raise ValueError("strings / sizes mismatch")
+        cap = (max(len(s) for s in strings) + 3) // 4 * 4
+        host = np.zeros((n, max(cap, 4)), dtype=np.uint8)
+        for i, s in enumerate(strings):
+            host[i, : len(s)] = np.frombuffer(s, dtype=np.uint8)
+        lens = np.array([len(s) for s in strings], dtype=np.uint32)
+        out = self._pinned("_pin_out", sum(3 * H * W for H, W in sizes))
+        Hs = (ctypes.c_int * n)(*[s[0] for s in sizes])
+        Ws = (ctypes.c_int * n)(*[s[1] for s in sizes])
+        with torch.cuda.device(self._device):
+            _lib.check(_lib.lib().lbic_decode_images_u8_host_mixed(h, host.ctypes.data, lens.ctypes.data, host.shape[1], n,
+                                                                   Hs, Ws, out.data_ptr(), lanes))
+        return self._unpack_u8(out, sizes)
+
     def compress(self, x, LRU=None, chlat=None):
         """NET:319-361: one image (1, 3B^2, Hb, Wb) -> (bitstream bytes, zhat)."""
         self._check_call(LRU, chlat)

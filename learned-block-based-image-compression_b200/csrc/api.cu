@@ -203,6 +203,18 @@ int dev_alloc(std::vector<void *> &list, void **p, size_t bytes, bool zero = fal
     return 0;
 }
 
+// A grow-only device buffer of at least `bytes`: a larger one replaces it once the device is idle (kernels enqueued
+// before may still use the old one).
+template <class T>
+int grow_buffer(T *&p, size_t &cap, size_t bytes) {
+    if (cap >= bytes) return 0;
+    if (p) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(p); p = nullptr; cap = 0; }
+    cudaError_t e = cudaMalloc((void **)&p, bytes);
+    if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
+    cap = bytes;
+    return 0;
+}
+
 void free_all(std::vector<void *> &list) {
     for (void *p : list) cudaFree(p);
     list.clear();
@@ -752,155 +764,27 @@ int run_range(lbic_model *m, int l0, int l1, const StepRows &rows, bool syms, cu
 // Step s (wavefront: h + 2v = s from s = 0, or -1 with KS[1] = 3; raster: block number s of every image that has it)
 // covers schedule rows [row0[k], row0[k+1]), k = s - s_first, in (img, v) order, and with KS[1] = 3 first the
 // ring-extended positions [ext0[k], ext0[k+1]) that become computable with it -- per image the positions the
-// equal-size loop of run_steps computes at that step (ring_steps).  The device copy (`geo`, d_ext, d_lane0, d_seg) is
-// one upload.
+// equal-size loop of run_steps computes at that step (ring_steps).  The device copy (`geo`, d_ext and the stream and
+// pixel tables the call's CallImages points to) is one upload (upload_mixed).
 struct MixedPlan {
     int n_img = 0, s_first = 0, s_last = 0;
-    bool raster = false;
-    int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0, n_lanes = 0, max_lanes = 0, max_hb = 0;
-    int64_t min_seg = 0;
+    int nblk = 0, n_ext = 0, max_rows = 0, max_ext = 0;
     std::vector<int> row0, ext0, lane0;
     // per step k: the largest block row of x it reads, and the block rows final in every image after it (an image with
     // fewer rows counts once all of its rows are final) -- what the host hooks of run_steps are told
     std::vector<int> x_hi, done;
-    // 8-bit host calls: pixel sizes and plane offsets per image, and the work-item spans of the conversions (BandPipe)
+    // 8-bit host calls: pixel sizes and plane offsets per image, and the work-item spans of the conversions (CallImages)
     std::vector<MixedPix> pix;
     std::vector<MixedSpan> spans;
-    const MixedPix *d_pix = nullptr;
-    const MixedSpan *d_span = nullptr;
     std::vector<int64_t> seg;           // encode: symbols of stream s = [seg[s], seg[s+1]) in packed order
     std::vector<int4> img, rows, ext;
     std::vector<int> sched, blk_img, g0row, stream;
     MixedGeo geo;
     const int4 *d_ext = nullptr;
-    const int *d_lane0 = nullptr;
-    const int64_t *d_seg = nullptr;
 };
 
 // steps of a call of one geometry: wavefront steps t = h + 2v, or (raster) blocks v * Wb + h
 int step_count(bool raster, int Hb, int Wb) { return raster ? Hb * Wb : Wb + 2 * (Hb - 1); }
-
-// lanes: 1 = one stream per image (reference container; decode in raster order), 0 = one lane per block row
-void plan_mixed(lbic_model *m, int n, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p) {
-    const bool k3 = m->k1 == 3;
-    p = MixedPlan();
-    p.n_img = n;
-    p.raster = raster;
-    p.lane0.assign(n + 1, 0);
-    int64_t npos = 0;
-    for (int i = 0; i < n; ++i) {
-        p.img.push_back(make_int4(Hb[i], Wb[i], p.nblk, (int)npos));
-        p.nblk += Hb[i] * Wb[i];
-        npos += (int64_t)(Hb[i] + 1) * (Wb[i] + 2);
-        const int L = lanes == 1 ? 1 : Hb[i];
-        p.lane0[i + 1] = p.lane0[i] + L;
-        p.max_lanes = L > p.max_lanes ? L : p.max_lanes;
-        const int last = step_count(raster, Hb[i], Wb[i]);
-        p.s_last = last > p.s_last ? last : p.s_last;
-        p.max_hb = Hb[i] > p.max_hb ? Hb[i] : p.max_hb;
-    }
-    p.n_lanes = p.lane0[n];
-    p.s_first = raster ? 0 : (k3 ? -1 : 0);
-    p.sched.assign(p.nblk, 0);
-    p.blk_img.assign(p.nblk, 0);
-    if (k3) p.g0row.assign(npos, 0);   // row 0 of the g0 store: the top ring row, the same for every image
-    for (int i = 0; i < n; ++i)
-        for (int b = 0; b < Hb[i] * Wb[i]; ++b) p.blk_img[p.img[i].z + b] = i;
-    auto add_ext = [&](int i, int v, int h) {
-        p.g0row[p.img[i].w + (v + 1) * (Wb[i] + 2) + (h + 1)] = 1 + p.n_ext++;
-        p.ext.push_back(make_int4(i, v, h, -1));
-    };
-    auto add_row = [&](int i, int v, int h) {
-        const int b = p.img[i].z + v * Wb[i] + h;
-        p.sched[b] = (int)p.rows.size();
-        p.rows.push_back(make_int4(i, v, h, b));
-        p.stream.push_back(p.lane0[i] + (lanes == 1 ? 0 : v));
-    };
-    for (int s = p.s_first; s < p.s_last; ++s) {
-        p.ext0.push_back(p.n_ext);
-        p.row0.push_back((int)p.rows.size());
-        int x_hi = -1, done = p.max_hb;
-        for (int i = 0; i < n; ++i) {
-            // block rows of image i final after step s (the closed forms of run_steps' equal-size calls)
-            const int d = raster ? (s + 1) / Wb[i] : (s >= Wb[i] - 1 ? (s - (Wb[i] - 1)) / 2 + 1 : 0);
-            if (d < Hb[i]) done = d < done ? d : done;
-            if (s >= step_count(raster, Hb[i], Wb[i])) continue;
-            StepDesc e[3];
-            const int n_ring = k3 ? ring_steps(s, raster, 1, Hb[i], Wb[i], e) : 0;
-            for (int j = 0; j < n_ring; ++j)
-                for (int v = e[j].vmin; v < e[j].vmin + e[j].nv; ++v) add_ext(i, v, e[j].t - 2 * v);
-            if (step_desc(s, raster, 1, Hb[i], Wb[i], e[0])) {
-                for (int v = e[0].vmin; v < e[0].vmin + e[0].nv; ++v) add_row(i, v, e[0].t - 2 * v);
-                x_hi = e[0].vmin + e[0].nv - 1 > x_hi ? e[0].vmin + e[0].nv - 1 : x_hi;
-            }
-        }
-        p.x_hi.push_back(x_hi);
-        p.done.push_back(done);
-        const int k = (int)p.row0.size() - 1;
-        const int R = (int)p.rows.size() - p.row0[k], Re = p.n_ext - p.ext0[k];
-        p.max_rows = R > p.max_rows ? R : p.max_rows;
-        p.max_ext = Re > p.max_ext ? Re : p.max_ext;
-    }
-    p.ext0.push_back(p.n_ext);
-    p.row0.push_back((int)p.rows.size());
-    // streams of the encoder: whole images (lanes = 1) or block rows, in packed symbol order
-    const int M = m->M;
-    p.min_seg = INT64_MAX;
-    for (int i = 0; i < n; ++i) {
-        const int L = lanes == 1 ? 1 : Hb[i];
-        const int64_t len = (int64_t)Hb[i] * Wb[i] * M / L;
-        for (int l = 0; l < L; ++l) p.seg.push_back((int64_t)M * p.img[i].z + l * len);
-        p.min_seg = len < p.min_seg ? len : p.min_seg;
-    }
-    p.seg.push_back((int64_t)M * p.nblk);
-}
-
-// One host-to-device copy of the plan's tables into the model's grow-only schedule buffer (on `st`, after the previous
-// call's kernels that read it: the workspace is held).
-int upload_mixed(lbic_model *m, MixedPlan &p, cudaStream_t st) {
-    size_t off = 0;
-    std::vector<std::pair<const void *, size_t>> parts;
-    std::vector<size_t> at;
-    auto add = [&](const void *src, size_t bytes) {
-        at.push_back(off);
-        parts.push_back({src, bytes});
-        off += (bytes + 15) / 16 * 16;
-    };
-    add(p.img.data(), sizeof(int4) * p.img.size());
-    add(p.rows.data(), sizeof(int4) * p.rows.size());
-    add(p.ext.data(), sizeof(int4) * p.ext.size());
-    add(p.sched.data(), sizeof(int) * p.sched.size());
-    add(p.blk_img.data(), sizeof(int) * p.blk_img.size());
-    add(p.g0row.data(), sizeof(int) * p.g0row.size());
-    add(p.stream.data(), sizeof(int) * p.stream.size());
-    add(p.lane0.data(), sizeof(int) * p.lane0.size());
-    add(p.seg.data(), sizeof(int64_t) * p.seg.size());
-    add(p.pix.data(), sizeof(MixedPix) * p.pix.size());
-    add(p.spans.data(), sizeof(MixedSpan) * p.spans.size());
-    if (m->mix_dev_bytes < off) {
-        if (m->mix_dev) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->mix_dev); m->mix_dev = nullptr; m->mix_dev_bytes = 0; }
-        cudaError_t e = cudaMalloc(&m->mix_dev, off);
-        if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", off, cudaGetErrorString(e));
-        m->mix_dev_bytes = off;
-    }
-    m->mix_host.resize(off);
-    for (size_t i = 0; i < parts.size(); ++i)
-        if (parts[i].second) memcpy(m->mix_host.data() + at[i], parts[i].first, parts[i].second);
-    LBIC_CUDA(cudaMemcpyAsync(m->mix_dev, m->mix_host.data(), off, cudaMemcpyHostToDevice, st));
-    char *d = (char *)m->mix_dev;
-    p.geo.img = (const int4 *)(d + at[0]);
-    p.geo.rows = (const int4 *)(d + at[1]);
-    p.d_ext = (const int4 *)(d + at[2]);
-    p.geo.sched = (const int *)(d + at[3]);
-    p.geo.blk_img = (const int *)(d + at[4]);
-    p.geo.g0row = (const int *)(d + at[5]);
-    p.geo.stream = (const int *)(d + at[6]);
-    p.d_lane0 = (const int *)(d + at[7]);
-    p.d_seg = (const int64_t *)(d + at[8]);
-    p.d_pix = (const MixedPix *)(d + at[9]);
-    p.d_span = (const MixedSpan *)(d + at[10]);
-    return 0;
-}
 
 // The steps [first, last) of a call.  at(s) gives step s's rows (R = 0: none, as step -1 of KS[1] = 3) and, with
 // KS[1] = 3, the ring-extended steps whose hidden map becomes computable with it (returns how many).  A call of one
@@ -945,21 +829,173 @@ struct CallSteps {
     }
 };
 
-CallSteps call_steps(const lbic_model *m, int n_img, int Hb, int Wb, bool raster) {
-    CallSteps c;
-    c.raster = raster; c.k3 = m->k1 == 3;
-    c.n_img = n_img; c.Hb = Hb; c.Wb = Wb;
-    c.first = !raster && c.k3 ? -1 : 0;
-    c.last = step_count(raster, Hb, Wb);
-    return c;
+// An encode or decode as its entry point built it: its images as the launchers see them, its steps and (mixed-size
+// call) its schedule, which call_begin uploads.  Built in place and not copied: im.geo and cs.plan point into `plan`.
+struct Call {
+    CallImages im;
+    CallSteps cs;
+    MixedPlan plan;
+    Call() = default;
+    Call(const Call &) = delete;
+    Call &operator=(const Call &) = delete;
+};
+
+// lanes: 1 = one stream per image (reference container; decode in raster order), 0 = one lane per block row
+void one_geometry_call(const lbic_model *m, Call &c, int n_img, int Hb, int Wb, int lanes, bool decode) {
+    const int L = lanes == 1 ? 1 : Hb;
+    c.im = one_geometry(n_img, Hb, Wb, L, (int64_t)Hb * Wb * m->M / L, lanes != 1);
+    CallSteps &cs = c.cs;
+    cs.raster = decode && lanes == 1; cs.k3 = m->k1 == 3;
+    cs.n_img = n_img; cs.Hb = Hb; cs.Wb = Wb;
+    cs.first = !cs.raster && cs.k3 ? -1 : 0;
+    cs.last = step_count(cs.raster, Hb, Wb);
 }
 
-CallSteps call_steps(const lbic_model *m, const MixedPlan &p) {
-    CallSteps c;
-    c.raster = p.raster; c.k3 = m->k1 == 3;
-    c.first = p.s_first; c.last = p.s_last;
-    c.plan = &p;
-    return c;
+// A mixed-size call: its schedule (MixedPlan), images and steps.
+void plan_mixed(const lbic_model *m, Call &c, int n, const int *Hb, const int *Wb, int lanes, bool decode) {
+    const bool k3 = m->k1 == 3, raster = decode && lanes == 1;
+    MixedPlan &p = c.plan;
+    CallImages &im = c.im;
+    p.n_img = n;
+    p.lane0.assign(n + 1, 0);
+    int64_t npos = 0;
+    int max_hb = 0;
+    for (int i = 0; i < n; ++i) {
+        p.img.push_back(make_int4(Hb[i], Wb[i], p.nblk, (int)npos));
+        p.nblk += Hb[i] * Wb[i];
+        npos += (int64_t)(Hb[i] + 1) * (Wb[i] + 2);
+        const int L = lanes == 1 ? 1 : Hb[i];
+        p.lane0[i + 1] = p.lane0[i] + L;
+        im.max_lanes = L > im.max_lanes ? L : im.max_lanes;
+        const int last = step_count(raster, Hb[i], Wb[i]);
+        p.s_last = last > p.s_last ? last : p.s_last;
+        max_hb = Hb[i] > max_hb ? Hb[i] : max_hb;
+    }
+    p.s_first = raster ? 0 : (k3 ? -1 : 0);
+    p.sched.assign(p.nblk, 0);
+    p.blk_img.assign(p.nblk, 0);
+    if (k3) p.g0row.assign(npos, 0);   // row 0 of the g0 store: the top ring row, the same for every image
+    for (int i = 0; i < n; ++i)
+        for (int b = 0; b < Hb[i] * Wb[i]; ++b) p.blk_img[p.img[i].z + b] = i;
+    auto add_ext = [&](int i, int v, int h) {
+        p.g0row[p.img[i].w + (v + 1) * (Wb[i] + 2) + (h + 1)] = 1 + p.n_ext++;
+        p.ext.push_back(make_int4(i, v, h, -1));
+    };
+    auto add_row = [&](int i, int v, int h) {
+        const int b = p.img[i].z + v * Wb[i] + h;
+        p.sched[b] = (int)p.rows.size();
+        p.rows.push_back(make_int4(i, v, h, b));
+        p.stream.push_back(p.lane0[i] + (lanes == 1 ? 0 : v));
+    };
+    for (int s = p.s_first; s < p.s_last; ++s) {
+        p.ext0.push_back(p.n_ext);
+        p.row0.push_back((int)p.rows.size());
+        int x_hi = -1, done = max_hb;
+        for (int i = 0; i < n; ++i) {
+            // block rows of image i final after step s (the closed forms of run_steps' equal-size calls)
+            const int d = raster ? (s + 1) / Wb[i] : (s >= Wb[i] - 1 ? (s - (Wb[i] - 1)) / 2 + 1 : 0);
+            if (d < Hb[i]) done = d < done ? d : done;
+            if (s >= step_count(raster, Hb[i], Wb[i])) continue;
+            StepDesc e[3];
+            const int n_ring = k3 ? ring_steps(s, raster, 1, Hb[i], Wb[i], e) : 0;
+            for (int j = 0; j < n_ring; ++j)
+                for (int v = e[j].vmin; v < e[j].vmin + e[j].nv; ++v) add_ext(i, v, e[j].t - 2 * v);
+            if (step_desc(s, raster, 1, Hb[i], Wb[i], e[0])) {
+                for (int v = e[0].vmin; v < e[0].vmin + e[0].nv; ++v) add_row(i, v, e[0].t - 2 * v);
+                x_hi = e[0].vmin + e[0].nv - 1 > x_hi ? e[0].vmin + e[0].nv - 1 : x_hi;
+            }
+        }
+        p.x_hi.push_back(x_hi);
+        p.done.push_back(done);
+        const int k = (int)p.row0.size() - 1;
+        const int R = (int)p.rows.size() - p.row0[k], Re = p.n_ext - p.ext0[k];
+        p.max_rows = R > p.max_rows ? R : p.max_rows;
+        p.max_ext = Re > p.max_ext ? Re : p.max_ext;
+    }
+    p.ext0.push_back(p.n_ext);
+    p.row0.push_back((int)p.rows.size());
+    // streams of the encoder: whole images (lanes = 1) or block rows, in packed symbol order
+    const int M = m->M;
+    im.min_sym = INT64_MAX;
+    for (int i = 0; i < n; ++i) {
+        const int L = lanes == 1 ? 1 : Hb[i];
+        const int64_t len = (int64_t)Hb[i] * Wb[i] * M / L;
+        for (int l = 0; l < L; ++l) p.seg.push_back((int64_t)M * p.img[i].z + l * len);
+        im.min_sym = len < im.min_sym ? len : im.min_sym;
+        im.max_sym = len > im.max_sym ? len : im.max_sym;
+    }
+    p.seg.push_back((int64_t)M * p.nblk);
+    im.n_img = n; im.nblk = p.nblk; im.Hb = max_hb;
+    im.n_streams = p.lane0[n];
+    im.lane_container = lanes != 1;
+    im.geo = &p.geo;
+    CallSteps &cs = c.cs;
+    cs.raster = raster; cs.k3 = k3;
+    cs.first = p.s_first; cs.last = p.s_last;
+    cs.plan = &p;
+}
+
+// One host-to-device copy of a mixed-size call's tables into the model's grow-only schedule buffer (on `st`, after the
+// previous call's kernels that read it: the workspace is held).  Nothing to do for a call of one geometry.
+int upload_mixed(lbic_model *m, Call &c, cudaStream_t st) {
+    if (!c.cs.plan) return 0;
+    MixedPlan &p = c.plan;
+    size_t off = 0;
+    std::vector<std::pair<const void *, size_t>> parts;
+    std::vector<size_t> at;
+    auto add = [&](const void *src, size_t bytes) {
+        at.push_back(off);
+        parts.push_back({src, bytes});
+        off += (bytes + 15) / 16 * 16;
+    };
+    add(p.img.data(), sizeof(int4) * p.img.size());
+    add(p.rows.data(), sizeof(int4) * p.rows.size());
+    add(p.ext.data(), sizeof(int4) * p.ext.size());
+    add(p.sched.data(), sizeof(int) * p.sched.size());
+    add(p.blk_img.data(), sizeof(int) * p.blk_img.size());
+    add(p.g0row.data(), sizeof(int) * p.g0row.size());
+    add(p.stream.data(), sizeof(int) * p.stream.size());
+    add(p.lane0.data(), sizeof(int) * p.lane0.size());
+    add(p.seg.data(), sizeof(int64_t) * p.seg.size());
+    add(p.pix.data(), sizeof(MixedPix) * p.pix.size());
+    add(p.spans.data(), sizeof(MixedSpan) * p.spans.size());
+    LBIC_TRY(grow_buffer(m->mix_dev, m->mix_dev_bytes, off));
+    m->mix_host.resize(off);
+    for (size_t i = 0; i < parts.size(); ++i)
+        if (parts[i].second) memcpy(m->mix_host.data() + at[i], parts[i].first, parts[i].second);
+    LBIC_CUDA(cudaMemcpyAsync(m->mix_dev, m->mix_host.data(), off, cudaMemcpyHostToDevice, st));
+    char *d = (char *)m->mix_dev;
+    p.geo.img = (const int4 *)(d + at[0]);
+    p.geo.rows = (const int4 *)(d + at[1]);
+    p.d_ext = (const int4 *)(d + at[2]);
+    p.geo.sched = (const int *)(d + at[3]);
+    p.geo.blk_img = (const int *)(d + at[4]);
+    p.geo.g0row = (const int *)(d + at[5]);
+    p.geo.stream = (const int *)(d + at[6]);
+    c.im.lane0 = (const int *)(d + at[7]);
+    c.im.seg = (const int64_t *)(d + at[8]);
+    c.im.pix = (const MixedPix *)(d + at[9]);
+    c.im.span = (const MixedSpan *)(d + at[10]);
+    return 0;
+}
+
+// What a call needs of the workspace: exactly its geometry (ensure_workspace), or (mixed-size call) its schedule's
+// largest steps, blocks, ring rows and lanes, in a workspace that only grows (ensure_workspace_mixed).
+int ensure_call_workspace(lbic_model *m, const Call &c) {
+    if (!c.cs.plan) return ensure_workspace(m, c.im.n_img, c.im.Hb, c.im.Wb);
+    const MixedPlan &p = c.plan;
+    WsNeed z;
+    z.rows = p.max_rows; z.ext_rows = p.max_ext; z.nblk = p.nblk; z.lanes = c.im.n_streams;
+    z.npos = m->k1 == 3 ? 1 + (size_t)p.n_ext : 0;
+    return ensure_workspace_mixed(m, z);
+}
+
+// KS[1] == 3: the top ring row of the g0 store, per image, or (mixed-size call) store row 0, which every image shares
+int fill_ring_top(lbic_model *m, const Call &c, cudaStream_t st) {
+    if (m->k1 != 3) return 0;
+    const bool per_img = !c.cs.plan;
+    return launch_fill_g0_top(m->L[L_E0].bias, m->E1, per_img ? c.im.n_img : 1, per_img ? c.im.Hb : 0,
+                              per_img ? c.im.Wb : -1, m->ws.G0.hi, m->ws.G0.lo, st);
 }
 
 // KS[1] == 3: hidden map g0 = lrelu(E0(zhat taps)) at the ring-extended positions of `ext` (single-position or
@@ -1019,14 +1055,15 @@ struct RowHooks {
     // launch where a hook has work to put between two steps)
     bool (*will_need)(void *ctx, int v_hi) = nullptr;
     bool (*will_done)(void *ctx, int v_done) = nullptr;
-    // mixed-size calls: adds the hooks' tables to the step schedule before its upload (and keeps the plan for the hooks)
-    void (*add_to_plan)(void *ctx, MixedPlan &p) = nullptr;
 };
 
 // The persistent wavefront kernel (gemm_wave.cu) takes over when every step of the call has at most wave_max_rows rows.
-bool wave_applies(const lbic_model *m, int n_img, int Hb, int Wb, bool raster, bool decode) {
-    if (!m->use_wave || m->gemm_core != 0 || m->force_bn || m->profiling || m->check_sat || !gemm_wave_supported())
+// (Mixed-size calls take no wavefront kernel.)
+bool wave_applies(const lbic_model *m, const CallSteps &cs, bool decode) {
+    if (cs.plan || !m->use_wave || m->gemm_core != 0 || m->force_bn || m->profiling || m->check_sat || !gemm_wave_supported())
         return false;
+    const int n_img = cs.n_img, Hb = cs.Hb, Wb = cs.Wb;
+    const bool raster = cs.raster;
     const int max_nv = Hb < (Wb + 1) / 2 ? Hb : (Wb + 1) / 2;
     if (m->k1 == 3) {
         // five-tap topologies: wavefront calls whose EXTENDED steps (two ring positions more per image) fit one row block
@@ -1108,8 +1145,7 @@ int decode_step(lbic_model *m, const StepRows &rows, int lanes, int32_t *sym, cu
 // The step loop of an encode or a decode.  Each step runs through `step(rows)` (per-layer or dataflow launches) after
 // the hidden-map ring positions (KS[1] == 3) that become computable with it, or, when `wave` (small steps: single images,
 // small batches), consecutive steps are collected into ONE launch of the persistent wavefront kernel, `wave_range(s0,
-// s1)`, cut only where a host hook has copies or conversions to put between two steps.  (Mixed-size calls take no
-// wavefront kernel.)
+// s1)`, cut only where a host hook has copies or conversions to put between two steps.
 template <class Step, class WaveRange>
 int run_steps(lbic_model *m, const CallSteps &cs, bool wave, const RowHooks *hk, Step step, WaveRange wave_range,
               cudaStream_t st) {
@@ -1165,12 +1201,12 @@ int ws_acquire(lbic_model *m, cudaStream_t st) {
 }
 
 // Start of an encode or decode on `st`: hold the workspace, clear the error flag and the zhat feedback buffer of its
-// nblk blocks (NET:336, NET:417).
-int call_begin(lbic_model *m, size_t nblk, cudaStream_t st) {
+// blocks (NET:336, NET:417), upload a mixed-size call's schedule.
+int call_begin(lbic_model *m, Call &c, cudaStream_t st) {
     LBIC_TRY(ws_acquire(m, st));
     LBIC_CUDA(cudaMemsetAsync(m->err_flag, 0, sizeof(int), st));
-    LBIC_CUDA(cudaMemsetAsync(m->ws.zhat_cl, 0, sizeof(float) * nblk * m->Cin, st));
-    return 0;
+    LBIC_CUDA(cudaMemsetAsync(m->ws.zhat_cl, 0, sizeof(float) * c.im.nblk * m->Cin, st));
+    return upload_mixed(m, c, st);
 }
 int ws_release(lbic_model *m, cudaStream_t st) {
     LBIC_CUDA(cudaEventRecord(m->ws_event, st));
@@ -1180,12 +1216,7 @@ int ws_release(lbic_model *m, cudaStream_t st) {
 }
 
 int ensure_aux(lbic_model *m, int which, size_t bytes, float **out) {
-    if (m->aux_bytes[which] < bytes) {
-        if (m->aux[which]) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->aux[which]); m->aux[which] = nullptr; m->aux_bytes[which] = 0; }
-        cudaError_t e = cudaMalloc(&m->aux[which], bytes);
-        if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-        m->aux_bytes[which] = bytes;
-    }
+    LBIC_TRY(grow_buffer(m->aux[which], m->aux_bytes[which], bytes));
     *out = m->aux[which];
     return 0;
 }
@@ -1203,18 +1234,109 @@ int take_error_flag(lbic_model *m) {
     return 0;
 }
 
-// info_cl: if set, the (n, Hb, Wb, M) channel-last self-information of the latents (lbic_validate)
-int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out,
-                uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
-                cudaStream_t st, const RowHooks *hk, float *info_cl = nullptr);
-int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img, int Hb,
-                int Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st, const RowHooks *hk);
-int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
-                      int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
-                      int lanes, cudaStream_t st, const RowHooks *hk);
-int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
-                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st,
-                      const RowHooks *hk);
+int check_lanes(int lanes) {
+    if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
+    return 0;
+}
+
+int check_mixed_args(int n_img, const int *Hb, const int *Wb, int lanes) {
+    if (n_img < 1 || !Hb || !Wb) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_lanes(lanes));
+    int64_t nblk = 0;
+    for (int i = 0; i < n_img; ++i) {
+        if (Hb[i] < 1 || Wb[i] < 1) return lbic_fail(LBIC_ERR_INVALID, "image %d has a %d x %d block grid", i, Hb[i], Wb[i]);
+        nblk += (int64_t)Hb[i] * Wb[i];
+    }
+    if (nblk > INT32_MAX / 4) return lbic_fail(LBIC_ERR_INVALID, "batch of %lld blocks is too large", (long long)nblk);
+    return 0;
+}
+
+// Symbols and indexes in packed order for the caller (sym_out / idx_out, if set) and for the stream coder (*sym, *idx,
+// when `coded`).  One geometry: the workspace holds them in packed order; they are coded from there and copied out as
+// asked.  A mixed-size call holds them in schedule order: both are reordered at once, into the caller's arrays or,
+// where the caller passed none, the model's buffer, and coded from there.
+int packed_symbols(lbic_model *m, const CallImages &c, int32_t *sym_out, uint8_t *idx_out, bool coded,
+                   const int32_t **sym, const uint8_t **idx, cudaStream_t st) {
+    Workspace &ws = m->ws;
+    *sym = ws.sym; *idx = ws.idx;
+    if (!c.geo) {
+        if (sym_out) LBIC_TRY(launch_packed_order(ws.sym, sym_out, m->M, c, st));
+        if (idx_out) LBIC_TRY(launch_packed_order(ws.idx, idx_out, m->M, c, st));
+        return 0;
+    }
+    if (!sym_out && !idx_out && !coded) return 0;
+    if (!sym_out || !idx_out) {
+        const size_t n = c.nblk * m->M;
+        LBIC_TRY(grow_buffer(m->mix_sym, m->mix_sym_bytes, n * (sizeof(int32_t) + 1)));
+        if (!sym_out) sym_out = (int32_t *)m->mix_sym;
+        if (!idx_out) idx_out = (uint8_t *)m->mix_sym + n * sizeof(int32_t);
+    }
+    LBIC_TRY(launch_packed_order(ws.sym, sym_out, m->M, c, st));
+    LBIC_TRY(launch_packed_order(ws.idx, idx_out, m->M, c, st));
+    *sym = sym_out; *idx = idx_out;
+    return 0;
+}
+
+// An encode of the call `c`: the images x (x = nullptr: the hooks convert them in) through the step loop to the
+// reconstruction (zhat_out), the symbols and indexes (sym_out, idx_out) and the streams (stream_out).
+// info_cl: if set, the (n, Hb, Wb, M) channel-last self-information of the latents (lbic_validate, one geometry)
+int encode_impl(lbic_model *m, Call &c, const float *x, float *zhat_out, int32_t *sym_out, uint8_t *idx_out,
+                uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, cudaStream_t st, const RowHooks *hk,
+                float *info_cl = nullptr) {
+    const CallImages &im = c.im;
+    LBIC_TRY(ensure_call_workspace(m, c));
+    Workspace &ws = m->ws;
+    LBIC_TRY(call_begin(m, c, st));
+    if (x) LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, m->Cin, im, st));
+    const bool want_syms = sym_out || idx_out || stream_out || info_cl;
+    LBIC_TRY(fill_ring_top(m, c, st));
+    auto step = [&](const StepRows &rows) -> int {
+        LBIC_TRY(encode_step(m, rows, want_syms, st));
+        return info_cl ? launch_selfinfo_step(rows.sd, rows.R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st) : 0;
+    };
+    auto wave_range = [&](int s0, int s1) {
+        return run_wave(m, false, false, s0, s1, c.cs.n_img, c.cs.Hb, c.cs.Wb, 0, nullptr, st);
+    };
+    // (the wavefront kernel does not compute the self-information)
+    const bool wave = !info_cl && wave_applies(m, c.cs, false);
+    LBIC_TRY(run_steps(m, c.cs, wave, hk, step, wave_range, st));
+    if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, m->Cin, im, st));
+    const int32_t *sym = nullptr;
+    const uint8_t *idx = nullptr;
+    LBIC_TRY(packed_symbols(m, im, sym_out, idx_out, stream_out != nullptr, &sym, &idx, st));
+    if (stream_out) {
+        // scratch words per stream: the reference container is coded straight into the caller's slot size; a lane gets
+        // its worst case (lane_bound), so only the caller's stream_cap can ever be the limit
+        const size_t per = (im.lane_container ? lane_bound((size_t)im.max_sym) : stream_cap) / 4;
+        LBIC_TRY(ensure_rans_scratch(m, (size_t)im.n_streams * per + 2 * (size_t)im.n_streams));
+        LBIC_TRY(launch_rans_encode(m->tables, sym, idx, im, ws.rans_scratch, per, im.lane_container ? nullptr : stream_out,
+                                    stream_cap, stream_len, m->err_flag, st));
+        if (im.lane_container)
+            LBIC_TRY(launch_lane_pack(ws.rans_scratch, per, im, stream_out, stream_cap, stream_len, m->err_flag, st));
+    }
+    return ws_release(m, st);
+}
+
+// A decode of the call `c` (the reference container: the rANS state threads through the blocks in raster order,
+// NET:420-450, one block of every image per step) to the reconstruction and, if sym_out is set, the symbols.
+int decode_impl(lbic_model *m, Call &c, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
+                float *zhat_out, int32_t *sym_out, cudaStream_t st, const RowHooks *hk) {
+    const CallImages &im = c.im;
+    LBIC_TRY(ensure_call_workspace(m, c));
+    Workspace &ws = m->ws;
+    LBIC_TRY(call_begin(m, c, st));
+    LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, im, ws.dec_states, ws.lane_ptr, m->err_flag, st));
+    LBIC_TRY(fill_ring_top(m, c, st));
+    int32_t *sym = sym_out ? ws.sym : nullptr;
+    auto step = [&](const StepRows &rows) { return decode_step(m, rows, im.lanes, sym, st); };
+    auto wave_range = [&](int s0, int s1) {
+        return run_wave(m, true, c.cs.raster, s0, s1, c.cs.n_img, c.cs.Hb, c.cs.Wb, im.lanes, sym, st);
+    };
+    LBIC_TRY(run_steps(m, c.cs, wave_applies(m, c.cs, true), hk, step, wave_range, st));
+    if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, m->Cin, im, st));
+    if (sym_out) LBIC_TRY(launch_packed_order(ws.sym, sym_out, m->M, im, st));
+    return ws_release(m, st);
+}
 
 }  // namespace
 
@@ -1467,54 +1589,16 @@ extern "C" int lbic_encode(lbic_model *m, const float *x, int n_img, int Hb, int
                            int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap,
                            uint32_t *stream_len, int lanes, void *stream) {
     if (!x) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    return encode_impl(m, x, n_img, Hb, Wb, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, lanes,
-                       (cudaStream_t)stream, nullptr);
-}
-
-namespace {
-int encode_impl(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out,
-                uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
-                cudaStream_t st, const RowHooks *hk, float *info_cl) {
     LBIC_TRY(check_ready(m, stream_out != nullptr));
-    if ((!x && !(hk && hk->need_rows)) || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
+    if (n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_lanes(lanes));
     if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
     Active act(m);
-    LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
-    Workspace &ws = m->ws;
-    const int HW = Hb * Wb;
-    const size_t nblk = (size_t)n_img * HW;
-    LBIC_TRY(call_begin(m, nblk, st));
-    if (x) LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, n_img, m->Cin, HW, st));
-    const bool want_syms = sym_out || idx_out || stream_out || info_cl;
-    if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
-    auto step = [&](const StepRows &rows) -> int {
-        LBIC_TRY(encode_step(m, rows, want_syms, st));
-        return info_cl ? launch_selfinfo_step(rows.sd, rows.R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st) : 0;
-    };
-    auto wave_range = [&](int s0, int s1) { return run_wave(m, false, false, s0, s1, n_img, Hb, Wb, 0, nullptr, st); };
-    // (the wavefront kernel does not compute the self-information)
-    const bool wave = !info_cl && wave_applies(m, n_img, Hb, Wb, false, false);
-    LBIC_TRY(run_steps(m, call_steps(m, n_img, Hb, Wb, false), wave, hk, step, wave_range, st));
-    if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
-    if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
-    if (idx_out) LBIC_CUDA(cudaMemcpyAsync(idx_out, ws.idx, nblk * m->M, cudaMemcpyDeviceToDevice, st));
-    if (stream_out) {
-        const int L = lanes == 1 ? 1 : Hb;
-        const int n_streams = n_img * L;
-        const int64_t n_sym = (int64_t)HW * m->M / L;
-        // scratch words per stream: the reference container is coded straight into the caller's slot size; a lane gets
-        // its worst case (lane_bound), so only the caller's stream_cap can ever be the limit
-        const size_t per = (lanes == 1 ? stream_cap : lane_bound((size_t)n_sym)) / 4;
-        LBIC_TRY(ensure_rans_scratch(m, (size_t)n_streams * per + 2 * (size_t)n_streams));
-        LBIC_TRY(launch_rans_encode(m->tables, ws.sym, ws.idx, n_streams, n_sym, n_sym, ws.rans_scratch, per,
-                                    lanes == 1 ? stream_out : nullptr, stream_cap, stream_len, m->err_flag, st));
-        if (lanes != 1)
-            LBIC_TRY(launch_lane_pack(ws.rans_scratch, per, n_img, L, stream_out, stream_cap, stream_len, m->err_flag, st));
-    }
-    return ws_release(m, st);
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, lanes, false);
+    return encode_impl(m, c, x, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, (cudaStream_t)stream,
+                       nullptr);
 }
-}  // namespace
 
 extern "C" int lbic_validate(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out,
                              float *selfinfo_out, void *stream) {
@@ -1525,8 +1609,11 @@ extern "C" int lbic_validate(lbic_model *m, const float *x, int n_img, int Hb, i
     LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
     float *cl = nullptr;
     LBIC_TRY(ensure_aux(m, 0, sizeof(float) * (size_t)n_img * Hb * Wb * m->M, &cl));
-    int rc = encode_impl(m, x, n_img, Hb, Wb, zhat_out, nullptr, nullptr, nullptr, 0, nullptr, 1, st, nullptr, cl);
-    if (rc == 0) rc = launch_cl_to_nchw(cl, selfinfo_out, n_img, m->M, Hb * Wb, st);   // -> (n, M, Hb, Wb) as AGENT:509
+    if (Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, 1, false);
+    int rc = encode_impl(m, c, x, zhat_out, nullptr, nullptr, nullptr, 0, nullptr, st, nullptr, cl);
+    if (rc == 0) rc = launch_cl_to_nchw(cl, selfinfo_out, m->M, c.im, st);   // -> (n, M, Hb, Wb) as AGENT:509
     if (rc == 0) rc = ws_release(m, st);
     return rc;
 }
@@ -1544,8 +1631,8 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
     cudaStream_t st = (cudaStream_t)stream;
     LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
     Workspace &ws = m->ws;
-    const int HW = Hb * Wb;
-    const long nblk = (long)n_img * HW;
+    const CallImages im = one_geometry(n_img, Hb, Wb);
+    const long nblk = (long)im.nblk;
     float *xhat_cl = nullptr, *info_cl = nullptr;
     int rc = 0;
     do {
@@ -1553,8 +1640,8 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
         P(ws_acquire(m, st));
         P(ensure_aux(m, 1, sizeof(float) * (size_t)nblk * m->Cin, &xhat_cl));
         if (selfinfo_out) P(ensure_aux(m, 0, sizeof(float) * (size_t)nblk * m->M, &info_cl));
-        P(launch_nchw_to_cl(x, ws.x_cl, n_img, m->Cin, HW, st));
-        P(launch_nchw_to_cl(zhat_in, ws.zhat_cl, n_img, m->Cin, HW, st));
+        P(launch_nchw_to_cl(x, ws.x_cl, m->Cin, im, st));
+        P(launch_nchw_to_cl(zhat_in, ws.zhat_cl, m->Cin, im, st));
         const int chunk = ws.R_cap;
         if (m->k1 == 3) {
             const size_t npos = (size_t)n_img * (Hb + 1) * (Wb + 2);
@@ -1584,8 +1671,8 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
             if (info_cl) P(launch_selfinfo_step(rows.sd, R, m->M, ws.KSI, ws.ldKSI, ws.sym, info_cl, st));
         }
         if (rc) break;
-        P(launch_cl_to_nchw(xhat_cl, xhat_out, n_img, m->Cin, HW, st));
-        if (info_cl) P(launch_cl_to_nchw(info_cl, selfinfo_out, n_img, m->M, HW, st));
+        P(launch_cl_to_nchw(xhat_cl, xhat_out, m->Cin, im, st));
+        if (info_cl) P(launch_cl_to_nchw(info_cl, selfinfo_out, m->M, im, st));
         if (sym_out && cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * (size_t)nblk * m->M, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
             rc = lbic_fail(LBIC_ERR_CUDA, "copy failed");
         if (rc == 0) rc = ws_release(m, st);
@@ -1596,22 +1683,41 @@ extern "C" int lbic_forward(lbic_model *m, const float *zhat_in, const float *x,
 
 extern "C" int lbic_decode(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                            int n_img, int Hb, int Wb, float *zhat_out, int32_t *sym_out, int lanes, void *stream) {
-    return decode_impl(m, streams, stream_len, stream_cap, n_img, Hb, Wb, zhat_out, sym_out, lanes, (cudaStream_t)stream,
-                       nullptr);
+    LBIC_TRY(check_ready(m, true));
+    if (!streams || !stream_len || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_lanes(lanes));
+    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, lanes, true);
+    return decode_impl(m, c, streams, stream_len, stream_cap, zhat_out, sym_out, (cudaStream_t)stream, nullptr);
 }
 
 extern "C" int lbic_encode_mixed(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
                                  int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap,
                                  uint32_t *stream_len, int lanes, void *stream) {
-    return encode_mixed_impl(m, x, n_img, Hb, Wb, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, lanes,
-                             (cudaStream_t)stream, nullptr);
+    LBIC_TRY(check_ready(m, stream_out != nullptr));
+    if (!x) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
+    if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    Call c;
+    plan_mixed(m, c, n_img, Hb, Wb, lanes, false);
+    return encode_impl(m, c, x, zhat_out, sym_out, idx_out, stream_out, stream_cap, stream_len, (cudaStream_t)stream,
+                       nullptr);
 }
 
 extern "C" int lbic_decode_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                                  int n_img, const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes,
                                  void *stream) {
-    return decode_mixed_impl(m, streams, stream_len, stream_cap, n_img, Hb, Wb, zhat_out, sym_out, lanes,
-                             (cudaStream_t)stream, nullptr);
+    LBIC_TRY(check_ready(m, true));
+    if (!streams || !stream_len) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
+    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    Call c;
+    plan_mixed(m, c, n_img, Hb, Wb, lanes, true);
+    return decode_impl(m, c, streams, stream_len, stream_cap, zhat_out, sym_out, (cudaStream_t)stream, nullptr);
 }
 
 // Synchronises `stream` and reports what the kernels enqueued on it flagged since the last encode / decode started:
@@ -1624,147 +1730,6 @@ extern "C" int lbic_check_errors(lbic_model *m, void *stream) {
 }
 
 namespace {
-int decode_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img, int Hb,
-                int Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st, const RowHooks *hk) {
-    LBIC_TRY(check_ready(m, true));
-    if (!streams || !stream_len || n_img < 1 || Hb < 1 || Wb < 1) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
-    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-    Active act(m);
-    LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
-    Workspace &ws = m->ws;
-    const int HW = Hb * Wb;
-    const size_t nblk = (size_t)n_img * HW;
-    const int L = lanes == 1 ? 1 : Hb;
-    LBIC_TRY(call_begin(m, nblk, st));
-    LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, n_img, L, lanes != 1, ws.dec_states, ws.lane_ptr,
-                                  m->err_flag, st));
-    if (m->k1 == 3) LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, n_img, Hb, Wb, ws.G0.hi, ws.G0.lo, st));
-    const bool raster = (L == 1 && lanes == 1);      // reference container: the rANS state threads through the blocks in
-                                                     // raster order (NET:420-450), one block of every image per step
-    int32_t *sym = sym_out ? ws.sym : nullptr;
-    auto step = [&](const StepRows &rows) { return decode_step(m, rows, L, sym, st); };
-    auto wave_range = [&](int s0, int s1) { return run_wave(m, true, raster, s0, s1, n_img, Hb, Wb, L, sym, st); };
-    LBIC_TRY(run_steps(m, call_steps(m, n_img, Hb, Wb, raster), wave_applies(m, n_img, Hb, Wb, raster, true), hk, step,
-                       wave_range, st));
-    if (zhat_out) LBIC_TRY(launch_cl_to_nchw(ws.zhat_cl, zhat_out, n_img, m->Cin, HW, st));
-    if (sym_out) LBIC_CUDA(cudaMemcpyAsync(sym_out, ws.sym, sizeof(int32_t) * nblk * m->M, cudaMemcpyDeviceToDevice, st));
-    return ws_release(m, st);
-}
-
-// ---- mixed-size batches ------------------------------------------------------------------------------------------
-int check_mixed_args(int n_img, const int *Hb, const int *Wb, int lanes) {
-    if (n_img < 1 || !Hb || !Wb) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    if (lanes != 0 && lanes != 1) return lbic_fail(LBIC_ERR_INVALID, "lanes must be 1 (reference) or 0 (per block row)");
-    int64_t nblk = 0;
-    for (int i = 0; i < n_img; ++i) {
-        if (Hb[i] < 1 || Wb[i] < 1) return lbic_fail(LBIC_ERR_INVALID, "image %d has a %d x %d block grid", i, Hb[i], Wb[i]);
-        nblk += (int64_t)Hb[i] * Wb[i];
-    }
-    if (nblk > INT32_MAX / 4) return lbic_fail(LBIC_ERR_INVALID, "batch of %lld blocks is too large", (long long)nblk);
-    return 0;
-}
-
-WsNeed mixed_need(const lbic_model *m, const MixedPlan &p) {
-    WsNeed z;
-    z.rows = p.max_rows; z.ext_rows = p.max_ext; z.nblk = p.nblk; z.lanes = p.n_lanes;
-    z.npos = m->k1 == 3 ? 1 + (size_t)p.n_ext : 0;
-    return z;
-}
-
-int mixed_begin(lbic_model *m, int n_img, const int *Hb, const int *Wb, bool raster, int lanes, MixedPlan &p,
-                cudaStream_t st, const RowHooks *hk) {
-    plan_mixed(m, n_img, Hb, Wb, raster, lanes, p);
-    if (hk && hk->add_to_plan) hk->add_to_plan(hk->ctx, p);
-    LBIC_TRY(ensure_workspace_mixed(m, mixed_need(m, p)));
-    LBIC_TRY(call_begin(m, p.nblk, st));
-    LBIC_TRY(upload_mixed(m, p, st));
-    if (m->k1 == 3)   // row 0 of the g0 store: the top ring row (fill_g0_top of a single position)
-        LBIC_TRY(launch_fill_g0_top(m->L[L_E0].bias, m->E1, 1, 0, -1, m->ws.G0.hi, m->ws.G0.lo, st));
-    return 0;
-}
-
-int encode_mixed_impl(lbic_model *m, const float *x, int n_img, const int *Hb, const int *Wb, float *zhat_out,
-                      int32_t *sym_out, uint8_t *idx_out, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
-                      int lanes, cudaStream_t st, const RowHooks *hk) {
-    LBIC_TRY(check_ready(m, stream_out != nullptr));
-    if (!x && !(hk && hk->need_rows)) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
-    if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-    Active act(m);
-    MixedPlan p;
-    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, false, lanes, p, st, hk));
-    Workspace &ws = m->ws;
-    const size_t nblk = p.nblk;
-    if (x) LBIC_TRY(launch_nchw_to_cl_mixed(x, ws.x_cl, m->Cin, p.geo, p.nblk, st));
-    const bool want_syms = sym_out || idx_out || stream_out;
-    auto step = [&](const StepRows &rows) { return encode_step(m, rows, want_syms, st); };
-    auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, call_steps(m, p), false, hk, step, no_wave, st));
-    if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
-    if (!want_syms) return ws_release(m, st);
-    // symbols and indexes in packed order: into the caller's arrays, or (streams only) a model buffer
-    int32_t *sym_p = sym_out;
-    uint8_t *idx_p = idx_out;
-    if (!sym_p || !idx_p) {
-        const size_t need = nblk * m->M * (sizeof(int32_t) + 1);
-        if (m->mix_sym_bytes < need) {
-            if (m->mix_sym) { LBIC_CUDA(cudaDeviceSynchronize()); cudaFree(m->mix_sym); m->mix_sym = nullptr; m->mix_sym_bytes = 0; }
-            cudaError_t e = cudaMalloc(&m->mix_sym, need);
-            if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", need, cudaGetErrorString(e));
-            m->mix_sym_bytes = need;
-        }
-        if (!sym_p) sym_p = (int32_t *)m->mix_sym;
-        if (!idx_p) idx_p = (uint8_t *)m->mix_sym + nblk * m->M * sizeof(int32_t);
-    }
-    LBIC_TRY(launch_unschedule_i32(ws.sym, sym_p, m->M, p.geo, p.nblk, st));
-    LBIC_TRY(launch_unschedule_u8(ws.idx, idx_p, m->M, p.geo, p.nblk, st));
-    if (stream_out) {
-        // scratch words per stream as in encode_impl: the caller's slot (reference container) or a lane's worst case
-        int64_t max_seg = 0;
-        for (size_t s = 0; s + 1 < p.seg.size(); ++s) max_seg = p.seg[s + 1] - p.seg[s] > max_seg ? p.seg[s + 1] - p.seg[s] : max_seg;
-        const size_t per = (lanes == 1 ? stream_cap : lane_bound((size_t)max_seg)) / 4;
-        LBIC_TRY(ensure_rans_scratch(m, (size_t)p.n_lanes * per + 2 * (size_t)p.n_lanes));
-        LBIC_TRY(launch_rans_encode_mixed(m->tables, sym_p, idx_p, p.n_lanes, p.d_seg, p.min_seg, ws.rans_scratch, per,
-                                          lanes == 1 ? stream_out : nullptr, stream_cap, stream_len, m->err_flag, st));
-        if (lanes != 1)
-            LBIC_TRY(launch_lane_pack_mixed(ws.rans_scratch, per, n_img, p.d_lane0, p.n_lanes, p.max_lanes, stream_out,
-                                            stream_cap, stream_len, m->err_flag, st));
-    }
-    return ws_release(m, st);
-}
-
-int decode_mixed_impl(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap, int n_img,
-                      const int *Hb, const int *Wb, float *zhat_out, int32_t *sym_out, int lanes, cudaStream_t st,
-                      const RowHooks *hk) {
-    LBIC_TRY(check_ready(m, true));
-    if (!streams || !stream_len) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    LBIC_TRY(check_mixed_args(n_img, Hb, Wb, lanes));
-    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-    Active act(m);
-    MixedPlan p;
-    const bool raster = lanes == 1;   // reference container: raster order, one block of every image per step
-    LBIC_TRY(mixed_begin(m, n_img, Hb, Wb, raster, lanes, p, st, hk));
-    Workspace &ws = m->ws;
-    LBIC_TRY(launch_rans_dec_init_mixed(streams, stream_len, stream_cap, n_img, p.d_lane0, p.n_lanes, lanes != 1,
-                                        ws.dec_states, ws.lane_ptr, m->err_flag, st));
-    int32_t *sym = sym_out ? ws.sym : nullptr;
-    auto step = [&](const StepRows &rows) { return decode_step(m, rows, 0, sym, st); };
-    auto no_wave = [&](int, int) { return 0; };
-    LBIC_TRY(run_steps(m, call_steps(m, p), false, hk, step, no_wave, st));
-    if (zhat_out) LBIC_TRY(launch_cl_to_nchw_mixed(ws.zhat_cl, zhat_out, m->Cin, p.geo, p.nblk, st));
-    if (sym_out) LBIC_TRY(launch_unschedule_i32(ws.sym, sym_out, m->M, p.geo, p.nblk, st));
-    return ws_release(m, st);
-}
-
-int ensure_io(lbic_model *m, size_t bytes) {
-    if (m->io_bytes >= bytes) return 0;
-    if (m->io_dev) { cudaDeviceSynchronize(); cudaFree(m->io_dev); m->io_dev = nullptr; m->io_bytes = 0; }
-    cudaError_t e = cudaMalloc(&m->io_dev, bytes);
-    if (e != cudaSuccess) return lbic_fail(LBIC_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-    m->io_bytes = bytes;
-    return 0;
-}
 size_t align256(size_t v) { return (v + 255) / 256 * 256; }
 
 // ---- host-buffer calls -----------------------------------------------------------------------------------------
@@ -1783,55 +1748,25 @@ int host_pipeline_init(lbic_model *m) {
 
 struct BandPipe {
     lbic_model *m = nullptr;
-    int n = 0, Hb = 0, Wb = 0;
+    const CallImages *c = nullptr;
+    int fmt = 0;                                  // 0: fp32 (n, Cin, Hb, Wb) block tensors, 1: u8 (n, 3, H, W) images
+    int B = 0;
+    size_t bytes = 0;                             // of the host buffer
     int nb = 0, vb[LBIC_MAX_BANDS + 1] = {};      // band b = block rows [vb[b], vb[b+1])
     int next_in = 0, next_out = 0;
-    int fmt = 0;                                  // 0: fp32 (n, Cin, Hb, Wb) block tensors, 1: u8 (n, 3, H, W) images
-    int H = 0, W = 0, B = 0;                      // fmt 1
     const uint8_t *h_in = nullptr; uint8_t *d_in = nullptr;
     uint8_t *h_out = nullptr; uint8_t *d_out = nullptr;
-    // mixed-size u8 call: per-image pixel sizes and plane offsets.  It moves in ONE band (copy, compute, copy): on a
-    // B200 host_bands 16 measured no faster than 1 for mixed batches (profiles/r3_mixed_u8_*.json), so the per-image
-    // band copies were not kept.  The plan's spans are the n images for the input conversion (tin work items), then
-    // the n images again for the output conversion (tout).
-    const int *Hs = nullptr, *Ws = nullptr, *Hbs = nullptr;
-    std::vector<size_t> off;
-    const MixedPlan *mp = nullptr;
-    long long tin = 0, tout = 0;
-    int rc = 0;
 
-    void plan(lbic_model *model, int n_img, int hb, int wb) {
-        m = model; n = n_img; Hb = hb; Wb = wb;
-        nb = hb < m->host_bands ? hb : m->host_bands;
-        for (int b = 0; b <= nb; ++b) vb[b] = (int)((long)hb * b / nb);
-    }
-    void plan_mixed(lbic_model *model, int n_img, const int *h, const int *w, const int *hb) {
-        int max_hb = 0;
-        Hs = h; Ws = w; Hbs = hb;
-        off.assign(n_img + 1, 0);
-        for (int i = 0; i < n_img; ++i) {
-            max_hb = hb[i] > max_hb ? hb[i] : max_hb;
-            off[i + 1] = off[i] + (size_t)3 * h[i] * w[i];
-        }
-        m = model; n = n_img; Hb = max_hb;
-        nb = 1; vb[0] = 0; vb[1] = max_hb;
-    }
-    static void add_to_plan(void *ctx, MixedPlan &p) {
-        BandPipe *q = (BandPipe *)ctx;
-        q->mp = &p;
-        for (int i = 0; i < q->n; ++i) p.pix.push_back(MixedPix{q->Hs[i], q->Ws[i], (long long)q->off[i]});
-        q->tin = q->tout = 0;
-        for (int i = 0; i < q->n; ++i) {              // padded pixels of the image
-            p.spans.push_back(MixedSpan{q->tin, i, 0});
-            q->tin += (long long)q->Hbs[i] * q->B * ((q->Ws[i] + q->B - 1) / q->B) * q->B;
-        }
-        for (int i = 0; i < q->n; ++i) {              // quads of output pixels of the image
-            p.spans.push_back(MixedSpan{q->tout, i, 0});
-            q->tout += (long long)q->Hs[i] * ((q->Ws[i] + 3) / 4);
-        }
+    // A mixed-size call moves in ONE band (copy, compute, copy): on a B200 host_bands 16 measured no faster than 1 for
+    // mixed batches (profiles/r3_mixed_u8_*.json), so the per-image band copies were not kept.
+    void plan(lbic_model *model, int format, const CallImages &im, size_t nbytes) {
+        m = model; c = &im; fmt = format; B = m->cfg.block_size; bytes = nbytes;
+        nb = im.geo ? 1 : im.Hb < m->host_bands ? im.Hb : m->host_bands;
+        for (int b = 0; b <= nb; ++b) vb[b] = (int)((long)im.Hb * b / nb);
     }
     // plane geometry of a band for the 2-D copies: `planes` rows of `pitch` bytes, the band is bytes [off, off + width)
     void geom(int b, size_t &planes, size_t &pitch, size_t &o, size_t &width) const {
+        const int n = c->n_img, Hb = c->Hb, Wb = c->Wb, H = c->H, W = c->W;
         if (fmt == 0) {
             planes = (size_t)n * m->Cin; pitch = sizeof(float) * (size_t)Hb * Wb;
             o = sizeof(float) * (size_t)vb[b] * Wb; width = sizeof(float) * (size_t)(vb[b + 1] - vb[b]) * Wb;
@@ -1843,8 +1778,8 @@ struct BandPipe {
     }
     // band b between host and device: one 2-D copy, or (mixed, one band) the packed images in one copy
     int copy(int b, uint8_t *dst, const uint8_t *src, cudaMemcpyKind kind, cudaStream_t st) const {
-        if (Hs) {
-            LBIC_CUDA(cudaMemcpyAsync(dst, src, off[n], kind, st));
+        if (c->geo) {
+            LBIC_CUDA(cudaMemcpyAsync(dst, src, bytes, kind, st));
             return 0;
         }
         size_t planes, pitch, o, width;
@@ -1869,30 +1804,26 @@ struct BandPipe {
     }
     static int need_rows(void *ctx, int v_hi, cudaStream_t st) {
         BandPipe *p = (BandPipe *)ctx;
+        const CallImages &c = *p->c;
         while (p->next_in < p->nb && p->vb[p->next_in] <= v_hi) {
             const int b = p->next_in++;
             LBIC_CUDA(cudaStreamWaitEvent(st, p->m->hev[b], 0));
-            if (p->mp)
-                LBIC_TRY(launch_u8_to_xcl_mixed(p->d_in, p->m->ws.x_cl, p->mp->geo, p->mp->d_pix, p->mp->d_span, p->n,
-                                                p->tin, p->B, st));
-            else if (p->fmt == 0)
-                LBIC_TRY(launch_nchw_to_cl_band((const float *)p->d_in, p->m->ws.x_cl, p->n, p->m->Cin, p->Hb, p->Wb, p->vb[b], p->vb[b + 1], st));
+            if (p->fmt == 0)
+                LBIC_TRY(launch_nchw_to_cl_band((const float *)p->d_in, p->m->ws.x_cl, c.n_img, p->m->Cin, c.Hb, c.Wb, p->vb[b], p->vb[b + 1], st));
             else
-                LBIC_TRY(launch_u8_to_xcl(p->d_in, p->m->ws.x_cl, p->n, p->H, p->W, p->Hb, p->Wb, p->B, p->vb[b], p->vb[b + 1], st));
+                LBIC_TRY(launch_u8_to_xcl(p->d_in, p->m->ws.x_cl, c, p->B, p->vb[b], p->vb[b + 1], st));
         }
         return 0;
     }
     static int rows_done(void *ctx, int v_done, cudaStream_t st) {
         BandPipe *p = (BandPipe *)ctx;
+        const CallImages &c = *p->c;
         while (p->next_out < p->nb && p->vb[p->next_out + 1] <= v_done) {
             const int b = p->next_out++;
-            if (p->mp)
-                LBIC_TRY(launch_zcl_to_u8_mixed(p->m->ws.zhat_cl, p->d_out, p->mp->geo, p->mp->d_pix, p->mp->d_span + p->n,
-                                                p->n, p->tout, p->B, st));
-            else if (p->fmt == 0)
-                LBIC_TRY(launch_cl_to_nchw_band(p->m->ws.zhat_cl, (float *)p->d_out, p->n, p->m->Cin, p->Hb, p->Wb, p->vb[b], p->vb[b + 1], st));
+            if (p->fmt == 0)
+                LBIC_TRY(launch_cl_to_nchw_band(p->m->ws.zhat_cl, (float *)p->d_out, c.n_img, p->m->Cin, c.Hb, c.Wb, p->vb[b], p->vb[b + 1], st));
             else
-                LBIC_TRY(launch_zcl_to_u8(p->m->ws.zhat_cl, p->d_out, p->n, p->H, p->W, p->Hb, p->Wb, p->B, p->vb[b], p->vb[b + 1], st));
+                LBIC_TRY(launch_zcl_to_u8(p->m->ws.zhat_cl, p->d_out, c, p->B, p->vb[b], p->vb[b + 1], st));
             LBIC_CUDA(cudaEventRecord(p->m->hev[LBIC_MAX_BANDS + b], st));
             LBIC_CUDA(cudaStreamWaitEvent(p->m->hs[2], p->m->hev[LBIC_MAX_BANDS + b], 0));
             LBIC_TRY(p->copy(b, p->h_out, p->d_out, cudaMemcpyDeviceToHost, p->m->hs[2]));
@@ -1901,40 +1832,28 @@ struct BandPipe {
     }
 };
 
-// fmt 0: x / zhat are fp32 (n, 3B^2, Hb, Wb) block tensors; fmt 1: 8-bit (n, 3, H, W) images (pad / crop fused), or
-// with Hv / Wv (mixed-size u8 call) the packed 8-bit images of pixel sizes Hv[i] x Wv[i] and block grids Hb[i] x Wb[i]
-// (Hbv / Wbv), `in_bytes` in all
-int encode_host_impl(lbic_model *m, int fmt, const void *in, int n_img, int H, int W, int Hb, int Wb, void *recon_out,
-                     uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes,
-                     const int *Hv = nullptr, const int *Wv = nullptr, const int *Hbv = nullptr, const int *Wbv = nullptr,
-                     size_t in_bytes = 0) {
-    LBIC_TRY(check_ready(m, stream_out != nullptr));
-    if (!in || n_img < 1 || (!Hv && (Hb < 1 || Wb < 1))) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
-    if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-    Active act(m);
+// fmt 0: `in` / recon_out are fp32 (n, 3B^2, Hb, Wb) block tensors; fmt 1: 8-bit (n, 3, H, W) images (pad / crop fused)
+// or, for a mixed-size call, the packed 8-bit images; `in_bytes` in all
+int encode_host_impl(lbic_model *m, int fmt, Call &c, const void *in, size_t in_bytes, void *recon_out,
+                     uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len) {
+    const int n_img = c.im.n_img;
     LBIC_TRY(host_pipeline_init(m));
-    const size_t nin = Hv ? in_bytes : fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
-    const size_t o_in = 0, o_out = align256(nin), o_len = o_out + (recon_out ? align256(nin) : 0),
+    const size_t o_in = 0, o_out = align256(in_bytes), o_len = o_out + (recon_out ? align256(in_bytes) : 0),
                  o_s = o_len + align256(4 * (size_t)n_img);
-    LBIC_TRY(ensure_io(m, o_s + (stream_out ? (size_t)n_img * stream_cap : 0)));
-    if (!Hv) LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
+    LBIC_TRY(grow_buffer(m->io_dev, m->io_bytes, o_s + (stream_out ? (size_t)n_img * stream_cap : 0)));
+    LBIC_TRY(ensure_call_workspace(m, c));
     uint8_t *io = (uint8_t *)m->io_dev;
     cudaStream_t s_cmp = m->hs[1], s_out = m->hs[2];
     BandPipe bp;
-    bp.fmt = fmt; bp.H = H; bp.W = W; bp.B = m->cfg.block_size;
-    if (Hv) bp.plan_mixed(m, n_img, Hv, Wv, Hbv);
-    else bp.plan(m, n_img, Hb, Wb);
+    bp.plan(m, fmt, c.im, in_bytes);
     bp.h_in = (const uint8_t *)in; bp.d_in = io + o_in;
     bp.h_out = (uint8_t *)recon_out; bp.d_out = io + o_out;
     LBIC_TRY(bp.queue_inputs());
     RowHooks hk;
     hk.ctx = &bp; hk.need_rows = BandPipe::need_rows; hk.rows_done = recon_out ? BandPipe::rows_done : nullptr;
     hk.will_need = BandPipe::will_need; hk.will_done = BandPipe::will_done;
-    if (Hv) hk.add_to_plan = BandPipe::add_to_plan;
-    int rc = Hv ? encode_mixed_impl(m, nullptr, n_img, Hbv, Wbv, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr,
-                                    stream_cap, (uint32_t *)(io + o_len), lanes, s_cmp, &hk)
-                : encode_impl(m, nullptr, n_img, Hb, Wb, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr, stream_cap,
-                              (uint32_t *)(io + o_len), lanes, s_cmp, &hk);
+    int rc = encode_impl(m, c, nullptr, nullptr, nullptr, nullptr, stream_out ? io + o_s : nullptr, stream_cap,
+                         (uint32_t *)(io + o_len), s_cmp, &hk);
     if (rc == 0 && stream_out && cudaMemcpyAsync(stream_len, io + o_len, 4 * (size_t)n_img, cudaMemcpyDeviceToHost, s_cmp) != cudaSuccess)
         rc = lbic_fail(LBIC_ERR_CUDA, "copy failed");
     cudaError_t e0 = cudaStreamSynchronize(m->hs[0]), e1 = cudaStreamSynchronize(s_cmp);
@@ -1955,44 +1874,50 @@ int encode_host_impl(lbic_model *m, int fmt, const void *in, int n_img, int H, i
     return rc;
 }
 
-int decode_host_impl(lbic_model *m, int fmt, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
-                     int n_img, int H, int W, int Hb, int Wb, void *out, int lanes, const int *Hv = nullptr,
-                     const int *Wv = nullptr, const int *Hbv = nullptr, const int *Wbv = nullptr, size_t out_bytes = 0) {
-    LBIC_TRY(check_ready(m, true));
-    if (!streams || !stream_len || !out || n_img < 1 || (!Hv && (Hb < 1 || Wb < 1))) return lbic_fail(LBIC_ERR_INVALID, "null argument");
-    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-    Active act(m);
+// fmt as in encode_host_impl; `out_bytes` of the host buffer `out`
+int decode_host_impl(lbic_model *m, int fmt, Call &c, const uint8_t *streams, const uint32_t *stream_len,
+                     size_t stream_cap, void *out, size_t out_bytes) {
+    const int n_img = c.im.n_img;
     LBIC_TRY(host_pipeline_init(m));
-    const size_t nout = Hv ? out_bytes : fmt == 0 ? sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img : (size_t)n_img * 3 * H * W;
-    const size_t o_out = 0, o_len = align256(nout), o_s = o_len + align256(4 * (size_t)n_img);
+    const size_t o_out = 0, o_len = align256(out_bytes), o_s = o_len + align256(4 * (size_t)n_img);
     size_t longest = 0;
-    for (int i = 0; i < n_img; ++i) {
-        if (stream_len[i] > stream_cap) return lbic_fail(LBIC_ERR_INVALID, "stream %d longer than stream_cap", i);
-        longest = stream_len[i] > longest ? stream_len[i] : longest;
-    }
-    LBIC_TRY(ensure_io(m, o_s + (size_t)n_img * stream_cap));
-    if (!Hv) LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
+    for (int i = 0; i < n_img; ++i) longest = stream_len[i] > longest ? stream_len[i] : longest;
+    LBIC_TRY(grow_buffer(m->io_dev, m->io_bytes, o_s + (size_t)n_img * stream_cap));
+    LBIC_TRY(ensure_call_workspace(m, c));
     uint8_t *io = (uint8_t *)m->io_dev;
     cudaStream_t s_cmp = m->hs[1], s_out = m->hs[2];
     LBIC_CUDA(cudaMemcpyAsync(io + o_len, stream_len, 4 * (size_t)n_img, cudaMemcpyHostToDevice, s_cmp));
     if (longest) LBIC_CUDA(cudaMemcpy2DAsync(io + o_s, stream_cap, streams, stream_cap, longest, n_img, cudaMemcpyHostToDevice, s_cmp));
     BandPipe bp;
-    bp.fmt = fmt; bp.H = H; bp.W = W; bp.B = m->cfg.block_size;
-    if (Hv) bp.plan_mixed(m, n_img, Hv, Wv, Hbv);
-    else bp.plan(m, n_img, Hb, Wb);
+    bp.plan(m, fmt, c.im, out_bytes);
     bp.h_out = (uint8_t *)out; bp.d_out = io + o_out;
     RowHooks hk;
     hk.ctx = &bp; hk.rows_done = BandPipe::rows_done; hk.will_done = BandPipe::will_done;
-    if (Hv) hk.add_to_plan = BandPipe::add_to_plan;
-    int rc = Hv ? decode_mixed_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hbv, Wbv, nullptr,
-                                    nullptr, lanes, s_cmp, &hk)
-                : decode_impl(m, io + o_s, (const uint32_t *)(io + o_len), stream_cap, n_img, Hb, Wb, nullptr, nullptr, lanes,
-                              s_cmp, &hk);
+    int rc = decode_impl(m, c, io + o_s, (const uint32_t *)(io + o_len), stream_cap, nullptr, nullptr, s_cmp, &hk);
     cudaError_t e1 = cudaStreamSynchronize(s_cmp), e2 = cudaStreamSynchronize(s_out);
     if (rc) return rc;
     if (e1 != cudaSuccess || e2 != cudaSuccess)
         return lbic_fail(LBIC_ERR_CUDA, "decode failed: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
     return take_error_flag(m);
+}
+
+// What every host-buffer encode checks after its sizes: the model, the input (`bad`) and the stream buffer.
+int check_host_encode(lbic_model *m, bool bad, const uint8_t *stream_out, const uint32_t *stream_len, size_t stream_cap) {
+    LBIC_TRY(check_ready(m, stream_out != nullptr));
+    if (bad) return lbic_fail(LBIC_ERR_INVALID, "bad arguments");
+    if (stream_out && (!stream_len || stream_cap % 4)) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    return 0;
+}
+
+// What every host-buffer decode checks after its sizes: the model, the buffers (`bad`, including a null stream_len)
+// and the stream lengths.
+int check_host_decode(lbic_model *m, bool bad, int n_img, const uint32_t *stream_len, size_t stream_cap) {
+    LBIC_TRY(check_ready(m, true));
+    if (bad) return lbic_fail(LBIC_ERR_INVALID, "null argument");
+    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    for (int i = 0; i < n_img; ++i)
+        if (stream_len[i] > stream_cap) return lbic_fail(LBIC_ERR_INVALID, "stream %d longer than stream_cap", i);
+    return 0;
 }
 
 // Arguments of the mixed-size u8 host calls: per-image block grids and the byte total of the packed images.
@@ -2015,34 +1940,83 @@ int u8_mixed_args(const lbic_model *m, int n_img, const int *H, const int *W, in
     *bytes = total;
     return 0;
 }
+
+// A mixed-size u8 host call: the plan of n_img images of H[i] x W[i] pixels with the tables of its conversions, image
+// i's pixel size and the byte offset of its planes in the packed buffer, and the work-item spans of the whole-image
+// conversions (padded pixels in, quads of output pixels out).
+void plan_mixed_u8(const lbic_model *m, Call &c, int n_img, const int *H, const int *W, const std::vector<int> &Hb,
+                   const std::vector<int> &Wb, int lanes, bool decode) {
+    plan_mixed(m, c, n_img, Hb.data(), Wb.data(), lanes, decode);
+    MixedPlan &p = c.plan;
+    const long long B = m->cfg.block_size;
+    long long off = 0, items = 0;
+    for (int i = 0; i < n_img; ++i) {
+        p.pix.push_back(MixedPix{H[i], W[i], off});
+        off += 3LL * H[i] * W[i];
+    }
+    for (int i = 0; i < n_img; ++i) {
+        p.spans.push_back(MixedSpan{items, i, 0});
+        items += Hb[i] * B * Wb[i] * B;
+    }
+    c.im.u8_items[0] = items;
+    items = 0;
+    for (int i = 0; i < n_img; ++i) {
+        p.spans.push_back(MixedSpan{items, i, 0});
+        items += (long long)H[i] * ((W[i] + 3) / 4);
+    }
+    c.im.u8_items[1] = items;
+}
 }  // namespace
 
 extern "C" int lbic_encode_host(lbic_model *m, const float *x, int n_img, int Hb, int Wb, float *zhat_out,
                                 uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes) {
-    return encode_host_impl(m, 0, x, n_img, 0, 0, Hb, Wb, zhat_out, stream_out, stream_cap, stream_len, lanes);
+    LBIC_TRY(check_host_encode(m, !x || n_img < 1 || Hb < 1 || Wb < 1, stream_out, stream_len, stream_cap));
+    LBIC_TRY(check_lanes(lanes));
+    Active act(m);
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, lanes, false);
+    return encode_host_impl(m, 0, c, x, sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img, zhat_out, stream_out,
+                            stream_cap, stream_len);
 }
 
 extern "C" int lbic_decode_host(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
                                 int n_img, int Hb, int Wb, float *zhat_out, int lanes) {
-    return decode_host_impl(m, 0, streams, stream_len, stream_cap, n_img, 0, 0, Hb, Wb, zhat_out, lanes);
+    LBIC_TRY(check_host_decode(m, !streams || !stream_len || !zhat_out || n_img < 1 || Hb < 1 || Wb < 1, n_img,
+                               stream_len, stream_cap));
+    LBIC_TRY(check_lanes(lanes));
+    Active act(m);
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, lanes, true);
+    return decode_host_impl(m, 0, c, streams, stream_len, stream_cap, zhat_out,
+                            sizeof(float) * (size_t)m->Cin * Hb * Wb * n_img);
 }
 
 extern "C" int lbic_encode_images_u8_host(lbic_model *m, const uint8_t *img, int n_img, int H, int W, uint8_t *recon_out,
                                           uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len, int lanes) {
     if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
     if (H < 1 || W < 1) return lbic_fail(LBIC_ERR_INVALID, "bad image size");
+    LBIC_TRY(check_host_encode(m, !img || n_img < 1, stream_out, stream_len, stream_cap));
+    LBIC_TRY(check_lanes(lanes));
+    Active act(m);
     const int B = m->cfg.block_size;
-    return encode_host_impl(m, 1, img, n_img, H, W, (H + B - 1) / B, (W + B - 1) / B, recon_out, stream_out, stream_cap,
-                            stream_len, lanes);
+    Call c;
+    one_geometry_call(m, c, n_img, (H + B - 1) / B, (W + B - 1) / B, lanes, false);
+    c.im.H = H; c.im.W = W;
+    return encode_host_impl(m, 1, c, img, (size_t)n_img * 3 * H * W, recon_out, stream_out, stream_cap, stream_len);
 }
 
 extern "C" int lbic_decode_images_u8_host(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len,
                                           size_t stream_cap, int n_img, int H, int W, uint8_t *img_out, int lanes) {
     if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
     if (H < 1 || W < 1) return lbic_fail(LBIC_ERR_INVALID, "bad image size");
+    LBIC_TRY(check_host_decode(m, !streams || !stream_len || !img_out || n_img < 1, n_img, stream_len, stream_cap));
+    LBIC_TRY(check_lanes(lanes));
+    Active act(m);
     const int B = m->cfg.block_size;
-    return decode_host_impl(m, 1, streams, stream_len, stream_cap, n_img, H, W, (H + B - 1) / B, (W + B - 1) / B, img_out,
-                            lanes);
+    Call c;
+    one_geometry_call(m, c, n_img, (H + B - 1) / B, (W + B - 1) / B, lanes, true);
+    c.im.H = H; c.im.W = W;
+    return decode_host_impl(m, 1, c, streams, stream_len, stream_cap, img_out, (size_t)n_img * 3 * H * W);
 }
 
 extern "C" int lbic_encode_images_u8_host_mixed(lbic_model *m, const uint8_t *img, int n_img, const int *H, const int *W,
@@ -2052,8 +2026,11 @@ extern "C" int lbic_encode_images_u8_host_mixed(lbic_model *m, const uint8_t *im
     std::vector<int> Hb, Wb;
     size_t bytes = 0;
     LBIC_TRY(u8_mixed_args(m, n_img, H, W, lanes, Hb, Wb, &bytes));
-    return encode_host_impl(m, 1, img, n_img, 0, 0, 0, 0, recon_out, stream_out, stream_cap, stream_len, lanes, H, W,
-                            Hb.data(), Wb.data(), bytes);
+    LBIC_TRY(check_host_encode(m, !img, stream_out, stream_len, stream_cap));
+    Active act(m);
+    Call c;
+    plan_mixed_u8(m, c, n_img, H, W, Hb, Wb, lanes, false);
+    return encode_host_impl(m, 1, c, img, bytes, recon_out, stream_out, stream_cap, stream_len);
 }
 
 extern "C" int lbic_decode_images_u8_host_mixed(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len,
@@ -2063,8 +2040,11 @@ extern "C" int lbic_decode_images_u8_host_mixed(lbic_model *m, const uint8_t *st
     std::vector<int> Hb, Wb;
     size_t bytes = 0;
     LBIC_TRY(u8_mixed_args(m, n_img, H, W, lanes, Hb, Wb, &bytes));
-    return decode_host_impl(m, 1, streams, stream_len, stream_cap, n_img, 0, 0, 0, 0, img_out, lanes, H, W, Hb.data(),
-                            Wb.data(), bytes);
+    LBIC_TRY(check_host_decode(m, !streams || !stream_len || !img_out, n_img, stream_len, stream_cap));
+    Active act(m);
+    Call c;
+    plan_mixed_u8(m, c, n_img, H, W, Hb, Wb, lanes, true);
+    return decode_host_impl(m, 1, c, streams, stream_len, stream_cap, img_out, bytes);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2128,12 +2108,12 @@ extern "C" int lbic_postprocess(lbic_model *m, const float *z, int n_img, int Hb
         LBIC_TRY(make_view(ws, m->vPPH, m->PPH, 4 * m->Cin));
         m->pp_rcap = ws.R_cap;
     }
-    const int HW = Hb * Wb;
-    const long nblk = (long)n_img * HW;
+    const CallImages im = one_geometry(n_img, Hb, Wb);
+    const long nblk = (long)im.nblk;
     float *out_cl = nullptr;
     LBIC_TRY(ws_acquire(m, st));
     LBIC_TRY(ensure_aux(m, 1, sizeof(float) * (size_t)nblk * m->Cin, &out_cl));
-    LBIC_TRY(launch_nchw_to_cl(z, ws.zhat_cl, n_img, m->Cin, HW, st));
+    LBIC_TRY(launch_nchw_to_cl(z, ws.zhat_cl, m->Cin, im, st));
     const int chunk = ws.R_cap;
     for (long r0 = 0; r0 < nblk; r0 += chunk) {
         const int R = (int)(nblk - r0 < chunk ? nblk - r0 : chunk);
@@ -2148,7 +2128,7 @@ extern "C" int lbic_postprocess(lbic_model *m, const float *z, int n_img, int Hb
         LBIC_TRY(run_gemm_layer(m, m->PP[1], -1, R, &m->vPPH, nullptr, e, st));
     }
     LBIC_TRY(launch_restore_border(ws.zhat_cl, out_cl, m->Cin, n_img, Hb, Wb, st));
-    LBIC_TRY(launch_cl_to_nchw(out_cl, out, n_img, m->Cin, HW, st));
+    LBIC_TRY(launch_cl_to_nchw(out_cl, out, m->Cin, im, st));
     return ws_release(m, st);
 }
 
@@ -2171,14 +2151,16 @@ extern "C" int lbic_band_begin(lbic_model *m, const float *x, int n_img, int Hb,
     if (m->k1 != 1) return lbic_fail(LBIC_ERR_INVALID, "band mode supports KS[1] = 1 (one halo block per step)");
     Active act(m);
     cudaStream_t st = (cudaStream_t)stream;
-    LBIC_TRY(ensure_workspace(m, n_img, Hb, Wb));
+    Call c;
+    one_geometry_call(m, c, n_img, Hb, Wb, 0, decode);   // one lane per block row
+    LBIC_TRY(ensure_call_workspace(m, c));
     Workspace &ws = m->ws;
-    LBIC_TRY(call_begin(m, (size_t)n_img * Hb * Wb, st));
+    LBIC_TRY(call_begin(m, c, st));
     if (decode) {
         if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
-        LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, n_img, Hb, 1, ws.dec_states, ws.lane_ptr, m->err_flag, st));
+        LBIC_TRY(launch_rans_dec_init(streams, stream_len, stream_cap, c.im, ws.dec_states, ws.lane_ptr, m->err_flag, st));
     } else {
-        LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, n_img, m->Cin, Hb * Wb, st));
+        LBIC_TRY(launch_nchw_to_cl(x, ws.x_cl, m->Cin, c.im, st));
     }
     m->band_n = n_img; m->band_Hb = Hb; m->band_Wb = Wb; m->band_decode = decode ? 1 : 0;
     return 0;
@@ -2219,12 +2201,12 @@ extern "C" int lbic_band_end(lbic_model *m, int v0, int v1, float *zhat_rows_out
                                     sizeof(float) * row_f * Hb, sizeof(float) * row_f * nr, n_img, cudaMemcpyDeviceToDevice, st));
     if (lane_out && !m->band_decode) {
         if (!lane_len || lane_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "lane_cap must be a multiple of 4");
-        const int64_t n_sym = (int64_t)Wb * m->M;
+        const CallImages band = one_geometry(1, nr, Wb, nr, (int64_t)Wb * m->M);   // one image's rows: a lane each
         const size_t per = lane_cap / 4;
         LBIC_TRY(ensure_rans_scratch(m, (size_t)nr * per + 2 * (size_t)nr));
         for (int i = 0; i < n_img; ++i) {
             const size_t o = ((size_t)i * Hb + v0) * Wb * m->M;
-            LBIC_TRY(launch_rans_encode(m->tables, ws.sym + o, ws.idx + o, nr, n_sym, n_sym, ws.rans_scratch, per,
+            LBIC_TRY(launch_rans_encode(m->tables, ws.sym + o, ws.idx + o, band, ws.rans_scratch, per,
                                         lane_out + (size_t)i * nr * lane_cap, lane_cap, lane_len + (size_t)i * nr, m->err_flag, st));
         }
     }
@@ -2252,8 +2234,8 @@ extern "C" int lbic_rans_encode(lbic_model *m, const int32_t *symbols, const uin
     if (m->ws.n_img == 0) LBIC_TRY(ensure_workspace(m, 1, 1, 2));
     const size_t per = stream_cap / 4;
     LBIC_TRY(ensure_rans_scratch(m, (size_t)n_streams * per + 2 * (size_t)n_streams));
-    return launch_rans_encode(m->tables, symbols, indexes, n_streams, n_sym, n_sym, m->ws.rans_scratch, per, stream_out,
-                              stream_cap, stream_len, m->err_flag, (cudaStream_t)stream);
+    return launch_rans_encode(m->tables, symbols, indexes, one_geometry(n_streams, 1, 1, 1, n_sym), m->ws.rans_scratch, per,
+                              stream_out, stream_cap, stream_len, m->err_flag, (cudaStream_t)stream);
 }
 
 extern "C" int lbic_rans_decode(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,

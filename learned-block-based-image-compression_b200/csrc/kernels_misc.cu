@@ -498,55 +498,64 @@ inline int grid_for(size_t total, int block) {
 
 }  // namespace
 
-int launch_nchw_to_cl(const float *src, float *dst, int n, int C, int HW, cudaStream_t st) {
-    dim3 grid((HW + 31) / 32, (C + 31) / 32, n), block(32, 8);
-    transpose_kernel<<<grid, block, 0, st>>>(src, dst, C, HW);
+int launch_nchw_to_cl(const float *src, float *dst, int C, const CallImages &c, cudaStream_t st) {
+    if (c.geo) {
+        dim3 grid((unsigned)((c.nblk + 31) / 32), (C + 31) / 32), block(32, 8);
+        nchw_cl_mixed_kernel<true><<<grid, block, 0, st>>>(src, dst, C, *c.geo, (int)c.nblk);
+    } else {
+        const int HW = c.Hb * c.Wb;
+        dim3 grid((HW + 31) / 32, (C + 31) / 32, c.n_img), block(32, 8);
+        transpose_kernel<<<grid, block, 0, st>>>(src, dst, C, HW);
+    }
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_cl_to_nchw(const float *src, float *dst, int n, int C, int HW, cudaStream_t st) {
-    dim3 grid((C + 31) / 32, (HW + 31) / 32, n), block(32, 8);
-    transpose_kernel<<<grid, block, 0, st>>>(src, dst, HW, C);
+int launch_cl_to_nchw(const float *src, float *dst, int C, const CallImages &c, cudaStream_t st) {
+    if (c.geo) {
+        dim3 grid((unsigned)((c.nblk + 31) / 32), (C + 31) / 32), block(32, 8);
+        nchw_cl_mixed_kernel<false><<<grid, block, 0, st>>>(src, dst, C, *c.geo, (int)c.nblk);
+    } else {
+        const int HW = c.Hb * c.Wb;
+        dim3 grid((C + 31) / 32, (HW + 31) / 32, c.n_img), block(32, 8);
+        transpose_kernel<<<grid, block, 0, st>>>(src, dst, HW, C);
+    }
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_u8_to_xcl(const uint8_t *img, float *x_cl, int n, int H, int W, int Hb, int Wb, int B, int v0, int v1,
-                     cudaStream_t st) {
-    if (v1 <= v0) return 0;
-    const size_t total = (size_t)n * (v1 - v0) * B * Wb * B;
-    u8_to_xcl_kernel<<<grid_for(total, 256), 256, 0, st>>>(img, x_cl, U8Batch{n, H, W, Hb, Wb, B, v0, v1});
+// (a mixed-size call converts its whole images: v0 = 0 in the kernels, the band arguments are not used)
+int launch_u8_to_xcl(const uint8_t *img, float *x_cl, const CallImages &c, int B, int v0, int v1, cudaStream_t st) {
+    if (c.geo) {
+        const long long total = c.u8_items[0];
+        if (c.n_img < 1 || total < 1) return 0;
+        u8_to_xcl_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(
+            img, x_cl, U8Mixed{*c.geo, c.pix, c.span, c.n_img, B, 0, total});
+    } else {
+        if (v1 <= v0) return 0;
+        const size_t total = (size_t)c.n_img * (v1 - v0) * B * c.Wb * B;
+        u8_to_xcl_kernel<<<grid_for(total, 256), 256, 0, st>>>(img, x_cl,
+                                                               U8Batch{c.n_img, c.H, c.W, c.Hb, c.Wb, B, v0, v1});
+    }
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_zcl_to_u8(const float *z_cl, uint8_t *img, int n, int H, int W, int Hb, int Wb, int B, int v0, int v1,
-                     cudaStream_t st) {
-    if (v1 <= v0 || v0 * B >= H) return 0;
-    const size_t total = (size_t)n * ((size_t)(v1 - v0) * B) * ((W + 3) / 4);
-    zcl_to_u8_kernel<<<grid_for(total, 256), 256, 0, st>>>(z_cl, img, U8Batch{n, H, W, Hb, Wb, B, v0, v1});
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_u8_to_xcl_mixed(const uint8_t *img, float *x_cl, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
-                           int n_span, long long total, int B, cudaStream_t st) {
-    if (n_span < 1 || total < 1) return 0;
-    u8_to_xcl_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(img, x_cl, U8Mixed{g, pix, span, n_span, B, 0, total});
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_zcl_to_u8_mixed(const float *z_cl, uint8_t *img, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
-                           int n_span, long long total, int B, cudaStream_t st) {
-    if (n_span < 1 || total < 1) return 0;
-    zcl_to_u8_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(z_cl, img, U8Mixed{g, pix, span, n_span, B, 0, total});
+int launch_zcl_to_u8(const float *z_cl, uint8_t *img, const CallImages &c, int B, int v0, int v1, cudaStream_t st) {
+    if (c.geo) {
+        const long long total = c.u8_items[1];
+        if (c.n_img < 1 || total < 1) return 0;
+        zcl_to_u8_kernel<<<grid_for((size_t)total, 256), 256, 0, st>>>(
+            z_cl, img, U8Mixed{*c.geo, c.pix, c.span + c.n_img, c.n_img, B, 0, total});
+    } else {
+        if (v1 <= v0 || v0 * B >= c.H) return 0;
+        const size_t total = (size_t)c.n_img * ((size_t)(v1 - v0) * B) * ((c.W + 3) / 4);
+        zcl_to_u8_kernel<<<grid_for(total, 256), 256, 0, st>>>(z_cl, img,
+                                                               U8Batch{c.n_img, c.H, c.W, c.Hb, c.Wb, B, v0, v1});
+    }
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
@@ -644,35 +653,19 @@ int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16
     return 0;
 }
 
-int launch_nchw_to_cl_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
-    dim3 grid((nblk + 31) / 32, (C + 31) / 32), block(32, 8);
-    nchw_cl_mixed_kernel<true><<<grid, block, 0, st>>>(src, dst, C, g, nblk);
+template <class T>
+int launch_packed_order(const T *src, T *dst, int C, const CallImages &c, cudaStream_t st) {
+    if (!c.geo) {   // one geometry: the schedule order is the packed order
+        LBIC_CUDA(cudaMemcpyAsync(dst, src, sizeof(T) * c.nblk * C, cudaMemcpyDeviceToDevice, st));
+        return 0;
+    }
+    unschedule_kernel<T><<<grid_for(c.nblk * C, 256), 256, 0, st>>>(src, dst, C, *c.geo, (int)c.nblk);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
-
-int launch_cl_to_nchw_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
-    dim3 grid((nblk + 31) / 32, (C + 31) / 32), block(32, 8);
-    nchw_cl_mixed_kernel<false><<<grid, block, 0, st>>>(src, dst, C, g, nblk);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_unschedule_i32(const int32_t *src, int32_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
-    unschedule_kernel<int32_t><<<grid_for((size_t)nblk * C, 256), 256, 0, st>>>(src, dst, C, g, nblk);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_unschedule_u8(const uint8_t *src, uint8_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st) {
-    unschedule_kernel<uint8_t><<<grid_for((size_t)nblk * C, 256), 256, 0, st>>>(src, dst, C, g, nblk);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
+template int launch_packed_order<int32_t>(const int32_t *, int32_t *, int, const CallImages &, cudaStream_t);
+template int launch_packed_order<uint8_t>(const uint8_t *, uint8_t *, int, const CallImages &, cudaStream_t);
 
 int launch_pack_conv(const float *w, const float *mask, int cout, int cin, int kh, int kw, const int *taps_host,
                      int ntaps, float *weff, int ld, cudaStream_t st) {

@@ -117,9 +117,9 @@ __host__ __device__ inline int ring_steps(int s, bool raster, int n_img, int Hb,
 // k holds the k-th block the call computes.  The GEMM layers then see each step as the raster chunk
 //   StepDesc{1, 0, 0, k0, 1, n_rows}      (row r -> block k0 + r, see step_row_to_block)
 // so their epilogues write the symbols, indexes and reconstruction of row r to schedule row k0 + r with the
-// equal-size kernels unchanged.  The kernels that look at an image's geometry read these tables: the gathers and the
-// rANS decode step through a row-source template parameter (one kernel body each, instantiated for StepDesc and for
-// the schedule's rows), the stream and layout kernels in mixed forms of their own.
+// equal-size kernels unchanged.  The kernels that look at an image's geometry read these tables through a template
+// parameter or a mixed form of the kernel, picked by the launcher: per step from StepRows (the gathers, the rANS decode
+// step), per call from CallImages (stream coding, layout and 8-bit conversions).
 // ------------------------------------------------------------------------------------------------
 struct MixedGeo {
     const int4 *rows;      // schedule row -> {img, v, h, packed block}      (packed block = P_img + v * Wb_img + h)
@@ -153,6 +153,39 @@ struct StepRows {
     const int4 *rows = nullptr;
     int g0_row0 = -1;      // ring rows of a mixed-size call: E0 writes them to g0 store rows g0_row0, ... (-1: by position)
 };
+
+// The images of a call as the call-level launchers see them (stream coding, layout and 8-bit conversions), the role
+// StepRows has for a step: n_img images of Hb x Wb blocks (geo == nullptr: the closed forms), or the schedule of a
+// mixed-size call.  Both carry their stream layout: `lanes` streams per image of min_sym = max_sym symbols each, or
+// (mixed) image i's streams lane0[i] .. lane0[i+1] - 1 with stream s holding packed symbols [seg[s], seg[s+1]).
+struct CallImages {
+    int n_img = 0;
+    size_t nblk = 0;                     // blocks of the batch
+    int Hb = 0, Wb = 0;                  // block grid of every image (mixed: Hb of the tallest, Wb unused)
+    int lanes = 0, max_lanes = 0;        // streams per image (mixed: lanes 0, per image from lane0), the most of one image
+    int n_streams = 0;
+    int64_t min_sym = 0, max_sym = 0;    // symbols of the shortest and of the longest stream
+    bool lane_container = false;         // streams are 'LBML' lane containers (also with one lane), else reference streams
+    const MixedGeo *geo = nullptr;       // mixed: the schedule's device tables, and (device) lane0 and seg
+    const int *lane0 = nullptr;
+    const int64_t *seg = nullptr;
+    // 8-bit calls: the pixel size of every image, or (mixed) per image, and the work items of the whole-image
+    // conversions: span[0, n_img) and u8_items[0] in, span[n_img, 2 n_img) and u8_items[1] out (device tables)
+    int H = 0, W = 0;
+    const MixedPix *pix = nullptr;
+    const MixedSpan *span = nullptr;
+    long long u8_items[2] = {0, 0};
+};
+
+// n_img images of Hb x Wb blocks, coded as `lanes` streams per image of n_sym symbols each
+inline CallImages one_geometry(int n_img, int Hb, int Wb, int lanes = 1, int64_t n_sym = 0, bool lane_container = false) {
+    CallImages c;
+    c.n_img = n_img; c.nblk = (size_t)n_img * Hb * Wb; c.Hb = Hb; c.Wb = Wb;
+    c.lanes = c.max_lanes = lanes; c.n_streams = n_img * lanes;
+    c.min_sym = c.max_sym = n_sym;
+    c.lane_container = lane_container;
+    return c;
+}
 
 // ------------------------------------------------------------------------------------------------
 // Epilogue of a GEMM layer (fused into both GEMM cores).
@@ -284,22 +317,20 @@ int make_tmap_2d(CUtensorMap *tm, const void *base, uint64_t inner, uint64_t out
 // ------------------------------------------------------------------------------------------------
 // elementwise / layout kernels (kernels_misc.cu)
 // ------------------------------------------------------------------------------------------------
-int launch_nchw_to_cl(const float *src, float *dst, int n, int C, int HW, cudaStream_t st);
-int launch_cl_to_nchw(const float *src, float *dst, int n, int C, int HW, cudaStream_t st);
+// (n, C, Hb, Wb) NCHW images <-> channel-last blocks, one launch for the batch.  Mixed-size call: the images packed back
+// to back, x_cl in packed block order (to_cl) and zhat_cl in schedule order (from_cl).
+int launch_nchw_to_cl(const float *src, float *dst, int C, const CallImages &c, cudaStream_t st);
+int launch_cl_to_nchw(const float *src, float *dst, int C, const CallImages &c, cudaStream_t st);
 // band-wise forms (block rows [v0, v1) of every image): the host calls convert while later bands are still in flight
 int launch_nchw_to_cl_band(const float *src, float *dst, int n, int C, int Hb, int Wb, int v0, int v1, cudaStream_t st);
 int launch_cl_to_nchw_band(const float *src, float *dst, int n, int C, int Hb, int Wb, int v0, int v1, cudaStream_t st);
-// 8-bit RGB images (n,3,H,W) <-> channel-last block tensors (pad / crop, +-0.5 and the 8-bit quantisation fused)
-int launch_u8_to_xcl(const uint8_t *img, float *x_cl, int n, int H, int W, int Hb, int Wb, int B, int v0, int v1,
-                     cudaStream_t st);
-int launch_zcl_to_u8(const float *z_cl, uint8_t *img, int n, int H, int W, int Hb, int Wb, int B, int v0, int v1,
-                     cudaStream_t st);
-// the same for the whole images of the n_span entries of `span` (device; `total` work items: padded pixels in, output
-// pixel quads out) of a mixed-size batch: x_cl in packed block order, zhat_cl in schedule order
-int launch_u8_to_xcl_mixed(const uint8_t *img, float *x_cl, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
-                           int n_span, long long total, int B, cudaStream_t st);
-int launch_zcl_to_u8_mixed(const float *z_cl, uint8_t *img, const MixedGeo &g, const MixedPix *pix, const MixedSpan *span,
-                           int n_span, long long total, int B, cudaStream_t st);
+// 8-bit RGB images (n,3,H,W) <-> channel-last block tensors (pad / crop, +-0.5 and the 8-bit quantisation fused), block
+// rows [v0, v1) of every image; a mixed-size call converts its whole images (c.pix, c.span)
+int launch_u8_to_xcl(const uint8_t *img, float *x_cl, const CallImages &c, int B, int v0, int v1, cudaStream_t st);
+int launch_zcl_to_u8(const float *z_cl, uint8_t *img, const CallImages &c, int B, int v0, int v1, cudaStream_t st);
+// the (block, C) symbols or indexes of the workspace (schedule order) -> packed block order: a copy for one geometry
+template <class T>
+int launch_packed_order(const T *src, T *dst, int C, const CallImages &c, cudaStream_t st);
 int launch_space_to_depth(const float *img, float *blk, int n, int C, int Hb, int Wb, int B, cudaStream_t st);
 int launch_depth_to_space(const float *blk, float *img, int n, int C, int Hb, int Wb, int B, cudaStream_t st);
 int launch_split_f32(const float *src, h16 *hi, h16 *lo, int64_t n, cudaStream_t st);
@@ -325,12 +356,6 @@ int launch_restore_border(const float *z_cl, float *out_cl, int Cin, int n_img, 
 int launch_gather5(const h16 *g0_hi, const h16 *g0_lo, int E1, const StepRows &s, h16 *out_hi, h16 *out_lo, int ld,
                    cudaStream_t st);
 int launch_fill_g0_top(const float *bias, int E1, int n_img, int Hb, int Wb, h16 *g_hi, h16 *g_lo, cudaStream_t st);
-// packed NCHW images <-> packed channel-last blocks (to_cl) or schedule-ordered channel-last blocks (from_cl), and a
-// schedule-ordered (block, C) array -> packed order; one launch for the whole batch
-int launch_nchw_to_cl_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
-int launch_cl_to_nchw_mixed(const float *src, float *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
-int launch_unschedule_i32(const int32_t *src, int32_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
-int launch_unschedule_u8(const uint8_t *src, uint8_t *dst, int C, const MixedGeo &g, int nblk, cudaStream_t st);
 int launch_add_vec(const float *a, const float *b, float *out, int n, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------------
@@ -360,19 +385,18 @@ struct RansStreamState {   // one per stream, device resident between decode ste
     uint32_t nwords;
 };
 
-// symbols/indexes: for stream s, symbol k lives at  base + s*stream_stride + k   (elements).
+// the c.n_streams streams of a call (CallImages: their symbols in packed order, stream after stream).
 // scratch holds n_streams*scratch_words words followed by start_word[n_streams] and n_words[n_streams];
 // out may be NULL (lane mode: launch_lane_pack assembles the containers from the scratch).
-int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, int64_t n_sym,
-                       int64_t stream_stride, uint32_t *scratch_words, size_t scratch_words_per_stream,
-                       uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st);
-// lane container: merges `lanes` consecutive single streams per image into header|lengths|payload
-int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, int n_img, int lanes, uint8_t *out,
-                     size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st);
-// lanes_container != 0: the streams are 'LBML' lane containers (also when lanes == 1, i.e. a one-block-row image)
-int launch_rans_dec_init(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
-                         int lanes, int lanes_container, RansStreamState *states, const uint8_t **lane_ptr, int *err_flag,
-                         cudaStream_t st);
+int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, const CallImages &c,
+                       uint32_t *scratch_words, size_t scratch_words_per_stream, uint8_t *out, size_t out_stride,
+                       uint32_t *out_len, int *err_flag, cudaStream_t st);
+// lane container: merges the streams of each image into header|lengths|payload
+int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, const CallImages &c, uint8_t *out, size_t out_stride,
+                     uint32_t *out_len, int *err_flag, cudaStream_t st);
+// decoder state of every stream of the call (c.lane_container: the streams are 'LBML' lane containers)
+int launch_rans_dec_init(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, const CallImages &c,
+                         RansStreamState *states, const uint8_t **lane_ptr, int *err_flag, cudaStream_t st);
 // decode M symbols for every row of a step; writes yq = sym + mean (hi/lo) and optionally symbols
 void rans_set_enc_block_max_streams(int n);    // encodes of at most this many streams use the CTA-per-stream kernel (0 = never)
 void rans_set_enc_thread_min_streams(int n);   // encodes of at least this many streams use the thread-per-stream kernel
@@ -384,17 +408,6 @@ int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t
                          int32_t *sym_out, cudaStream_t st);
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,
                          cudaStream_t st);
-// Mixed-size forms.  Encode: stream s holds symbols [seg[s], seg[s+1]) (device array, min_sym = the shortest stream);
-// lane s of image i is stream lane0[i] + s (lane0: device, n_img + 1 entries, max_lanes = the most lanes of one image).
-int launch_rans_encode_mixed(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
-                             int64_t min_sym, uint32_t *scratch_words, size_t scratch_words_per_stream, uint8_t *out,
-                             size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st);
-int launch_lane_pack_mixed(const uint32_t *scratch, size_t scratch_words, int n_img, const int *lane0, int n_lanes,
-                           int max_lanes, uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag,
-                           cudaStream_t st);
-int launch_rans_dec_init_mixed(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
-                               const int *lane0, int n_lanes, int lanes_container, RansStreamState *states,
-                               const uint8_t **lane_ptr, int *err_flag, cudaStream_t st);
 // CDF index of n scales by both routines of the decoders (bisection; hint with bisection fallback), for tests
 int launch_scale_index(const float *scales, int n, const float *tab, int32_t *idx_bisect, int32_t *idx_hinted, cudaStream_t st);
 int launch_rans_decode_full(const Tables &T, const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride,

@@ -871,64 +871,44 @@ int rans_encode_any(const Tables &T, const int32_t *sym, const uint8_t *idx, int
     return 0;
 }
 
-int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, int64_t n_sym,
-                       int64_t stream_stride, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
-                       uint32_t *out_len, int *err_flag, cudaStream_t st) {
-    return rans_encode_any(T, sym, idx, n_streams, EqualSegs{(long)n_sym, (long)stream_stride},
-                           n_sym % 4 == 0 && stream_stride % 4 == 0, n_sym, n_sym == stream_stride, (long)n_sym, scratch, scratch_words, out, out_stride,
-                           out_len, err_flag, st);
+int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, const CallImages &c, uint32_t *scratch,
+                       size_t scratch_words, uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag,
+                       cudaStream_t st) {
+    // (mixed: every stream is a whole number of blocks of M symbols, M a multiple of 16; the streams differ in length,
+    // so the CTA-per-stream form, which is for few long streams of one size, is not used)
+    if (c.geo)
+        return rans_encode_any(T, sym, idx, c.n_streams, MixedSegs{c.seg}, true, c.min_sym, false, 0L, scratch,
+                               scratch_words, out, out_stride, out_len, err_flag, st);
+    const long n_sym = (long)c.min_sym;
+    return rans_encode_any(T, sym, idx, c.n_streams, EqualSegs{n_sym, n_sym}, n_sym % 4 == 0, n_sym, true, n_sym, scratch,
+                           scratch_words, out, out_stride, out_len, err_flag, st);
 }
 
-int launch_rans_encode_mixed(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
-                             int64_t min_sym, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
-                             uint32_t *out_len, int *err_flag, cudaStream_t st) {
-    // (every stream is a whole number of blocks of M symbols, M a multiple of 16; the streams differ in length, so
-    // the CTA-per-stream form, which is for few long streams of one size, is not used)
-    return rans_encode_any(T, sym, idx, n_streams, MixedSegs{seg}, true, min_sym, false, 0L, scratch, scratch_words, out,
-                           out_stride, out_len, err_flag, st);
-}
-
-int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, int n_img, int lanes, uint8_t *out,
-                     size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st) {
-    const uint32_t *start_word = scratch + (size_t)n_img * lanes * scratch_words;
-    const uint32_t *n_words = start_word + (size_t)n_img * lanes;
-    lane_pack_kernel<EqualLanes><<<n_img, 256, sizeof(uint32_t) * (lanes + 1), st>>>(
-        scratch, (long)scratch_words, start_word, n_words, EqualLanes{lanes}, out, out_stride, out_len, err_flag);
+int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, const CallImages &c, uint8_t *out, size_t out_stride,
+                     uint32_t *out_len, int *err_flag, cudaStream_t st) {
+    const uint32_t *start_word = scratch + (size_t)c.n_streams * scratch_words;
+    const uint32_t *n_words = start_word + (size_t)c.n_streams;
+    const size_t smem = sizeof(uint32_t) * (c.max_lanes + 1);
+    if (c.geo)
+        lane_pack_kernel<MixedLanes><<<c.n_img, 256, smem, st>>>(scratch, (long)scratch_words, start_word, n_words,
+                                                                 MixedLanes{c.lane0}, out, out_stride, out_len, err_flag);
+    else
+        lane_pack_kernel<EqualLanes><<<c.n_img, 256, smem, st>>>(scratch, (long)scratch_words, start_word, n_words,
+                                                                 EqualLanes{c.lanes}, out, out_stride, out_len, err_flag);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;
 }
 
-int launch_lane_pack_mixed(const uint32_t *scratch, size_t scratch_words, int n_img, const int *lane0, int n_lanes,
-                           int max_lanes, uint8_t *out, size_t out_stride, uint32_t *out_len, int *err_flag,
-                           cudaStream_t st) {
-    const uint32_t *start_word = scratch + (size_t)n_lanes * scratch_words;
-    const uint32_t *n_words = start_word + (size_t)n_lanes;
-    lane_pack_kernel<MixedLanes><<<n_img, 256, sizeof(uint32_t) * (max_lanes + 1), st>>>(
-        scratch, (long)scratch_words, start_word, n_words, MixedLanes{lane0}, out, out_stride, out_len, err_flag);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_rans_dec_init(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img, int lanes,
-                         int lanes_container, RansStreamState *states, const uint8_t **lane_ptr, int *err_flag,
-                         cudaStream_t st) {
-    const int n = n_img * lanes;
-    rans_dec_init_kernel<EqualLanes><<<(n + 127) / 128, 128, 0, st>>>(streams, stream_len, stream_stride, n_img,
-                                                                      EqualLanes{lanes}, lanes_container, states,
-                                                                      lane_ptr, err_flag);
-    count_launch(1);
-    LBIC_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int launch_rans_dec_init_mixed(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, int n_img,
-                               const int *lane0, int n_lanes, int lanes_container, RansStreamState *states,
-                               const uint8_t **lane_ptr, int *err_flag, cudaStream_t st) {
-    rans_dec_init_kernel<MixedLanes><<<(n_lanes + 127) / 128, 128, 0, st>>>(streams, stream_len, stream_stride, n_img,
-                                                                            MixedLanes{lane0}, lanes_container, states,
-                                                                            lane_ptr, err_flag);
+int launch_rans_dec_init(const uint8_t *streams, const uint32_t *stream_len, size_t stream_stride, const CallImages &c,
+                         RansStreamState *states, const uint8_t **lane_ptr, int *err_flag, cudaStream_t st) {
+    const int grid = (c.n_streams + 127) / 128, container = c.lane_container ? 1 : 0;
+    if (c.geo)
+        rans_dec_init_kernel<MixedLanes><<<grid, 128, 0, st>>>(streams, stream_len, stream_stride, c.n_img,
+                                                               MixedLanes{c.lane0}, container, states, lane_ptr, err_flag);
+    else
+        rans_dec_init_kernel<EqualLanes><<<grid, 128, 0, st>>>(streams, stream_len, stream_stride, c.n_img,
+                                                               EqualLanes{c.lanes}, container, states, lane_ptr, err_flag);
     count_launch(1);
     LBIC_CUDA(cudaGetLastError());
     return 0;

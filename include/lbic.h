@@ -297,6 +297,32 @@ int lbic_debug_selfinfo(lbic_model *m, const float *ksi, int ld_ksi, const int32
 int lbic_debug_scale_index(lbic_model *m, const float *scales, int n, const float *scale_table, int32_t *idx_bisect,
                            int32_t *idx_hinted, void *stream);
 
+/* Test hooks for the entropy coder: each runs the one kernel form it is asked for and returns LBIC_ERR_INVALID where that
+ * form's preconditions do not hold (never another form).  Device pointers unless stated; they synchronise `stream`.
+ *
+ * lbic_debug_rans_encode: stream s codes symbols / indexes [seg[s], seg[s+1]) (seg: device int64 [n_streams + 1],
+ * seg[0] = 0, non-decreasing) as lbic_rans_encode does.  form 1 = one warp per stream, 2 = one CTA per stream (streams of
+ * equal length), 3 = one thread per stream (compact tables present, every length and start a multiple of 4, symbols
+ * 16-byte and indexes 4-byte aligned).  Outputs as lbic_rans_encode. */
+int lbic_debug_rans_encode(lbic_model *m, const int32_t *symbols, const uint8_t *indexes, int n_streams,
+                           const int64_t *seg, int form, uint8_t *stream_out, size_t stream_cap, uint32_t *stream_len,
+                           void *stream);
+/* lbic_debug_rans_decode_steps: n_streams reference-container streams (slot s at s * stream_cap, stream_len[s] bytes)
+ * decoded in n_steps steps of M symbols per stream, as the decode steps of the codec do: step k decodes row
+ * k * n_streams + s of ksi ((n_steps * n_streams, 2M) fp32: scales, then means) from stream s.  form 0 = the whole-stream
+ * decoder of lbic_rans_decode with the indexes of the scales (writes sym_out only); 1 = warp per row on the int32 tables,
+ * 2 = warp per row on shared-memory copies of the compact rows, 3 = thread per row (compact tables, M % 4 == 0).
+ * Outputs: sym_out (n_steps * n_streams, M) int32; yq_hi / yq_lo the same shape as fp16 bit patterns of sym + mean;
+ * pos_out [n_streams] uint32 = the 32-bit words of each stream consumed at the end. */
+int lbic_debug_rans_decode_steps(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len, size_t stream_cap,
+                                 int n_streams, int M, int n_steps, const float *ksi, int form, int32_t *sym_out,
+                                 uint16_t *yq_hi, uint16_t *yq_lo, uint32_t *pos_out, void *stream);
+/* lbic_debug_compact_tables: the compact tables of the installed CDFs (HOST outputs, each may be NULL): *total = entries of
+ * the 16-bit rows (0: the tables are too large for the compact form), rows [*total] uint16 (row l from offsets[l], its
+ * cdf_length - 1 entries without the final 65536), offsets [65] int32, lut [64 * 257] uint16 (lut[l][b] = first k with
+ * cdf[l][k] > 256 b). */
+int lbic_debug_compact_tables(lbic_model *m, int *total, uint16_t *rows, int32_t *offsets, uint16_t *lut);
+
 /* Tuning hook: times `iters` back-to-back launches of the D = A W^T tile kernel (EPI_RAW or a PREGDN-style
  * epilogue when with_epilogue != 0) on synthetic operands with CUDA events; returns the mean ms per launch. */
 int lbic_debug_gemm_bench(lbic_model *m, int R, int K, int cout, int with_epilogue, int iters, double *ms_per_launch);

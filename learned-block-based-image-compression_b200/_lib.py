@@ -89,6 +89,9 @@ PROTOTYPES = {
     "lbic_debug_layer": (_i, [_vp, ctypes.POINTER(LbicDebugLayerArgs), _vp]),
     "lbic_debug_selfinfo": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _vp]),
     "lbic_debug_scale_index": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
+    "lbic_debug_rans_encode": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _sz, _vp, _vp]),
+    "lbic_debug_rans_decode_steps": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "lbic_debug_compact_tables": (_i, [_vp, ctypes.POINTER(_i), _vp, _vp, _vp]),
     "lbic_debug_gemm_bench": (_i, [_vp, _i, _i, _i, _i, _i, ctypes.POINTER(ctypes.c_double)]),
     "lbic_saturation_count": (_i, [_vp, _vp, ctypes.POINTER(ctypes.c_int64), _i]),
     "lbic_launch_count": (_i64, [_vp]),

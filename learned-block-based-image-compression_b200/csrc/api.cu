@@ -3,6 +3,7 @@
 #include <math.h>
 #include <cmath>
 #include <stdarg.h>
+#include <stddef.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -2386,6 +2387,129 @@ extern "C" int lbic_debug_scale_index(lbic_model *m, const float *scales, int n,
     cudaStream_t st = (cudaStream_t)stream;
     LBIC_TRY(launch_scale_index(scales, n, scale_table, idx_bisect, idx_hinted, st));
     LBIC_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int lbic_debug_rans_encode(lbic_model *m, const int32_t *symbols, const uint8_t *indexes, int n_streams,
+                                      const int64_t *seg, int form, uint8_t *stream_out, size_t stream_cap,
+                                      uint32_t *stream_len, void *stream) {
+    if (!m || !symbols || !indexes || !seg || !stream_out || !stream_len || n_streams < 1 || form < 1 || form > 3)
+        return lbic_fail(LBIC_ERR_INVALID, "bad argument");
+    if (!m->tables.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");
+    if (stream_cap % 4) return lbic_fail(LBIC_ERR_INVALID, "stream_cap must be a multiple of 4");
+    Active act(m);
+    cudaStream_t st = (cudaStream_t)stream;
+    std::vector<int64_t> seg_host(n_streams + 1);
+    LBIC_CUDA(cudaMemcpyAsync(seg_host.data(), seg, sizeof(int64_t) * (n_streams + 1), cudaMemcpyDeviceToHost, st));
+    LBIC_CUDA(cudaStreamSynchronize(st));
+    if (seg_host[0] != 0) return lbic_fail(LBIC_ERR_INVALID, "seg[0] must be 0");
+    for (int s = 0; s < n_streams; ++s)
+        if (seg_host[s + 1] < seg_host[s]) return lbic_fail(LBIC_ERR_INVALID, "seg must be non-decreasing");
+    if (m->ws.n_img == 0) LBIC_TRY(ensure_workspace(m, 1, 1, 2));
+    const size_t per = stream_cap / 4;
+    LBIC_TRY(ensure_rans_scratch(m, (size_t)n_streams * per + 2 * (size_t)n_streams));
+    LBIC_TRY(launch_rans_encode_form(m->tables, symbols, indexes, n_streams, seg, seg_host.data(), form, m->ws.rans_scratch,
+                                     per, stream_out, stream_cap, stream_len, m->err_flag, st));
+    LBIC_CUDA(cudaStreamSynchronize(st));
+    return take_error_flag(m);
+}
+
+extern "C" int lbic_debug_rans_decode_steps(lbic_model *m, const uint8_t *streams, const uint32_t *stream_len,
+                                            size_t stream_cap, int n_streams, int M, int n_steps, const float *ksi, int form,
+                                            int32_t *sym_out, uint16_t *yq_hi, uint16_t *yq_lo, uint32_t *pos_out,
+                                            void *stream) {
+    if (!m || !streams || !stream_len || !ksi || !sym_out || n_streams < 1 || M < 1 || n_steps < 1 || form < 0 || form > 3 ||
+        (form > 0 && (!yq_hi || !yq_lo || !pos_out)))
+        return lbic_fail(LBIC_ERR_INVALID, "bad argument");
+    if (!m->tables.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");
+    if (form == 3 && ((reinterpret_cast<uintptr_t>(ksi) | reinterpret_cast<uintptr_t>(sym_out)) & 15 ||
+                      (reinterpret_cast<uintptr_t>(yq_hi) | reinterpret_cast<uintptr_t>(yq_lo)) & 7))
+        return lbic_fail(LBIC_ERR_INVALID, "the thread-per-row decode step needs 16-byte aligned ksi / symbols, 8-byte aligned yq");
+    Active act(m);
+    cudaStream_t st = (cudaStream_t)stream;
+    const Tables &T = m->tables;
+    const size_t rows = (size_t)n_steps * n_streams, n = rows * M, ld_row = sizeof(float) * 2 * M;
+    std::vector<void *> tmp;
+    int rc = 0;
+    do {
+#define P(call) if ((rc = (call)) != 0) break
+        if (form == 0) {
+            // stream-major scales -> indexes (the decoders' bisection) -> the whole-stream decoder -> step-major symbols
+            const size_t step_bytes = sizeof(float) * (size_t)M, sm_pitch = step_bytes * n_steps;
+            float *scales;
+            int32_t *idx32, *idx32b, *sym_sm;
+            uint8_t *idx8;
+            P(dev_alloc(tmp, (void **)&scales, sizeof(float) * n));
+            P(dev_alloc(tmp, (void **)&idx32, sizeof(int32_t) * n));
+            P(dev_alloc(tmp, (void **)&idx32b, sizeof(int32_t) * n));
+            P(dev_alloc(tmp, (void **)&sym_sm, sizeof(int32_t) * n));
+            P(dev_alloc(tmp, (void **)&idx8, n));
+            for (int k = 0; k < n_steps && rc == 0; ++k)
+                rc = cudaMemcpy2DAsync((char *)scales + k * step_bytes, sm_pitch, ksi + (size_t)k * n_streams * 2 * M, ld_row,
+                                       step_bytes, n_streams, cudaMemcpyDeviceToDevice, st) == cudaSuccess
+                         ? 0 : lbic_fail(LBIC_ERR_CUDA, "scale copy failed");
+            if (rc) break;
+            P(launch_scale_index(scales, (int)n, T.d_scale_table, idx32, idx32b, st));
+            if (cudaMemcpy2DAsync(idx8, 1, idx32, 4, 1, n, cudaMemcpyDeviceToDevice, st) != cudaSuccess) {   // low bytes
+                rc = lbic_fail(LBIC_ERR_CUDA, "index copy failed");
+                break;
+            }
+            P(launch_rans_decode_full(T, streams, stream_len, stream_cap, idx8, n_streams, (int64_t)n_steps * M, sym_sm, st));
+            for (int k = 0; k < n_steps && rc == 0; ++k)
+                rc = cudaMemcpy2DAsync(sym_out + (size_t)k * n_streams * M, step_bytes, (char *)sym_sm + k * step_bytes,
+                                       sm_pitch, step_bytes, n_streams, cudaMemcpyDeviceToDevice, st) == cudaSuccess
+                         ? 0 : lbic_fail(LBIC_ERR_CUDA, "symbol copy failed");
+            break;
+        }
+        // the decode steps of a mixed-size call whose schedule row k * n_streams + s reads stream s
+        RansStreamState *states;
+        const uint8_t **lane_ptr;
+        int *stream_of;
+        P(dev_alloc(tmp, (void **)&states, sizeof(RansStreamState) * n_streams));
+        P(dev_alloc(tmp, (void **)&lane_ptr, sizeof(void *) * n_streams));
+        P(dev_alloc(tmp, (void **)&stream_of, sizeof(int) * rows));
+        std::vector<int> h_stream(rows);
+        for (size_t r = 0; r < rows; ++r) h_stream[r] = (int)(r % n_streams);
+        if (cudaMemcpyAsync(stream_of, h_stream.data(), sizeof(int) * rows, cudaMemcpyHostToDevice, st) != cudaSuccess) {
+            rc = lbic_fail(LBIC_ERR_CUDA, "stream table copy failed");
+            break;
+        }
+        P(launch_rans_dec_init(streams, stream_len, stream_cap, one_geometry(n_streams, 1, 1), states, lane_ptr, m->err_flag, st));
+        MixedGeo geo{};
+        geo.stream = stream_of;
+        for (int k = 0; k < n_steps && rc == 0; ++k) {
+            StepRows r;
+            r.sd = StepDesc{1, 0, 0, k * n_streams, 1, (int)rows};
+            r.R = n_streams;
+            r.geo = &geo;
+            const size_t o = (size_t)k * n_streams * M;
+            rc = launch_rans_dec_step(T, states, lane_ptr, 0, r, M, ksi + 2 * o, 2 * M, reinterpret_cast<h16 *>(yq_hi) + o,
+                                      reinterpret_cast<h16 *>(yq_lo) + o, M, sym_out, st, form);
+        }
+        if (rc) break;
+        if (cudaMemcpy2DAsync(pos_out, sizeof(uint32_t), (char *)states + offsetof(RansStreamState, pos),
+                              sizeof(RansStreamState), sizeof(uint32_t), n_streams, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            rc = lbic_fail(LBIC_ERR_CUDA, "position copy failed");
+#undef P
+    } while (0);
+    cudaError_t ce = cudaStreamSynchronize(st);
+    free_all(tmp);
+    if (rc) return rc;
+    if (ce != cudaSuccess) return lbic_fail(LBIC_ERR_CUDA, "debug decode failed: %s", cudaGetErrorString(ce));
+    return take_error_flag(m);
+}
+
+extern "C" int lbic_debug_compact_tables(lbic_model *m, int *total, uint16_t *rows, int32_t *offsets, uint16_t *lut) {
+    if (!m) return lbic_fail(LBIC_ERR_INVALID, "null model");
+    const Tables &T = m->tables;
+    if (!T.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");
+    Active act(m);
+    if (total) *total = T.cdf16_total;
+    if (T.cdf16_total <= 0) return 0;
+    LBIC_CUDA(cudaDeviceSynchronize());
+    if (rows) LBIC_CUDA(cudaMemcpy(rows, T.cdf16, sizeof(uint16_t) * T.cdf16_total, cudaMemcpyDeviceToHost));
+    if (offsets) LBIC_CUDA(cudaMemcpy(offsets, T.cdf16_off, sizeof(int32_t) * 65, cudaMemcpyDeviceToHost));
+    if (lut) LBIC_CUDA(cudaMemcpy(lut, T.cdf16 + T.cdf16_total, sizeof(uint16_t) * 64 * 257, cudaMemcpyDeviceToHost));
     return 0;
 }
 

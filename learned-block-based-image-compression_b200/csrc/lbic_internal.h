@@ -403,9 +403,17 @@ void rans_set_enc_thread_min_streams(int n);   // encodes of at least this many 
 void rans_set_dec_smem_warp(int on);           // 1 (default): warp-per-row decode steps run on shared-memory tables
 void rans_set_dec_thread_min_rows(int rows);   // steps with at least this many rows use the thread-per-stream kernel
 // (one geometry: row r reads stream img * lanes + v, or img for lanes <= 1; a mixed-size step: stream geo->stream[row])
+// form: 0 = the kernel the policy picks; 1 warp per row on the int32 tables, 2 warp per row on shared-memory tables,
+// 3 thread per row (tests: LBIC_ERR_INVALID where that kernel does not apply)
 int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
                          const StepRows &s, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq,
-                         int32_t *sym_out, cudaStream_t st);
+                         int32_t *sym_out, cudaStream_t st, int form = 0);
+// test hook: n_streams streams, stream s = symbols [seg[s], seg[s+1]) (seg device, seg_host its host copy), through
+// encoder form 1 (warp per stream), 2 (CTA per stream; equal streams back to back) or 3 (thread per stream; compact tables,
+// 4-symbol aligned streams); LBIC_ERR_INVALID where the form does not apply
+int launch_rans_encode_form(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
+                            const int64_t *seg_host, int form, uint32_t *scratch, size_t scratch_words, uint8_t *out,
+                            size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st);
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,
                          cudaStream_t st);
 // CDF index of n scales by both routines of the decoders (bisection; hint with bisection fallback), for tests

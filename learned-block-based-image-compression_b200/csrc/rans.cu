@@ -831,17 +831,24 @@ static int g_enc_block_max_streams = 592;     // up to 4 CTAs per SM: one CTA pe
 // (`aligned`: every stream starts and ends on a multiple of 4 symbols and the arrays are 16 / 4-byte aligned;
 // `min_sym`: the shortest stream)
 // (`block_form`: streams of block_n_sym symbols back to back may take the CTA-per-stream form)
+// (`form`: 0 = by the policy below; 1 warp, 2 CTA, 3 thread per stream = that form, LBIC_ERR_INVALID if it does not apply)
 template <class Segs>
 int rans_encode_any(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, Segs seg, bool aligned,
                     int64_t min_sym, bool block_form, long block_n_sym, uint32_t *scratch, size_t scratch_words, uint8_t *out, size_t out_stride,
-                    uint32_t *out_len, int *err_flag, cudaStream_t st) {
+                    uint32_t *out_len, int *err_flag, cudaStream_t st, int form = 0) {
     if (!T.cdf) return lbic_fail(LBIC_ERR_STATE, "Uninitialized CDFs. Run update() first");
     uint32_t *start_word = scratch + (size_t)n_streams * scratch_words;
     uint32_t *n_words = start_word + n_streams;
+    const bool thread_ok = T.cdf16_total > 0 && aligned && (reinterpret_cast<uintptr_t>(sym) & 15) == 0 &&
+                           (reinterpret_cast<uintptr_t>(idx) & 3) == 0;
+    if (form < 0 || form > 3 || (form == 3 && !thread_ok) || (form == 2 && !block_form))
+        return lbic_fail(LBIC_ERR_INVALID, "rANS encoder form %d does not apply to these streams", form);
     // many streams: one thread per stream with the tables in shared memory; few (single images): one warp per stream
-    const bool thread_form = T.cdf16_total > 0 && n_streams >= g_enc_thread_min_streams && aligned &&
-                             (reinterpret_cast<uintptr_t>(sym) & 15) == 0 && (reinterpret_cast<uintptr_t>(idx) & 3) == 0;
-    if (thread_form) {
+    if (form == 0)
+        form = thread_ok && n_streams >= g_enc_thread_min_streams                          ? 3
+               : block_form && n_streams <= g_enc_block_max_streams && min_sym >= 256 ? 2
+                                                                                        : 1;
+    if (form == 3) {
         const size_t smem = 16 * (((size_t)T.cdf16_total + 7) / 8) + 3 * 64 * 4;
         static unsigned long long attr_mask = 0;
         if (lbic_first_use_on_device(attr_mask))
@@ -849,7 +856,7 @@ int rans_encode_any(const Tables &T, const int32_t *sym, const uint8_t *idx, int
         rans_encode_thread_kernel<Segs><<<(n_streams + ENC_T_THREADS - 1) / ENC_T_THREADS, ENC_T_THREADS, smem, st>>>(
             T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, sym, idx, n_streams, seg, scratch,
             (long)scratch_words, start_word, n_words, err_flag);
-    } else if (block_form && n_streams <= g_enc_block_max_streams && min_sym >= 256) {
+    } else if (form == 2) {
         // few long streams (single images, the reference container): one CTA per stream, serial chain on one thread
         rans_encode_block_kernel<<<n_streams, ENC_B_THREADS, 0, st>>>(
             T.cdf, T.stride, T.cdf_length, T.offset, sym, idx, n_streams, block_n_sym, block_n_sym, scratch,
@@ -882,6 +889,26 @@ int launch_rans_encode(const Tables &T, const int32_t *sym, const uint8_t *idx, 
     const long n_sym = (long)c.min_sym;
     return rans_encode_any(T, sym, idx, c.n_streams, EqualSegs{n_sym, n_sym}, n_sym % 4 == 0, n_sym, true, n_sym, scratch,
                            scratch_words, out, out_stride, out_len, err_flag, st);
+}
+
+int launch_rans_encode_form(const Tables &T, const int32_t *sym, const uint8_t *idx, int n_streams, const int64_t *seg,
+                            const int64_t *seg_host, int form, uint32_t *scratch, size_t scratch_words, uint8_t *out,
+                            size_t out_stride, uint32_t *out_len, int *err_flag, cudaStream_t st) {
+    const int64_t n0 = seg_host[1] - seg_host[0];
+    bool equal = seg_host[0] == 0, aligned = true;
+    int64_t min_sym = n0;
+    for (int s = 0; s < n_streams; ++s) {
+        const int64_t n = seg_host[s + 1] - seg_host[s];
+        equal = equal && n == n0;
+        aligned = aligned && n % 4 == 0 && seg_host[s] % 4 == 0;
+        min_sym = n < min_sym ? n : min_sym;
+    }
+    // equal streams back to back take the closed form, as an equal-size call codes them; any others the segment table
+    if (equal)
+        return rans_encode_any(T, sym, idx, n_streams, EqualSegs{(long)n0, (long)n0}, aligned, min_sym, true, (long)n0,
+                               scratch, scratch_words, out, out_stride, out_len, err_flag, st, form);
+    return rans_encode_any(T, sym, idx, n_streams, MixedSegs{seg}, aligned, min_sym, false, 0L, scratch, scratch_words, out,
+                           out_stride, out_len, err_flag, st, form);
 }
 
 int launch_lane_pack(const uint32_t *scratch, size_t scratch_words, const CallImages &c, uint8_t *out, size_t out_stride,
@@ -921,14 +948,22 @@ void rans_set_dec_thread_min_rows(int rows) { g_dec_thread_min_rows = rows < 1 ?
 void rans_set_enc_thread_min_streams(int n) { g_enc_thread_min_streams = n < 1 ? 1 : n; }
 void rans_set_enc_block_max_streams(int n) { g_enc_block_max_streams = n < 0 ? 0 : n; }
 
+// (`form`: 0 = by the policy below; 1 warp per row on the int32 tables, 2 warp per row on shared-memory tables, 3 thread per
+// row = that form, LBIC_ERR_INVALID if it does not apply)
 template <class Rows>
 int rans_dec_step_any(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes, const Rows &s,
                       int R, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq, int32_t *sym_out,
-                      cudaStream_t st) {
+                      cudaStream_t st, int form) {
     if (R <= 0) return 0;
     if (M > 256) return lbic_fail(LBIC_ERR_INVALID, "M > 256 unsupported by the decode step");
+    const bool thread_ok = T.cdf16_total > 0 && M % 4 == 0 && ld_ksi % 4 == 0 && ld_yq % 4 == 0;
+    const size_t smem_s = 16 * (((size_t)T.cdf16_total + 7) / 8) + 1024 + (size_t)DEC_S_WARPS * RANS_ROW_SCRATCH(M);
+    const bool smem_ok = T.cdf16_total > 0 && smem_s <= 200 * 1024;
+    if (form < 0 || form > 3 || (form == 3 && !thread_ok) || (form == 2 && !smem_ok))
+        return lbic_fail(LBIC_ERR_INVALID, "rANS decode step form %d does not apply", form);
     // many streams: one thread per stream with the tables in shared memory; few (single images): one warp per stream
-    if (T.cdf16_total > 0 && R >= g_dec_thread_min_rows && M % 4 == 0 && ld_ksi % 4 == 0 && ld_yq % 4 == 0) {
+    if (form == 0) form = thread_ok && R >= g_dec_thread_min_rows ? 3 : smem_ok && g_dec_smem_warp ? 2 : 1;
+    if (form == 3) {
         const size_t smem = 16 * (((size_t)T.cdf16_total + 64 * 257 + 7) / 8) + 4 * 64 * 4;
         static unsigned long long attr_mask = 0;
         if (lbic_first_use_on_device(attr_mask))
@@ -940,20 +975,17 @@ int rans_dec_step_any(const Tables &T, RansStreamState *states, const uint8_t *c
         LBIC_CUDA(cudaGetLastError());
         return 0;
     }
-    if (T.cdf16_total > 0 && g_dec_smem_warp) {
+    if (form == 2) {
         // few rows: one warp per row on shared-memory tables
-        const size_t smem = 16 * (((size_t)T.cdf16_total + 7) / 8) + 1024 + (size_t)DEC_S_WARPS * RANS_ROW_SCRATCH(M);
         static unsigned long long attr_mask2 = 0;
         if (lbic_first_use_on_device(attr_mask2))
             LBIC_CUDA(cudaFuncSetAttribute(rans_dec_step_smem_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        if (smem <= 200 * 1024) {
-            rans_dec_step_smem_kernel<Rows><<<(R + DEC_S_WARPS - 1) / DEC_S_WARPS, DEC_S_WARPS * 32, smem, st>>>(
-                T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, T.d_scale_table, states, lane_ptr, lanes, s, R, M,
-                ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out);
-            count_launch(1);
-            LBIC_CUDA(cudaGetLastError());
-            return 0;
-        }
+        rans_dec_step_smem_kernel<Rows><<<(R + DEC_S_WARPS - 1) / DEC_S_WARPS, DEC_S_WARPS * 32, smem_s, st>>>(
+            T.cdf16, T.cdf16_off, T.cdf16_total, T.cdf_length, T.offset, T.d_scale_table, states, lane_ptr, lanes, s, R, M,
+            ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out);
+        count_launch(1);
+        LBIC_CUDA(cudaGetLastError());
+        return 0;
     }
     const int warps_per_block = 4;
     rans_dec_step_kernel<Rows><<<(R + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(
@@ -966,11 +998,11 @@ int rans_dec_step_any(const Tables &T, RansStreamState *states, const uint8_t *c
 
 int launch_rans_dec_step(const Tables &T, RansStreamState *states, const uint8_t *const *lane_ptr, int lanes,
                          const StepRows &s, int M, const float *ksi, int ld_ksi, h16 *yq_hi, h16 *yq_lo, int ld_yq,
-                         int32_t *sym_out, cudaStream_t st) {
+                         int32_t *sym_out, cudaStream_t st, int form) {
     if (s.geo)   // schedule rows [sd.t, sd.t + R)
         return rans_dec_step_any(T, states, lane_ptr, 0, MixedDecRows{s.geo->stream + s.sd.t, s.sd.t}, s.R, M, ksi,
-                                 ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
-    return rans_dec_step_any(T, states, lane_ptr, lanes, s.sd, s.R, M, ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st);
+                                 ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st, form);
+    return rans_dec_step_any(T, states, lane_ptr, lanes, s.sd, s.R, M, ksi, ld_ksi, yq_hi, yq_lo, ld_yq, sym_out, st, form);
 }
 
 int launch_selfinfo_step(const StepDesc &s, int R, int M, const float *ksi, int ld_ksi, const int32_t *sym, float *info,

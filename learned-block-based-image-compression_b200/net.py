@@ -691,6 +691,58 @@ class BlockBasedImgCompLossyNetv9:
                                                          ib.data_ptr(), ih.data_ptr(), self._stream()))
         return ib, ih
 
+    def debug_rans_encode(self, sym, idx, seg, form, stream_cap):
+        """The streams [seg[s], seg[s+1]) of sym (int32) / idx (uint8) CUDA tensors through rANS encoder form 1 (warp), 2
+        (CTA) or 3 (thread per stream) (test hook, lbic_debug_rans_encode) -> list of stream bytes."""
+        seg = torch.as_tensor(seg, dtype=torch.int64).to(sym.device)
+        n = seg.numel() - 1
+        if sym.numel() == 0:                 # streams of no symbols: any valid (non-null) arrays
+            sym, idx = torch.zeros(4, dtype=torch.int32, device=sym.device), torch.zeros(4, dtype=torch.uint8, device=sym.device)
+        out = torch.zeros(n, stream_cap, dtype=torch.uint8, device=sym.device)
+        lens = torch.zeros(n, dtype=torch.int32, device=sym.device)
+        with torch.cuda.device(sym.device):
+            _lib.check(_lib.lib().lbic_debug_rans_encode(self._need(), sym.data_ptr(), idx.data_ptr(), n, seg.data_ptr(),
+                                                         int(form), out.data_ptr(), stream_cap, lens.data_ptr(),
+                                                         self._stream()))
+        out_h, lens_h = out.cpu().numpy(), lens.cpu().numpy()
+        return [out_h[s, :lens_h[s]].tobytes() for s in range(n)]
+
+    def debug_rans_decode_steps(self, streams, ksi, M, n_steps, form):
+        """Reference-container streams (list of bytes) decoded in n_steps steps of M symbols with scales | means from ksi
+        (n_steps * n_streams, 2M) CUDA fp32 through decode form 0 (whole stream), 1 (warp, int32 tables), 2 (warp,
+        shared-memory tables) or 3 (thread per row) (test hook, lbic_debug_rans_decode_steps) -> (sym (n_steps, n_streams,
+        M) int32, yq_hi, yq_lo fp16 of that shape, words consumed per stream); form 0 returns symbols only."""
+        n, dev = len(streams), ksi.device
+        cap = max(8, max(len(s) for s in streams) + 3) // 4 * 4
+        buf = np.zeros((n, cap), dtype=np.uint8)
+        for s, b in enumerate(streams):
+            buf[s, :len(b)] = np.frombuffer(b, dtype=np.uint8)
+        d_buf = torch.from_numpy(buf).to(dev)
+        lens = torch.tensor([len(b) for b in streams], dtype=torch.int32, device=dev)
+        ksi = ksi.contiguous().float()
+        sym = torch.empty(n_steps, n, M, dtype=torch.int32, device=dev)
+        hi, lo = (torch.empty(n_steps, n, M, dtype=torch.float16, device=dev) for _ in range(2))
+        pos = torch.zeros(n, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().lbic_debug_rans_decode_steps(self._need(), d_buf.data_ptr(), lens.data_ptr(), cap, n, M,
+                                                               n_steps, ksi.data_ptr(), int(form), sym.data_ptr(),
+                                                               hi.data_ptr(), lo.data_ptr(), pos.data_ptr(), self._stream()))
+        return (sym, None, None, None) if form == 0 else (sym, hi, lo, pos)
+
+    def debug_compact_tables(self):
+        """The compact tables of the installed CDFs (test hook, lbic_debug_compact_tables) -> (total, rows uint16 [total],
+        offsets int32 [65], lut uint16 [64, 257]); total 0 (and None for the arrays) when the tables are too large for them."""
+        total = ctypes.c_int()
+        h = self._need()
+        _lib.check(_lib.lib().lbic_debug_compact_tables(h, ctypes.byref(total), None, None, None))
+        if total.value == 0:
+            return 0, None, None, None
+        rows = np.empty(total.value, dtype=np.uint16)
+        off = np.empty(65, dtype=np.int32)
+        lut = np.empty((64, 257), dtype=np.uint16)
+        _lib.check(_lib.lib().lbic_debug_compact_tables(h, None, rows.ctypes.data, off.ctypes.data, lut.ctypes.data))
+        return total.value, rows, off, lut
+
 
 class BlkBasedPostProcessing:
     """Mirror of the reference's optional post-processing module (graphs/models/BlockBasedImgCompLossy_net.py:455-476,

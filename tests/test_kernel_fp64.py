@@ -285,10 +285,10 @@ def test_saturation_count_matches_fp64(model, dev):
 
 
 # ---- C. each epilogue mode, isolated from GEMM noise ----------------------------------------------------------------
-def nongeometric_table():
+def nongeometric_table(top=256.0):
     """An increasing scale table that is not geometric (quadratic in the level), as a checkpoint may carry."""
     i = torch.arange(64, dtype=torch.float64)
-    return (0.11 + (256.0 - 0.11) * (i / 63) ** 2).float()
+    return (0.11 + (top - 0.11) * (i / 63) ** 2).float()
 
 
 def crafted_scales(tab):
@@ -454,14 +454,37 @@ def test_selfinfo_vs_reference_formula(model, dev):
 
 
 # ---- E. end to end with a non-geometric installed table ------------------------------------------------------------
+# (top scale, entries of the compact 16-bit rows): 52 776 fit the shared-memory tables of the thread-per-stream coders, the
+# warp decoder on shared memory and the wave kernel's entropy CTAs; 67 512 do not, and every call takes the int32 tables
+NONGEOMETRIC = {"fits_compact": (200.0, 52776), "beyond_compact": (256.0, 0)}
+
+
 def test_nongeometric_table_end_to_end(dev):
+    """nongeometric_end_to_end on the KS3111 topology, with the table that fits the compact form and the one that does
+    not."""
+    for table in NONGEOMETRIC:
+        nongeometric_end_to_end(dev, table, "B8_lowrate")
+
+
+@pytest.mark.parametrize("table", list(NONGEOMETRIC))
+def test_nongeometric_table_end_to_end_ks3311(dev, table):
+    """nongeometric_end_to_end on a KS3311 topology (five-tap second entropy layer, ring-extended wave steps)."""
+    nongeometric_end_to_end(dev, table, "B8_highrate")
+
+
+def nongeometric_end_to_end(dev, table, cfgname):
     """A checkpoint whose conditional_gaussian_model buffers carry a non-geometric scale table (CDFs built by the
     oracle's restatement of update_scale_table / pmf_to_quantized_cdf): encode / decode are exact for both containers,
-    with the wave kernel on and off and with both decoder forms, and the indexes are build_indexes of the oracle's
-    teacher-forced ksi except at rounding boundaries (scale within 2e-4 of a level, one step)."""
-    cfgname = "B8_lowrate"
+    with the wave kernel on and off, with the thread-per-stream encoder and decoder and the warp-per-row decoder, and the
+    bytes equal the oracle's; the indexes are build_indexes of the oracle's teacher-forced ksi except at rounding
+    boundaries (scale within 2e-4 of a level, one step).  Encodes run in the wave kernel (a handful of launches per
+    call); decodes do where the table fits the compact form, whose rows the kernel's entropy CTAs read, and otherwise
+    fall back to the per-layer launches."""
+    from oracle import native as onative
     cfg = lbic_b200.load_config(cfgname)
-    tab = nongeometric_table()
+    case = f"{cfgname} {table}"
+    top, compact_total = NONGEOMETRIC[table]
+    tab = nongeometric_table(top)
     cdf, ln, off = nets.build_tables(tab)
     sd = weights.synth_state_dict(cfg, 1337)
     sd["conditional_gaussian_model._quantized_cdf"] = cdf
@@ -470,35 +493,54 @@ def test_nongeometric_table_end_to_end(dev):
     sd["conditional_gaussian_model.scale_table"] = tab
     m = BlockBasedImgCompLossyNetv9(cfg, device=dev)
     m.load_state_dict(sd)
+    assert m.debug_compact_tables()[0] == compact_total, f"{case}: compact tables"
     img = weights.synth_images(2, 48, 72)
     x = nets.arrange_block_pixels_to_channel_dim(img - 0.5, 8).contiguous().to(dev)
     P = nets.effective_params(sd, cfg)
     P.scale_table = tab
-    runs = {}
+    T = onative.Tables(cdf.numpy(), ln.numpy(), off.numpy())
+    runs, streams = {}, {}
     try:
         for wave in (1, 0):
             m.set_option("wave", wave)
+            # wave off: the thread-per-stream encoder for every stream count (it needs the compact tables)
+            m.set_option("enc_thread_streams", 1 if wave == 0 else 4096)
             for lanes in (1, 0):
+                l0 = m.launch_count()
                 strings, zhat, sym, idx = m.compress_batch(x, lanes=lanes, return_symbols=True)
+                if wave:
+                    assert m.launch_count() - l0 < 20, f"{case} lanes={lanes}: the encode should run in the wave kernel"
+                assert streams.setdefault(lanes, strings) == strings, f"{case} wave={wave} lanes={lanes}: bytes differ"
+                if lanes == 1:
+                    for i in range(x.shape[0]):
+                        want = onative.rans_encode(sym[i].cpu().numpy().reshape(-1), idx[i].cpu().numpy().reshape(-1), T)
+                        assert strings[i] == want, f"{case} wave={wave} image {i}: bytes differ from the oracle"
                 for rows in (1, 1 << 30):
                     m.set_option("dec_thread_rows", rows)
+                    l0 = m.launch_count()
                     zdec = m.decompress_batch(strings, x.shape, lanes=lanes)
-                    assert torch.equal(zdec, zhat), f"wave={wave} lanes={lanes} dec_thread_rows={rows}: decode differs"
+                    if wave and not (m.KS[1] == 3 and lanes == 1):   # (KS3311 has no raster mode in the wave kernel)
+                        assert (m.launch_count() - l0 < 20) == (compact_total > 0), f"{case} lanes={lanes}: wave decode use"
+                    assert torch.equal(zdec, zhat), \
+                        f"{case} wave={wave} lanes={lanes} dec_thread_rows={rows}: decode differs"
                 runs[(wave, lanes)] = (sym, idx, zhat)
     finally:
         m.set_option("dec_thread_rows", 4096)
+        m.set_option("enc_thread_streams", 4096)
         m.set_option("wave", 1)
     sym, idx, zhat = runs[(1, 1)]
     for k, (s2, i2, z2) in runs.items():
-        assert torch.equal(s2, sym) and torch.equal(i2, idx) and torch.equal(z2, zhat), f"{k} differs from wave=1 lanes=1"
+        assert torch.equal(s2, sym) and torch.equal(i2, idx) and torch.equal(z2, zhat), \
+            f"{case} {k} differs from wave=1 lanes=1"
     _, i_or, _, _, ksi = nets.whole_image_eval(P, x.cpu(), zhat.cpu())
     M = cfg.M
     sc = torch.clamp(ksi[:, :M], min=0.11).permute(0, 2, 3, 1)
     mis = i_or != idx.cpu().int()
     dist = ((sc[..., None] - tab).abs() / tab).min(dim=-1).values
-    assert int((i_or - idx.cpu().int()).abs().max()) <= 1
-    assert bool((dist[mis] < 2e-4).all()), f"index mismatches away from a table level: {float(dist[mis].max()):.2e}"
-    assert int(mis.sum()) <= max(1, mis.numel() // 10000)
-    assert len(set(idx.unique().tolist())) > 10
-    report(test="nongeometric_e2e", symbols=int(idx.numel()), index_mismatches=int(mis.sum()),
-           levels_used=len(set(idx.unique().tolist())), stream_bytes=len(m.compress_batch(x, lanes=1)[0][0]))
+    assert int((i_or - idx.cpu().int()).abs().max()) <= 1, case
+    assert bool((dist[mis] < 2e-4).all()), f"{case} index mismatches away from a table level: {float(dist[mis].max()):.2e}"
+    assert int(mis.sum()) <= max(1, mis.numel() // 10000), f"{case}: {int(mis.sum())} index mismatches"
+    assert len(set(idx.unique().tolist())) > 10, case
+    report(test="nongeometric_e2e", config=cfgname, table=table, compact_total=compact_total, symbols=int(idx.numel()),
+           index_mismatches=int(mis.sum()), levels_used=len(set(idx.unique().tolist())),
+           stream_bytes=len(streams[1][0]))
